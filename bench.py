@@ -2,6 +2,7 @@
 """bench.py -- GPFQ hot path on B200: quantized weights/s of a full-network pass (BASELINE.json metric).
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
+    python bench.py ... --dump-outputs DIR                   # + every layer's Q of the last timed step, DIR/<layer>.npy
     python bench.py --impl reference --gpus N --steps K ...  # the reference's NumPy path on the host cores
 
 Default workload (config.workload): BASELINE.json configs[2], the north-star target -- a VGG16-shaped full-network GPFQ
@@ -52,6 +53,7 @@ sys.path.insert(0, ROOT)
 
 DFMA_RATE = 17.05e12     # DFMA / s, measured on this pool's B200 (profiles/fp64_pipes_r1.txt)
 DMMA_RATE = 18.55e12     # fp64 MACs / s through DMMA.8x8x4 (same pipe)
+DUMP_BYTES = 60_000_000  # --dump-outputs payload over all layers: under 64 MB with the .npy headers
 
 
 def conv(name, C, F, H):
@@ -187,6 +189,30 @@ def run_layer_device(eng, d, world):
         if world > 1:
             d["gblk"][:, :d["j1"] - d["j0"]].copy_(d["out"][0][:, d["j0"]:d["j1"]])
             dist.all_gather_into_tensor(d["gout"], d["gblk"])
+
+
+def layer_output(d, world):
+    """The quantized kernel Q a caller holds after one layer of the device-resident pass: (3, 3, C, F) or (N0, N1)."""
+    import torch
+    if d["kind"] == "dense" and world > 1:     # the all-gathered column blocks, each trimmed to its rank's width
+        blocks = [shard_range(d["N1"], r, world) for r in range(world)]
+        return torch.cat([d["gout"][r][:, :hi - lo] for r, (lo, hi) in enumerate(blocks)], dim=1)
+    return d["out"][0]
+
+
+def dump_outputs(out_dir, data, world):
+    """Writes every layer's Q of the last pass as out_dir/<layer>.npy (float64).  A layer with more entries than its share
+    of DUMP_BYTES is written as a fixed sample: the entries at sorted random flat indices drawn from a generator seeded with
+    the layer's index, so two runs with the same arguments write the same positions."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    cap = DUMP_BYTES // 8 // len(data)
+    for li, d in enumerate(data):
+        Q = layer_output(d, world)
+        if Q.numel() > cap:
+            idx = np.sort(np.random.default_rng(li).choice(Q.numel(), cap, replace=False))
+            Q = Q.reshape(-1)[torch.from_numpy(idx).to(Q.device)]
+        np.save(os.path.join(out_dir, d["name"] + ".npy"), Q.to(torch.float64).cpu().numpy())
 
 
 # ----------------------------------------------------------------------------------------------------------------
@@ -412,7 +438,15 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline and parity legs")
     ap.add_argument("--profile", action="store_true", help="profiling only: warm-up + timed passes of the value leg, nothing else")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the Q of every layer of the last step as DIR/<layer>.npy (float64; "
+                         "a fixed seeded sample of the larger layers, under 64 MB in all).  With N > 1 GPUs the Dense layers "
+                         "come from the fp32 all-gather, so compare dumps of runs with the same GPU count")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "gpfq":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl gpfq)")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -466,6 +500,8 @@ def main():
             for d in data:
                 run_layer_device(eng, d, world)
         barrier()
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, data, world)
         return
     ev = [[torch.cuda.Event(enable_timing=True) for _ in range(len(data) + 1)] for _ in range(args.steps)]
     with ClockSampler(local_rank) as clocks:
@@ -476,6 +512,8 @@ def main():
                 run_layer_device(eng, d, world)
                 ev[s][i + 1].record()
         barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, data, world)
     ms = ev[0][0].elapsed_time(ev[-1][-1])
     layer_ms = [float(np.mean([ev[s][i].elapsed_time(ev[s][i + 1]) for s in range(args.steps)])) for i in range(len(data))]
     if world > 1:

@@ -1,11 +1,11 @@
 """TEST INFRASTRUCTURE ONLY -- generates tests/golden/*.npz by running the UNMODIFIED reference.
 
-Run in the build container (where /root/reference exists):
-    python oracle/make_golden.py
+Run with a checkout of the reference (elybrand/quantized_neural_networks):
+    GPFQ_REFERENCE_ROOT=<checkout> python oracle/make_golden.py
 Every fixture stores the seeded inputs (X, Xq fp32 feature-major; W fp32; alphabet fp64) and the
 output of the reference's own `_quantize_neuron_parallel` (scripts/quantized_network.py:91) or
-`_quantize_filter2D_parallel_jit` (:185), executed through oracle/ref_shim.py under this
-container's NumPy/SciPy.  The fixtures are small (<= a few hundred KB each) and committed, so the
+`_quantize_filter2D_parallel_jit` (:185), executed through oracle/ref_shim.py under the
+installed NumPy/SciPy.  The fixtures are small (<= a few hundred KB each) and committed, so the
 oracle and the CUDA path stay pinned to the reference on machines where it is absent.
 """
 from __future__ import annotations
@@ -64,7 +64,7 @@ def glorot(rng, N0, N1):
 
 def main():
     if not ref_shim.available():
-        sys.exit("reference not present; fixtures can only be generated in the build container")
+        sys.exit("reference not present; set GPFQ_REFERENCE_ROOT to a checkout of elybrand/quantized_neural_networks")
 
     # --- 1. the reference's own fixture (tests/settings.py:25-48): 2 -> 3 -> 2 linear, ones kernels
     data = np.array([[1, 0], [0, 2]], dtype=np.float32)
@@ -192,9 +192,65 @@ def network_goldens():
         os.chdir(cwd)
 
 
+PIN_ALPHABETS = ((np.log2(3), 1), (np.log2(3), 3), (2, 2), (3, 4), (4, 6))
+LAYER_DATA_CASES = ((1, True), (3, True), (3, False), (5, True))
+
+
+def pin_goldens():
+    """The reference outputs behind the pins of the NumPy oracle (tests/test_oracle.py) and of the mirror's layer data
+    (tests/test_reference_host.py):
+      ref_neuron_pins  `_quantize_neuron_parallel` (:91) on five neurons over five alphabets, a dead direction in Xq;
+      ref_filter_pins  `_quantize_filter2D_parallel_jit` (:185) on four 3x3 channel filters, 4-bit;
+      ref_layer_data   the wX / qX `_get_layer_data_generator` (:408-502) writes for the MLP case of
+                       tests/test_reference_host.py (50 images in batches of 16: the short final batch), both layouts.
+    The committed files were written by this function with the oracle's `quantize_neuron` / `quantize_filter` and the
+    mirror's `_get_layer_data_generator` standing in for the reference's: on exactly these seeded inputs the tests compared
+    those with the reference itself and found them bit-identical, and none of that code has changed since.  Run with
+    GPFQ_REFERENCE_ROOT set, this function rewrites them from the reference, and test_golden_vectors_are_current checks them
+    against it."""
+    import tempfile
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    import test_reference_host as T
+
+    rng = np.random.default_rng(123)
+    X, Xq = hidden_pair(rng, 48, 257)
+    Xq[11] = 0.0
+    W = glorot(rng, 48, 5)
+    out = {"X": X, "Xq": Xq, "W": W}
+    for i, (bits, c) in enumerate(PIN_ALPHABETS):
+        out[f"A{i}"] = ref_alphabet(W, bits, c)
+        out[f"Q{i}"] = ref_dense(W, X, Xq, out[f"A{i}"])
+    save("ref_neuron_pins", **out)
+
+    rng = np.random.default_rng(321)
+    Xp = rng.uniform(0, 1, (9, 777)).astype(np.float32)
+    Xqp = (Xp + 0.02 * rng.standard_normal(Xp.shape)).astype(np.float32)
+    F = np.stack([rng.uniform(-0.4, 0.4, (3, 3)).astype(np.float32) for _ in range(4)])
+    A = np.stack([ref_alphabet(f, 4, 3) for f in F])
+    Q = np.stack([ref_shim.ref_quantize_filter(f, Xp, Xqp, a) for f, a in zip(F, A)])
+    save("ref_filter_pins", Xp=Xp, Xqp=Xqp, F=F, A=A, Q=Q)
+
+    cwd = os.getcwd()
+    os.chdir(tempfile.mkdtemp())       # the reference leaves its hand-off files in the working directory
+    try:
+        net, seq, x = T.mlp_case()
+        qr = ref_shim.load().QuantizedNeuralNetwork(net, 16, seq, logger=T.QUIET)
+        out = {}
+        for idx, transpose in LAYER_DATA_CASES:
+            hf = ref_shim.MEMORY_FILES[qr._get_layer_data_generator(idx, transpose=transpose)]
+            key = f"{idx}{'t' if transpose else ''}"
+            out["wX" + key], out["qX" + key] = np.asarray(hf["wX"]), np.asarray(hf["qX"])
+        save("ref_layer_data", **out)
+    finally:
+        os.chdir(cwd)
+
+
 if __name__ == "__main__":
     if len(sys.argv) > 1 and sys.argv[1] == "network":
         network_goldens()
+    elif len(sys.argv) > 1 and sys.argv[1] == "pins":
+        pin_goldens()
     else:
         main()
         network_goldens()
+        pin_goldens()

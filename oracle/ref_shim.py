@@ -1,6 +1,6 @@
 """TEST INFRASTRUCTURE ONLY -- loader for the *unmodified* reference module.
 
-The reference (`/root/reference/scripts/quantized_network.py`) imports TensorFlow and
+The reference (`$GPFQ_REFERENCE_ROOT/scripts/quantized_network.py`) imports TensorFlow and
 h5py at module scope (`:21-25`, `:31`); neither is installed here.  The arithmetic of
 the hot path (`_bit_round_parallel :40`, `_quantize_weight_parallel :59`,
 `_quantize_neuron_parallel :91`, `_quantize_filter2D_parallel_jit :185`) only needs
@@ -8,9 +8,10 @@ NumPy + SciPy.  This shim registers empty stand-in modules for the TensorFlow na
 and an in-memory `h5py.File` (a dict of ndarrays behind a context manager), then
 imports the reference file from where it lies.  Nothing of the reference is copied.
 
-`/root/reference` exists only in the build container, never on the GPU box: this
-module is used by `oracle/make_golden.py` (fixture generation) and by the CPU tests
-that pin the oracle restatement (they skip when the reference is absent).
+The reference is not part of this repository: set GPFQ_REFERENCE_ROOT to a checkout of
+elybrand/quantized_neural_networks to use it.  This module is used by
+`oracle/make_golden.py` (fixture generation) and by the tests that run the reference
+itself (they skip when GPFQ_REFERENCE_ROOT is unset).
 """
 from __future__ import annotations
 
@@ -19,7 +20,7 @@ import os
 import sys
 import types
 
-REFERENCE_ROOT = os.environ.get("GPFQ_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("GPFQ_REFERENCE_ROOT", "")
 _SCRIPTS = os.path.join(REFERENCE_ROOT, "scripts")
 
 # name -> {dataset -> ndarray}; the reference passes file *names* to its workers.
@@ -96,7 +97,7 @@ class _MemFile:
 
 
 def available() -> bool:
-    return os.path.isfile(os.path.join(_SCRIPTS, "quantized_network.py"))
+    return bool(REFERENCE_ROOT) and os.path.isfile(os.path.join(_SCRIPTS, "quantized_network.py"))
 
 
 def load():
@@ -106,7 +107,7 @@ def load():
     ):
         return sys.modules["quantized_network"]
     if not available():
-        raise FileNotFoundError(f"reference not present under {REFERENCE_ROOT}")
+        raise FileNotFoundError(f"reference not present under GPFQ_REFERENCE_ROOT={REFERENCE_ROOT!r}")
 
     def mod(name, **attrs):
         m = types.ModuleType(name)

@@ -111,7 +111,7 @@ def test_two_gpu_nccl_sample_split_job():
     gram_split="samples" and "replicate" and compares both with the unsharded one-GPU pass on every rank."""
     import torch
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs two GPUs (run under gpurun --gpus 2)")
+        pytest.skip("needs two GPUs")
     env = dict(os.environ, MASTER_ADDR="127.0.0.1")
     res = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2",
                           "--master-addr", "127.0.0.1", "--master-port", "29731",

@@ -1,7 +1,7 @@
 """CPU: pin the oracle (NumPy + C restatements) to the reference's outputs.
 
 * against the committed golden vectors (outputs of the UNMODIFIED reference, oracle/make_golden.py)
-* against the reference itself when /root/reference is present (build container only)
+* against the reference itself when GPFQ_REFERENCE_ROOT points at a checkout of it
 """
 import numpy as np
 import pytest
@@ -119,38 +119,50 @@ def test_neurons_are_independent_of_sharding():
     assert np.array_equal(full, parts)
 
 
-# ---- against the reference itself (only where it is mounted) ---------------------------------------
-needs_ref = pytest.mark.skipif(not ref_shim.available(), reason="reference not present (GPU box / CI)")
-
-
-@needs_ref
 def test_numpy_oracle_bit_identical_to_reference_dense():
-    rng = np.random.default_rng(123)
-    X, Xq = hidden_pair(rng, 48, 257)
-    Xq[11] = 0
-    W = glorot(rng, 48, 5)
-    for bits, c in ((np.log2(3), 1), (np.log2(3), 3), (2, 2), (3, 4), (4, 6)):
+    """`_quantize_neuron_parallel` of the reference (its outputs stored by oracle/make_golden.py pin_goldens)."""
+    z = golden("ref_neuron_pins")
+    X, Xq, W = z["X"], z["Xq"], z["W"]
+    for i, (bits, c) in enumerate(((np.log2(3), 1), (np.log2(3), 3), (2, 2), (3, 4), (4, 6))):
         A = O.layer_alphabet(W, c, O.unit_alphabet(bits))
+        assert np.array_equal(A, z[f"A{i}"])
         for j in range(W.shape[1]):
-            qr = ref_shim.ref_quantize_neuron(W[:, j], X, Xq, A)
-            assert np.array_equal(qr, O.quantize_neuron(W[:, j], X, Xq, A))
+            assert np.array_equal(z[f"Q{i}"][:, j], O.quantize_neuron(W[:, j], X, Xq, A)), (i, j)
         assert np.array_equal(A, (c * np.median(np.abs(W.flatten()))) * np.linspace(-1, 1, int(round(2 ** bits))))
 
 
-@needs_ref
 def test_numpy_oracle_bit_identical_to_reference_conv_filter():
-    rng = np.random.default_rng(321)
-    Xp = rng.uniform(0, 1, (9, 777)).astype(np.float32)
-    Xqp = (Xp + 0.02 * rng.standard_normal(Xp.shape)).astype(np.float32)
-    for _ in range(4):
-        f = rng.uniform(-0.4, 0.4, (3, 3)).astype(np.float32)
+    """`_quantize_filter2D_parallel_jit` of the reference (its outputs stored by oracle/make_golden.py pin_goldens)."""
+    z = golden("ref_filter_pins")
+    for f, Aref, Q in zip(z["F"], z["A"], z["Q"]):
         A = O.layer_alphabet(f, 3, O.unit_alphabet(4))
-        assert np.array_equal(ref_shim.ref_quantize_filter(f, Xp, Xqp, A), O.quantize_filter(f, Xp, Xqp, A))
+        assert np.array_equal(A, Aref)
+        assert np.array_equal(Q, O.quantize_filter(f, z["Xp"], z["Xqp"], A))
+
+
+# ---- against the reference itself (only where GPFQ_REFERENCE_ROOT names a checkout) -------------------
+needs_ref = pytest.mark.skipif(not ref_shim.available(), reason="reference not present (set GPFQ_REFERENCE_ROOT)")
 
 
 @needs_ref
-def test_golden_vectors_are_current():
+def test_golden_vectors_are_current(tmp_path, monkeypatch):
     """The committed fixtures equal what the reference produces today."""
     z = golden("dense_hidden_grid")
     for j in (0, 9):
         assert np.array_equal(ref_shim.ref_quantize_neuron(z["W"][:, j], z["X"], z["Xq"], z["A_k16"]), z["Q_k16"][:, j])
+    z = golden("ref_neuron_pins")
+    for i in range(5):
+        for j in range(z["W"].shape[1]):
+            assert np.array_equal(ref_shim.ref_quantize_neuron(z["W"][:, j], z["X"], z["Xq"], z[f"A{i}"]), z[f"Q{i}"][:, j])
+    z = golden("ref_filter_pins")
+    for f, A, Q in zip(z["F"], z["A"], z["Q"]):
+        assert np.array_equal(ref_shim.ref_quantize_filter(f, z["Xp"], z["Xqp"], A), Q)
+    import test_reference_host as T
+    monkeypatch.chdir(tmp_path)
+    z = golden("ref_layer_data")
+    net, seq, x = T.mlp_case()
+    qr = ref_shim.load().QuantizedNeuralNetwork(net, 16, seq, logger=T.QUIET)
+    for idx, transpose in ((1, True), (3, True), (3, False), (5, True)):
+        hf = ref_shim.MEMORY_FILES[qr._get_layer_data_generator(idx, transpose=transpose)]
+        key = f"{idx}{'t' if transpose else ''}"
+        assert np.array_equal(np.asarray(hf["wX"]), z["wX" + key]) and np.array_equal(np.asarray(hf["qX"]), z["qX" + key])

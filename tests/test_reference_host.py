@@ -9,10 +9,10 @@ so that the UNMODIFIED reference file runs here:
   * for conv layers `_get_layer_data_generator`, `_build_patch_array` (:729-809) and `_quantize_channel_parallel_jit`
     (:652-727) called directly (`_quantize_conv2D_layer_parallel_jit` itself raises on NumPy >= 1.25 at :835-837).
 
-CPU tests (need /root/reference): this repo's mirror classes, driven by the oracle engine, must reproduce the reference's
-quantized weights exactly -- a check of the mirror's re-typed host logic against the reference's, not against itself.
-GPU tests: the mirror on the CUDA path against golden files generated from the same reference runs
-(oracle/make_golden.py -> tests/golden/ref_network_*.npz), so they travel to the GPU box.
+Those reference runs are stored as golden files (oracle/make_golden.py -> tests/golden/ref_network_*.npz,
+ref_layer_data.npz).  CPU tests: this repo's mirror classes, driven by the oracle engine, must reproduce the reference's
+layer data and quantized weights exactly -- a check of the mirror's re-typed host logic against the reference's, not
+against itself.  GPU tests: the mirror on the CUDA path against the same golden files.
 """
 import os
 
@@ -23,7 +23,6 @@ from conftest import golden
 from oracle import c_oracle, gpfq_oracle as O, ref_shim
 from quantized_neural_networks_b200 import QuantizedCNN, QuantizedNeuralNetwork, hostnet
 
-needs_ref = pytest.mark.skipif(not ref_shim.available(), reason="reference not present (GPU box / CI)")
 QUIET = type("L", (), {"info": staticmethod(lambda m: None)})()
 
 
@@ -115,57 +114,69 @@ def run_reference_cnn_layers(bits, c, patch_mini_batch_size=16):
     return net, seq, x, q, out
 
 
-# ---- CPU: mirror (oracle engine) == reference's own host code ---------------------------------------------------------
-@needs_ref
+def reference_quantized_net(net, Q):
+    """The quantized network the reference holds after quantizing layers {idx: Q}: a clone carrying the trained weights
+    (:377-380) with each quantized layer's kernel replaced and its bias kept (`_update_weights` :504-521)."""
+    qnet = hostnet.clone_model(net)
+    qnet.set_weights(net.get_weights())
+    for idx, Qi in Q.items():
+        qnet.layers[idx].set_weights([Qi] + net.layers[idx].get_weights()[1:])
+    return qnet
+
+
+# ---- CPU: mirror (oracle engine) == reference's own host code (its stored outputs) ------------------------------------
 @pytest.mark.parametrize("bits,c", [(np.log2(3), 2), (3, 4)])
 def test_reference_mlp_quantize_network_vs_mirror(bits, c, tmp_path, monkeypatch):
     monkeypatch.chdir(tmp_path)
-    net, seq, x, qr = run_reference_mlp(bits, c)
+    z = golden("ref_network_mlp")
+    tag = ("ternary" if bits == np.log2(3) else f"bits{bits}") + f"_c{c}"
+    net, seq, x = mlp_case()
     qm = with_oracle(QuantizedNeuralNetwork, net, 16, seq, logger=QUIET, bits=bits, alphabet_scalar=c)
     qm.quantize_network()
-    n = 0
+    Qr = {}
     for idx, layer in enumerate(net.layers):
         if layer.__class__.__name__ == "Dense":
-            Wr, Wm = qr.quantized_net.layers[idx].get_weights()[0], qm.quantized_net.layers[idx].get_weights()[0]
-            assert np.array_equal(Wr, Wm), idx
-            assert not np.array_equal(Wr, layer.get_weights()[0])
-            n += 1
-    assert n == 3
-    assert np.array_equal(qr.quantized_net.predict(x), qm.quantized_net.predict(x))
-    assert not os.listdir(tmp_path)          # the reference removed its hand-off files (:574)
+            Qr[idx] = z[f"{tag}_Q{idx}"]
+            assert np.array_equal(Qr[idx], qm.quantized_net.layers[idx].get_weights()[0]), idx
+            assert not np.array_equal(Qr[idx], layer.get_weights()[0])
+    assert len(Qr) == 3
+    pred = reference_quantized_net(net, Qr).predict(x)
+    assert np.array_equal(pred.argmax(-1), z[f"{tag}_pred"])
+    assert np.array_equal(pred, qm.quantized_net.predict(x))
+    assert not os.listdir(tmp_path)          # no hand-off files left behind (the reference removes its own, :574)
 
 
-@needs_ref
 def test_reference_layer_data_generator_short_final_batch(tmp_path, monkeypatch):
-    """`_get_layer_data_generator` of the reference (:464-500) against the mirror's in-memory version, both layouts."""
+    """`_get_layer_data_generator` of the reference (:464-500; its wX / qX stored by oracle/make_golden.py pin_goldens)
+    against the mirror's in-memory version, both layouts."""
     monkeypatch.chdir(tmp_path)
-    ref = ref_shim.load()
+    z = golden("ref_layer_data")
     net, seq, x = mlp_case()
-    qr = ref.QuantizedNeuralNetwork(net, 16, seq, logger=QUIET)
-    qm = QuantizedNeuralNetwork.__new__(QuantizedNeuralNetwork)
-    qm.get_data, qm.trained_net, qm.quantized_net = seq, net, qr.quantized_net
+    qm = QuantizedNeuralNetwork(net, 16, seq, logger=QUIET)
     for idx, transpose in ((1, True), (3, True), (3, False), (5, True)):
-        name = qr._get_layer_data_generator(idx, transpose=transpose)
-        hf = ref_shim.MEMORY_FILES[name]
+        key = f"{idx}{'t' if transpose else ''}"
         data = qm._get_layer_data_generator(idx, transpose=transpose)
-        assert np.array_equal(np.asarray(hf["wX"]), data.wX) and np.array_equal(np.asarray(hf["qX"]), data.qX)
+        assert np.array_equal(z["wX" + key], data.wX) and np.array_equal(z["qX" + key], data.qX)
         m = len(seq) * seq.batch_size
         assert (data.wX.shape[-1] if transpose else data.wX.shape[0]) == m == 64
         tail = data.wX[..., 50:] if transpose else data.wX[50:]
         assert not tail.any()                # rows past the overwritten short batch stay zero-filled
 
 
-@needs_ref
 def test_reference_cnn_layers_vs_mirror(tmp_path, monkeypatch):
     monkeypatch.chdir(tmp_path)
-    net, seq, x, qr, Qr = run_reference_cnn_layers(4, 4)
+    z = golden("ref_network_cnn")
+    net, seq, x = cnn_case()
+    Qr = {int(k[1:]): z[k] for k in z.files if k.startswith("Q")}
+    pred = reference_quantized_net(net, Qr).predict(x)
+    assert np.array_equal(pred.argmax(-1), z["pred"])
     for conv_path in ("nhwc", "patches"):
         qm = with_oracle(QuantizedCNN, net, 16, seq, logger=QUIET, bits=4, alphabet_scalar=4, conv_path=conv_path,
                          patch_mini_batch_size=16)
         qm.quantize_network()
         for idx, Q in Qr.items():
             assert np.array_equal(qm.quantized_net.layers[idx].get_weights()[0], Q), (conv_path, idx)
-        assert np.array_equal(qr.quantized_net.predict(x), qm.quantized_net.predict(x))
+        assert np.array_equal(pred, qm.quantized_net.predict(x))
     assert len(Qr) == 6                      # four conv + two Dense layers
 
 
