@@ -94,15 +94,10 @@ int gpfq_set_stream(gpfq_ctx *ctx, void *cuda_stream);
  *   "corr_rows"    correlation form: image rows per band (0 auto by image height, or 4 / 6 / 8)
  *   "corr_strip"   correlation form on small images (widths 8, 14, 16, 28, 32, 56, 64): 0 the strip kernel (whole strips of <= 16 columns as
  *                  straight-line code), 2 the band kernel
- *   "sweep_kernel"  0 pipelined range walk (panel of block b+1 contracted during the walk of block b) when every CTA is
- *                  resident, else the persistent tile kernel; 1 one launch pair per block; 2 always the persistent tile kernel
- *   "sweep_wq"     residual-form sweep on tcgen05: 0 auto, 1 W part of the residual update on an aux stream underneath the walk,
- *                  2 W and Q part as one two-product launch
- *   "sweep_range"  residual-form sweep on tcgen05: directions per range (0 auto, else a multiple of 128)
- *   "sweep_groups" residual-form sweep on tcgen05: independent neuron groups in flight (0 auto, 1, 2 or 4)
- *   "sweep_nt"     pipelined range walk: neurons per CTA (0 auto, 8, 16 or 32)
- *   "sweep_walk"   range walk of the sweep for one symmetric equispaced alphabet: 0 auto (the tensor-core walk sweep_tc_kernel in the
- *                  residual form and for Gram-row sweeps from 2048 directions), 1 always the tensor-core walk, 2 sweep_pipe / sweep_tile
+ *   "sweep_walk"   range walk of the Gram-row sweep for one symmetric equispaced alphabet: 0 auto (the tensor-core walk
+ *                  sweep_tc_kernel from 2048 directions, below that sweep_pipe / sweep_tile), 1 always the tensor-core walk,
+ *                  2 always sweep_pipe / sweep_tile.  The residual form walks with sweep_tc_kernel when its contractions run on
+ *                  tcgen05, with sweep_pipe / sweep_tile when they run on the fp64 pipe ("sweep_i8")
  *   "sweep_i8"     contractions of the residual-form sweep: 0 auto, 1 int8 slices on tcgen05, 2 fp64 DMMA
  *   "sweep_outer"  0 auto, 1 Gram rows of all earlier directions, 2 carried residuals (3 m N0 N1 MACs: wins when m << N0),
  *                  3 carried residuals as one chain (default: two halves of the neurons on two streams, so that one half's

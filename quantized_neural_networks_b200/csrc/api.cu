@@ -130,12 +130,6 @@ extern "C" int gpfq_create(int device, gpfq_ctx **out) {
         return GPFQ_ERR_CUDA;
     }
     ctx->stream = ctx->own_stream;
-    if (const char *v = getenv("GPFQ_CONV_KERNEL"))  // A/B switch for profiling: tma (default) | ldg | generic
-        ctx->conv_variant = !strcmp(v, "ldg") ? 1 : (!strcmp(v, "generic") ? 2 : 0);
-    if (const char *v = getenv("GPFQ_SWEEP_KERNEL"))  // A/B switch: tile (default) | blocks
-        ctx->sweep_variant = !strcmp(v, "blocks") ? 1 : 0;
-    if (const char *v = getenv("GPFQ_GRAM_KERNEL"))   // A/B switch: auto (default) | dmma | i8
-        ctx->gram_variant = !strcmp(v, "dmma") ? 1 : (!strcmp(v, "i8") ? 2 : 0);
     *out = ctx;
     return GPFQ_OK;
 }
@@ -204,30 +198,13 @@ extern "C" int gpfq_set_option(gpfq_ctx *ctx, const char *key, int64_t value) {
         // 3 carried residuals as ONE chain (no two-stream split of the neurons)
         if (value < 0 || value > 3) return gpfq_fail(ctx, GPFQ_ERR_ARG, "sweep_outer must be 0, 1, 2 or 3");
         ctx->lowrank_variant = (int)value;
-    } else if (!strcmp(key, "sweep_wq")) {      // residual-form sweep on tcgen05: W part of the update on the aux stream (1) or
-                                                 // together with the Q part as one two-product launch (2); 0 auto
-        if (value < 0 || value > 2) return gpfq_fail(ctx, GPFQ_ERR_ARG, "sweep_wq must be 0, 1 or 2");
-        ctx->sweep_wq = (int)value;
-    } else if (!strcmp(key, "sweep_range")) {   // residual-form sweep on tcgen05: directions per range (0 auto)
-        if (value < 0 || value > 8192 || value % 128) return gpfq_fail(ctx, GPFQ_ERR_ARG, "sweep_range must be 0 or a multiple of 128 up to 8192");
-        ctx->sweep_range = (int)value;
-    } else if (!strcmp(key, "sweep_groups")) {  // residual-form sweep: independent neuron groups in flight (0 auto)
-        if (value != 0 && value != 1 && value != 2 && value != 4) return gpfq_fail(ctx, GPFQ_ERR_ARG, "sweep_groups must be 0, 1, 2 or 4");
-        ctx->sweep_groups = (int)value;
-    } else if (!strcmp(key, "sweep_nt")) {      // pipelined range walk: neurons per CTA (0 auto)
-        if (value != 0 && value != 8 && value != 16 && value != 32) return gpfq_fail(ctx, GPFQ_ERR_ARG, "sweep_nt must be 0, 8, 16 or 32");
-        ctx->sweep_nt = (int)value;
-    } else if (!strcmp(key, "sweep_walk")) {    // range walk of the residual-form sweep (ternary alphabets): 0 auto, 1 tensor-core
-                                                 // walk (sweep_tc.cu), 2 sweep_pipe / sweep_tile kernels
+    } else if (!strcmp(key, "sweep_walk")) {    // range walk of the Gram-row sweep (one symmetric equispaced alphabet): 0 auto,
+                                                 // 1 tensor-core walk (sweep_tc.cu), 2 sweep_pipe / sweep_tile kernels
         if (value < 0 || value > 2) return gpfq_fail(ctx, GPFQ_ERR_ARG, "sweep_walk must be 0, 1 or 2");
         ctx->sweep_walk = (int)value;
     } else if (!strcmp(key, "sweep_i8")) {      // residual-form sweep contractions: 0 auto, 1 int8 slices on tcgen05, 2 fp64 DMMA
         if (value < 0 || value > 2) return gpfq_fail(ctx, GPFQ_ERR_ARG, "sweep_i8 must be 0, 1 or 2");
         ctx->sweep_i8 = (int)value;
-    } else if (!strcmp(key, "sweep_kernel")) {  // 0 pipelined range walk where it applies, else the neuron-tile kernel;
-                                                 // 1 one launch pair per block; 2 always the (unpipelined) neuron-tile kernel
-        if (value < 0 || value > 2) return gpfq_fail(ctx, GPFQ_ERR_ARG, "sweep_kernel must be 0, 1 or 2");
-        ctx->sweep_variant = (int)value;
     } else {
         return gpfq_fail(ctx, GPFQ_ERR_ARG, "unknown option '%s'", key);
     }

@@ -53,9 +53,6 @@ struct gpfq_ctx {
     cudaStream_t aux_stream[8] = {};   // residual-form sweep, up to 4 neuron groups: [g] the W part of group g's residual update,
                                        // [4 + g] the main chain of group g >= 1 (group 0 runs on `stream`)
     cudaEvent_t ev_chain[12] = {};     // ... [3 g] residuals sliced (main -> aux), [3 g + 1] W part landed (aux -> main), [3 g + 2] done
-    int sweep_wq = 0;                  // ... 0 auto, 1 W part of the update on the aux stream, 2 W and Q parts as one two-product launch
-    int sweep_range = 0;               // ... directions per range (0 auto; a multiple of 128)
-    int sweep_groups = 0;              // ... neuron groups (0 auto, 1 / 2 / 4)
     std::string err = "";
     int launches = 0;
     int conv_variant = 0;         // 3x3 patch-Gram kernel: 0 TMA-staged / correlation form (default), 1 direct LDG, 2 generic,
@@ -66,18 +63,14 @@ struct gpfq_ctx {
     int corr_rb = 0;              // correlation-form conv Grams: rows per band (0: chosen per image height)
     int corr_strip_occ[2][2][3] = {};  // strip kernel: resident CTAs per SM by [X~ == X][rows per band 1 / 4][strip width 8 / 14 / 16]
     int corr_strip = 0;           // ... small images (W in {8, 14, 16, 28, 32, 56, 64}): 0 the strip kernel, 2 the band kernel
-    int sweep_variant = 0;        // triangular sweep: 0 persistent neuron-tile kernel (default), 1 one launch pair per block
     bool stream_literal = false;  // streaming walk: reproduce the reference's fp32-rounded w*X products (set per call)
     int gram_variant = 0;         // Dense Gram stage: 0 auto, 1 fp64 DMMA (mma.sync), 2 int8 slices on tcgen05 (gram_i8.cu)
     int lowrank_variant = 0;      // sweep outer level: 0 auto, 1 Gram rows, 2 residual (low-rank) form
-    int sweep_nt = 0;             // pipelined range walk: neurons per CTA (0 auto, 8 / 16 / 32)
-    int sweep_walk = 0;           // range walk of the residual-form sweep: 0 auto, 1 tensor-core walk (sweep_tc.cu), 2 sweep_pipe / sweep_tile
-    int last_sweep_tc = 0;        // the last residual-form sweep walked its ranges with sweep_tc_kernel
+    int sweep_walk = 0;           // range walk of the Gram-row sweep: 0 auto, 1 tensor-core walk (sweep_tc.cu), 2 sweep_pipe / sweep_tile
     int sweep_i8 = 0;             // sweep contractions of the residual form: 0 auto, 1 int8 slices on tcgen05, 2 fp64 DMMA
     int i8_pairs_d = 0;           // int8 Gram: keep slice pairs with k + l <= this (0: the default of gram_i8.cu)
     const double *h_alph = nullptr;  // host copy of the current call's alphabets (levels back to back) and their offsets
     const int *h_koff = nullptr, *h_flags = nullptr;
-    int last_sweep_i8 = 0;        // the last residual-form sweep ran its contractions on tcgen05 (int8 slices)
     double *gram_only_out = nullptr;  // set for the duration of gpfq_conv_gram_nhwc: conv_finish hands the Grams out, no walk
     int last_gram_kernel = 0;     // what the last Dense Gram stage ran (1 DMMA, 2 int8 tcgen05)
     size_t i8_oom_bytes = 0;      // smallest int8-Gram workspace that failed to allocate (0: none yet)

@@ -5,9 +5,9 @@
 // fp32 products) the residual dot of step t is
 //     d_t = <Xq_t, u_{t-1}> = sum_{s<t} ( w_s G1[t,s] - q_s G2[t,s] )
 // so q_t = Q( (d_t + w_t G1[t,t]) / fl32(sqrt(G2[t,t]))^2 ) with the two guards of :83-87 intact.
-// The sweep walks blocks of 32 directions: contributions of earlier blocks are one NT contraction
-// per block (gemm_nt.cuh, two segments), the 32 in-block steps run warp-per-neuron with the running
-// d held one-per-lane and exchanged by shuffles.
+// The sweep walks ranges of directions: what the earlier ranges contribute to a range is one NT contraction
+// (gemm_nt.cuh, two segments), then one persistent kernel walks the range's blocks of 32 directions for a tile of
+// neurons (sweep_pipe_kernel / sweep_tile_kernel below, or the tensor-core walk of sweep_tc.cu).
 #include <algorithm>
 
 #include "gemm_nt.cuh"
@@ -47,53 +47,6 @@ __global__ void transpose_q_kernel(const double *__restrict__ Qt, int64_t N0, in
         const int64_t t = tb + r, j = jb + threadIdx.x;
         if (t < N0 && j < nj) Q[t * ldq + col0 + j] = tile[threadIdx.x][r];
     }
-}
-
-// In-block steps of the sweep.  One warp per neuron, lane = direction within the block.
-//   G1, G2 : (N0, N0) fp64, lower triangle + diagonal valid
-//   Wt     : (nj, N0) fp64;  Dt : (n_alph, nj, 32) prior-block part of d (ignored for block 0)
-//   Qt     : (n_alph, nj, N0) fp64 output
-__global__ void __launch_bounds__(256)
-sweep_inblock_kernel(const double *__restrict__ G1, const double *__restrict__ G2, int64_t ldg,
-                     int64_t N0, int blk, const double *__restrict__ Wt, const double *__restrict__ Dt,
-                     double *__restrict__ Qt, int64_t nj, const double *__restrict__ alphabets,
-                     const int *__restrict__ Koff, const int *__restrict__ Flags) {
-    __shared__ double g1[SWEEP_B][SWEEP_B + 1], g2[SWEEP_B][SWEEP_B + 1];
-    __shared__ double nrm[SWEEP_B];
-    __shared__ double alph[GPFQ_MAX_K];
-    const int64_t t0 = (int64_t)blk * SWEEP_B;
-    const int nb = (int)((N0 - t0) < SWEEP_B ? (N0 - t0) : SWEEP_B);
-    const int a = blockIdx.y;
-    const int K = Koff[a + 1] - Koff[a];
-    for (int e = threadIdx.x; e < SWEEP_B * SWEEP_B; e += blockDim.x) {
-        const int r = e / SWEEP_B, c = e % SWEEP_B;
-        const bool ok = r < nb && c <= r;
-        g1[r][c] = ok ? G1[(t0 + r) * ldg + t0 + c] : 0.0;
-        g2[r][c] = ok ? G2[(t0 + r) * ldg + t0 + c] : 0.0;
-    }
-    for (int e = threadIdx.x; e < K; e += blockDim.x) alph[e] = alphabets[Koff[a] + e];
-    __syncthreads();
-    if (threadIdx.x < SWEEP_B)
-        nrm[threadIdx.x] = threadIdx.x < nb ? (double)(float)sqrt(g2[threadIdx.x][threadIdx.x]) : 0.0;
-    __syncthreads();
-    const double inv_step = gpfq_inv_step(alph, K, Flags[a]);
-
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int64_t j = (int64_t)blockIdx.x * (blockDim.x >> 5) + warp;
-    if (j >= nj) return;
-    const int64_t t = t0 + lane;
-    const double w = (lane < nb) ? Wt[j * N0 + t] : 0.0;
-    double d = (blk > 0 && lane < nb) ? Dt[((int64_t)a * nj + j) * SWEEP_B + lane] : 0.0;
-    double myq = 0.0;
-    for (int tt = 0; tt < nb; ++tt) {
-        const double dtt = __shfl_sync(0xffffffffu, d, tt);
-        const double wtt = __shfl_sync(0xffffffffu, w, tt);
-        const double num = fma(wtt, g1[tt][tt], dtt);
-        const double q = gpfq_decide(nrm[tt], dtt, num, wtt, alph, K, inv_step);
-        if (lane == tt) myq = q;
-        if (lane > tt) d += g1[lane][tt] * wtt - g2[lane][tt] * q;
-    }
-    if (lane < nb) Qt[((int64_t)a * nj + j) * N0 + t] = myq;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -142,10 +95,7 @@ sweep_tile_kernel(const double *__restrict__ G1, const double *__restrict__ G2, 
                   const double *__restrict__ Wt, double *__restrict__ Qt, int64_t nj,
                   const double *__restrict__ alphabets, const int *__restrict__ Koff,
                   const int *__restrict__ Flags, int64_t t_begin, int64_t t_end, const double *__restrict__ Dt,
-                  int64_t ldd, int8_t *__restrict__ Kq, int64_t krows, int64_t krow0, double inv_h) {
-    // Kq (nullable): the decisions also go out as int8 level indices k' = q / h (one digit slice of the int8 contractions
-    // of the residual-form sweep, slgemm_i8.cu) in its K-block-tiled layout (sl_offset): krows rows, this launch's neuron 0 is
-    // row krow0.
+                  int64_t ldd) {
     // Directions [t_begin, t_end) (t_begin a multiple of 32).  Dt (nullable): (n_alph, nj, ldd) contributions of the
     // directions before t_begin, from one large NT contraction on the host side (two-level blocking).
     using Cfg = SweepCfg<NT>;
@@ -356,11 +306,7 @@ sweep_tile_kernel(const double *__restrict__ G1, const double *__restrict__ G2, 
         __syncthreads();
         for (int e = tid; e < NT * B; e += THREADS) {
             const int j = e / B, t = e % B;
-            if (jt + j < nj && t < nb) {
-                const double q = qblk[j * (B + 1) + t];
-                Qa[(jt + j) * N0 + t0 + t] = q;
-                if (Kq) Kq[sl_offset(t0 + t, 0, krow0 + jt + j, krows, 1)] = (int8_t)__double2int_rn(q * inv_h);
-            }
+            if (jt + j < nj && t < nb) Qa[(jt + j) * N0 + t0 + t] = qblk[j * (B + 1) + t];
         }
         __syncthreads();  // Q block visible to this CTA's later panel loads
     }
@@ -375,7 +321,7 @@ sweep_tile_kernel(const double *__restrict__ G1, const double *__restrict__ G2, 
 // 32-direction chunk, G2[block b + 1, block b] x Q_b, remains between two walks.  Two working sets (block operands, prior
 // dots, decisions) alternate between the roles; named barriers hand them over:
 //   READY[s]      contractors -> walkers: set s holds block b's operands and residual dots
-//   WALK_DONE[s]  walkers -> contractors: the decisions of block b are in set s (and in Qt / the int8 index slice)
+//   WALK_DONE[s]  walkers -> contractors: the decisions of block b are in set s (and in Qt)
 // One CTA per SM (up to 200 KB of shared memory); the host uses it when every CTA of the launch is resident at once.
 // ---------------------------------------------------------------------------------------------
 __device__ __forceinline__ void named_bar_sync(int id, int count) { asm volatile("bar.sync %0, %1;\n" ::"r"(id), "r"(count) : "memory"); }
@@ -396,7 +342,7 @@ __global__ void __launch_bounds__(256, 1)
 sweep_pipe_kernel(const double *__restrict__ G1, const double *__restrict__ G2, int64_t ldg, int64_t N0,
                   const double *__restrict__ Wt, double *__restrict__ Qt, int64_t nj, const double *__restrict__ alphabets,
                   const int *__restrict__ Koff, const int *__restrict__ Flags, int64_t t_begin, int64_t t_end,
-                  const double *__restrict__ Dt, int64_t ldd, int8_t *__restrict__ Kq, int64_t krows, int64_t krow0, double inv_h) {
+                  const double *__restrict__ Dt, int64_t ldd) {
     using Cfg = PipeCfg<NT>;
     constexpr int B = Cfg::B, KC = Cfg::KC, LD = Cfg::LD, STAGES = Cfg::STAGES, CT = Cfg::CT, NA = NT / 8, NW = 4 * NT;
     constexpr int BAR_C = 1, BAR_READY = 2, BAR_WALK_DONE = 4, BAR_Q_STORED = 6, HANDOVER = NW + CT;
@@ -621,16 +567,12 @@ sweep_pipe_kernel(const double *__restrict__ G1, const double *__restrict__ G2, 
             // shared memory for the one chunk that separates this walk from the next
             __threadfence_block();
             named_bar_arrive(BAR_WALK_DONE + s, HANDOVER);
-            // ---- this lane's own decisions (directions = r mod 4) go out: Qt for later ranges / the result, and the int8 index.
+            // ---- this lane's own decisions (directions = r mod 4) go out to Qt, for later ranges and the result.
             // qblk of this set is rewritten only after the contractors have seen Q_STORED of this block (two blocks on).
 #pragma unroll
             for (int i = 0; i < 8; ++i) {
                 const int tt = 4 * i + r;
-                if (jt + j < nj && tt < nb) {
-                    const double q = qrow[tt];
-                    Qa[(jt + j) * N0 + t0 + tt] = q;
-                    if (Kq) Kq[sl_offset(t0 + tt, 0, krow0 + jt + j, krows, 1)] = (int8_t)__double2int_rn(q * inv_h);
-                }
+                if (jt + j < nj && tt < nb) Qa[(jt + j) * N0 + t0 + tt] = qrow[tt];
             }
             if (b + 2 < nblk) {   // somebody will wait for it
                 __threadfence_block();
@@ -643,14 +585,12 @@ sweep_pipe_kernel(const double *__restrict__ G1, const double *__restrict__ G2, 
 template <int NT>
 static int launch_sweep_pipe(gpfq_ctx *ctx, const double *G1, const double *G2, int64_t ldg, int64_t N0, const double *Wt,
                              double *Qt, int64_t nj, const double *d_alph, const int *d_koff, const int *d_flags,
-                             int n_alph, int64_t t_begin, int64_t t_end, const double *Dt, int64_t ldd, int8_t *Kq,
-                             int64_t krows, int64_t krow0, double inv_h) {
+                             int n_alph, int64_t t_begin, int64_t t_end, const double *Dt, int64_t ldd) {
     const size_t smem = PipeCfg<NT>::SMEM;
     dim3 grid((unsigned)ceil_div64(nj, NT), (unsigned)n_alph);
     auto k = sweep_pipe_kernel<NT>;
     CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    k<<<grid, 256, smem, ctx->stream>>>(G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, t_begin, t_end, Dt, ldd, Kq, krows,
-                                        krow0, inv_h);
+    k<<<grid, 256, smem, ctx->stream>>>(G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, t_begin, t_end, Dt, ldd);
     KERNEL_CHECK(ctx);
     return GPFQ_OK;
 }
@@ -658,8 +598,7 @@ static int launch_sweep_pipe(gpfq_ctx *ctx, const double *G1, const double *G2, 
 template <int NT>
 static int launch_sweep_tile(gpfq_ctx *ctx, const double *G1, const double *G2, int64_t ldg, int64_t N0, const double *Wt,
                              double *Qt, int64_t nj, const double *d_alph, const int *d_koff, const int *d_flags,
-                             int n_alph, int64_t t_begin, int64_t t_end, const double *Dt, int64_t ldd, int8_t *Kq = nullptr,
-                             int64_t krows = 0, int64_t krow0 = 0, double inv_h = 0.0) {
+                             int n_alph, int64_t t_begin, int64_t t_end, const double *Dt, int64_t ldd) {
     const size_t smem = SweepCfg<NT>::SMEM;
     dim3 grid((unsigned)ceil_div64(nj, NT), (unsigned)n_alph);
     const bool aligned = (N0 % 2 == 0) && (ldg % 2 == 0) && ((uintptr_t)G1 % 16 == 0) && ((uintptr_t)G2 % 16 == 0) &&
@@ -667,11 +606,11 @@ static int launch_sweep_tile(gpfq_ctx *ctx, const double *G1, const double *G2, 
     if (aligned) {
         auto k = sweep_tile_kernel<NT, true>;
         CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k<<<grid, 256, smem, ctx->stream>>>(G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, t_begin, t_end, Dt, ldd, Kq, krows, krow0, inv_h);
+        k<<<grid, 256, smem, ctx->stream>>>(G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, t_begin, t_end, Dt, ldd);
     } else {
         auto k = sweep_tile_kernel<NT, false>;
         CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k<<<grid, 256, smem, ctx->stream>>>(G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, t_begin, t_end, Dt, ldd, Kq, krows, krow0, inv_h);
+        k<<<grid, 256, smem, ctx->stream>>>(G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, t_begin, t_end, Dt, ldd);
     }
     KERNEL_CHECK(ctx);
     return GPFQ_OK;
@@ -782,7 +721,7 @@ __global__ void widen_transpose_kernel(const float *__restrict__ X, int64_t ldx,
 }
 
 static bool dense_uses_lowrank(gpfq_ctx *ctx, int64_t N0, int64_t m, int64_t nj, int n_alph, bool same, bool i8_ok) {
-    if (ctx->sweep_variant == 1 || ctx->lowrank_variant == 1) return false;
+    if (ctx->lowrank_variant == 1) return false;
     if (ctx->lowrank_variant >= 2) return N0 > 64;
     if (!i8_ok) return 3 * m < N0 && N0 >= 4096 && nj >= 256;   // fp64 (DMMA) contractions: the measured rule of round 1
     // int8-slice contractions (slgemm_i8.cu) and the tensor-core range walk (sweep_tc.cu).  Both forms calibrated on this pool's B200
@@ -821,31 +760,23 @@ static int64_t pick_range_length(gpfq_ctx *ctx, int64_t nj, int n_alph) {
 
 static int dispatch_sweep_tile(gpfq_ctx *ctx, int NT, const double *G1, const double *G2, int64_t ldg, int64_t N0,
                                const double *Wt, double *Qt, int64_t nj, const double *d_alph, const int *d_koff,
-                               const int *d_flags, int n_alph, int64_t tb, int64_t te, const double *Dp, int64_t R,
-                               int8_t *Kq = nullptr, int64_t krows = 0, int64_t krow0 = 0, double inv_h = 0.0) {
+                               const int *d_flags, int n_alph, int64_t tb, int64_t te, const double *Dp, int64_t R) {
     // The pipelined walk (one CTA per SM) when its 16-byte copies are possible and every CTA of the launch is resident at
-    // once; the narrowest neuron tile that allows it.  ctx->sweep_variant == 2 keeps the unpipelined tile kernel (A/B).
+    // once; the narrowest neuron tile that allows it.
     const bool aligned = (N0 % 2 == 0) && (ldg % 2 == 0) && ((uintptr_t)G1 % 16 == 0) && ((uintptr_t)G2 % 16 == 0) &&
                          ((uintptr_t)Wt % 16 == 0) && ((uintptr_t)Qt % 16 == 0) && ((nj * N0) % 2 == 0);
-    if (aligned && ctx->sweep_variant != 2) {
+    if (aligned) {
         const int64_t sms = ctx->sm_count;
-        const int force = ctx->sweep_nt;
-        if (force == 32 || (force == 0 && false)) {
-            if (ceil_div64(nj, 32) * n_alph <= sms)
-                return launch_sweep_pipe<32>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R, Kq, krows, krow0, inv_h);
-        } else if (force == 16) {
-            if (ceil_div64(nj, 16) * n_alph <= sms)
-                return launch_sweep_pipe<16>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R, Kq, krows, krow0, inv_h);
-        } else if (ceil_div64(nj, 8) * n_alph <= sms)
-            return launch_sweep_pipe<8>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R, Kq, krows, krow0, inv_h);
+        if (ceil_div64(nj, 8) * n_alph <= sms)
+            return launch_sweep_pipe<8>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R);
         if (ceil_div64(nj, 16) * n_alph <= sms)
-            return launch_sweep_pipe<16>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R, Kq, krows, krow0, inv_h);
+            return launch_sweep_pipe<16>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R);
         if (ceil_div64(nj, 32) * n_alph <= sms)
-            return launch_sweep_pipe<32>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R, Kq, krows, krow0, inv_h);
+            return launch_sweep_pipe<32>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R);
     }
-    if (NT == 32) return launch_sweep_tile<32>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R, Kq, krows, krow0, inv_h);
-    if (NT == 16) return launch_sweep_tile<16>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R, Kq, krows, krow0, inv_h);
-    return launch_sweep_tile<8>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R, Kq, krows, krow0, inv_h);
+    if (NT == 32) return launch_sweep_tile<32>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R);
+    if (NT == 16) return launch_sweep_tile<16>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R);
+    return launch_sweep_tile<8>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R);
 }
 
 // Sweep with the low-rank outer level.  Wt (nj, N0) is ready; Qt (n_alph, nj, N0) receives the result.
@@ -1079,27 +1010,23 @@ static bool dense_lowrank_uses_i8(gpfq_ctx *ctx, int64_t N0, int64_t m, int64_t 
 }
 
 static int dense_lowrank_sweep_i8(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ldx, int64_t N0, int64_t m,
-                                  const double *Wt, double *Qt, int64_t nj, const double *d_alph, const int *d_koff,
-                                  const int *d_flags, int NT, double h, gpfq_stats *stats, const float *W, int64_t ldw, int64_t j0,
-                                  double *Qd, int64_t ldq, int64_t col0) {
+                                  const double *Wt, int64_t nj, const double *d_alph, double h, gpfq_stats *stats, const float *W,
+                                  int64_t ldw, int64_t j0, double *Qd, int64_t ldq, int64_t col0) {
     const bool same = (Xq == X);
     cudaStream_t st = ctx->stream, side = ctx->copy_stream;
     int64_t R = pick_range_length(ctx, nj, 1);
     R = std::max<int64_t>(128, R / 128 * 128);      // K blocks of the update are 128 directions
-    if (ctx->sweep_walk != 2) R = std::min<int64_t>(R, stc::MAX_R);   // the tensor-core walk keeps a range's level indices in shared memory
-    if (ctx->sweep_range) R = ctx->sweep_range;
+    R = std::min<int64_t>(R, stc::MAX_R);           // the tensor-core walk keeps a range's level indices in shared memory
     // Ternary alphabets: the tensor-core range walk (sweep_tc.cu) -- the W terms of every range as ONE batched product before the
     // sweep, the Q terms inside the walk kernel, one thread per neuron
     const int K_levels = ctx->h_koff[1] - ctx->h_koff[0];
     const double a_top = ctx->h_alph[ctx->h_koff[0] + K_levels - 1];
     const double *d_levels = d_alph;   // one alphabet per call on this path: its levels start the device array
-    const bool use_tc = ctx->sweep_walk != 2 && R <= stc::MAX_R;
-    ctx->last_sweep_tc = use_tc ? 1 : 0;
     const int64_t N0P = ceil_div64(N0, R) * R, mP = ceil_div64(m, 128) * 128, njP = ceil_div64(nj, 128) * 128;   // whole ranges
     constexpr int S = 5;
     int8_t *sW = nullptr, *sXT = nullptr, *sXqT = nullptr, *sXq = nullptr, *sU = nullptr, *sKq = nullptr;
     int32_t *e = nullptr;
-    double *Ut = nullptr, *Gc1 = nullptr, *Gc2 = nullptr, *Do = nullptr;
+    double *Ut = nullptr, *Gc1 = nullptr, *Gc2 = nullptr;
     GPFQ_TRY(gpfq_ws(ctx, WS_SL_W, (size_t)S * njP * N0P, (void **)&sW));
     GPFQ_TRY(gpfq_ws(ctx, WS_SL_XT, (size_t)S * mP * N0P, (void **)&sXT));
     if (same) sXqT = sXT;
@@ -1115,7 +1042,6 @@ static int dense_lowrank_sweep_i8(gpfq_ctx *ctx, const float *X, const float *Xq
     GPFQ_TRY(gpfq_ws(ctx, WS_G2, gc_bytes, (void **)&Gc2));
     if (same) Gc1 = Gc2;
     else GPFQ_TRY(gpfq_ws(ctx, WS_G1, gc_bytes, (void **)&Gc1));
-    GPFQ_TRY(gpfq_ws(ctx, WS_DT, (size_t)nj * R * sizeof(double), (void **)&Do));
     constexpr int D_DOTS_GRAM = 6;
 
     CUDA_TRY(ctx, gpfq_record(ctx, 2, st));
@@ -1152,10 +1078,10 @@ static int dense_lowrank_sweep_i8(gpfq_ctx *ctx, const float *X, const float *Xq
     GPFQ_TRY(sl_make_operand(ctx, &oW, sW, njP, N0P, S, eW, 0, false));
     TcTables tct;
     double *Dsplit = nullptr;   // K-split partials of the residual dots (few neurons)
-    if (use_tc && ceil_div64(nj, 128) * (R / 64) * 3 <= ctx->sm_count) GPFQ_TRY(gpfq_ws(ctx, WS_PART, (size_t)6 * njP * R * sizeof(double), (void **)&Dsplit));
+    if (ceil_div64(nj, 128) * (R / 64) * 3 <= ctx->sm_count) GPFQ_TRY(gpfq_ws(ctx, WS_PART, (size_t)6 * njP * R * sizeof(double), (void **)&Dsplit));
     double *Pd = nullptr;   // (nj, N0P): per range the W terms of the range itself, then + D_r (what the earlier ranges contribute)
     float *Wn = nullptr;    // (nj, N0P): the weights neuron-major, fp32
-    if (use_tc) {
+    {
         GPFQ_TRY(gpfq_ws(ctx, WS_TC_W, (size_t)njP * N0P * sizeof(float), (void **)&Wn));   // (rows >= nj: never written, never used)
         GPFQ_TRY(sweep_tc_weights(ctx, W, ldw, j0, N0, N0P, nj, Wn));
         int8_t *sG1 = nullptr;
@@ -1199,7 +1125,7 @@ static int dense_lowrank_sweep_i8(gpfq_ctx *ctx, const float *X, const float *Xq
         // measured (VGG16 fc1 / fc2): with thousands of neurons the sweep is bound by the SUM of its contraction launches -- W and Q
         // part as ONE two-product launch (25.5 vs 27.3 ms); a shard of a few hundred neurons is bound by the LATENCY of the
         // chain -- W part off it, on the aux stream (11.0 vs 11.6 ms)
-        const bool merged = ctx->sweep_wq == 2 || (ctx->sweep_wq == 0 && nj >= 2048);
+        const bool merged = nj >= 2048;
         auto cu = [&](cudaError_t e) { if (e != cudaSuccess && rc == GPFQ_OK) rc = gpfq_fail(ctx, GPFQ_ERR_CUDA, "%s", cudaGetErrorString(e)); };
         for (int64_t tb = 0, pb = 0; tb < N0 && rc == GPFQ_OK; pb = tb, tb += R) {
             const int64_t te = tb + R < N0 ? tb + R : N0;
@@ -1227,7 +1153,7 @@ static int dense_lowrank_sweep_i8(gpfq_ctx *ctx, const float *X, const float *Xq
                 int ns = 1;
                 for (int c : {6, 4, 3})   // (two-way splits measured slower than none: fc3's 1000 neurons 1.64 -> 1.76 ms)
                     if (ns == 1 && dtiles * c <= ctx->sm_count && (mP / 64) % c == 0 && mP / c >= 256) ns = c;
-                if (use_tc && ns > 1 && Dsplit) {
+                if (ns > 1 && Dsplit) {
                     SlBatch sb;
                     sb.n = ns;
                     sb.a_k = sb.b_k = mP / ns;
@@ -1236,8 +1162,7 @@ static int dense_lowrank_sweep_i8(gpfq_ctx *ctx, const float *X, const float *Xq
                     rc = slgemm_i8_ex(ctx, &dps, 1, Dsplit + j_lo * R, R, njh, te - tb, false, sb);
                     if (rc == GPFQ_OK)
                         rc = sweep_tc_add_partials(ctx, Pd + j_lo * N0P + tb, N0P, Dsplit + j_lo * R, ns, njP * R, R, njh, te - tb);
-                } else if (use_tc) rc = slgemm_i8(ctx, &dp, 1, Pd + j_lo * N0P + tb, N0P, njh, te - tb, true);   // P_r += U X~_r^T
-                else rc = slgemm_i8(ctx, &dp, 1, Do + j_lo * R, R, njh, te - tb, false);   // D_r = U X~_r^T
+                } else rc = slgemm_i8(ctx, &dp, 1, Pd + j_lo * N0P + tb, N0P, njh, te - tb, true);   // P_r += U X~_r^T
                 if (rc != GPFQ_OK) break;
             }
             if (te < N0 && !merged) {   // the W part of THIS range, for the ranges after it
@@ -1250,30 +1175,22 @@ static int dense_lowrank_sweep_i8(gpfq_ctx *ctx, const float *X, const float *Xq
                 ctx->stream = on;
                 if (rc != GPFQ_OK) break;
             }
-            if (use_tc)
-                rc = sweep_tc_range(ctx, tct, tb, te, j_lo, njh, sKq, njP, j_lo, a_top, d_levels, K_levels);   // {-a, 0, a}: h = a / 2
-            else
-                rc = dispatch_sweep_tile(ctx, NT, Gc1 - tb, Gc2 - tb, R, N0, Wt + j_lo * N0, Qt + j_lo * N0, njh, d_alph, d_koff,
-                                         d_flags, 1, tb, te, tb > 0 ? Do + j_lo * R : nullptr, R, sKq, njP, j_lo, 1.0 / h);
+            rc = sweep_tc_range(ctx, tct, tb, te, j_lo, njh, sKq, njP, j_lo, a_top, d_levels, K_levels);   // {-a, 0, a}: h = a / 2
         }
         ctx->stream = keep;
         return rc;
     };
     if (stats) {
         stats->flops_algorithmic = 2LL * (19 + 5 + 15) * nj * m * N0;   // int8 operations of the 39 slice-pair products
-        stats->reserved |= 1;
-        if (use_tc) stats->reserved |= 2;   // ... and the ranges were walked by sweep_tc_kernel
+        stats->reserved |= 1 | 2;   // int8-slice contractions, ranges walked by sweep_tc_kernel
     }
-    ctx->last_sweep_i8 = 1;
-    int G = ctx->sweep_groups ? ctx->sweep_groups : (nj >= 4096 ? 4 : (nj >= 2048 ? 2 : 1));
+    int G = nj >= 4096 ? 4 : (nj >= 2048 ? 2 : 1);
     if (ctx->lowrank_variant == 3) G = 1;
     while (G > 1 && ceil_div64(nj, G) < 256) G >>= 1;
     if (G > 1) {
         // Independent groups of neurons, one chain each on its own stream: while one group sits in the latency-bound walk of a
-        // range (which is given few SMs: 32 neurons per CTA) the contractions of the other groups have the rest of the chip.
+        // range (which is given few SMs: 128 neurons per CTA) the contractions of the other groups have the rest of the chip.
         const int64_t gs = ceil_div64(ceil_div64(nj, G), 128) * 128;
-        const int keep_nt = ctx->sweep_nt;
-        if (!keep_nt) ctx->sweep_nt = 32;
         CUDA_TRY(ctx, cudaEventRecord(ctx->ev_copy[0], st));
         int rc = GPFQ_OK;
         for (int g = 0; g < G && rc == GPFQ_OK; ++g) {
@@ -1287,13 +1204,12 @@ static int dense_lowrank_sweep_i8(gpfq_ctx *ctx, const float *X, const float *Xq
                 CUDA_TRY(ctx, cudaStreamWaitEvent(st, ctx->ev_chain[3 * g + 2], 0));
             }
         }
-        ctx->sweep_nt = keep_nt;
         if (rc != GPFQ_OK) return rc;
     } else {
         GPFQ_TRY(chain(0, st, 0, nj));
     }
     // the tensor-core walk leaves level indices only: the layer's fp64 values are made from them here
-    if (use_tc) GPFQ_TRY(sweep_tc_q_from_kq(ctx, sKq, njP, N0, nj, d_levels, K_levels, Qd, ldq, col0));
+    GPFQ_TRY(sweep_tc_q_from_kq(ctx, sKq, njP, N0, nj, d_levels, K_levels, Qd, ldq, col0));
     return GPFQ_OK;
 }
 
@@ -1307,7 +1223,7 @@ int dense_gram_path(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ldx,
     // gpfq_dense_layer_from_gram); X / Xq / m are then unused and the sweep starts from the given (N0, N0) matrices.
     const bool pre = (G2_pre != nullptr);
     const bool same = pre ? (G1_pre == nullptr || G1_pre == G2_pre) : (Xq == X);
-    double *G1 = nullptr, *G2 = nullptr, *Wt = nullptr, *Qt = nullptr, *Dt = nullptr;
+    double *G1 = nullptr, *G2 = nullptr, *Wt = nullptr, *Qt = nullptr;
     double h_step = 0.0;
     const bool i8_sweep = !pre && dense_lowrank_uses_i8(ctx, N0, m, nj, n_alph, &h_step);
     const bool lowrank = !pre && dense_uses_lowrank(ctx, N0, m, nj, n_alph, same, i8_sweep);
@@ -1316,30 +1232,30 @@ int dense_gram_path(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ldx,
     const int64_t slots = 2LL * ctx->sm_count;
     const int NT = ceil_div64(nj, 8) * n_alph <= slots ? 8 : (ceil_div64(nj, 16) * n_alph <= slots ? 16 : 32);
     GPFQ_TRY(gpfq_ws(ctx, WS_WT, (size_t)nj * N0 * sizeof(double), (void **)&Wt));
-    GPFQ_TRY(gpfq_ws(ctx, WS_QT, (size_t)n_alph * nj * N0 * sizeof(double), (void **)&Qt));
+    // Qt (neuron-major decisions): every form but the int8 residual form, whose walk leaves level indices only
+    if (!(lowrank && i8_sweep)) GPFQ_TRY(gpfq_ws(ctx, WS_QT, (size_t)n_alph * nj * N0 * sizeof(double), (void **)&Qt));
     {
         dim3 grid((unsigned)ceil_div64(N0, 32), (unsigned)ceil_div64(nj, 32));
         transpose_w_kernel<<<grid, dim3(32, 8), 0, ctx->stream>>>(W, ldw, N0, j0, nj, Wt);
         KERNEL_CHECK(ctx);
     }
     if (lowrank) {
-        ctx->last_sweep_i8 = 0;
-        if (i8_sweep)
-            GPFQ_TRY(dense_lowrank_sweep_i8(ctx, X, Xq, ldx, N0, m, Wt, Qt, nj, d_alph, d_koff, d_flags, NT, h_step, st, W, ldw, j0, Qd, ldq,
-                                            col0));
-        else
+        if (i8_sweep) {   // writes Qd itself
+            GPFQ_TRY(dense_lowrank_sweep_i8(ctx, X, Xq, ldx, N0, m, Wt, nj, d_alph, h_step, st, W, ldw, j0, Qd, ldq, col0));
+        } else {
             GPFQ_TRY(dense_lowrank_sweep(ctx, X, Xq, ldx, N0, m, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, NT));
-        for (int a = 0; a < n_alph && !(i8_sweep && ctx->last_sweep_tc); ++a) {
-            dim3 grid((unsigned)ceil_div64(N0, 32), (unsigned)ceil_div64(nj, 32));
-            transpose_q_kernel<<<grid, dim3(32, 8), 0, ctx->stream>>>(Qt + (int64_t)a * nj * N0, N0, nj,
-                                                                      Qd + (int64_t)a * N0 * ldq, ldq, col0);
-            KERNEL_CHECK(ctx);
+            for (int a = 0; a < n_alph; ++a) {
+                dim3 grid((unsigned)ceil_div64(N0, 32), (unsigned)ceil_div64(nj, 32));
+                transpose_q_kernel<<<grid, dim3(32, 8), 0, ctx->stream>>>(Qt + (int64_t)a * nj * N0, N0, nj,
+                                                                          Qd + (int64_t)a * N0 * ldq, ldq, col0);
+                KERNEL_CHECK(ctx);
+            }
         }
         CUDA_TRY(ctx, gpfq_record(ctx, 4, ctx->stream));
         if (st) {
             st->method = GPFQ_METHOD_GRAM >> 4;
             st->gram_kernel = 3;
-            if (!ctx->last_sweep_i8) st->flops_algorithmic = 6 * m * N0 * nj * n_alph;
+            if (!i8_sweep) st->flops_algorithmic = 6 * m * N0 * nj * n_alph;
             st->bytes_algorithmic = (same ? 1 : 2) * 4 * N0 * m;
         }
         return GPFQ_OK;
@@ -1352,143 +1268,113 @@ int dense_gram_path(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ldx,
         if (same) G1 = G2;
         else GPFQ_TRY(gpfq_ws(ctx, WS_G1, (size_t)N0 * N0 * sizeof(double), (void **)&G1));
     }
-    if (ctx->sweep_variant == 1)
-        GPFQ_TRY(gpfq_ws(ctx, WS_DT, (size_t)n_alph * nj * SWEEP_B * sizeof(double), (void **)&Dt));
-
     CUDA_TRY(ctx, gpfq_record(ctx, 2, ctx->stream));
     if (!pre) GPFQ_TRY(dense_gram_only(ctx, X, Xq, ldx, N0, m, G1, G2));
     else ctx->last_gram_kernel = 0;
     CUDA_TRY(ctx, gpfq_record(ctx, 3, ctx->stream));
 
-    if (ctx->sweep_variant != 1) {
-        // Two-level blocking: directions in ranges of R; what the earlier ranges contribute to a range is ONE large NT
-        // contraction (all SMs, split over neurons x directions, and over K when that is too few tiles), the
-        // persistent neuron-tile kernel then walks the range.
-        const int64_t tiles_m = ceil_div64(nj, 128) * n_alph;
-        int64_t R = pick_range_length(ctx, nj, n_alph);
-        double *Do = nullptr, *Dpart = nullptr;
-        // One symmetric equispaced alphabet: the tensor-core range walk (sweep_tc.cu).  P = (what the earlier ranges contribute:
-        // the Gram-row contraction below) + (the W terms of the range itself: one batched product on the fp64 pipe up front).
-        double h_tc = 0.0;
-        // (measured, profiles/dense_methods_r2.md: below ~2048 directions the few extra launches of the preparation cost more than the
-        //  walk saves -- MNIST's layers 0.65 -> 0.73 ms -- so those keep sweep_pipe_kernel; sweep_walk = 1 forces the new walk)
-        const bool use_tc = n_alph == 1 && ctx->sweep_walk != 2 && (N0 >= 2048 || ctx->sweep_walk == 1) && ctx->h_alph && ctx->h_koff &&
-                            ctx->h_flags && N0 < ((int64_t)1 << 30) &&
-                            alphabet_symmetric_equispaced(ctx->h_alph + ctx->h_koff[0], ctx->h_koff[1] - ctx->h_koff[0], ctx->h_flags[0], &h_tc);
-        ctx->last_sweep_tc = use_tc ? 1 : 0;
-        TcTables tct;
-        double *Pd = nullptr, *G1m = nullptr;
-        float *Wn = nullptr;
-        int8_t *sKq = nullptr;
-        int64_t N0P = 0, njP = 0;
-        const int K_levels = use_tc ? ctx->h_koff[1] - ctx->h_koff[0] : 0;
-        const double a_top = use_tc ? ctx->h_alph[ctx->h_koff[0] + K_levels - 1] : 0.0;
-        if (use_tc) {
-            R = std::min<int64_t>(R, stc::MAX_R);
-            N0P = ceil_div64(N0, R) * R;
-            njP = ceil_div64(nj, 128) * 128;
-            GPFQ_TRY(gpfq_ws(ctx, WS_TC_P, (size_t)njP * N0P * sizeof(double), (void **)&Pd));
-            GPFQ_TRY(gpfq_ws(ctx, WS_TC_W, (size_t)njP * N0P * sizeof(float), (void **)&Wn));
-            GPFQ_TRY(gpfq_ws(ctx, WS_TC_G1M, (size_t)N0P * R * sizeof(double), (void **)&G1m));
-            GPFQ_TRY(gpfq_ws(ctx, WS_SL_KQ, (size_t)njP * N0P, (void **)&sKq));
-            CUDA_TRY(ctx, cudaMemsetAsync(Pd, 0, (size_t)njP * N0P * sizeof(double), ctx->stream));
-            GPFQ_TRY(sweep_tc_weights(ctx, W, ldw, j0, N0, N0P, nj, Wn));
-            GPFQ_TRY(sweep_tc_prepare(ctx, G1, G2, N0, false, N0, N0P, R, h_tc, &tct));
-            GPFQ_TRY(sweep_tc_bind(ctx, &tct, Pd, Wn, njP, N0P));
-            GPFQ_TRY(sweep_tc_mask_g1_lower(ctx, G1, N0, N0, N0P, R, G1m));
-            const int64_t nfull = N0 / R;
-            GemmArgs g = {};   // P[:, range] = Wt[:, range] strict_lower(G1[range, range])^T, every full range a batch
-            g.seg[0] = {Wt, G1m, N0, R, R, 1.0};
-            g.nseg = 1;
+    // Two-level blocking: directions in ranges of R; what the earlier ranges contribute to a range is ONE large NT
+    // contraction (all SMs, split over neurons x directions, and over K when that is too few tiles), the
+    // persistent neuron-tile kernel then walks the range.
+    const int64_t tiles_m = ceil_div64(nj, 128) * n_alph;
+    int64_t R = pick_range_length(ctx, nj, n_alph);
+    double *Do = nullptr, *Dpart = nullptr;
+    // One symmetric equispaced alphabet: the tensor-core range walk (sweep_tc.cu).  P = (what the earlier ranges contribute:
+    // the Gram-row contraction below) + (the W terms of the range itself: one batched product on the fp64 pipe up front).
+    double h_tc = 0.0;
+    // (measured, profiles/dense_methods_r2.md: below ~2048 directions the few extra launches of the preparation cost more than the
+    //  walk saves -- MNIST's layers 0.65 -> 0.73 ms -- so those keep sweep_pipe_kernel; sweep_walk = 1 forces the new walk)
+    const bool use_tc = n_alph == 1 && ctx->sweep_walk != 2 && (N0 >= 2048 || ctx->sweep_walk == 1) && ctx->h_alph && ctx->h_koff &&
+                        ctx->h_flags && N0 < ((int64_t)1 << 30) &&
+                        alphabet_symmetric_equispaced(ctx->h_alph + ctx->h_koff[0], ctx->h_koff[1] - ctx->h_koff[0], ctx->h_flags[0], &h_tc);
+    TcTables tct;
+    double *Pd = nullptr, *G1m = nullptr;
+    float *Wn = nullptr;
+    int8_t *sKq = nullptr;
+    int64_t N0P = 0, njP = 0;
+    const int K_levels = use_tc ? ctx->h_koff[1] - ctx->h_koff[0] : 0;
+    const double a_top = use_tc ? ctx->h_alph[ctx->h_koff[0] + K_levels - 1] : 0.0;
+    if (use_tc) {
+        R = std::min<int64_t>(R, stc::MAX_R);
+        N0P = ceil_div64(N0, R) * R;
+        njP = ceil_div64(nj, 128) * 128;
+        GPFQ_TRY(gpfq_ws(ctx, WS_TC_P, (size_t)njP * N0P * sizeof(double), (void **)&Pd));
+        GPFQ_TRY(gpfq_ws(ctx, WS_TC_W, (size_t)njP * N0P * sizeof(float), (void **)&Wn));
+        GPFQ_TRY(gpfq_ws(ctx, WS_TC_G1M, (size_t)N0P * R * sizeof(double), (void **)&G1m));
+        GPFQ_TRY(gpfq_ws(ctx, WS_SL_KQ, (size_t)njP * N0P, (void **)&sKq));
+        CUDA_TRY(ctx, cudaMemsetAsync(Pd, 0, (size_t)njP * N0P * sizeof(double), ctx->stream));
+        GPFQ_TRY(sweep_tc_weights(ctx, W, ldw, j0, N0, N0P, nj, Wn));
+        GPFQ_TRY(sweep_tc_prepare(ctx, G1, G2, N0, false, N0, N0P, R, h_tc, &tct));
+        GPFQ_TRY(sweep_tc_bind(ctx, &tct, Pd, Wn, njP, N0P));
+        GPFQ_TRY(sweep_tc_mask_g1_lower(ctx, G1, N0, N0, N0P, R, G1m));
+        const int64_t nfull = N0 / R;
+        GemmArgs g = {};   // P[:, range] = Wt[:, range] strict_lower(G1[range, range])^T, every full range a batch
+        g.seg[0] = {Wt, G1m, N0, R, R, 1.0};
+        g.nseg = 1;
+        g.M = nj;
+        g.N = R;
+        g.C = Pd;
+        g.ldc = N0P;
+        g.nsplit = 1;
+        g.batch_strideA0 = R;
+        g.batch_strideB = R * R;
+        g.batch_strideC = R;
+        for (int64_t b0 = 0; b0 < nfull; b0 += 65535) {
+            GemmArgs gb = g;
+            gb.seg[0].A = Wt + b0 * R;
+            gb.seg[0].B = G1m + b0 * R * R;
+            gb.C = Pd + b0 * R;
+            GPFQ_TRY((launch_gemm_nt<double, 128, 64, 16>(ctx, gb, (int)std::min<int64_t>(65535, nfull - b0))));
+        }
+        if (nfull * R < N0) {   // the ragged last range
+            const int64_t tb = nfull * R;
+            GemmArgs gl = g;
+            gl.seg[0] = {Wt + tb, G1m + tb * R, N0, R, N0 - tb, 1.0};
+            gl.N = N0 - tb;
+            gl.C = Pd + tb;
+            GPFQ_TRY((launch_gemm_nt<double, 128, 64, 16>(ctx, gl, 1)));
+        }
+    }
+    if (N0 > R) GPFQ_TRY(gpfq_ws(ctx, WS_DT, (size_t)n_alph * nj * R * sizeof(double), (void **)&Do));
+    for (int64_t tb = 0; tb < N0; tb += R) {
+        const int64_t te = tb + R < N0 ? tb + R : N0;
+        if (tb > 0) {
+            GemmArgs g = {};
+            g.seg[0] = {Wt, G1 + tb * N0, N0, N0, tb, 1.0};
+            g.seg[1] = {Qt, G2 + tb * N0, N0, N0, tb, -1.0};
+            g.nseg = 2;
             g.M = nj;
-            g.N = R;
-            g.C = Pd;
-            g.ldc = N0P;
+            g.N = te - tb;
+            g.C = Do;
+            g.ldc = R;
             g.nsplit = 1;
-            g.batch_strideA0 = R;
-            g.batch_strideB = R * R;
-            g.batch_strideC = R;
-            for (int64_t b0 = 0; b0 < nfull; b0 += 65535) {
-                GemmArgs gb = g;
-                gb.seg[0].A = Wt + b0 * R;
-                gb.seg[0].B = G1m + b0 * R * R;
-                gb.C = Pd + b0 * R;
-                GPFQ_TRY((launch_gemm_nt<double, 128, 64, 16>(ctx, gb, (int)std::min<int64_t>(65535, nfull - b0))));
-            }
-            if (nfull * R < N0) {   // the ragged last range
-                const int64_t tb = nfull * R;
-                GemmArgs gl = g;
-                gl.seg[0] = {Wt + tb, G1m + tb * R, N0, R, N0 - tb, 1.0};
-                gl.N = N0 - tb;
-                gl.C = Pd + tb;
-                GPFQ_TRY((launch_gemm_nt<double, 128, 64, 16>(ctx, gl, 1)));
-            }
-        }
-        if (N0 > R) GPFQ_TRY(gpfq_ws(ctx, WS_DT, (size_t)n_alph * nj * R * sizeof(double), (void **)&Do));
-        for (int64_t tb = 0; tb < N0; tb += R) {
-            const int64_t te = tb + R < N0 ? tb + R : N0;
-            if (tb > 0) {
-                GemmArgs g = {};
-                g.seg[0] = {Wt, G1 + tb * N0, N0, N0, tb, 1.0};
-                g.seg[1] = {Qt, G2 + tb * N0, N0, N0, tb, -1.0};
-                g.nseg = 2;
-                g.M = nj;
-                g.N = te - tb;
-                g.C = Do;
-                g.ldc = R;
-                g.nsplit = 1;
-                g.batch_strideA1 = nj * N0;
-                g.batch_strideC = nj * R;
-                // few neurons: split K (the earlier directions) so that every SM gets a CTA; fixed-order reduction
-                const int64_t tiles = tiles_m * ceil_div64(te - tb, 64);
-                int64_t ns = tiles >= ctx->sm_count ? 1 : ctx->sm_count / tiles;
-                ns = std::min<int64_t>(std::min<int64_t>(ns, 16), std::max<int64_t>(1, tb / 128));
-                if (ns > 1) {
-                    const size_t one = (size_t)n_alph * nj * R;
-                    GPFQ_TRY(gpfq_ws(ctx, WS_PART, (size_t)ns * one * sizeof(double), (void **)&Dpart));
-                    g.C = Dpart;
-                    g.nsplit = (int)ns;
-                    g.split_stride = (int64_t)one;
-                    GPFQ_TRY((launch_gemm_nt<double, 128, 64, 16>(ctx, g, n_alph)));
-                    int blocks = (int)std::min<int64_t>(ceil_div64((int64_t)one, 256), 4096);
-                    reduce_splits_kernel<<<blocks, 256, 0, ctx->stream>>>(Dpart, (int)ns, (int64_t)one, Do, (int64_t)one);
-                    KERNEL_CHECK(ctx);
-                } else {
-                    GPFQ_TRY((launch_gemm_nt<double, 128, 64, 16>(ctx, g, n_alph)));
-                }
-            }
-            if (use_tc) {
-                if (tb > 0) GPFQ_TRY(sweep_tc_add_outer(ctx, Pd + tb, N0P, Do, R, nj, te - tb));
-                GPFQ_TRY(sweep_tc_range(ctx, tct, tb, te, 0, nj, sKq, njP, 0, a_top, d_alph, K_levels));
-                GPFQ_TRY(sweep_tc_qt_from_kq(ctx, sKq, njP, tb, te, nj, d_alph, K_levels, Qt, N0));
+            g.batch_strideA1 = nj * N0;
+            g.batch_strideC = nj * R;
+            // few neurons: split K (the earlier directions) so that every SM gets a CTA; fixed-order reduction
+            const int64_t tiles = tiles_m * ceil_div64(te - tb, 64);
+            int64_t ns = tiles >= ctx->sm_count ? 1 : ctx->sm_count / tiles;
+            ns = std::min<int64_t>(std::min<int64_t>(ns, 16), std::max<int64_t>(1, tb / 128));
+            if (ns > 1) {
+                const size_t one = (size_t)n_alph * nj * R;
+                GPFQ_TRY(gpfq_ws(ctx, WS_PART, (size_t)ns * one * sizeof(double), (void **)&Dpart));
+                g.C = Dpart;
+                g.nsplit = (int)ns;
+                g.split_stride = (int64_t)one;
+                GPFQ_TRY((launch_gemm_nt<double, 128, 64, 16>(ctx, g, n_alph)));
+                int blocks = (int)std::min<int64_t>(ceil_div64((int64_t)one, 256), 4096);
+                reduce_splits_kernel<<<blocks, 256, 0, ctx->stream>>>(Dpart, (int)ns, (int64_t)one, Do, (int64_t)one);
+                KERNEL_CHECK(ctx);
             } else {
-                GPFQ_TRY(dispatch_sweep_tile(ctx, NT, G1, G2, N0, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te,
-                                             tb > 0 ? Do : nullptr, R));
+                GPFQ_TRY((launch_gemm_nt<double, 128, 64, 16>(ctx, g, n_alph)));
             }
         }
-    } else {
-        // multi-launch reference: one NT contraction + one in-block kernel per 32 directions
-        const int nblk = (int)ceil_div64(N0, SWEEP_B);
-        for (int b = 0; b < nblk; ++b) {
-            const int64_t p = (int64_t)b * SWEEP_B;
-            const int64_t nb = (N0 - p) < SWEEP_B ? (N0 - p) : SWEEP_B;
-            if (b > 0) {
-                GemmArgs g = {};
-                g.seg[0] = {Wt, G1 + p * N0, N0, N0, p, 1.0};
-                g.seg[1] = {Qt, G2 + p * N0, N0, N0, p, -1.0};
-                g.nseg = 2;
-                g.M = nj;
-                g.N = nb;
-                g.C = Dt;
-                g.ldc = SWEEP_B;
-                g.nsplit = 1;
-                g.batch_strideA1 = nj * N0;
-                g.batch_strideC = nj * SWEEP_B;
-                GPFQ_TRY((launch_gemm_nt<double, 128, 32, 16>(ctx, g, n_alph)));
-            }
-            dim3 grid((unsigned)ceil_div64(nj, 8), (unsigned)n_alph);
-            sweep_inblock_kernel<<<grid, 256, 0, ctx->stream>>>(G1, G2, N0, N0, b, Wt, Dt, Qt, nj, d_alph, d_koff, d_flags);
-            KERNEL_CHECK(ctx);
+        if (use_tc) {
+            if (tb > 0) GPFQ_TRY(sweep_tc_add_outer(ctx, Pd + tb, N0P, Do, R, nj, te - tb));
+            GPFQ_TRY(sweep_tc_range(ctx, tct, tb, te, 0, nj, sKq, njP, 0, a_top, d_alph, K_levels));
+            GPFQ_TRY(sweep_tc_qt_from_kq(ctx, sKq, njP, tb, te, nj, d_alph, K_levels, Qt, N0));
+        } else {
+            GPFQ_TRY(dispatch_sweep_tile(ctx, NT, G1, G2, N0, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te,
+                                         tb > 0 ? Do : nullptr, R));
         }
     }
     for (int a = 0; a < n_alph; ++a) {
@@ -1501,7 +1387,7 @@ int dense_gram_path(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ldx,
     if (st) {
         st->method = GPFQ_METHOD_GRAM >> 4;
         st->gram_kernel = ctx->last_gram_kernel;
-        if (ctx->sweep_variant != 1 && ctx->last_sweep_tc) st->reserved |= 2;   // ranges walked by sweep_tc_kernel
+        if (use_tc) st->reserved |= 2;   // ranges walked by sweep_tc_kernel
         st->flops_algorithmic = pre ? 2 * N0 * N0 * nj * n_alph : (same ? 1 : 2) * m * N0 * (N0 + 1);  // lower triangles
         st->bytes_algorithmic = (pre ? 0 : (same ? 1 : 2) * 4 * N0 * m) + (same ? 1 : 2) * 8 * N0 * N0;
     }

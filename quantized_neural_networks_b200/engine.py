@@ -73,7 +73,8 @@ class GpfqEngine:
         self._check(self._lib.gpfq_trim(self._ctx))
 
     def set_option(self, key: str, value: int):
-        """A/B switches of include/gpfq.h (`gram_kernel`, `i8_pairs_d`, `conv_kernel`, `sweep_kernel`)."""
+        """A/B switches of include/gpfq.h (`gram_kernel`, `i8_pairs_d`, `conv_kernel`, `corr_*`, `sweep_outer`, `sweep_walk`,
+        `sweep_i8`)."""
         self._check(self._lib.gpfq_set_option(self._ctx, key.encode(), int(value)))
 
     def _bind_stream(self, dev):

@@ -355,12 +355,10 @@ def test_streaming_neuron_tiles(engine, J_neurons):
         assert O.agreement(engine.dense_layer(X, Xq, W, A, method="stream_fast"), Qref) >= AGREE, m
 
 
-def test_conv_gram_kernel_variants_agree():
+def test_conv_gram_kernel_variants_agree(engine):
     """The three 3x3 patch-Gram kernels (TMA-staged, direct LDG, generic) produce the same quantized kernel, on
     ragged column counts (tail stages, several chunks) and on the unaligned fallback (n % 4 != 0)."""
-    import os
     import torch
-    from quantized_neural_networks_b200 import GpfqEngine
     rng = np.random.default_rng(77)
     C, F = 3, 5
     W = (rng.uniform(-1, 1, (3, 3, C, F)) * 0.3).astype(np.float32)
@@ -374,18 +372,14 @@ def test_conv_gram_kernel_variants_agree():
             G2 = Xqp[c].astype(np.float64) @ Xqp[c].astype(np.float64).T
             Qref[:, :, c, :] = O.gram_quantize_layer(W[:, :, c, :].reshape(9, F), None, None, A, grams=(G1, G2)).reshape(3, 3, F)
         outs = {}
-        for variant in ("tma", "ldg", "generic"):
-            os.environ["GPFQ_CONV_KERNEL"] = variant
-            try:
-                with GpfqEngine(0) as eng:
-                    outs[variant] = eng.conv_channels(list(Xp), list(Xqp), W, A)
-                    same = eng.conv_channels(list(Xqp), None, W, A)
-                    dev = eng.conv_channels([torch.from_numpy(x).cuda() for x in Xp], [torch.from_numpy(x).cuda() for x in Xqp],
-                                            torch.from_numpy(W).cuda(), A).cpu().numpy()
-                    assert np.array_equal(dev, outs[variant]), (variant, n)
-                    outs[variant + "_same"] = same
-            finally:
-                os.environ.pop("GPFQ_CONV_KERNEL", None)
+        for variant, kernel in (("tma", 0), ("ldg", 1), ("generic", 2)):
+            with _conv_options(engine, conv_kernel=kernel):
+                outs[variant] = engine.conv_channels(list(Xp), list(Xqp), W, A)
+                same = engine.conv_channels(list(Xqp), None, W, A)
+                dev = engine.conv_channels([torch.from_numpy(x).cuda() for x in Xp], [torch.from_numpy(x).cuda() for x in Xqp],
+                                           torch.from_numpy(W).cuda(), A).cpu().numpy()
+                assert np.array_equal(dev, outs[variant]), (variant, n)
+                outs[variant + "_same"] = same
         assert O.agreement(outs["tma"], Qref) == 1.0, n
         assert np.array_equal(outs["tma"], outs["ldg"]) and np.array_equal(outs["tma"], outs["generic"]), n
         assert np.array_equal(outs["tma_same"], outs["ldg_same"]) and np.array_equal(outs["tma_same"], outs["generic_same"]), n
@@ -394,13 +388,11 @@ def test_conv_gram_kernel_variants_agree():
 @pytest.mark.parametrize("n_img,H,Wd,C,F,pad", [(5, 7, 12, 5, 4, "SAME"), (9, 10, 8, 8, 3, "VALID"), (3, 32, 32, 16, 6, "SAME"),
                                                 (70, 6, 6, 3, 2, "VALID"), (2, 40, 44, 12, 2, "SAME"),
                                                 (4, 14, 14, 8, 3, "SAME"), (3, 9, 7, 4, 2, "SAME"), (6, 5, 5, 9, 2, "VALID")])
-def test_conv_nhwc_fused_matches_patch_path(n_img, H, Wd, C, F, pad):
+def test_conv_nhwc_fused_matches_patch_path(engine, n_img, H, Wd, C, F, pad):
     """The fused NHWC kernel (planes in shared memory, no patch matrices) against the im2col + patch-Gram path and the
     oracle: ragged channel groups (scalar loader), full groups (LDG.128 loader), SAME / VALID, several bands, output widths that
     are not a multiple of four (VGG block 5 is 14 x 14)."""
-    import os
     import torch
-    from quantized_neural_networks_b200 import GpfqEngine
     rng = np.random.default_rng(n_img * 31 + C)
     act = np.maximum(rng.standard_normal((n_img, H, Wd, C)), 0).astype(np.float32)
     actq = np.maximum(act + 0.05 * rng.standard_normal(act.shape), 0).astype(np.float32)
@@ -409,19 +401,15 @@ def test_conv_nhwc_fused_matches_patch_path(n_img, H, Wd, C, F, pad):
     patches = lambda ch: (O.channel_patches(act, ch, (3, 3), (1, 1), pad), O.channel_patches(actq, ch, (3, 3), (1, 1), pad))
     Qref = c_oracle.quantize_conv_layer(W, patches, A)
     outs = {}
-    for variant in ("tma", "ldg"):
-        os.environ["GPFQ_CONV_KERNEL"] = variant
-        try:
-            with GpfqEngine(0) as eng:
-                outs[variant] = eng.conv_layer_nhwc(act, actq, W, A, padding=pad)
-                outs[variant + "_same"] = eng.conv_layer_nhwc(actq, None, W, A, padding=pad)
-                dev = eng.conv_layer_nhwc(torch.from_numpy(act).cuda(), torch.from_numpy(actq).cuda(), torch.from_numpy(W).cuda(),
-                                          A, padding=pad).cpu().numpy()
-                assert np.array_equal(dev, outs[variant])
-                part = eng.conv_layer_nhwc(act, actq, W, A, padding=pad, c0=1, n_channels=C - 2)
-                assert np.array_equal(part[:, :, 1:C - 1], outs[variant][:, :, 1:C - 1]) and np.all(part[:, :, 0] == 0)
-        finally:
-            os.environ.pop("GPFQ_CONV_KERNEL", None)
+    for variant, kernel in (("tma", 0), ("ldg", 1)):
+        with _conv_options(engine, conv_kernel=kernel):
+            outs[variant] = engine.conv_layer_nhwc(act, actq, W, A, padding=pad)
+            outs[variant + "_same"] = engine.conv_layer_nhwc(actq, None, W, A, padding=pad)
+            dev = engine.conv_layer_nhwc(torch.from_numpy(act).cuda(), torch.from_numpy(actq).cuda(), torch.from_numpy(W).cuda(),
+                                         A, padding=pad).cpu().numpy()
+            assert np.array_equal(dev, outs[variant])
+            part = engine.conv_layer_nhwc(act, actq, W, A, padding=pad, c0=1, n_channels=C - 2)
+            assert np.array_equal(part[:, :, 1:C - 1], outs[variant][:, :, 1:C - 1]) and np.all(part[:, :, 0] == 0)
     assert O.agreement(outs["tma"], Qref) == 1.0
     assert np.array_equal(outs["tma"], outs["ldg"]) and np.array_equal(outs["tma_same"], outs["ldg_same"])
 
@@ -620,7 +608,8 @@ def test_dense_gram_kernels_match_the_oracle(engine, variant):
                                            (600, 2200, 64, False), (520, 2048, 48, True)])
 def test_sweep_lowrank_outer_level_matches_the_oracle(engine, N0, N1, m, first):
     """`sweep_outer = 2`: the earlier ranges enter through the residuals U (nj x m) instead of Gram rows, and only
-    block-diagonal Gram tiles exist.  Same decisions as the literal oracle walk and as the Gram-row form."""
+    block-diagonal Gram tiles exist.  Same decisions as the literal oracle walk and as the Gram-row form; the int8 form
+    (tensor-core walk) and the fp64 form (sweep_pipe / sweep_tile) agree bit for bit on every alphabet."""
     rng = np.random.default_rng(N0 + N1 + m)
     if first:
         X = (rng.uniform(0, 1, (N0, m)) * (rng.uniform(0, 1, (N0, m)) < 0.5)).astype(np.float32)
@@ -634,27 +623,22 @@ def test_sweep_lowrank_outer_level_matches_the_oracle(engine, N0, N1, m, first):
     engine.set_option("sweep_outer", 2)
     try:
         Q = engine.dense_layer(X, None if first else Xq, W, A, method="gram")       # contractions on tcgen05 (int8 slices)
-        assert engine.last_stats["gram_kernel"] == 3 and engine.last_stats["reserved"] & 1
-        engine.set_option("sweep_i8", 2)                                            # the same on the fp64 DMMA pipe
-        try:
-            Qf = engine.dense_layer(X, None if first else Xq, W, A, method="gram")
-            assert engine.last_stats["gram_kernel"] == 3 and not engine.last_stats["reserved"] & 1
-        finally:
-            engine.set_option("sweep_i8", 0)
-        assert np.array_equal(Q, Qf)
+        assert engine.last_stats["gram_kernel"] == 3 and (engine.last_stats["reserved"] & 3) == 3   # ... and sweep_tc_kernel
         A2 = O.layer_alphabet(W, 4, O.unit_alphabet(3))
         Qm = engine.dense_layer(X, None if first else Xq, W, [A, A2], method="gram", j0=1, j1=N1 - 1)
         # alphabets with more than three levels through the tensor-core walk (even K: no zero level; the 16 levels of 4 bits)
         Q16 = {bits: engine.dense_layer(X, None if first else Xq, W, O.layer_alphabet(W, 3, O.unit_alphabet(bits)), method="gram")
                for bits in (2, 4)}
-        engine.set_option("sweep_walk", 2)                                          # the same walks by sweep_pipe / sweep_tile
-        try:
-            assert np.array_equal(engine.dense_layer(X, None if first else Xq, W, A, method="gram"), Q)
+        engine.set_option("sweep_i8", 2)                                            # the same on the fp64 DMMA pipe, the ranges
+        try:                                                                        # walked by sweep_pipe / sweep_tile
+            Qf = engine.dense_layer(X, None if first else Xq, W, A, method="gram")
+            assert engine.last_stats["gram_kernel"] == 3 and not engine.last_stats["reserved"] & 3
             for bits, Qb in Q16.items():
                 Ab = O.layer_alphabet(W, 3, O.unit_alphabet(bits))
                 assert np.array_equal(engine.dense_layer(X, None if first else Xq, W, Ab, method="gram"), Qb)
         finally:
-            engine.set_option("sweep_walk", 0)
+            engine.set_option("sweep_i8", 0)
+        assert np.array_equal(Q, Qf)
     finally:
         engine.set_option("sweep_outer", 0)
     for bits, Qb in Q16.items():

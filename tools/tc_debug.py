@@ -1,4 +1,4 @@
-"""Debug: tensor-core walk vs oracle / old walk on one lowrank test case."""
+"""Debug: tensor-core walk (int8 residual form) vs oracle / sweep_pipe walk (fp64 residual form) on the lowrank test cases."""
 import os, sys
 import numpy as np
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -22,9 +22,9 @@ for (N0, N1, m, first) in ((520, 2048, 48, True), (600, 2200, 64, False)):
         Qref = c_oracle.quantize_layer(W, X, Xq, A)
         eng.set_option("sweep_outer", 2)
         Q = eng.dense_layer(X, None if first else Xq, W, A, method="gram")
-        eng.set_option("sweep_walk", 2)
+        eng.set_option("sweep_i8", 2)
         Qo = eng.dense_layer(X, None if first else Xq, W, A, method="gram")
-        eng.set_option("sweep_walk", 0)
+        eng.set_option("sweep_i8", 0)
         eng.set_option("sweep_outer", 0)
         bad = np.argwhere(Q != Qref)
         print((N0, N1, m, first), "bits", bits, "K", len(A), "agree tc/oracle", O.agreement(Q, Qref), "old/oracle", O.agreement(Qo, Qref),
