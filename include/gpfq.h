@@ -185,6 +185,8 @@ int gpfq_conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float *actq, int
  *   gpfq_conv_layer_from_gram  the walks of every filter of channels c0 .. c0+n_ch-1 from such matrices (device pointer,
  *                              GPFQ_X_DEVICE; channel i of the range at gram + i * 2 kk^2).  W / Q_out as in
  *                              gpfq_conv_channels (GPFQ_W_DEVICE / GPFQ_Q_DEVICE say where they live).
+ * Both serve only the kernel sizes with their own Gram and walk kernels, kh * kw in {1, 2, 3, 4, 6, 9}; any other size returns
+ * GPFQ_ERR_UNSUPPORTED (gpfq_conv_layer_nhwc still takes it, one Dense problem per channel).
  */
 int gpfq_conv_gram_nhwc(gpfq_ctx *ctx, const float *act, const float *actq, int64_t n_img, int64_t H, int64_t Wd,
                         int64_t C, int32_t kh, int32_t kw, int32_t stride_h, int32_t stride_w, int32_t rate_h,

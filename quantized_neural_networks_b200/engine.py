@@ -17,6 +17,10 @@ except Exception:  # pragma: no cover
 _METHODS = {"auto": _lib.METHOD_AUTO, "stream": _lib.METHOD_STREAM, "gram": _lib.METHOD_GRAM,
             "stream_fast": _lib.METHOD_STREAM_FAST}
 
+# Conv kernel sizes kh * kw with their own Gram and walk kernels: the set of `conv_supported_kk` in csrc/conv.cu.  Only these
+# have the Gram-only entry points (`conv_gram_nhwc`, `conv_layer_from_gram`); other sizes run one Dense problem per channel.
+CONV_SUPPORTED_KK = frozenset({1, 2, 3, 4, 6, 9})
+
 
 def _is_torch(x):
     return torch is not None and isinstance(x, torch.Tensor)
@@ -359,7 +363,8 @@ class GpfqEngine:
                        sync=True):
         """Gram stage of a conv layer alone: per-channel [G1 | G2] of channels c0..c0+n_channels-1 over the given images,
         as a float64 CUDA tensor (n_channels, 2, kh*kw, kh*kw) (lower triangles + diagonals valid).  act / actq: NHWC
-        NumPy arrays or CUDA tensors.  The per-rank part of an image-split multi-GPU job (`conv_layer_from_gram`)."""
+        NumPy arrays or CUDA tensors.  The per-rank part of an image-split multi-GPU job (`conv_layer_from_gram`).  Raises
+        GpfqError for kh * kw outside CONV_SUPPORTED_KK."""
         act = self._f32(act, "act")
         same = actq is None or actq is act
         actq = act if same else self._f32(actq, "actq")

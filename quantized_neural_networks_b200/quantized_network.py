@@ -23,7 +23,7 @@ import numpy as np
 from numpy import abs, array, linspace, log2, median, zeros
 
 from . import hostnet
-from .engine import get_engine
+from .engine import CONV_SUPPORTED_KK, get_engine
 from .replicate import image_split_conv_gram, prefer_sample_split, replicate_leading_axis, sample_split_gram, shard_range
 
 try:  # real Keras if present, the TF-free shim otherwise (same call surface, SURVEY.md App. D)
@@ -403,9 +403,10 @@ class QuantizedCNN(QuantizedNeuralNetwork):
         tic = time()
         if self.conv_path == "nhwc":
             try:
-                if self._nccl_job() and self.gram_split != "replicate":
+                if self._nccl_job() and self.gram_split != "replicate" and W.shape[0] * W.shape[1] in CONV_SUPPORTED_KK:
                     # image split: every rank contracts n_img / world images of ALL channels, one tiny all-reduce sums the
-                    # per-channel Grams, then every rank walks every channel (cheap: kk steps per filter) -- no Q gather
+                    # per-channel Grams, then every rank walks every channel (cheap: kk steps per filter) -- no Q gather.
+                    # Other kernel sizes (5 x 5, 7 x 7, ...) have no Gram-only path and take the channel shards below.
                     gram = image_split_conv_gram(self.engine, data.wX, None if data.same else data.qX, W.shape[:2],
                                                  layer.strides, layer.padding.upper(), rate, *self.shard)
                     self.layer_stats[layer_idx] = dict(self.engine.last_stats)

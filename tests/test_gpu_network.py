@@ -112,6 +112,28 @@ def test_cnn_with_5x5_and_7x7_kernels_through_the_default_path():
     _compare(qg, qo, x[:32], {"Dense", "Conv2D"})
 
 
+@pytest.mark.parametrize("conv_path", ["nhwc", "patches"])
+def test_cnn_with_non_square_strided_dilated_and_depthwise_layers(conv_path):
+    """Kernels 1x3, 3x1, 2x3 and 1x2 (kk = 3, 6, 2: the patch-path kernels of those sizes), strides (2, 1) and (1, 2), dilation on
+    one axis and on both, a VALID layer, and a DepthwiseConv2D with depth_multiplier 2 (its (kh, kw, C, 2) kernel is walked like a
+    Conv2D kernel with two filters per channel), through both conv paths."""
+    rng = np.random.default_rng(15)
+    L = hostnet
+    net = L.Sequential([L.Conv2D(6, (1, 3), padding="same", activation="relu"),
+                        L.Conv2D(6, (3, 1), strides=(2, 1), padding="same", activation="relu"),
+                        L.DepthwiseConv2D(3, padding="same", depth_multiplier=2, dilation_rate=2, activation="relu"),
+                        L.Conv2D(8, (2, 3), strides=(1, 2), padding="valid", activation="relu"),
+                        L.Conv2D(4, (1, 2), dilation_rate=(1, 2), padding="same", activation="relu"),
+                        L.Flatten(), L.Dense(10, activation="softmax")], input_shape=(16, 16, 3), seed=4)
+    x = rng.random((64, 16, 16, 3)).astype(np.float32)
+    seq = hostnet.ArraySequence(x, rng.integers(0, 10, 64), 16)
+    qg = QuantizedCNN(net, 16, seq, bits=3, alphabet_scalar=3, conv_path=conv_path)
+    qg.quantize_network()
+    qo = _with_oracle(QuantizedCNN, net, 16, seq, bits=3, alphabet_scalar=3)
+    qo.quantize_network()
+    _compare(qg, qo, x[:32], {"Dense", "Conv2D", "DepthwiseConv2D"})
+
+
 def test_vgg_like_full_network_matches_the_oracle_walk():
     """BASELINE config 3 shape family (Keras VGG16, quantize_pretrained_imagenet.py:43-50): InputLayer, 13 conv 3x3
     'same', 5 pools, fc1 / fc2 / predictions -- a thin copy (channels / 16, 32 x 32 inputs), ternary alphabet."""

@@ -16,18 +16,46 @@ from quantized_neural_networks_b200.quantized_network import (  # noqa: E402
     LayerData, QuantizedCNN, QuantizedNeuralNetwork, shard_range)
 
 
+def _unfold_patches(act, c, kernel_size, strides, padding, rate):
+    """Patch matrix of channel c by torch.nn.functional.unfold on an explicitly padded input, TensorFlow's SAME split
+    (pad before = total // 2): a restatement that shares no loop with the oracle or hostnet."""
+    import torch
+    (kh, kw), (sh, sw), (rh, rw) = kernel_size, strides, rate
+    n, H, Wd = act.shape[:3]
+    pads = []
+    for size, k, s, r in ((Wd, kw, sw, rw), (H, kh, sh, rh)):   # F.pad order: (left, right, top, bottom)
+        total = max((-(-size // s) - 1) * s + (k - 1) * r + 1 - size, 0) if padding == "SAME" else 0
+        pads += [total // 2, total - total // 2]
+    x = torch.nn.functional.pad(torch.from_numpy(np.ascontiguousarray(act[..., c]))[:, None], pads)
+    p = torch.nn.functional.unfold(x, (kh, kw), dilation=(rh, rw), stride=(sh, sw))   # (n, kh*kw, Ho*Wo)
+    return p.permute(1, 0, 2).reshape(kh * kw, -1).numpy()
+
+
 @pytest.mark.parametrize("padding,strides,rate", [("SAME", (1, 1), (1, 1)), ("VALID", (1, 1), (1, 1)),
                                                   ("SAME", (2, 2), (1, 1)), ("VALID", (1, 2), (1, 1)),
-                                                  ("SAME", (1, 1), (2, 2))])
+                                                  ("SAME", (1, 1), (2, 2)), ("SAME", (2, 1), (1, 1)),
+                                                  ("VALID", (2, 1), (2, 1)), ("SAME", (1, 3), (1, 2)),
+                                                  ("VALID", (1, 3), (2, 3)), ("SAME", (3, 2), (2, 3)),
+                                                  ("VALID", (1, 1), (1, 2)), ("SAME", (4, 4), (1, 1))])
 def test_extract_patches_matches_oracle_im2col(padding, strides, rate):
+    """Three restatements of the patch geometry agree exactly: hostnet.extract_patches, the oracle's loop and torch's unfold,
+    for non-square kernels (taps r * kw + col), asymmetric strides and rates, strides beyond the kernel extent, SAME padding
+    with a nonzero top / left pad and VALID outputs one pixel high or wide.  The GPU conv tests compare with the oracle."""
     rng = np.random.default_rng(3)
-    act = rng.standard_normal((3, 7, 6, 2)).astype(np.float32)
-    for c in range(2):
-        ch = act[..., c:c + 1]
-        p = hostnet.extract_patches(ch, [1, 3, 3, 1], [1, *strides, 1], [1, *rate, 1], padding)
-        mine = p.reshape(-1, p.shape[-1]).T
-        ref = O.channel_patches(act, c, (3, 3), strides, padding, rate)
-        assert np.array_equal(mine, ref)
+    for shape in ((3, 7, 6, 2), (2, 9, 13, 2)):
+        act = rng.standard_normal(shape).astype(np.float32)
+        H, Wd = shape[1:3]
+        for ks in ((3, 3), (1, 2), (2, 1), (1, 3), (3, 1), (2, 3), (3, 2), (1, 4), (1, 6), (1, 9), (9, 1), (1, 5), (2, 5),
+                   (5, 5)):
+            if padding == "VALID" and ((ks[0] - 1) * rate[0] + 1 > H or (ks[1] - 1) * rate[1] + 1 > Wd):
+                continue
+            for c in range(2):
+                ch = act[..., c:c + 1]
+                p = hostnet.extract_patches(ch, [1, *ks, 1], [1, *strides, 1], [1, *rate, 1], padding)
+                mine = p.reshape(-1, p.shape[-1]).T
+                ref = O.channel_patches(act, c, ks, strides, padding, rate)
+                assert np.array_equal(mine, ref), (shape, ks)
+                assert np.array_equal(_unfold_patches(act, c, ks, strides, padding, rate), ref), (shape, ks)
 
 
 @pytest.mark.parametrize("n,world", [(10, 1), (10, 3), (128, 8), (3, 8), (37, 4)])
