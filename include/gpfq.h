@@ -108,6 +108,10 @@ int gpfq_set_option(gpfq_ctx *ctx, const char *key, int64_t value);
 int gpfq_query_stats(gpfq_ctx *ctx, int32_t calls_back, gpfq_stats *out);
 /* Release cached device/pinned workspaces (they are otherwise kept between calls). */
 int gpfq_trim(gpfq_ctx *ctx);
+/* Bytes of partial Gram workspace the last conv call (gpfq_conv_channels, gpfq_conv_layer_nhwc, gpfq_conv_gram_nhwc) asked
+ * for: 0 for kernels above 128 taps.  For the kernel sizes without a specialised kernel it stays within 1 GiB unless a single
+ * partial slot of every channel is larger. */
+int64_t gpfq_conv_partial_bytes(gpfq_ctx *ctx);
 
 /* ---- Dense layer ---------------------------------------------------------------------------
  * Replaces QuantizedNeuralNetwork._quantize_layer_parallel after data collection
@@ -185,8 +189,8 @@ int gpfq_conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float *actq, int
  *   gpfq_conv_layer_from_gram  the walks of every filter of channels c0 .. c0+n_ch-1 from such matrices (device pointer,
  *                              GPFQ_X_DEVICE; channel i of the range at gram + i * 2 kk^2).  W / Q_out as in
  *                              gpfq_conv_channels (GPFQ_W_DEVICE / GPFQ_Q_DEVICE say where they live).
- * Both serve only the kernel sizes with their own Gram and walk kernels, kh * kw in {1, 2, 3, 4, 6, 9}; any other size returns
- * GPFQ_ERR_UNSUPPORTED (gpfq_conv_layer_nhwc still takes it, one Dense problem per channel).
+ * Both serve every kernel up to 128 taps, kh * kw <= 128 (11 x 11 included); a larger kernel returns GPFQ_ERR_UNSUPPORTED
+ * (gpfq_conv_layer_nhwc and gpfq_conv_channels still take it, one Dense problem per channel).
  */
 int gpfq_conv_gram_nhwc(gpfq_ctx *ctx, const float *act, const float *actq, int64_t n_img, int64_t H, int64_t Wd,
                         int64_t C, int32_t kh, int32_t kw, int32_t stride_h, int32_t stride_w, int32_t rate_h,

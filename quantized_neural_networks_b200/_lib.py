@@ -49,6 +49,7 @@ EXPORTS = {
     "gpfq_set_stream": (c_int, [c_void_p, c_void_p]),
     "gpfq_set_option": (c_int, [c_void_p, c_char_p, c_int64]),
     "gpfq_trim": (c_int, [c_void_p]),
+    "gpfq_conv_partial_bytes": (c_int64, [c_void_p]),
     "gpfq_query_stats": (c_int, [c_void_p, c_int32, POINTER(GpfqStats)]),
     "gpfq_dense_layer": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int64,
                                  c_int64, c_int64, c_int64, POINTER(c_double), POINTER(c_int32), c_int32,

@@ -18,7 +18,8 @@ int dense_stream_path(gpfq_ctx *, const float *, const float *, int64_t, int64_t
 int dense_gram_only(gpfq_ctx *, const float *, const float *, int64_t, int64_t, int64_t, double *, double *);
 bool dense_gram_uses_i8(gpfq_ctx *, int64_t, int64_t, bool);
 int conv_supported_kk(int kk);
-int conv_pick_chunks(gpfq_ctx *, int64_t, int, int64_t *, int, bool);
+int conv_pick_chunks(gpfq_ctx *, int64_t, int, int64_t *, int, bool, int64_t part_rows = 0);
+bool conv_specialised_kk(int kk);
 int conv_gram_stage(gpfq_ctx *, int, ConvPtrs, bool, int64_t, int, int, int64_t, double *, bool, int);
 int conv_finalize_stage(gpfq_ctx *, const double *, int, int, int, bool, double *);
 int conv_sweep_stage(gpfq_ctx *, int, const double *, const float *, double *, int64_t, int64_t, int64_t, int,
@@ -133,6 +134,8 @@ extern "C" int gpfq_create(int device, gpfq_ctx **out) {
     *out = ctx;
     return GPFQ_OK;
 }
+
+extern "C" int64_t gpfq_conv_partial_bytes(gpfq_ctx *ctx) { return ctx ? ctx->conv_part_bytes : 0; }
 
 extern "C" int gpfq_trim(gpfq_ctx *ctx) {
     if (!ctx) return GPFQ_ERR_ARG;
@@ -621,6 +624,9 @@ static void conv_stats(gpfq_ctx *ctx, gpfq_stats *st, int kk, int64_t n, int64_t
     st->method = GPFQ_METHOD_GRAM >> 4;
     st->bytes_algorithmic = (same ? 1 : 2) * 4LL * kk * n * n_ch;
     st->flops_algorithmic = (same ? 0 : 2LL * kk * kk * n * n_ch) + (int64_t)kk * (kk + 1) * n * n_ch;
+    // conv_gramx_kernel forms the lower triangles + diagonals of both Grams (of G2 alone in the first-layer form):
+    // kk (kk + 1) / 2 MACs = kk (kk + 1) flops per column, channel and Gram
+    if (!conv_specialised_kk(kk)) st->flops_algorithmic = (same ? 1 : 2) * (int64_t)kk * (kk + 1) * n * n_ch;
 }
 
 extern "C" int gpfq_conv_channels(gpfq_ctx *ctx, const float *const *Xp, const float *const *Xqp, int64_t n,
@@ -636,6 +642,7 @@ extern "C" int gpfq_conv_channels(gpfq_ctx *ctx, const float *const *Xp, const f
                          (long long)C, (long long)F, (long long)c0, (long long)n_ch);
     if ((flags & GPFQ_NO_SYNC) && (flags & GPFQ_ALL_DEVICE) != GPFQ_ALL_DEVICE)
         return gpfq_fail(ctx, GPFQ_ERR_ARG, "GPFQ_NO_SYNC needs all-device pointers");
+    ctx->conv_part_bytes = 0;
     if (n_ch == 0) return GPFQ_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     bool same = (Xqp == nullptr);
@@ -647,7 +654,7 @@ extern "C" int gpfq_conv_channels(gpfq_ctx *ctx, const float *const *Xp, const f
         if (!Xp[i] || (!same && !Xqp[i])) return gpfq_fail(ctx, GPFQ_ERR_ARG, "NULL patch pointer for channel %lld", (long long)i);
 
     if (!conv_supported_kk(kk)) {
-        // generic kernel sizes: each channel is a (kk, F) Dense problem over n_patches samples
+        // kernels above 128 taps: each channel is a (kk, F) Dense problem over n_patches samples
         int64_t launches = 0;
         for (int64_t i = 0; i < n_ch; ++i) {
             const int64_t c = c0 + i;
@@ -673,7 +680,8 @@ extern "C" int gpfq_conv_channels(gpfq_ctx *ctx, const float *const *Xp, const f
     int64_t chunk_cols = 0;
     const int n_chunks = conv_pick_chunks(ctx, n, (int)n_ch, &chunk_cols, kk, vec_ok);
     double *partial = nullptr;
-    GPFQ_TRY(gpfq_ws(ctx, WS_CPART, (size_t)n_ch * n_chunks * 2 * kk * kk * sizeof(double), (void **)&partial));
+    ctx->conv_part_bytes = (int64_t)n_ch * n_chunks * 2 * kk * kk * (int64_t)sizeof(double);
+    GPFQ_TRY(gpfq_ws(ctx, WS_CPART, (size_t)ctx->conv_part_bytes, (void **)&partial));
     const float **d_ptrs = nullptr;
     GPFQ_TRY(gpfq_ws(ctx, WS_PTRS, (size_t)2 * n_ch * sizeof(float *), (void **)&d_ptrs));
     std::vector<const float *> h_ptrs(2 * n_ch);
@@ -753,6 +761,7 @@ extern "C" int gpfq_conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float
         c0 < 0 || n_ch < 0 || c0 + n_ch > C || H > 65535 || Wd > 65535)
         return gpfq_fail(ctx, GPFQ_ERR_ARG, "bad conv geometry");
     const int kk = kh * kw;
+    ctx->conv_part_bytes = 0;
     if (n_ch == 0) return GPFQ_OK;
     // TensorFlow extract_patches geometry (quantized_network.py:158-172)
     const int keh = (kh - 1) * rh + 1, kew = (kw - 1) * rw + 1;
@@ -774,8 +783,8 @@ extern "C" int gpfq_conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float
     cudaStream_t s = ctx->stream;
     const bool same = (actq == nullptr || actq == act);
     if (!conv_supported_kk(kk)) {
-        // Kernel sizes without a dedicated Gram / walk kernel (5 x 5, 7 x 7, ...; the reference takes any size,
-        // quantized_network.py:686-727): patches of one channel at a time on the device (im2col), then that channel is a
+        // Kernels above 128 taps (13 x 11, 12 x 12, ...; the reference takes any size, quantized_network.py:686-727) have no
+        // batched Gram / walk kernel: patches of one channel at a time on the device (im2col), then that channel is a
         // (kk, F) Dense problem over n patches -- what gpfq_conv_channels does for such sizes from host patch matrices.
         if (ctx->gram_only_out) return gpfq_fail(ctx, GPFQ_ERR_UNSUPPORTED, "kernel %dx%d has no Gram-only (image split) path", kh, kw);
         const size_t abytes_g = (size_t)n_img * H * Wd * C * sizeof(float);
@@ -827,7 +836,16 @@ extern "C" int gpfq_conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float
         ipc = std::max<int64_t>(ipc, ceil_div64(n_img, 32));  // at most 32 chunks
         ipc = std::min<int64_t>(ceil_div64(ipc, 4) * 4, n_img);
     }
-    const int n_ic = (int)ceil_div64(n_img, ipc);
+    int n_ic = (int)ceil_div64(n_img, ipc);
+    if (host_act && !conv_specialised_kk(kk)) {
+        // every image chunk adds partial slots: keep the partial workspace of conv_gramx_kernel within CONV_PART_LIMIT
+        // (conv_pick_chunks trims the column chunks), with fewer, larger image chunks when many channels meet a large kernel
+        const int64_t max_ic = std::max<int64_t>(1, CONV_PART_LIMIT / (n_ch * 2 * kk * kk * (int64_t)sizeof(double)));
+        if (n_ic > max_ic) {
+            ipc = std::min<int64_t>(ceil_div64(ceil_div64(n_img, max_ic), 4) * 4, n_img);
+            n_ic = (int)ceil_div64(n_img, ipc);
+        }
+    }
     if (host_act) {
         float *ba = nullptr, *bq = nullptr;
         GPFQ_TRY(gpfq_ws(ctx, WS_ACT_A, abytes, (void **)&ba));
@@ -880,6 +898,7 @@ extern "C" int gpfq_conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float
         float *pkA = nullptr, *pkQ = nullptr;
         const size_t part_bytes = (size_t)vch * slots * 78 * sizeof(double);      // 2 passes x 3 column classes x 13 sums
         const size_t bpart_bytes = (size_t)vch * bslots * 78 * sizeof(double);
+        ctx->conv_part_bytes = (int64_t)part_bytes;
         GPFQ_TRY(gpfq_ws(ctx, WS_CPART, part_bytes, (void **)&partial));
         GPFQ_TRY(gpfq_ws(ctx, WS_CORR_B, bpart_bytes, (void **)&bpartial));
         GPFQ_TRY(gpfq_ws(ctx, WS_CG, (size_t)n_ch * 2 * kk * kk * sizeof(double), (void **)&gram));
@@ -941,6 +960,7 @@ extern "C" int gpfq_conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float
         const int slots = (int)(n_ic * per_ic);
         double *partial = nullptr;
         const size_t part_bytes = (size_t)groups * 8 * slots * 2 * kk * kk * sizeof(double);
+        ctx->conv_part_bytes = (int64_t)part_bytes;
         GPFQ_TRY(gpfq_ws(ctx, WS_CPART, part_bytes, (void **)&partial));
         CUDA_TRY(ctx, cudaMemsetAsync(partial, 0, part_bytes, s));  // short chunks leave slots unused
         CUDA_TRY(ctx, gpfq_record(ctx, 2, s));
@@ -978,11 +998,12 @@ extern "C" int gpfq_conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float
     const int64_t n_c = ipc * hw_out;  // patch columns of a full image chunk
     bool vec_ok = n_c % 4 == 0 && ((n_img - (int64_t)(n_ic - 1) * ipc) * hw_out) % 4 == 0;
     int64_t chunk_cols = 0;
-    const int n_chunks = conv_pick_chunks(ctx, n_c, (int)std::min<int64_t>(n_ch, 64), &chunk_cols, kk, vec_ok);
+    const int n_chunks = conv_pick_chunks(ctx, n_c, (int)std::min<int64_t>(n_ch, 64), &chunk_cols, kk, vec_ok, n_ch * n_ic);
     const int slots = n_ic * n_chunks;
     double *partial = nullptr;
     const size_t part_bytes = (size_t)n_ch * slots * 2 * kk * kk * sizeof(double);
-    GPFQ_TRY(gpfq_ws(ctx, WS_CPART, part_bytes, (void **)&partial));
+    ctx->conv_part_bytes = (int64_t)part_bytes;
+        GPFQ_TRY(gpfq_ws(ctx, WS_CPART, part_bytes, (void **)&partial));
     if (n_ic > 1) CUDA_TRY(ctx, cudaMemsetAsync(partial, 0, part_bytes, s));  // a short last chunk leaves slots unused
     const size_t ch_elems = (size_t)kk * n_c;
     const size_t per_ch = ch_elems * sizeof(float);

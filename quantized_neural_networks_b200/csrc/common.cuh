@@ -71,6 +71,7 @@ struct gpfq_ctx {
     int i8_pairs_d = 0;           // int8 Gram: keep slice pairs with k + l <= this (0: the default of gram_i8.cu)
     const double *h_alph = nullptr;  // host copy of the current call's alphabets (levels back to back) and their offsets
     const int *h_koff = nullptr, *h_flags = nullptr;
+    int64_t conv_part_bytes = 0;      // partial Gram workspace of the last conv call (gpfq_conv_partial_bytes)
     double *gram_only_out = nullptr;  // set for the duration of gpfq_conv_gram_nhwc: conv_finish hands the Grams out, no walk
     int last_gram_kernel = 0;     // what the last Dense Gram stage ran (1 DMMA, 2 int8 tcgen05)
     size_t i8_oom_bytes = 0;      // smallest int8-Gram workspace that failed to allocate (0: none yet)
@@ -117,6 +118,10 @@ int gpfq_pinned(gpfq_ctx *ctx, int slot, size_t bytes, void **out);     // pinne
             return gpfq_fail((ctx), GPFQ_ERR_CUDA, "kernel launch failed: %s (%s:%d)",        \
                              cudaGetErrorString(_e), __FILE__, __LINE__);                     \
     } while (0)
+
+// Partial Gram workspace (WS_CPART) of the conv kernels for sizes without a kernel of their own: at most 1 GiB, reached
+// through fewer column chunks / image chunks (conv_pick_chunks, gpfq_conv_layer_nhwc) unless one slot per channel exceeds it.
+static constexpr int64_t CONV_PART_LIMIT = (int64_t)1 << 30;
 
 static inline int64_t ceil_div64(int64_t a, int64_t b) { return (a + b - 1) / b; }
 

@@ -8,6 +8,8 @@
 //                                 accumulation of exact fp32 products, per-CTA partials
 //   stage 2  conv_finalize_kernel fixed-order sum of the partials (deterministic)
 //   stage 3  conv_sweep_kernel    one thread per (channel, filter): the kk-step walk in registers
+// Stages 1 and 3 have kernels of their own for kk in {1, 2, 3, 4, 6, 9}; every other kk <= 128 (5 x 5, 7 x 7, 11 x 11, ...)
+// takes conv_gramx_kernel (DMMA tiles for a runtime kk) and conv_walkx_kernel (one warp per filter).
 // Also here: the on-device single-channel im2col that serves gpfq_conv_layer_nhwc (the reference's
 // _build_patch_array :729-809 / tf.image.extract_patches :158-172) and the MSQ baseline.
 #include "common.cuh"
@@ -543,6 +545,166 @@ conv_gram9_nhwc_kernel(const float *__restrict__ act, const float *__restrict__ 
     }
 }
 
+// ---- stage 1, any kk <= 128 on the fp64 tensor pipe ---------------------------------------------
+// The sizes without a kernel above (5 x 5, 7 x 7, 11 x 11, 1 x 7, ...).  The kk patch rows are padded with zero rows to
+// KP = 8 NB and cut into NB blocks of eight; the lower-triangular 8 x 8 tiles (I >= J) of G2 = Xq Xq^T and G1 = Xq X^T are one
+// DMMA.8x8x4 each per four columns (exact fp32 products, fp64 sums: the Gram form of DESIGN section 3).  A CTA stages TC
+// columns of Xq (and X) in shared memory, converted to fp64 once; the next stage's loads are in flight in registers while
+// the current one is multiplied.  Warp (p, cg) owns the tiles of block rows p and NB-1-p (NB + 1 tiles per Gram, the A fragment
+// of a row loaded once per four columns) over the four-column steps cg, cg + CG, ... of every stage; the CG column groups are
+// added in index order at the end, so the summation order is fixed and the result bit-reproducible.  Padding rows are zero, so
+// they add nothing; a tap that only ever reads padding has an exactly zero row.  Any n and any row alignment (scalar loads).
+// Writes the partial layout of conv_gram_kernel: lower triangle + diagonal of G2, of G1 too (its upper triangle is written 0).
+namespace gramx {
+constexpr int MAX_KK = 128;
+template <int NB>
+struct Cfg {
+    static constexpr int KP = 8 * NB;
+    static constexpr int NP = (NB + 1) / 2;                  // block-row pairs
+    static constexpr int CG = 8 / NP >= 1 ? 8 / NP : 1;      // column groups
+    static constexpr int NW = NP * CG;                       // warps (5..8)
+    static constexpr int NT = NW * 32;
+    static constexpr int TC = 2048 / KP >= 256 ? 256 : 2048 / KP >= 128 ? 128 : 2048 / KP >= 64 ? 64 : 2048 / KP >= 32 ? 32 : 16;
+    static constexpr int LTC = TC == 256 ? 8 : TC == 128 ? 7 : TC == 64 ? 6 : TC == 32 ? 5 : 4;
+    static constexpr int PITCH = TC + 4;                     // doubles: lanes (g, k) of an LDS.64 half-warp on distinct banks
+    static constexpr int MINB = NB == 1 ? 3 : NB <= 4 ? 2 : 1;   // CTAs per SM the registers allow without spills
+    static_assert((TC / 4) % CG == 0, "every column group gets the same steps");
+};
+// dynamic shared memory: the fp64 stage, reused for the column-group sum (CG > 1)
+template <int NB, bool SAME>
+constexpr size_t smem_bytes() {
+    using C = Cfg<NB>;
+    const size_t stage = (size_t)(SAME ? 1 : 2) * C::KP * C::PITCH * sizeof(double);
+    const size_t red = C::CG > 1 ? (size_t)2 * C::KP * C::KP * sizeof(double) : 0;
+    return stage > red ? stage : red;
+}
+}  // namespace gramx
+
+template <int NB, bool SAME>
+__global__ void __launch_bounds__(gramx::Cfg<NB>::NT, gramx::Cfg<NB>::MINB)
+conv_gramx_kernel(ConvPtrs ptrs, int64_t n, int kk, int64_t chunk_cols, double *__restrict__ partial, int slots) {
+    using C = gramx::Cfg<NB>;
+    constexpr int KP = C::KP, TC = C::TC, PITCH = C::PITCH, NT = C::NT, NMAT = SAME ? 1 : 2;
+    constexpr int E = (NMAT * KP * TC + NT - 1) / NT;   // staged elements per thread and stage
+    extern __shared__ __align__(16) double gramx_smem[];
+    double *sq = gramx_smem;                            // KP x PITCH: Xq
+    double *sx = SAME ? sq : sq + KP * PITCH;           // KP x PITCH: X
+    const int ch = blockIdx.y, chunk = blockIdx.x;
+    const float *X = ptrs.Xp[ch];
+    const float *Xq = SAME ? X : ptrs.Xqp[ch];
+    const int64_t c_beg = (int64_t)chunk * chunk_cols;
+    const int64_t c_end = (c_beg + chunk_cols < n) ? c_beg + chunk_cols : n;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int g = lane >> 2, k = lane & 3;
+    const int p = warp % C::NP, cg = warp / C::NP;
+    const int I1 = p, I2 = NB - 1 - p;
+    const int real = NMAT * kk * TC;                    // staged elements of the kk real rows
+
+    // padding rows kk .. KP-1 stay zero for the whole kernel
+    for (int e = tid; e < NMAT * (KP - kk) * PITCH; e += NT) {
+        const int m = e / ((KP - kk) * PITCH), rc = e % ((KP - kk) * PITCH);
+        gramx_smem[m * KP * PITCH + kk * PITCH + rc] = 0.0;
+    }
+    float pre[E];
+    auto load = [&](int64_t c0) {
+#pragma unroll
+        for (int i = 0; i < E; ++i) {
+            const int e = tid + i * NT;
+            const int c = e & (TC - 1), mr = e >> C::LTC;
+            const int m = mr >= kk ? 1 : 0, r = mr - m * kk;
+            const int64_t col = c0 + c;
+            const float *src = m ? X : Xq;
+            pre[i] = (e < real && col < c_end) ? __ldg(src + (int64_t)r * n + col) : 0.f;
+        }
+    };
+    double acc2[NB + 1][2] = {}, acc1[NB + 1][2] = {};
+    load(c_beg);
+    for (int64_t c0 = c_beg; c0 < c_end; c0 += TC) {
+        __syncthreads();  // the previous stage has been read
+#pragma unroll
+        for (int i = 0; i < E; ++i) {
+            const int e = tid + i * NT;
+            if (e < real) {
+                const int c = e & (TC - 1), mr = e >> C::LTC;
+                const int m = mr >= kk ? 1 : 0, r = mr - m * kk;
+                gramx_smem[(m * KP + r) * PITCH + c] = (double)pre[i];
+            }
+        }
+        __syncthreads();
+        if (c0 + TC < c_end) load(c0 + TC);  // in flight while this stage is multiplied
+        for (int ks = cg; ks < TC / 4; ks += C::CG) {
+            const int col = 4 * ks + k;
+            const double a1 = sq[(8 * I1 + g) * PITCH + col], a2 = sq[(8 * I2 + g) * PITCH + col];
+#pragma unroll
+            for (int j = 0; j <= NB; ++j) {
+                // tile j: (I1, j) for j <= I1, else (I2, j - I1 - 1); the middle row of an odd NB has no second row
+                const bool r1 = j <= I1;
+                if (!r1 && I2 == I1) continue;
+                const int J = r1 ? j : j - I1 - 1;
+                const double a = r1 ? a1 : a2;
+                dmma884(acc2[j][0], acc2[j][1], a, sq[(8 * J + g) * PITCH + col]);
+                if (!SAME) dmma884(acc1[j][0], acc1[j][1], a, sx[(8 * J + g) * PITCH + col]);
+            }
+        }
+    }
+
+    double *out = partial + ((size_t)ch * slots + chunk) * (2 * kk * kk);
+    // lane (g, k) of tile (I, J) holds entries (8 I + g, 8 J + 2 k + u), u = 0, 1
+    auto tile_of = [&](int j, int &I, int &J) {
+        const bool r1 = j <= I1;
+        I = r1 ? I1 : I2;
+        J = r1 ? j : j - I1 - 1;
+        return r1 || I2 != I1;
+    };
+    if (!SAME)
+        for (int e = tid; e < kk * kk; e += NT)
+            if (e % kk > e / kk) out[e] = 0.0;  // upper triangle of G1: not computed
+    if (C::CG == 1) {
+#pragma unroll
+        for (int j = 0; j <= NB; ++j) {
+            int I, J;
+            if (!tile_of(j, I, J)) continue;
+            const int t = 8 * I + g;
+#pragma unroll
+            for (int u = 0; u < 2; ++u) {
+                const int s = 8 * J + 2 * k + u;
+                if (t < kk && s <= t) {
+                    out[kk * kk + t * kk + s] = acc2[j][u];
+                    if (!SAME) out[t * kk + s] = acc1[j][u];
+                }
+            }
+        }
+        return;
+    }
+    // column groups in index order through shared memory: red[which][t][s], KP x KP each
+    double *red = gramx_smem;
+    for (int c = 0; c < C::CG; ++c) {
+        __syncthreads();
+        if (cg == c) {
+#pragma unroll
+            for (int j = 0; j <= NB; ++j) {
+                int I, J;
+                if (!tile_of(j, I, J)) continue;
+                const int t = 8 * I + g;
+#pragma unroll
+                for (int u = 0; u < 2; ++u) {
+                    const int s = 8 * J + 2 * k + u;
+                    double *r2 = red + KP * KP + t * KP + s, *r1 = red + t * KP + s;
+                    *r2 = c == 0 ? acc2[j][u] : *r2 + acc2[j][u];
+                    if (!SAME) *r1 = c == 0 ? acc1[j][u] : *r1 + acc1[j][u];
+                }
+            }
+        }
+    }
+    __syncthreads();
+    for (int e = tid; e < kk * kk; e += NT) {
+        const int t = e / kk, s = e % kk;
+        if (s > t) continue;
+        out[kk * kk + e] = red[KP * KP + t * KP + s];
+        if (!SAME) out[e] = red[t * KP + s];
+    }
+}
+
 // ---- stage 2 ---------------------------------------------------------------------------------
 // gram: (n_channels, 2*kk*kk): [G1 | G2], lower triangle + diagonal of each valid.
 __global__ void conv_finalize_kernel(const double *__restrict__ partial, int n_chunks, int kk, int same,
@@ -593,6 +755,74 @@ conv_sweep_kernel(const double *__restrict__ gram, const float *__restrict__ W, 
         const double num = fma(w[t], g1[t * KK + t], d);
         q[t] = gpfq_decide(nrm[t], d, num, w[t], alph, K, inv_step);
         Q[(int64_t)a * q_alph_stride + (int64_t)t * CF + base] = q[t];
+    }
+}
+
+// The same walk for any kk <= 128: one warp per (channel, filter, alphabet).  The channel's lower triangles sit in shared
+// memory packed by columns (column s holds rows s .. kk-1, so the lanes of one update read consecutive words).  Lane l holds the
+// running dots d[t'] of the directions t' = l, l + 32, ...; after step t every later direction adds its term
+// w_t G1[t', t] - q_t G2[t', t], so d[t'] is summed over s < t' in ascending s, as in conv_sweep_kernel.  The lane that owns t
+// decides and q_t goes to the others by shuffle.
+namespace walkx {
+constexpr int MAXW = 16;  // warps (filters) per CTA
+__host__ __device__ constexpr int col_off(int s, int kk) { return s * kk - s * (s - 1) / 2; }
+}  // namespace walkx
+
+__global__ void __launch_bounds__(walkx::MAXW * 32)
+conv_walkx_kernel(const double *__restrict__ gram, int kk, const float *__restrict__ W, double *__restrict__ Q, int64_t CF,
+                  int64_t F, int64_t c0, const double *__restrict__ alphabets, const int *__restrict__ Koff,
+                  const int *__restrict__ Flags, int64_t q_alph_stride) {
+    extern __shared__ double walkx_smem[];
+    const int tri = kk * (kk + 1) / 2;
+    double *g1 = walkx_smem, *g2 = g1 + tri, *nrm = g2 + tri, *alph = nrm + kk;
+    const int ch = blockIdx.y, a = blockIdx.z;
+    const int K = Koff[a + 1] - Koff[a];
+    const double *gc = gram + (size_t)ch * 2 * kk * kk;
+    for (int e = threadIdx.x; e < kk * kk; e += blockDim.x) {
+        const int t = e / kk, s = e % kk;
+        if (s > t) continue;
+        const int o = walkx::col_off(s, kk) + t - s;
+        g1[o] = gc[e];
+        g2[o] = gc[kk * kk + e];
+    }
+    for (int e = threadIdx.x; e < K; e += blockDim.x) alph[e] = alphabets[Koff[a] + e];
+    __syncthreads();
+    for (int t = threadIdx.x; t < kk; t += blockDim.x) nrm[t] = (double)(float)sqrt(g2[walkx::col_off(t, kk)]);
+    __syncthreads();
+    const double inv_step = gpfq_inv_step(alph, K, Flags[a]);
+    const int lane = threadIdx.x & 31;
+    const int64_t f = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (f >= F) return;
+    const int64_t base = (c0 + ch) * F + f;
+    double *q_out = Q + (int64_t)a * q_alph_stride + base;
+    double w[4], d[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+        const int t = 32 * j + lane;
+        w[j] = t < kk ? (double)W[(int64_t)t * CF + base] : 0.0;
+        d[j] = 0.0;
+    }
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+        if (32 * j >= kk) break;
+        const int o_end = kk - 32 * j < 32 ? kk - 32 * j : 32;
+        for (int o = 0; o < o_end; ++o) {
+            const int t = 32 * j + o;
+            const int off = walkx::col_off(t, kk) - t;  // g[off + t'] = G[t', t]
+            double qt = 0.0;
+            if (lane == o) {
+                const double num = fma(w[j], g1[off + t], d[j]);
+                qt = gpfq_decide(nrm[t], d[j], num, w[j], alph, K, inv_step);
+                q_out[(int64_t)t * CF] = qt;
+            }
+            qt = __shfl_sync(0xffffffffu, qt, o);
+            const double wt = __shfl_sync(0xffffffffu, w[j], o);
+#pragma unroll
+            for (int j2 = j; j2 < 4; ++j2) {
+                const int t2 = 32 * j2 + lane;
+                if (t2 > t && t2 < kk) d[j2] += wt * g1[off + t2] - qt * g2[off + t2];
+            }
+        }
     }
 }
 
@@ -663,19 +893,46 @@ static int launch_conv_gram(gpfq_ctx *ctx, ConvPtrs ptrs, bool same, int64_t n, 
     return GPFQ_OK;
 }
 
-int conv_supported_kk(int kk) { return kk == 1 || kk == 2 || kk == 3 || kk == 4 || kk == 6 || kk == 9; }
+template <int NB, bool SAME>
+static int launch_conv_gramx(gpfq_ctx *ctx, ConvPtrs ptrs, int64_t n, int kk, int n_ch, int n_chunks, int64_t chunk_cols,
+                             double *partial, int slots) {
+    constexpr size_t smem = gramx::smem_bytes<NB, SAME>();
+    CUDA_TRY(ctx, cudaFuncSetAttribute(conv_gramx_kernel<NB, SAME>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    conv_gramx_kernel<NB, SAME><<<dim3((unsigned)n_chunks, (unsigned)n_ch), gramx::Cfg<NB>::NT, smem, ctx->stream>>>(
+        ptrs, n, kk, chunk_cols, partial, slots);
+    KERNEL_CHECK(ctx);
+    return GPFQ_OK;
+}
+
+// kh * kw with a kernel of its own (conv_gram_kernel<KK> and friends, conv_sweep_kernel<KK>)
+bool conv_specialised_kk(int kk) { return kk == 1 || kk == 2 || kk == 3 || kk == 4 || kk == 6 || kk == 9; }
+
+// kh * kw with batched Gram and walk kernels: the specialised sizes above, every other size through conv_gramx_kernel /
+// conv_walkx_kernel.  Larger kernels run one Dense problem per channel.
+int conv_supported_kk(int kk) { return kk >= 1 && kk <= gramx::MAX_KK; }
 
 // Column chunks per channel: grid = n_chunks x n_ch CTAs.  TMA kernel (kk == 9, vectorisable): one CTA per SM, whole
 // waves of sm_count CTAs, chunks a multiple of the 512-column stage; the other kernels: two CTAs per SM.
-int conv_pick_chunks(gpfq_ctx *ctx, int64_t n, int n_ch, int64_t *chunk_cols, int kk, bool vec_ok) {
+// conv_gramx_kernel: chunks a multiple of its widest stage (256 columns); from 8 block rows (kk > 56) a column costs
+// 72 DMMAs or more, so 1024-column chunks are already long enough.
+int conv_pick_chunks(gpfq_ctx *ctx, int64_t n, int n_ch, int64_t *chunk_cols, int kk, bool vec_ok, int64_t part_rows) {
     const bool tma = (kk == 9 && vec_ok && (ctx->conv_variant == 0 || ctx->conv_variant == 3));
+    const bool gx = !conv_specialised_kk(kk);
     const int64_t per_wave = tma ? ctx->sm_count : 2LL * ctx->sm_count;
-    const int64_t min_cols = tma ? 32768 : 4096, align = tma ? tma9::COLS : 128;
+    const int64_t min_cols = tma ? 32768 : (gx && kk > 56) ? 1024 : 4096, align = tma ? tma9::COLS : gx ? 256 : 128;
     int64_t waves = ((int64_t)n * n_ch) / (per_wave * min_cols);
     waves = waves < 1 ? 1 : (waves > 4 ? 4 : waves);
     int64_t want = (waves * per_wave) / n_ch;
     const int64_t max_chunks = ceil_div64(n, min_cols) > 0 ? ceil_div64(n, min_cols) : 1;
     if (want > max_chunks) want = max_chunks;
+    if (gx) {
+        // The partial workspace is part_rows (channels, times image chunks where those add slots; 0: n_ch) x n_chunks slots of
+        // 2 kk^2 doubles, 256 KB at kk = 128.  Keep it within CONV_PART_LIMIT: fewer, longer column chunks when many channels
+        // meet a large kernel (at least one chunk).
+        const int64_t per_slot = (part_rows > 0 ? part_rows : n_ch) * 2 * kk * kk * (int64_t)sizeof(double);
+        const int64_t cap = CONV_PART_LIMIT / per_slot;
+        if (want > cap) want = cap;
+    }
     if (want < 1) want = 1;
     int64_t cols = ceil_div64(n, want);
     cols = ceil_div64(cols, align) * align;
@@ -696,7 +953,17 @@ int conv_gram_stage(gpfq_ctx *ctx, int kk, ConvPtrs d_ptrs, bool same, int64_t n
         case 6: return launch_conv_gram<6>(ctx, d_ptrs, same, n, n_ch, n_chunks, chunk_cols, partial, vec_ok, slots);
         case 9: return launch_conv_gram<9>(ctx, d_ptrs, same, n, n_ch, n_chunks, chunk_cols, partial, vec_ok, slots);
     }
-    return gpfq_fail(ctx, GPFQ_ERR_UNSUPPORTED, "conv kernel size kk=%d has no specialised kernel", kk);
+    if (!conv_supported_kk(kk)) return gpfq_fail(ctx, GPFQ_ERR_UNSUPPORTED, "conv kernel size kk=%d has no Gram kernel", kk);
+#define GRAMX_CASE(NBV)                                                                                          \
+    case NBV:                                                                                                    \
+        return same ? launch_conv_gramx<NBV, true>(ctx, d_ptrs, n, kk, n_ch, n_chunks, chunk_cols, partial, slots) \
+                    : launch_conv_gramx<NBV, false>(ctx, d_ptrs, n, kk, n_ch, n_chunks, chunk_cols, partial, slots);
+    switch ((kk + 7) / 8) {
+        GRAMX_CASE(1) GRAMX_CASE(2) GRAMX_CASE(3) GRAMX_CASE(4) GRAMX_CASE(5) GRAMX_CASE(6) GRAMX_CASE(7) GRAMX_CASE(8)
+        GRAMX_CASE(9) GRAMX_CASE(10) GRAMX_CASE(11) GRAMX_CASE(12) GRAMX_CASE(13) GRAMX_CASE(14) GRAMX_CASE(15) GRAMX_CASE(16)
+    }
+#undef GRAMX_CASE
+    return gpfq_fail(ctx, GPFQ_ERR_UNSUPPORTED, "conv kernel size kk=%d has no Gram kernel", kk);
 }
 
 int conv_finalize_stage(gpfq_ctx *ctx, const double *partial, int n_ch, int n_chunks, int kk, bool same,
@@ -715,7 +982,15 @@ int conv_sweep_stage(gpfq_ctx *ctx, int kk, const double *gram, const float *W, 
     case KKV: conv_sweep_kernel<KKV><<<grid, 128, 0, ctx->stream>>>(gram, W, Q, CF, F, c0, d_alph, d_koff, d_flags, qs); break;
     switch (kk) {
         SWEEP_CASE(1) SWEEP_CASE(2) SWEEP_CASE(3) SWEEP_CASE(4) SWEEP_CASE(6) SWEEP_CASE(9)
-        default: return gpfq_fail(ctx, GPFQ_ERR_UNSUPPORTED, "conv kernel size kk=%d has no specialised kernel", kk);
+        default: {
+            if (!conv_supported_kk(kk)) return gpfq_fail(ctx, GPFQ_ERR_UNSUPPORTED, "conv kernel size kk=%d has no walk kernel", kk);
+            using namespace walkx;
+            const int warps = F < MAXW ? (int)F : MAXW;
+            const size_t smem = ((size_t)kk * (kk + 1) + kk + GPFQ_MAX_K) * sizeof(double);
+            CUDA_TRY(ctx, cudaFuncSetAttribute(conv_walkx_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            dim3 wgrid((unsigned)ceil_div64(F, warps), (unsigned)n_ch, (unsigned)n_alph);
+            conv_walkx_kernel<<<wgrid, warps * 32, smem, ctx->stream>>>(gram, kk, W, Q, CF, F, c0, d_alph, d_koff, d_flags, qs);
+        }
     }
 #undef SWEEP_CASE
     KERNEL_CHECK(ctx);

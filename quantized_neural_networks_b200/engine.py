@@ -17,9 +17,10 @@ except Exception:  # pragma: no cover
 _METHODS = {"auto": _lib.METHOD_AUTO, "stream": _lib.METHOD_STREAM, "gram": _lib.METHOD_GRAM,
             "stream_fast": _lib.METHOD_STREAM_FAST}
 
-# Conv kernel sizes kh * kw with their own Gram and walk kernels: the set of `conv_supported_kk` in csrc/conv.cu.  Only these
-# have the Gram-only entry points (`conv_gram_nhwc`, `conv_layer_from_gram`); other sizes run one Dense problem per channel.
-CONV_SUPPORTED_KK = frozenset({1, 2, 3, 4, 6, 9})
+# Conv kernel sizes kh * kw with batched Gram and walk kernels (every size up to 128 taps, 11 x 11 included): the set of
+# `conv_supported_kk` in csrc/conv.cu.  Only these have the Gram-only entry points (`conv_gram_nhwc`, `conv_layer_from_gram`)
+# and so the image split of a multi-GPU job; larger kernels run one Dense problem per channel.
+CONV_SUPPORTED_KK = frozenset(range(1, 129))
 
 
 def _is_torch(x):
@@ -75,6 +76,10 @@ class GpfqEngine:
 
     def trim(self):
         self._check(self._lib.gpfq_trim(self._ctx))
+
+    def conv_partial_bytes(self) -> int:
+        """Bytes of partial Gram workspace the last conv call asked for (0 for kernels above 128 taps)."""
+        return int(self._lib.gpfq_conv_partial_bytes(self._ctx))
 
     def set_option(self, key: str, value: int):
         """A/B switches of include/gpfq.h (`gram_kernel`, `i8_pairs_d`, `conv_kernel`, `corr_*`, `sweep_outer`, `sweep_walk`,
@@ -364,7 +369,7 @@ class GpfqEngine:
         """Gram stage of a conv layer alone: per-channel [G1 | G2] of channels c0..c0+n_channels-1 over the given images,
         as a float64 CUDA tensor (n_channels, 2, kh*kw, kh*kw) (lower triangles + diagonals valid).  act / actq: NHWC
         NumPy arrays or CUDA tensors.  The per-rank part of an image-split multi-GPU job (`conv_layer_from_gram`).  Raises
-        GpfqError for kh * kw outside CONV_SUPPORTED_KK."""
+        GpfqError for kh * kw outside CONV_SUPPORTED_KK (kernels above 128 taps)."""
         act = self._f32(act, "act")
         same = actq is None or actq is act
         actq = act if same else self._f32(actq, "actq")

@@ -406,7 +406,7 @@ class QuantizedCNN(QuantizedNeuralNetwork):
                 if self._nccl_job() and self.gram_split != "replicate" and W.shape[0] * W.shape[1] in CONV_SUPPORTED_KK:
                     # image split: every rank contracts n_img / world images of ALL channels, one tiny all-reduce sums the
                     # per-channel Grams, then every rank walks every channel (cheap: kk steps per filter) -- no Q gather.
-                    # Other kernel sizes (5 x 5, 7 x 7, ...) have no Gram-only path and take the channel shards below.
+                    # Kernels above 128 taps (13 x 11, ...) have no Gram-only path and take the channel shards below.
                     gram = image_split_conv_gram(self.engine, data.wX, None if data.same else data.qX, W.shape[:2],
                                                  layer.strides, layer.padding.upper(), rate, *self.shard)
                     self.layer_stats[layer_idx] = dict(self.engine.last_stats)

@@ -71,9 +71,11 @@ def main():
     xi_eval = rng.random((256, 16, 16, 3)).astype(np.float32)
 
     def run_cnn(**kw):
-        # a 5 x 5 layer after the first conv: kernel sizes without a Gram-only path leave the image split for channel shards
+        # after the first conv a 5 x 5 layer (image split, like the 3 x 3 layers) and a 13 x 11 layer: kernels above 128 taps
+        # have no Gram-only path and leave the image split for channel shards
         base = hostnet.cifar10_cnn(seed=5, size=16, widths=(32, 32, 64), dense=64, n_out=10).layers
-        net = hostnet.Sequential(base[:2] + [hostnet.Conv2D(32, 5, padding="same", activation="relu")] + base[2:],
+        net = hostnet.Sequential(base[:2] + [hostnet.Conv2D(32, 5, padding="same", activation="relu"),
+                                             hostnet.Conv2D(32, (13, 11), padding="same", activation="relu")] + base[2:],
                                  input_shape=(16, 16, 3), seed=5)
         q = QuantizedCNN(net, 32, hostnet.ArraySequence(xi, np.zeros(320), 32), logger=quiet, bits=2, alphabet_scalar=3,
                          device=local, **kw)
