@@ -200,6 +200,26 @@ int gpfq_conv_layer_from_gram(gpfq_ctx *ctx, const double *gram, int32_t kk, con
                               int64_t c0, int64_t n_channels, const double *alphabets, const int32_t *K,
                               int32_t n_alphabets, double *Q_out, uint32_t flags, gpfq_stats *stats);
 
+/* ---- grouped Conv2D (groups > 1: ResNeXt, RegNet, ConvNeXt's Conv2D(groups=C), ShuffleNet) ---------------------------------
+ * The counterparts of gpfq_conv_layer_nhwc and gpfq_conv_layer_from_gram for a Conv2D with `groups` groups, in one call.  C is the
+ * number of INPUT channels (of the activations / Grams); W and Q_out are the (kh, kw, Cg, F) kernel of the layer, Cg = C / groups:
+ * tap t of input channel c and filter f < Fg = F / groups of c's group g = c / Cg is W[t*Cg*F + (c % Cg)*F + g*Fg + f], and input
+ * channel c is walked against those Fg filters only (the filters of other groups never see it).  c0 / n_channels index input
+ * channels as in the Gram stage (gpfq_conv_gram_nhwc is shared: Grams do not depend on groups), so a channel range may start or
+ * end inside a group; only its channels' entries of Q_out are written.  The a-th alphabet's tensor starts at
+ * Q_out + a*kk*Cg*F.  groups must be >= 1 and divide both C and F (GPFQ_ERR_ARG otherwise); groups = 1 is the ungrouped call.
+ * stats.weights counts kk * n_channels * Fg * n_alphabets.  A depthwise layer (groups = C) is a DepthwiseConv2D with
+ * depth_multiplier Fg whose kernel is stored (kh, kw, 1, C*Fg).
+ */
+int gpfq_conv_layer_nhwc_grouped(gpfq_ctx *ctx, const float *act, const float *actq, int64_t n_img, int64_t H, int64_t Wd,
+                                 int64_t C, int32_t kh, int32_t kw, int32_t stride_h, int32_t stride_w, int32_t rate_h,
+                                 int32_t rate_w, int32_t padding_same, const float *W, int64_t F, int64_t c0,
+                                 int64_t n_channels, const double *alphabets, const int32_t *K, int32_t n_alphabets,
+                                 double *Q_out, uint32_t flags, gpfq_stats *stats, int32_t groups);
+int gpfq_conv_layer_from_gram_grouped(gpfq_ctx *ctx, const double *gram, int32_t kk, const float *W, int64_t C, int64_t F,
+                                      int64_t c0, int64_t n_channels, const double *alphabets, const int32_t *K,
+                                      int32_t n_alphabets, double *Q_out, uint32_t flags, gpfq_stats *stats, int32_t groups);
+
 /* ---- MSQ baseline ---------------------------------------------------------------------------
  * Plain nearest-level rounding of every weight (_bit_round_parallel :40-57 applied elementwise,
  * as in quantize_pretrained_mlp.py:97-117).  n elements, contiguous. */

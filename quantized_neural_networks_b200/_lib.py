@@ -69,6 +69,13 @@ EXPORTS = {
     "gpfq_conv_layer_from_gram": (c_int, [c_void_p, c_void_p, c_int32, c_void_p, c_int64, c_int64, c_int64, c_int64,
                                           POINTER(c_double), POINTER(c_int32), c_int32, c_void_p, c_uint32,
                                           POINTER(GpfqStats)]),
+    "gpfq_conv_layer_nhwc_grouped": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int64, c_int64, c_int32,
+                                             c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_void_p, c_int64,
+                                             c_int64, c_int64, POINTER(c_double), POINTER(c_int32), c_int32, c_void_p,
+                                             c_uint32, POINTER(GpfqStats), c_int32]),
+    "gpfq_conv_layer_from_gram_grouped": (c_int, [c_void_p, c_void_p, c_int32, c_void_p, c_int64, c_int64, c_int64, c_int64,
+                                                  POINTER(c_double), POINTER(c_int32), c_int32, c_void_p, c_uint32,
+                                                  POINTER(GpfqStats), c_int32]),
     "gpfq_msq": (c_int, [c_void_p, c_void_p, c_int64, POINTER(c_double), c_int32, c_void_p, c_uint32]),
     "gpfq_bit_round": (c_int, [c_void_p, c_void_p, c_int64, POINTER(c_double), c_int32, c_void_p, c_uint32]),
     "gpfq_gram_matrices": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_void_p,

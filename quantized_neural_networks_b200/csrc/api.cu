@@ -23,7 +23,7 @@ bool conv_specialised_kk(int kk);
 int conv_gram_stage(gpfq_ctx *, int, ConvPtrs, bool, int64_t, int, int, int64_t, double *, bool, int);
 int conv_finalize_stage(gpfq_ctx *, const double *, int, int, int, bool, double *);
 int conv_sweep_stage(gpfq_ctx *, int, const double *, const float *, double *, int64_t, int64_t, int64_t, int,
-                     const double *, const int *, const int *, int);
+                     const double *, const int *, const int *, int, int64_t);
 int im2col_stage(gpfq_ctx *, const float *, int64_t, int, int, int64_t, int64_t, int, int, int, int, int, int, int,
                  int, int, int, int, float *, int64_t);
 int msq_stage(gpfq_ctx *, const void *, int, int64_t, const double *, int, int, double *);
@@ -579,9 +579,40 @@ extern "C" int gpfq_gram_matrices(gpfq_ctx *ctx, const float *X, const float *Xq
 // ---------------------------------------------------------------------------------------------
 // Conv
 // ---------------------------------------------------------------------------------------------
+// Host Q of a grouped layer, (kk, Cg, F) per alphabet: channel c's entries are row c % Cg of its group's Fg columns in every
+// tap.  Channels c0 .. c0+n_ch-1 cover a partial first group, whole groups and a partial last group; whole groups are one
+// pitched copy over all taps, a partial group one per tap.
+static int conv_copy_q_grouped(gpfq_ctx *ctx, double *Q_out, const double *dQ, int kk, int64_t Cg, int64_t F, int64_t Fg,
+                               int64_t c0, int64_t n_ch, int n_alph, size_t wcount) {
+    cudaStream_t s = ctx->stream;
+    const size_t pitch = (size_t)F * sizeof(double);
+    auto box = [&](int64_t r0, int64_t r1, int64_t g0, int64_t g1) -> int {  // rows [r0, r1) of groups [g0, g1)
+        if (r1 <= r0 || g1 <= g0) return GPFQ_OK;
+        const size_t width = (size_t)(g1 - g0) * Fg * sizeof(double);
+        for (int a = 0; a < n_alph; ++a) {
+            const size_t off = (size_t)a * wcount + (size_t)r0 * F + (size_t)g0 * Fg;
+            if (r0 == 0 && r1 == Cg) {
+                CUDA_TRY(ctx, cudaMemcpy2DAsync(Q_out + off, pitch, dQ + off, pitch, width, (size_t)kk * Cg, cudaMemcpyDeviceToHost, s));
+                continue;
+            }
+            for (int t = 0; t < kk; ++t) {
+                const size_t o = off + (size_t)t * Cg * F;
+                CUDA_TRY(ctx, cudaMemcpy2DAsync(Q_out + o, pitch, dQ + o, pitch, width, (size_t)(r1 - r0), cudaMemcpyDeviceToHost, s));
+            }
+        }
+        return GPFQ_OK;
+    };
+    const int64_t c1 = c0 + n_ch, w0 = ceil_div64(c0, Cg), w1 = c1 / Cg;  // whole groups [w0, w1)
+    if (w0 > w1) return box(c0 % Cg, c1 % Cg, c0 / Cg, c0 / Cg + 1);    // inside one group
+    GPFQ_TRY(box(c0 % Cg, Cg, c0 / Cg, w0));
+    GPFQ_TRY(box(0, Cg, w0, w1));
+    return box(0, c1 % Cg, w1, w1 + 1);
+}
+
+// W / Q_out: (kk, C / groups, F); channel c walks the F / groups filters of its group c / (C / groups).
 static int conv_finish(gpfq_ctx *ctx, int kk, const double *partial, int n_ch, int n_chunks, bool same,
                        const float *W, int64_t C, int64_t F, int64_t c0, const Alphabets &al, int n_alph,
-                       double *Q_out, uint32_t flags, double *gram_ready = nullptr) {
+                       double *Q_out, uint32_t flags, double *gram_ready = nullptr, int64_t groups = 1) {
     cudaStream_t s = ctx->stream;
     double *gram = gram_ready;  // per-channel [G1 | G2] already assembled (correlation form): no partials to sum
     if (!gram) {
@@ -597,7 +628,8 @@ static int conv_finish(gpfq_ctx *ctx, int kk, const double *partial, int n_ch, i
         return GPFQ_OK;
     }
     const float *dW = W;
-    const size_t wcount = (size_t)kk * C * F;
+    const int64_t Cg = C / groups;
+    const size_t wcount = (size_t)kk * Cg * F;
     if (!(flags & GPFQ_W_DEVICE)) {
         float *bw = nullptr;
         GPFQ_TRY(gpfq_ws(ctx, WS_W, wcount * sizeof(float), (void **)&bw));
@@ -606,8 +638,10 @@ static int conv_finish(gpfq_ctx *ctx, int kk, const double *partial, int n_ch, i
     }
     double *dQ = Q_out;
     if (!(flags & GPFQ_Q_DEVICE)) GPFQ_TRY(gpfq_ws(ctx, WS_Q, (size_t)n_alph * wcount * sizeof(double), (void **)&dQ));
-    GPFQ_TRY(conv_sweep_stage(ctx, kk, gram, dW, dQ, C, F, c0, n_ch, al.d_levels, al.d_koff, al.d_flags, n_alph));
+    GPFQ_TRY(conv_sweep_stage(ctx, kk, gram, dW, dQ, C, F, c0, n_ch, al.d_levels, al.d_koff, al.d_flags, n_alph, groups));
     CUDA_TRY(ctx, gpfq_record(ctx, 4, s));
+    if (!(flags & GPFQ_Q_DEVICE) && groups > 1)
+        return conv_copy_q_grouped(ctx, Q_out, dQ, kk, Cg, F, F / groups, c0, n_ch, n_alph, wcount);
     if (!(flags & GPFQ_Q_DEVICE)) {
         for (int a = 0; a < n_alph; ++a) {
             const size_t off = (size_t)a * wcount + (size_t)c0 * F;
@@ -748,11 +782,11 @@ extern "C" int gpfq_conv_channels(gpfq_ctx *ctx, const float *const *Xp, const f
     return GPFQ_OK;
 }
 
-extern "C" int gpfq_conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float *actq, int64_t n_img, int64_t H,
-                                    int64_t Wd, int64_t C, int32_t kh, int32_t kw, int32_t sh, int32_t sw, int32_t rh,
-                                    int32_t rw, int32_t padding_same, const float *W, int64_t F, int64_t c0,
-                                    int64_t n_ch, const double *alphabets, const int32_t *K, int32_t n_alph,
-                                    double *Q_out, uint32_t flags, gpfq_stats *stats) {
+// gpfq_conv_layer_nhwc(_grouped): W / Q_out (kh, kw, C / groups, F).
+static int conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float *actq, int64_t n_img, int64_t H, int64_t Wd, int64_t C,
+                           int32_t kh, int32_t kw, int32_t sh, int32_t sw, int32_t rh, int32_t rw, int32_t padding_same,
+                           const float *W, int64_t F, int64_t c0, int64_t n_ch, const double *alphabets, const int32_t *K,
+                           int32_t n_alph, double *Q_out, uint32_t flags, gpfq_stats *stats, int64_t groups) {
     if (!ctx) return GPFQ_ERR_ARG;
     ctx->err.clear();
     if (stats) memset(stats, 0, sizeof(*stats));
@@ -760,6 +794,9 @@ extern "C" int gpfq_conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float
     if (n_img < 1 || H < 1 || Wd < 1 || C < 1 || F < 1 || kh < 1 || kw < 1 || sh < 1 || sw < 1 || rh < 1 || rw < 1 ||
         c0 < 0 || n_ch < 0 || c0 + n_ch > C || H > 65535 || Wd > 65535)
         return gpfq_fail(ctx, GPFQ_ERR_ARG, "bad conv geometry");
+    if (groups < 1 || C % groups || F % groups)
+        return gpfq_fail(ctx, GPFQ_ERR_ARG, "bad groups=%lld for C=%lld, F=%lld", (long long)groups, (long long)C, (long long)F);
+    const int64_t Cg = C / groups, Fg = F / groups;
     const int kk = kh * kw;
     ctx->conv_part_bytes = 0;
     if (n_ch == 0) return GPFQ_OK;
@@ -810,12 +847,14 @@ extern "C" int gpfq_conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float
             GPFQ_TRY(im2col_stage(ctx, gA, n_img, (int)H, (int)Wd, C, c, 1, kh, kw, sh, sw, rh, rw, pt, pl, Ho, Wo, pa, (int64_t)kk * n));
             if (!same)
                 GPFQ_TRY(im2col_stage(ctx, gAq, n_img, (int)H, (int)Wd, C, c, 1, kh, kw, sh, sw, rh, rw, pt, pl, Ho, Wo, pq, (int64_t)kk * n));
-            // per-alphabet outputs are kk*C*F apart, which is exactly N0*ldq for N0 = kk, ldq = C*F
-            GPFQ_TRY(gpfq_dense_layer(ctx, pa, same ? pa : pq, n, kk, n, W + c * F, C * F, F, 0, F, alphabets, K, n_alph, Q_out + c * F,
-                                      C * F, ((flags & ~GPFQ_NO_SYNC) | GPFQ_X_DEVICE | GPFQ_METHOD_GRAM), stats));
+            // channel c against the Fg filters of its group (all F when ungrouped); per-alphabet outputs are kk*Cg*F apart, which is
+            // exactly N0*ldq for N0 = kk, ldq = Cg*F
+            const int64_t off = (c % Cg) * F + (c / Cg) * Fg;
+            GPFQ_TRY(gpfq_dense_layer(ctx, pa, same ? pa : pq, n, kk, n, W + off, Cg * F, Fg, 0, Fg, alphabets, K, n_alph, Q_out + off,
+                                      Cg * F, ((flags & ~GPFQ_NO_SYNC) | GPFQ_X_DEVICE | GPFQ_METHOD_GRAM), stats));
             launches += (stats ? stats->kernel_launches : 0) + (same ? 1 : 2);
         }
-        if (stats) { stats->kernel_launches = (int)launches; stats->weights = (int64_t)kk * n_ch * F * n_alph; }
+        if (stats) { stats->kernel_launches = (int)launches; stats->weights = (int64_t)kk * n_ch * Fg * n_alph; }
         return GPFQ_OK;
     }
     begin_call(ctx, 2);
@@ -938,11 +977,11 @@ extern "C" int gpfq_conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float
         }
         GPFQ_TRY(conv_corr9_assemble_stage(ctx, partial, slots, bpartial, bslots, same, (int)n_ch, pack ? corr_G : 1, gram));
         CUDA_TRY(ctx, gpfq_record(ctx, 3, s));
-        GPFQ_TRY(conv_finish(ctx, kk, nullptr, (int)n_ch, 0, same, W, C, F, c0, al, n_alph, Q_out, flags, gram));
+        GPFQ_TRY(conv_finish(ctx, kk, nullptr, (int)n_ch, 0, same, W, C, F, c0, al, n_alph, Q_out, flags, gram, groups));
         CUDA_TRY(ctx, gpfq_record(ctx, 1, s));
         gpfq_stats local = {};
         gpfq_stats *st = stats ? stats : &local;
-        conv_stats(ctx, st, kk, n, n_ch, F, same, n_alph);
+        conv_stats(ctx, st, kk, n, n_ch, Fg, same, n_alph);
         st->bytes_algorithmic = (same ? 1 : 2) * 4LL * n_img * H * Wd * n_ch;  // the activations, once
         st->flops_algorithmic = (same ? 1 : 2) * 26LL * n_img * H * Wd * n_ch;  // 13 MACs per pixel, channel and Gram
         st->gram_kernel = pack ? 5 : 4;
@@ -954,12 +993,12 @@ extern "C" int gpfq_conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float
     int planeP = 0, bandR = 0;
     if ((ctx->conv_variant == 0 || ctx->conv_variant == 3) && nhwc9_plan(kh, kw, sh, sw, rh, rw, Ho, Wo, &planeP, &bandR)) {
         // ---- fused path: Grams straight from the activations, no patch matrices
-        const int64_t groups = ceil_div64(n_ch, 8);
-        int64_t per_ic = ceil_div64(4LL * 2 * ctx->sm_count, groups * n_ic);  // ~4 waves of two CTAs per SM overall
+        const int64_t ctas = ceil_div64(n_ch, 8);                            // CTAs of 8 channels per image slot
+        int64_t per_ic = ceil_div64(4LL * 2 * ctx->sm_count, ctas * n_ic);  // ~4 waves of two CTAs per SM overall
         per_ic = std::max<int64_t>(1, std::min<int64_t>(per_ic, ipc));
         const int slots = (int)(n_ic * per_ic);
         double *partial = nullptr;
-        const size_t part_bytes = (size_t)groups * 8 * slots * 2 * kk * kk * sizeof(double);
+        const size_t part_bytes = (size_t)ctas * 8 * slots * 2 * kk * kk * sizeof(double);
         ctx->conv_part_bytes = (int64_t)part_bytes;
         GPFQ_TRY(gpfq_ws(ctx, WS_CPART, part_bytes, (void **)&partial));
         CUDA_TRY(ctx, cudaMemsetAsync(partial, 0, part_bytes, s));  // short chunks leave slots unused
@@ -983,11 +1022,11 @@ extern "C" int gpfq_conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float
                                            planeP, bandR, (int)per_ic, partial + (size_t)ic * per_ic * 2 * kk * kk, slots));
         }
         CUDA_TRY(ctx, gpfq_record(ctx, 3, s));
-        GPFQ_TRY(conv_finish(ctx, kk, partial, (int)n_ch, slots, same, W, C, F, c0, al, n_alph, Q_out, flags));
+        GPFQ_TRY(conv_finish(ctx, kk, partial, (int)n_ch, slots, same, W, C, F, c0, al, n_alph, Q_out, flags, nullptr, groups));
         CUDA_TRY(ctx, gpfq_record(ctx, 1, s));
         gpfq_stats local = {};
         gpfq_stats *st = stats ? stats : &local;
-        conv_stats(ctx, st, kk, n, n_ch, F, same, n_alph);
+        conv_stats(ctx, st, kk, n, n_ch, Fg, same, n_alph);
         st->bytes_algorithmic = (same ? 1 : 2) * 4LL * n_img * H * Wd * n_ch;  // the activations, once
         const bool synced = !(flags & GPFQ_NO_SYNC);
         if (synced) CUDA_TRY(ctx, cudaStreamSynchronize(s));
@@ -1055,14 +1094,32 @@ extern "C" int gpfq_conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float
         }
     }
     CUDA_TRY(ctx, gpfq_record(ctx, 3, s));
-    GPFQ_TRY(conv_finish(ctx, kk, partial, (int)n_ch, slots, same, W, C, F, c0, al, n_alph, Q_out, flags));
+    GPFQ_TRY(conv_finish(ctx, kk, partial, (int)n_ch, slots, same, W, C, F, c0, al, n_alph, Q_out, flags, nullptr, groups));
     CUDA_TRY(ctx, gpfq_record(ctx, 1, s));
     gpfq_stats local = {};
-    conv_stats(ctx, stats ? stats : &local, kk, n, n_ch, F, same, n_alph);
+    conv_stats(ctx, stats ? stats : &local, kk, n, n_ch, Fg, same, n_alph);
     const bool synced = !(flags & GPFQ_NO_SYNC);
     if (synced) CUDA_TRY(ctx, cudaStreamSynchronize(s));
     end_call(ctx, stats ? stats : &local, synced);
     return GPFQ_OK;
+}
+
+extern "C" int gpfq_conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float *actq, int64_t n_img, int64_t H,
+                                    int64_t Wd, int64_t C, int32_t kh, int32_t kw, int32_t sh, int32_t sw, int32_t rh,
+                                    int32_t rw, int32_t padding_same, const float *W, int64_t F, int64_t c0,
+                                    int64_t n_ch, const double *alphabets, const int32_t *K, int32_t n_alph,
+                                    double *Q_out, uint32_t flags, gpfq_stats *stats) {
+    return conv_layer_nhwc(ctx, act, actq, n_img, H, Wd, C, kh, kw, sh, sw, rh, rw, padding_same, W, F, c0, n_ch, alphabets, K,
+                           n_alph, Q_out, flags, stats, 1);
+}
+
+extern "C" int gpfq_conv_layer_nhwc_grouped(gpfq_ctx *ctx, const float *act, const float *actq, int64_t n_img, int64_t H,
+                                            int64_t Wd, int64_t C, int32_t kh, int32_t kw, int32_t sh, int32_t sw, int32_t rh,
+                                            int32_t rw, int32_t padding_same, const float *W, int64_t F, int64_t c0,
+                                            int64_t n_ch, const double *alphabets, const int32_t *K, int32_t n_alph,
+                                            double *Q_out, uint32_t flags, gpfq_stats *stats, int32_t groups) {
+    return conv_layer_nhwc(ctx, act, actq, n_img, H, Wd, C, kh, kw, sh, sw, rh, rw, padding_same, W, F, c0, n_ch, alphabets, K,
+                           n_alph, Q_out, flags, stats, groups);
 }
 
 // Gram stage of a conv layer alone (see include/gpfq.h): the same planner and kernels as gpfq_conv_layer_nhwc, stopped
@@ -1086,16 +1143,18 @@ extern "C" int gpfq_conv_gram_nhwc(gpfq_ctx *ctx, const float *act, const float 
     return rc;
 }
 
-// Walk stage of a conv layer from per-channel Gram matrices on the device (see include/gpfq.h).
-extern "C" int gpfq_conv_layer_from_gram(gpfq_ctx *ctx, const double *gram, int32_t kk, const float *W, int64_t C, int64_t F,
-                                         int64_t c0, int64_t n_ch, const double *alphabets, const int32_t *K, int32_t n_alph,
-                                         double *Q_out, uint32_t flags, gpfq_stats *stats) {
+// Walk stage of a conv layer from per-channel Gram matrices on the device (see include/gpfq.h); W / Q_out (kk, C / groups, F).
+static int conv_layer_from_gram(gpfq_ctx *ctx, const double *gram, int32_t kk, const float *W, int64_t C, int64_t F, int64_t c0,
+                                int64_t n_ch, const double *alphabets, const int32_t *K, int32_t n_alph, double *Q_out,
+                                uint32_t flags, gpfq_stats *stats, int64_t groups) {
     if (!ctx) return GPFQ_ERR_ARG;
     ctx->err.clear();
     if (stats) memset(stats, 0, sizeof(*stats));
     if (!gram || !W || !Q_out) return gpfq_fail(ctx, GPFQ_ERR_ARG, "NULL gram, W or Q_out");
     if (!(flags & GPFQ_X_DEVICE)) return gpfq_fail(ctx, GPFQ_ERR_ARG, "gram must be a device pointer (GPFQ_X_DEVICE)");
     if (C < 1 || F < 1 || c0 < 0 || n_ch < 0 || c0 + n_ch > C) return gpfq_fail(ctx, GPFQ_ERR_ARG, "bad channel range");
+    if (groups < 1 || C % groups || F % groups)
+        return gpfq_fail(ctx, GPFQ_ERR_ARG, "bad groups=%lld for C=%lld, F=%lld", (long long)groups, (long long)C, (long long)F);
     if (!conv_supported_kk(kk)) return gpfq_fail(ctx, GPFQ_ERR_UNSUPPORTED, "kernel size kk=%d has no walk kernel", kk);
     if (n_ch == 0) return GPFQ_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
@@ -1107,16 +1166,30 @@ extern "C" int gpfq_conv_layer_from_gram(gpfq_ctx *ctx, const double *gram, int3
     CUDA_TRY(ctx, gpfq_record(ctx, 5, s));
     CUDA_TRY(ctx, gpfq_record(ctx, 2, s));
     CUDA_TRY(ctx, gpfq_record(ctx, 3, s));
-    GPFQ_TRY(conv_finish(ctx, kk, nullptr, (int)n_ch, 0, false, W, C, F, c0, al, n_alph, Q_out, flags, const_cast<double *>(gram)));
+    GPFQ_TRY(conv_finish(ctx, kk, nullptr, (int)n_ch, 0, false, W, C, F, c0, al, n_alph, Q_out, flags, const_cast<double *>(gram),
+                         groups));
     CUDA_TRY(ctx, gpfq_record(ctx, 1, s));
     gpfq_stats local = {};
     gpfq_stats *st = stats ? stats : &local;
-    st->weights = (int64_t)kk * n_ch * F * n_alph;
+    st->weights = (int64_t)kk * n_ch * (F / groups) * n_alph;
     st->method = GPFQ_METHOD_GRAM >> 4;
     const bool synced = !(flags & GPFQ_NO_SYNC);
     if (synced) CUDA_TRY(ctx, cudaStreamSynchronize(s));
     end_call(ctx, st, synced);
     return GPFQ_OK;
+}
+
+extern "C" int gpfq_conv_layer_from_gram(gpfq_ctx *ctx, const double *gram, int32_t kk, const float *W, int64_t C, int64_t F,
+                                         int64_t c0, int64_t n_ch, const double *alphabets, const int32_t *K, int32_t n_alph,
+                                         double *Q_out, uint32_t flags, gpfq_stats *stats) {
+    return conv_layer_from_gram(ctx, gram, kk, W, C, F, c0, n_ch, alphabets, K, n_alph, Q_out, flags, stats, 1);
+}
+
+extern "C" int gpfq_conv_layer_from_gram_grouped(gpfq_ctx *ctx, const double *gram, int32_t kk, const float *W, int64_t C,
+                                                 int64_t F, int64_t c0, int64_t n_ch, const double *alphabets, const int32_t *K,
+                                                 int32_t n_alph, double *Q_out, uint32_t flags, gpfq_stats *stats,
+                                                 int32_t groups) {
+    return conv_layer_from_gram(ctx, gram, kk, W, C, F, c0, n_ch, alphabets, K, n_alph, Q_out, flags, stats, groups);
 }
 
 static int round_elements(gpfq_ctx *ctx, const void *W, int is_f64, int64_t n, const double *alphabet, int32_t K,

@@ -722,12 +722,20 @@ __global__ void conv_finalize_kernel(const double *__restrict__ partial, int n_c
 }
 
 // ---- stage 3 ---------------------------------------------------------------------------------
-// One thread per (channel, filter, alphabet).  W/Q tap stride CF = C*F; channel c at offset c*F.
-template <int KK>
+// One thread per (channel, filter, alphabet).  W/Q tap stride CF = Cg*F, where a group of Cg = C / groups input channels
+// feeds Fg = F / groups filters.  Ungrouped (Cg = C, Fg = F): channel c, filter f at c*F + f.  GROUPED: channel c walks only
+// the Fg filters of its group g = c / Cg, filter f < Fg at (c % Cg)*F + g*Fg + f -- the (kh, kw, C / groups, F) kernel of a
+// grouped Conv2D, indexed in place.
+template <bool GROUPED>
+__device__ __forceinline__ int64_t conv_wq_offset(int64_t c, int64_t f, int64_t F, int64_t Cg, int64_t Fg) {
+    return GROUPED ? (c % Cg) * F + (c / Cg) * Fg + f : c * F + f;
+}
+
+template <int KK, bool GROUPED>
 __global__ void __launch_bounds__(128)
 conv_sweep_kernel(const double *__restrict__ gram, const float *__restrict__ W, double *__restrict__ Q,
                   int64_t CF, int64_t F, int64_t c0, const double *__restrict__ alphabets,
-                  const int *__restrict__ Koff, const int *__restrict__ Flags, int64_t q_alph_stride) {
+                  const int *__restrict__ Koff, const int *__restrict__ Flags, int64_t q_alph_stride, int64_t Cg, int64_t Fg) {
     __shared__ double g1[KK * KK], g2[KK * KK], nrm[KK], alph[GPFQ_MAX_K];
     const int ch = blockIdx.y, a = blockIdx.z;
     const int K = Koff[a + 1] - Koff[a];
@@ -741,8 +749,8 @@ conv_sweep_kernel(const double *__restrict__ gram, const float *__restrict__ W, 
     __syncthreads();
     const double inv_step = gpfq_inv_step(alph, K, Flags[a]);
     const int64_t f = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (f >= F) return;
-    const int64_t base = (c0 + ch) * F + f;
+    if (f >= (GROUPED ? Fg : F)) return;
+    const int64_t base = conv_wq_offset<GROUPED>(c0 + ch, f, F, Cg, Fg);
     double w[KK], q[KK];
 #pragma unroll
     for (int t = 0; t < KK; ++t) w[t] = (double)W[(int64_t)t * CF + base];
@@ -768,10 +776,11 @@ constexpr int MAXW = 16;  // warps (filters) per CTA
 __host__ __device__ constexpr int col_off(int s, int kk) { return s * kk - s * (s - 1) / 2; }
 }  // namespace walkx
 
+template <bool GROUPED>
 __global__ void __launch_bounds__(walkx::MAXW * 32)
 conv_walkx_kernel(const double *__restrict__ gram, int kk, const float *__restrict__ W, double *__restrict__ Q, int64_t CF,
                   int64_t F, int64_t c0, const double *__restrict__ alphabets, const int *__restrict__ Koff,
-                  const int *__restrict__ Flags, int64_t q_alph_stride) {
+                  const int *__restrict__ Flags, int64_t q_alph_stride, int64_t Cg, int64_t Fg) {
     extern __shared__ double walkx_smem[];
     const int tri = kk * (kk + 1) / 2;
     double *g1 = walkx_smem, *g2 = g1 + tri, *nrm = g2 + tri, *alph = nrm + kk;
@@ -792,8 +801,8 @@ conv_walkx_kernel(const double *__restrict__ gram, int kk, const float *__restri
     const double inv_step = gpfq_inv_step(alph, K, Flags[a]);
     const int lane = threadIdx.x & 31;
     const int64_t f = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    if (f >= F) return;
-    const int64_t base = (c0 + ch) * F + f;
+    if (f >= (GROUPED ? Fg : F)) return;
+    const int64_t base = conv_wq_offset<GROUPED>(c0 + ch, f, F, Cg, Fg);
     double *q_out = Q + (int64_t)a * q_alph_stride + base;
     double w[4], d[4];
 #pragma unroll
@@ -973,23 +982,38 @@ int conv_finalize_stage(gpfq_ctx *ctx, const double *partial, int n_ch, int n_ch
     return GPFQ_OK;
 }
 
+// W / Q: (kk, C / groups, F); channels c0 .. c0+n_ch-1 walk the F / groups filters of their group (groups = 1: all F).
 int conv_sweep_stage(gpfq_ctx *ctx, int kk, const double *gram, const float *W, double *Q, int64_t C,
                      int64_t F, int64_t c0, int n_ch, const double *d_alph, const int *d_koff, const int *d_flags,
-                     int n_alph) {
-    dim3 grid((unsigned)ceil_div64(F, 128), (unsigned)n_ch, (unsigned)n_alph);
-    const int64_t CF = C * F, qs = (int64_t)kk * CF;
-#define SWEEP_CASE(KKV) \
-    case KKV: conv_sweep_kernel<KKV><<<grid, 128, 0, ctx->stream>>>(gram, W, Q, CF, F, c0, d_alph, d_koff, d_flags, qs); break;
+                     int n_alph, int64_t groups) {
+    const int64_t Cg = C / groups, Fg = F / groups;
+    const bool grouped = groups > 1;
+    dim3 grid((unsigned)ceil_div64(Fg, 128), (unsigned)n_ch, (unsigned)n_alph);
+    const int64_t CF = Cg * F, qs = (int64_t)kk * CF;
+#define SWEEP_CASE(KKV)                                                                                                 \
+    case KKV:                                                                                                           \
+        if (grouped)                                                                                                    \
+            conv_sweep_kernel<KKV, true><<<grid, 128, 0, ctx->stream>>>(gram, W, Q, CF, F, c0, d_alph, d_koff, d_flags, qs, Cg, Fg); \
+        else                                                                                                            \
+            conv_sweep_kernel<KKV, false><<<grid, 128, 0, ctx->stream>>>(gram, W, Q, CF, F, c0, d_alph, d_koff, d_flags, qs, Cg, Fg); \
+        break;
     switch (kk) {
         SWEEP_CASE(1) SWEEP_CASE(2) SWEEP_CASE(3) SWEEP_CASE(4) SWEEP_CASE(6) SWEEP_CASE(9)
         default: {
             if (!conv_supported_kk(kk)) return gpfq_fail(ctx, GPFQ_ERR_UNSUPPORTED, "conv kernel size kk=%d has no walk kernel", kk);
             using namespace walkx;
-            const int warps = F < MAXW ? (int)F : MAXW;
+            const int warps = Fg < MAXW ? (int)Fg : MAXW;
             const size_t smem = ((size_t)kk * (kk + 1) + kk + GPFQ_MAX_K) * sizeof(double);
-            CUDA_TRY(ctx, cudaFuncSetAttribute(conv_walkx_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            dim3 wgrid((unsigned)ceil_div64(F, warps), (unsigned)n_ch, (unsigned)n_alph);
-            conv_walkx_kernel<<<wgrid, warps * 32, smem, ctx->stream>>>(gram, kk, W, Q, CF, F, c0, d_alph, d_koff, d_flags, qs);
+            dim3 wgrid((unsigned)ceil_div64(Fg, warps), (unsigned)n_ch, (unsigned)n_alph);
+            if (grouped) {
+                CUDA_TRY(ctx, cudaFuncSetAttribute(conv_walkx_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+                conv_walkx_kernel<true><<<wgrid, warps * 32, smem, ctx->stream>>>(gram, kk, W, Q, CF, F, c0, d_alph, d_koff, d_flags,
+                                                                                 qs, Cg, Fg);
+            } else {
+                CUDA_TRY(ctx, cudaFuncSetAttribute(conv_walkx_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+                conv_walkx_kernel<false><<<wgrid, warps * 32, smem, ctx->stream>>>(gram, kk, W, Q, CF, F, c0, d_alph, d_koff, d_flags,
+                                                                                  qs, Cg, Fg);
+            }
         }
     }
 #undef SWEEP_CASE

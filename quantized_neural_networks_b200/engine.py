@@ -316,9 +316,20 @@ class GpfqEngine:
         self.last_stats = st.as_dict()
         return out[0] if single else out
 
+    @staticmethod
+    def _check_groups(groups, C, Cg, F):
+        """A grouped kernel is (kh, kw, C / groups, F) and F is a multiple of groups."""
+        groups = int(groups)
+        if groups < 1 or Cg * groups != C or F % groups:
+            raise ValueError(f"groups={groups} does not fit {C} input channels, a kernel with {Cg} input channels and {F} filters "
+                             "(need C == W.shape[2] * groups and F % groups == 0)")
+        return groups
+
     def conv_layer_nhwc(self, act, actq, W, alphabets, strides=(1, 1), padding="SAME", rate=(1, 1), c0=0,
-                        n_channels=None, out=None, sync=True):
-        """Quantize a Conv2D kernel straight from the NHWC activations (on-device patch extraction)."""
+                        n_channels=None, out=None, sync=True, groups=1):
+        """Quantize a Conv2D kernel straight from the NHWC activations (on-device patch extraction).  With `groups` > 1, W is the
+        (kh, kw, C / groups, F) kernel of a grouped Conv2D: input channel c is walked against the F / groups filters of its group
+        c // (C / groups); c0 / n_channels index input channels.  The result has W's shape."""
         flat, K, n_alph, als = _alph_args(alphabets)
         single = isinstance(alphabets, np.ndarray) and alphabets.ndim == 1
         W = self._f32(W, "W")
@@ -334,10 +345,13 @@ class GpfqEngine:
             W = np.ascontiguousarray(W)
         elif not (act.is_contiguous() and actq.is_contiguous() and W.is_contiguous()):
             raise ValueError("device tensors must be contiguous")
-        kh, kw, C, F = (int(v) for v in W.shape)
-        n_img, H, Wd, Ca = (int(v) for v in act.shape)
-        if Ca != C or tuple(actq.shape) != tuple(act.shape):
+        kh, kw, Cg, F = (int(v) for v in W.shape)
+        n_img, H, Wd, C = (int(v) for v in act.shape)
+        if tuple(actq.shape) != tuple(act.shape):
             raise ValueError("activation / kernel channel mismatch")
+        if groups == 1 and Cg != C:
+            raise ValueError("activation / kernel channel mismatch")
+        groups = self._check_groups(groups, C, Cg, F)
         n_channels = (C - c0) if n_channels is None else int(n_channels)
         rate = tuple(rate) if rate else (1, 1)
         ptr = (lambda t: t.data_ptr()) if dev else (lambda t: t.ctypes.data)
@@ -346,20 +360,20 @@ class GpfqEngine:
         if dev:
             flags |= _lib.ALL_DEVICE
             if out is None:
-                out = torch.zeros((n_alph, kh, kw, C, F), dtype=torch.float64, device=W.device)
+                out = torch.zeros((n_alph, kh, kw, Cg, F), dtype=torch.float64, device=W.device)
             pout = out.data_ptr()
             if not sync:
                 flags |= _lib.NO_SYNC
         else:
             if out is None:
-                out = np.zeros((n_alph, kh, kw, C, F), dtype=np.float64)
+                out = np.zeros((n_alph, kh, kw, Cg, F), dtype=np.float64)
             pout = out.ctypes.data
         st = _lib.GpfqStats()
-        rc = self._lib.gpfq_conv_layer_nhwc(self._ctx, c_void_p(ptr(act)), c_void_p(ptr(actq)), n_img, H, Wd, C, kh, kw,
-                                            int(strides[0]), int(strides[1]), int(rate[0]), int(rate[1]),
-                                            1 if str(padding).upper() == "SAME" else 0, c_void_p(ptr(W)), F, int(c0),
-                                            n_channels, flat.ctypes.data_as(POINTER(c_double)),
-                                            K.ctypes.data_as(POINTER(c_int32)), n_alph, c_void_p(pout), flags, byref(st))
+        args = (self._ctx, c_void_p(ptr(act)), c_void_p(ptr(actq)), n_img, H, Wd, C, kh, kw, int(strides[0]), int(strides[1]),
+                int(rate[0]), int(rate[1]), 1 if str(padding).upper() == "SAME" else 0, c_void_p(ptr(W)), F, int(c0), n_channels,
+                flat.ctypes.data_as(POINTER(c_double)), K.ctypes.data_as(POINTER(c_int32)), n_alph, c_void_p(pout), flags,
+                byref(st))
+        rc = (self._lib.gpfq_conv_layer_nhwc_grouped(*args, groups) if groups > 1 else self._lib.gpfq_conv_layer_nhwc(*args))
         self._check(rc)
         self.last_stats = st.as_dict()
         return out[0] if single else out
@@ -400,16 +414,20 @@ class GpfqEngine:
         self.last_stats = self.query_stats(0)
         return gram
 
-    def conv_layer_from_gram(self, gram, W, alphabets, c0=0, n_channels=None, out=None, sync=True):
+    def conv_layer_from_gram(self, gram, W, alphabets, c0=0, n_channels=None, out=None, sync=True, groups=1):
         """Walks of every filter of channels c0..c0+n_channels-1 from per-channel Gram matrices on the device
-        (`conv_gram_nhwc`, summed over the ranks of an image-split job).  W: (kh, kw, C, F) NumPy array or CUDA tensor."""
+        (`conv_gram_nhwc`, summed over the ranks of an image-split job).  W: (kh, kw, C, F) NumPy array or CUDA tensor; with
+        `groups` > 1 the (kh, kw, C / groups, F) kernel of a grouped Conv2D, each input channel walked against the F / groups
+        filters of its group (c0 / n_channels index input channels, as in the Gram stage)."""
         flat, K, n_alph, als = _alph_args(alphabets)
         single = isinstance(alphabets, np.ndarray) and alphabets.ndim == 1
         W = self._f32(W, "W")
         wdev = _is_torch(W)
         W = W.contiguous() if wdev else np.ascontiguousarray(W)
-        kh, kw, C, F = (int(v) for v in W.shape)
+        kh, kw, Cg, F = (int(v) for v in W.shape)
         kk = kh * kw
+        C = Cg * int(groups)
+        groups = self._check_groups(groups, C, Cg, F)
         n_channels = (C - c0) if n_channels is None else int(n_channels)
         if (not _is_torch(gram) or gram.dtype != torch.float64 or not gram.is_cuda or not gram.is_contiguous()
                 or gram.numel() != n_channels * 2 * kk * kk):
@@ -419,18 +437,19 @@ class GpfqEngine:
         if wdev:
             flags |= _lib.W_DEVICE | _lib.Q_DEVICE
             if out is None:
-                out = torch.zeros((n_alph, kh, kw, C, F), dtype=torch.float64, device=W.device)
+                out = torch.zeros((n_alph, kh, kw, Cg, F), dtype=torch.float64, device=W.device)
             pout, pw = out.data_ptr(), W.data_ptr()
             if not sync:
                 flags |= _lib.NO_SYNC
         else:
             if out is None:
-                out = np.zeros((n_alph, kh, kw, C, F), dtype=np.float64)
+                out = np.zeros((n_alph, kh, kw, Cg, F), dtype=np.float64)
             pout, pw = out.ctypes.data, W.ctypes.data
         st = _lib.GpfqStats()
-        rc = self._lib.gpfq_conv_layer_from_gram(self._ctx, c_void_p(gram.data_ptr()), kk, c_void_p(pw), C, F, int(c0),
-                                                 n_channels, flat.ctypes.data_as(POINTER(c_double)),
-                                                 K.ctypes.data_as(POINTER(c_int32)), n_alph, c_void_p(pout), flags, byref(st))
+        args = (self._ctx, c_void_p(gram.data_ptr()), kk, c_void_p(pw), C, F, int(c0), n_channels,
+                flat.ctypes.data_as(POINTER(c_double)), K.ctypes.data_as(POINTER(c_int32)), n_alph, c_void_p(pout), flags, byref(st))
+        rc = (self._lib.gpfq_conv_layer_from_gram_grouped(*args, groups) if groups > 1
+              else self._lib.gpfq_conv_layer_from_gram(*args))
         self._check(rc)
         self.last_stats = st.as_dict()
         return out[0] if single else out

@@ -110,7 +110,9 @@ class QuantizedCNNGrid:
                     Q = eng.dense_layer(Xd, Xqd, Wd, A)
                 else:
                     rate = getattr(layer, "dilation_rate", None)
-                    Q = eng.conv_layer_nhwc(Xd, Xqd, Wd, A, strides=layer.strides, padding=layer.padding.upper(), rate=rate)
+                    groups = int(getattr(layer, "groups", 1)) if kind == "Conv2D" else 1
+                    Q = eng.conv_layer_nhwc(Xd, Xqd, Wd, A, strides=layer.strides, padding=layer.padding.upper(), rate=rate,
+                                            **({"groups": groups} if groups > 1 else {}))
                 Q = Q.cpu().numpy()
                 for a, g in enumerate(members):
                     Qs[g] = Q[a]

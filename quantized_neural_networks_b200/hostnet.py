@@ -173,8 +173,11 @@ def extract_patches(images, sizes, strides, rates, padding):
 
 class Conv2D(Layer):
     def __init__(self, filters, kernel_size, strides=(1, 1), padding="valid", dilation_rate=(1, 1), activation=None,
-                 use_bias=True, kernel_initializer="he_uniform", **kw):
+                 use_bias=True, kernel_initializer="he_uniform", groups=1, **kw):
         super().__init__(kw.get("name"), kw.get("input_shape"))
+        # Keras' `groups`: input channels and filters split into `groups` groups, filters of group g see only the input channels
+        # of group g; the kernel is (kh, kw, c_in // groups, filters)
+        self.groups = int(groups)
         ks = (kernel_size, kernel_size) if np.isscalar(kernel_size) else tuple(kernel_size)
         self.filters, self.kernel_size = int(filters), (int(ks[0]), int(ks[1]))
         self.strides = (strides, strides) if np.isscalar(strides) else tuple(strides)
@@ -183,12 +186,14 @@ class Conv2D(Layer):
         self.kernel_initializer = kernel_initializer
 
     def _kernel_shape(self, c_in):
-        return (*self.kernel_size, c_in, self.filters)
+        if c_in % self.groups or self.filters % self.groups:
+            raise ValueError(f"groups={self.groups} must divide the {c_in} input channels and the {self.filters} filters")
+        return (*self.kernel_size, c_in // self.groups, self.filters)
 
     def build(self, in_shape, rng):
         c_in = int(in_shape[-1])
         shape = self._kernel_shape(c_in)
-        fan_in = self.kernel_size[0] * self.kernel_size[1] * c_in
+        fan_in = self.kernel_size[0] * self.kernel_size[1] * shape[2]
         k = _he(rng, shape, fan_in) if self.kernel_initializer == "he_uniform" else \
             _glorot(rng, shape, fan_in, self.kernel_size[0] * self.kernel_size[1] * self.filters)
         n_out = self._n_out(c_in)
@@ -214,8 +219,14 @@ class Conv2D(Layer):
 
     def call(self, x):
         p = self._patches(x)                                   # (n, Ho, Wo, kh*kw*C)
-        k = self.weights[0].reshape(-1, self.weights[0].shape[-1])  # (kh*kw*C, F)
-        y = p.reshape(-1, p.shape[-1]) @ k
+        if self.groups == 1:
+            k = self.weights[0].reshape(-1, self.weights[0].shape[-1])  # (kh*kw*C, F)
+            y = p.reshape(-1, p.shape[-1]) @ k
+        else:
+            kk, G = self.kernel_size[0] * self.kernel_size[1], self.groups
+            Cg, F = self.weights[0].shape[2:]
+            k = self.weights[0].reshape(kk, Cg, G, F // G)     # filter g*Fg + f of group g
+            y = np.einsum("ptgc,tcgf->pgf", p.reshape(-1, kk, G, Cg), k).reshape(-1, F)
         y = y.reshape(*p.shape[:3], -1)
         if self.use_bias:
             y = y + self.weights[1]

@@ -398,8 +398,14 @@ class QuantizedCNN(QuantizedNeuralNetwork):
         rate = getattr(layer, "dilation_rate", None)
         W = layer.get_weights()[0]
         alphabet = self._layer_alphabet(W)
-        num_channels = W.shape[-2]
-        lo, hi = shard_range(num_channels, *self.shard)
+        # a grouped Conv2D has a (kh, kw, C / groups, F) kernel: input channel c meets only the Fg filters of its group c // Cg,
+        # so ranks take whole groups and gather their filters (groups == 1: channels, all filters)
+        groups = int(getattr(layer, "groups", 1)) if layer.__class__.__name__ == "Conv2D" else 1
+        grouped = {"groups": groups} if groups > 1 else {}   # the ungrouped call keeps its signature
+        Cg, Fg = W.shape[-2], W.shape[-1] // groups
+        num_channels = Cg * groups
+        unit = Cg if groups > 1 else 1
+        lo, hi = (u * unit for u in shard_range(num_channels // unit, *self.shard))
         tic = time()
         if self.conv_path == "nhwc":
             try:
@@ -410,7 +416,8 @@ class QuantizedCNN(QuantizedNeuralNetwork):
                     gram = image_split_conv_gram(self.engine, data.wX, None if data.same else data.qX, W.shape[:2],
                                                  layer.strides, layer.padding.upper(), rate, *self.shard)
                     self.layer_stats[layer_idx] = dict(self.engine.last_stats)
-                    Q = self.engine.conv_layer_from_gram(gram, np.ascontiguousarray(W), np.asarray(alphabet, dtype=np.float64))
+                    Q = self.engine.conv_layer_from_gram(gram, np.ascontiguousarray(W), np.asarray(alphabet, dtype=np.float64),
+                                                         **grouped)
                     lo, hi = 0, num_channels
                 elif self._nccl_job():
                     import torch
@@ -418,11 +425,12 @@ class QuantizedCNN(QuantizedNeuralNetwork):
                     Wd = torch.from_numpy(np.ascontiguousarray(W)).to(Ad.device)
                     Q = self.engine.conv_layer_nhwc(Ad, Aqd, Wd, np.asarray(alphabet, dtype=np.float64), strides=layer.strides,
                                                     padding=layer.padding.upper(), rate=rate, c0=lo,
-                                                    n_channels=hi - lo).cpu().numpy()
+                                                    n_channels=hi - lo, **grouped).cpu().numpy()
                 else:
                     Q = self.engine.conv_layer_nhwc(data.wX, None if data.same else data.qX, np.ascontiguousarray(W),
                                                     np.asarray(alphabet, dtype=np.float64), strides=layer.strides,
-                                                    padding=layer.padding.upper(), rate=rate, c0=lo, n_channels=hi - lo)
+                                                    padding=layer.padding.upper(), rate=rate, c0=lo, n_channels=hi - lo,
+                                                    **grouped)
             except Exception as exc:
                 self._log(f"\t\tChannels {lo}:{hi} generated an exception: {exc}")
                 raise exc
@@ -430,10 +438,14 @@ class QuantizedCNN(QuantizedNeuralNetwork):
         else:
             Q = zeros(W.shape)
             for channel_idx in range(lo, hi):
-                Q[:, :, channel_idx, :] = self._quantize_channel_parallel_jit(
-                    channel_idx, W[:, :, channel_idx, :], data, strides=layer.strides, padding=layer.padding.upper(),
+                ci, f0 = channel_idx % Cg, (channel_idx // Cg) * Fg   # the channel's kernel slice and its group's filters
+                Q[:, :, ci, f0:f0 + Fg] = self._quantize_channel_parallel_jit(
+                    channel_idx, W[:, :, ci, f0:f0 + Fg], data, strides=layer.strides, padding=layer.padding.upper(),
                     rate=rate, alphabet=alphabet, patch_mini_batch_size=self.patch_mini_batch_size)
-        if (lo, hi) != (0, num_channels):
+        if (lo, hi) != (0, num_channels) and groups > 1:
+            # this rank wrote the filters of groups lo / Cg .. hi / Cg: gather along the group axis of (kh, kw, Cg, groups, Fg)
+            Q = self._gather_columns(Q.reshape(*Q.shape[:3], groups, Fg), lo // Cg, hi // Cg, axis=3).reshape(W.shape)
+        elif (lo, hi) != (0, num_channels):
             Q = self._gather_columns(Q, lo, hi, axis=2)
         self._log(f"\t\t{num_channels} channels x {W.shape[-1]} filters quantized in {time()-tic:.2f} seconds.")
         self._update_weights(layer_idx, Q)
