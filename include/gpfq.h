@@ -220,6 +220,43 @@ int gpfq_conv_layer_from_gram_grouped(gpfq_ctx *ctx, const double *gram, int32_t
                                       int64_t c0, int64_t n_channels, const double *alphabets, const int32_t *K,
                                       int32_t n_alphabets, double *Q_out, uint32_t flags, gpfq_stats *stats, int32_t groups);
 
+/* ---- per-channel alphabets --------------------------------------------------------------------------------------------------
+ * The counterparts of the entry points above with one scale per unit: unit u (a Dense neuron, or the kernel slice W[:, :, ci, f] of
+ * a conv layer, ci < Cw = C / groups) walks with the levels fl64(s_u * alphabet[k]) -- one correctly rounded product per level,
+ * what NumPy's `rad_u * alphabet` gives for a scalar rad_u -- instead of the alphabet itself.  Every decision and guard is the
+ * reference's, taken with the unit's own levels; the outputs are those levels, or the literal 0 of a dead direction.  s_u = 0 gives
+ * the unit an all-zero Q.  `scales` is HOST memory, like the alphabets: every scale a call reads must be finite and >= 0
+ * (GPFQ_ERR_ARG otherwise, before any work); GPFQ_NO_SYNC all-device calls stay asynchronous.
+ *   Dense:  scales[a * N1 + j] for the global neuron j (a shard j0..j1 reads its own slice).
+ *   Conv:   scales[a * Cw * F + ci * F + f]; groups as in the _grouped entry points (1 = ungrouped; gpfq_conv_channels: C = Cw).
+ *   MSQ:    element i of W rounds with scales[i % n_units] (n_units >= 1: the last axis of a Dense or conv kernel, or its (Cw, F)).
+ * A scaled call runs the kernels its per-layer counterpart runs (the tensor-core walk and the int8 residual form apply each neuron's
+ * own level step; stats.reserved reports them as for per-layer calls).
+ */
+int gpfq_dense_layer_scaled(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ldx, int64_t N0, int64_t m, const float *W,
+                            int64_t ldw, int64_t N1, int64_t j0, int64_t j1, const double *alphabets, const int32_t *K,
+                            int32_t n_alphabets, double *Q_out, int64_t ldq, uint32_t flags, gpfq_stats *stats,
+                            const double *scales);
+int gpfq_dense_layer_from_gram_scaled(gpfq_ctx *ctx, const double *G1, const double *G2, int64_t N0, const float *W, int64_t ldw,
+                                      int64_t N1, int64_t j0, int64_t j1, const double *alphabets, const int32_t *K,
+                                      int32_t n_alphabets, double *Q_out, int64_t ldq, uint32_t flags, gpfq_stats *stats,
+                                      const double *scales);
+int gpfq_conv_channels_scaled(gpfq_ctx *ctx, const float *const *Xp, const float *const *Xqp, int64_t n_patches, int32_t kk,
+                              const float *W, int64_t C, int64_t F, int64_t c0, int64_t n_channels, const double *alphabets,
+                              const int32_t *K, int32_t n_alphabets, double *Q_out, uint32_t flags, gpfq_stats *stats,
+                              const double *scales);
+int gpfq_conv_layer_nhwc_scaled(gpfq_ctx *ctx, const float *act, const float *actq, int64_t n_img, int64_t H, int64_t Wd,
+                                int64_t C, int32_t kh, int32_t kw, int32_t stride_h, int32_t stride_w, int32_t rate_h,
+                                int32_t rate_w, int32_t padding_same, const float *W, int64_t F, int64_t c0, int64_t n_channels,
+                                const double *alphabets, const int32_t *K, int32_t n_alphabets, double *Q_out, uint32_t flags,
+                                gpfq_stats *stats, int32_t groups, const double *scales);
+int gpfq_conv_layer_from_gram_scaled(gpfq_ctx *ctx, const double *gram, int32_t kk, const float *W, int64_t C, int64_t F,
+                                     int64_t c0, int64_t n_channels, const double *alphabets, const int32_t *K,
+                                     int32_t n_alphabets, double *Q_out, uint32_t flags, gpfq_stats *stats, int32_t groups,
+                                     const double *scales);
+int gpfq_msq_scaled(gpfq_ctx *ctx, const float *W, int64_t n, const double *alphabet, int32_t K, const double *scales,
+                    int64_t n_units, double *Q_out, uint32_t flags);
+
 /* ---- MSQ baseline ---------------------------------------------------------------------------
  * Plain nearest-level rounding of every weight (_bit_round_parallel :40-57 applied elementwise,
  * as in quantize_pretrained_mlp.py:97-117).  n elements, contiguous. */

@@ -76,7 +76,25 @@ EXPORTS = {
     "gpfq_conv_layer_from_gram_grouped": (c_int, [c_void_p, c_void_p, c_int32, c_void_p, c_int64, c_int64, c_int64, c_int64,
                                                   POINTER(c_double), POINTER(c_int32), c_int32, c_void_p, c_uint32,
                                                   POINTER(GpfqStats), c_int32]),
+    "gpfq_dense_layer_scaled": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_int64,
+                                        c_int64, c_int64, c_int64, POINTER(c_double), POINTER(c_int32), c_int32,
+                                        c_void_p, c_int64, c_uint32, POINTER(GpfqStats), POINTER(c_double)]),
+    "gpfq_dense_layer_from_gram_scaled": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_int64, c_int64,
+                                                  c_int64, POINTER(c_double), POINTER(c_int32), c_int32, c_void_p, c_int64,
+                                                  c_uint32, POINTER(GpfqStats), POINTER(c_double)]),
+    "gpfq_conv_channels_scaled": (c_int, [c_void_p, POINTER(c_void_p), POINTER(c_void_p), c_int64, c_int32, c_void_p,
+                                          c_int64, c_int64, c_int64, c_int64, POINTER(c_double), POINTER(c_int32),
+                                          c_int32, c_void_p, c_uint32, POINTER(GpfqStats), POINTER(c_double)]),
+    "gpfq_conv_layer_nhwc_scaled": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int64, c_int64, c_int32,
+                                            c_int32, c_int32, c_int32, c_int32, c_int32, c_int32, c_void_p, c_int64,
+                                            c_int64, c_int64, POINTER(c_double), POINTER(c_int32), c_int32, c_void_p,
+                                            c_uint32, POINTER(GpfqStats), c_int32, POINTER(c_double)]),
+    "gpfq_conv_layer_from_gram_scaled": (c_int, [c_void_p, c_void_p, c_int32, c_void_p, c_int64, c_int64, c_int64, c_int64,
+                                                 POINTER(c_double), POINTER(c_int32), c_int32, c_void_p, c_uint32,
+                                                 POINTER(GpfqStats), c_int32, POINTER(c_double)]),
     "gpfq_msq": (c_int, [c_void_p, c_void_p, c_int64, POINTER(c_double), c_int32, c_void_p, c_uint32]),
+    "gpfq_msq_scaled": (c_int, [c_void_p, c_void_p, c_int64, POINTER(c_double), c_int32, POINTER(c_double), c_int64, c_void_p,
+                                c_uint32]),
     "gpfq_bit_round": (c_int, [c_void_p, c_void_p, c_int64, POINTER(c_double), c_int32, c_void_p, c_uint32]),
     "gpfq_gram_matrices": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_int64, c_int64, c_void_p, c_void_p,
                                    c_uint32]),

@@ -11,10 +11,10 @@
 // kernels / stages implemented in the other translation units
 int dense_gram_path(gpfq_ctx *, const float *, const float *, int64_t, int64_t, int64_t, const float *, int64_t,
                     int64_t, int64_t, const double *, const int *, const int *, int, double *, int64_t, int64_t,
-                    gpfq_stats *, const double *G1_pre = nullptr, const double *G2_pre = nullptr);
+                    gpfq_stats *, const double *G1_pre = nullptr, const double *G2_pre = nullptr, const double *d_scales = nullptr);
 int dense_stream_path(gpfq_ctx *, const float *, const float *, int64_t, int64_t, int64_t, const float *, int64_t,
                       int64_t, int64_t, const double *, const int *, const int *, int, double *, int64_t, int64_t,
-                      gpfq_stats *);
+                      gpfq_stats *, const double *d_scales);
 int dense_gram_only(gpfq_ctx *, const float *, const float *, int64_t, int64_t, int64_t, double *, double *);
 bool dense_gram_uses_i8(gpfq_ctx *, int64_t, int64_t, bool);
 int conv_supported_kk(int kk);
@@ -23,10 +23,10 @@ bool conv_specialised_kk(int kk);
 int conv_gram_stage(gpfq_ctx *, int, ConvPtrs, bool, int64_t, int, int, int64_t, double *, bool, int);
 int conv_finalize_stage(gpfq_ctx *, const double *, int, int, int, bool, double *);
 int conv_sweep_stage(gpfq_ctx *, int, const double *, const float *, double *, int64_t, int64_t, int64_t, int,
-                     const double *, const int *, const int *, int, int64_t);
+                     const double *, const int *, const int *, int, int64_t, const double *);
 int im2col_stage(gpfq_ctx *, const float *, int64_t, int, int, int64_t, int64_t, int, int, int, int, int, int, int,
                  int, int, int, int, float *, int64_t);
-int msq_stage(gpfq_ctx *, const void *, int, int64_t, const double *, int, int, double *);
+int msq_stage(gpfq_ctx *, const void *, int, int64_t, const double *, int, int, double *, const double *, int64_t);
 int nhwc9_plan(int, int, int, int, int, int, int, int, int *, int *);
 int corr9_plan(int, int, int, int, int, int, int, int, int, int);
 int corr9_pack_stage(gpfq_ctx *, const float *, int64_t, int, int, int64_t, int64_t, int, int, int64_t, int64_t, float *);
@@ -294,6 +294,29 @@ static int upload_alphabets(gpfq_ctx *ctx, const double *alphabets, const int32_
     return GPFQ_OK;
 }
 
+// Per-unit scales (per-channel alphabets): n_alph rows of n scales, row a read from scales + a * lds, each finite and >= 0.
+static int check_scales(gpfq_ctx *ctx, const double *scales, int n_alph, int64_t n, int64_t lds) {
+    if (!scales) return gpfq_fail(ctx, GPFQ_ERR_ARG, "NULL scales");
+    for (int a = 0; a < n_alph; ++a)
+        for (int64_t j = 0; j < n; ++j) {
+            const double v = scales[a * lds + j];
+            if (!(v >= 0.0) || !std::isfinite(v))
+                return gpfq_fail(ctx, GPFQ_ERR_ARG, "scale %lld of alphabet %d is %g (scales must be finite and >= 0)", (long long)j, a, v);
+        }
+    return GPFQ_OK;
+}
+
+// ... staged on the device as (n_alph, n) on the call's stream, like the alphabets (pageable source: staged before the call
+// returns, so GPFQ_NO_SYNC calls stay asynchronous).  The kernels of the call read them in stream order.
+static int upload_scales(gpfq_ctx *ctx, const double *scales, int n_alph, int64_t n, int64_t lds, const double **out) {
+    double *d = nullptr;
+    GPFQ_TRY(gpfq_ws(ctx, WS_SCALES, (size_t)n_alph * n * sizeof(double), (void **)&d));
+    CUDA_TRY(ctx, cudaMemcpy2DAsync(d, n * sizeof(double), scales, lds * sizeof(double), n * sizeof(double), n_alph,
+                                    cudaMemcpyHostToDevice, ctx->stream));
+    *out = d;
+    return GPFQ_OK;
+}
+
 cudaError_t gpfq_record(gpfq_ctx *ctx, int which, cudaStream_t s) {
     ctx->cur->rec[which] = true;
     return cudaEventRecord(ctx->cur->e[which], s);
@@ -379,10 +402,10 @@ static int choose_dense_method(gpfq_ctx *ctx, uint32_t flags, int64_t N0, int64_
     return t_gram < t_stream ? GPFQ_METHOD_GRAM : GPFQ_METHOD_STREAM_FAST;
 }
 
-extern "C" int gpfq_dense_layer(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ldx, int64_t N0, int64_t m,
-                                const float *W, int64_t ldw, int64_t N1, int64_t j0, int64_t j1,
-                                const double *alphabets, const int32_t *K, int32_t n_alph, double *Q_out,
-                                int64_t ldq, uint32_t flags, gpfq_stats *stats) {
+// scales (nullable, host): per-neuron scales, neuron j of alphabet a at scales[a * lds + j].
+static int dense_layer(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ldx, int64_t N0, int64_t m, const float *W,
+                       int64_t ldw, int64_t N1, int64_t j0, int64_t j1, const double *alphabets, const int32_t *K, int32_t n_alph,
+                       double *Q_out, int64_t ldq, uint32_t flags, gpfq_stats *stats, const double *scales, int64_t lds) {
     if (!ctx) return GPFQ_ERR_ARG;
     ctx->err.clear();
     if (stats) memset(stats, 0, sizeof(*stats));
@@ -395,6 +418,7 @@ extern "C" int gpfq_dense_layer(gpfq_ctx *ctx, const float *X, const float *Xq, 
     if ((flags & GPFQ_NO_SYNC) && (flags & GPFQ_ALL_DEVICE) != GPFQ_ALL_DEVICE)
         return gpfq_fail(ctx, GPFQ_ERR_ARG, "GPFQ_NO_SYNC needs all-device pointers");
     const int64_t nj = j1 - j0;
+    if (scales && n_alph >= 1) GPFQ_TRY(check_scales(ctx, scales + j0, n_alph, nj, lds));
     if (nj == 0) return GPFQ_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     const bool same = (Xq == nullptr || Xq == X);
@@ -405,6 +429,8 @@ extern "C" int gpfq_dense_layer(gpfq_ctx *ctx, const float *X, const float *Xq, 
 
     Alphabets al;
     GPFQ_TRY(upload_alphabets(ctx, alphabets, K, n_alph, &al));
+    const double *d_scales = nullptr;
+    if (scales) GPFQ_TRY(upload_scales(ctx, scales + j0, n_alph, nj, lds, &d_scales));
 
     const float *dX = X, *dXq = same ? X : Xq, *dW = W;
     int64_t dldx = ldx, dldw = ldw, dj0 = j0;
@@ -442,11 +468,11 @@ extern "C" int gpfq_dense_layer(gpfq_ctx *ctx, const float *X, const float *Xq, 
 
     if (method == GPFQ_METHOD_GRAM)
         GPFQ_TRY(dense_gram_path(ctx, dX, dXq, dldx, N0, m, dW, dldw, dj0, nj, al.d_levels, al.d_koff, al.d_flags, n_alph, dQ,
-                                 dldq, col0, stats));
+                                 dldq, col0, stats, nullptr, nullptr, d_scales));
     else {
         ctx->stream_literal = (method == GPFQ_METHOD_STREAM);
         GPFQ_TRY(dense_stream_path(ctx, dX, dXq, dldx, N0, m, dW, dldw, dj0, nj, al.d_levels, al.h_koff.data(),
-                                   al.h_flags.data(), n_alph, dQ, dldq, col0, stats));
+                                   al.h_flags.data(), n_alph, dQ, dldq, col0, stats, d_scales));
         if (stats) stats->method = method >> 4;
     }
     CUDA_TRY(ctx, gpfq_record(ctx, 6, s));
@@ -464,13 +490,27 @@ extern "C" int gpfq_dense_layer(gpfq_ctx *ctx, const float *X, const float *Xq, 
     return GPFQ_OK;
 }
 
+extern "C" int gpfq_dense_layer(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ldx, int64_t N0, int64_t m,
+                                const float *W, int64_t ldw, int64_t N1, int64_t j0, int64_t j1,
+                                const double *alphabets, const int32_t *K, int32_t n_alph, double *Q_out,
+                                int64_t ldq, uint32_t flags, gpfq_stats *stats) {
+    return dense_layer(ctx, X, Xq, ldx, N0, m, W, ldw, N1, j0, j1, alphabets, K, n_alph, Q_out, ldq, flags, stats, nullptr, 0);
+}
+
+extern "C" int gpfq_dense_layer_scaled(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ldx, int64_t N0, int64_t m,
+                                       const float *W, int64_t ldw, int64_t N1, int64_t j0, int64_t j1,
+                                       const double *alphabets, const int32_t *K, int32_t n_alph, double *Q_out,
+                                       int64_t ldq, uint32_t flags, gpfq_stats *stats, const double *scales) {
+    if (ctx && !scales) return gpfq_fail(ctx, GPFQ_ERR_ARG, "NULL scales");
+    return dense_layer(ctx, X, Xq, ldx, N0, m, W, ldw, N1, j0, j1, alphabets, K, n_alph, Q_out, ldq, flags, stats, scales, N1);
+}
+
 // Sweep stage alone, from Gram matrices the caller already holds on the device (sample-split Gram stage of a multi-GPU
 // job: every rank contracts its m / world samples with gpfq_gram_matrices, the (N0, N0) partial Grams are summed with
 // one NCCL all-reduce, then each rank sweeps its own neurons from the summed matrices).
-extern "C" int gpfq_dense_layer_from_gram(gpfq_ctx *ctx, const double *G1, const double *G2, int64_t N0, const float *W,
-                                          int64_t ldw, int64_t N1, int64_t j0, int64_t j1, const double *alphabets,
-                                          const int32_t *K, int32_t n_alph, double *Q_out, int64_t ldq, uint32_t flags,
-                                          gpfq_stats *stats) {
+static int dense_layer_from_gram(gpfq_ctx *ctx, const double *G1, const double *G2, int64_t N0, const float *W, int64_t ldw,
+                                 int64_t N1, int64_t j0, int64_t j1, const double *alphabets, const int32_t *K, int32_t n_alph,
+                                 double *Q_out, int64_t ldq, uint32_t flags, gpfq_stats *stats, const double *scales) {
     if (!ctx) return GPFQ_ERR_ARG;
     ctx->err.clear();
     if (stats) memset(stats, 0, sizeof(*stats));
@@ -482,6 +522,7 @@ extern "C" int gpfq_dense_layer_from_gram(gpfq_ctx *ctx, const double *G1, const
     if ((flags & GPFQ_NO_SYNC) && (flags & GPFQ_ALL_DEVICE) != GPFQ_ALL_DEVICE)
         return gpfq_fail(ctx, GPFQ_ERR_ARG, "GPFQ_NO_SYNC needs all-device pointers");
     const int64_t nj = j1 - j0;
+    if (scales && n_alph >= 1) GPFQ_TRY(check_scales(ctx, scales + j0, n_alph, nj, N1));
     if (nj == 0) return GPFQ_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     cudaStream_t s = ctx->stream;
@@ -489,6 +530,8 @@ extern "C" int gpfq_dense_layer_from_gram(gpfq_ctx *ctx, const double *G1, const
     CUDA_TRY(ctx, gpfq_record(ctx, 0, s));
     Alphabets al;
     GPFQ_TRY(upload_alphabets(ctx, alphabets, K, n_alph, &al));
+    const double *d_scales = nullptr;
+    if (scales) GPFQ_TRY(upload_scales(ctx, scales + j0, n_alph, nj, N1, &d_scales));
     const float *dW = W;
     int64_t dldw = ldw, dj0 = j0;
     if (!(flags & GPFQ_W_DEVICE)) {
@@ -509,7 +552,7 @@ extern "C" int gpfq_dense_layer_from_gram(gpfq_ctx *ctx, const double *G1, const
     }
     CUDA_TRY(ctx, gpfq_record(ctx, 5, s));
     GPFQ_TRY(dense_gram_path(ctx, nullptr, nullptr, 0, N0, 0, dW, dldw, dj0, nj, al.d_levels, al.d_koff, al.d_flags, n_alph,
-                             dQ, dldq, col0, stats, (G1 == nullptr || G1 == G2) ? nullptr : G1, G2));
+                             dQ, dldq, col0, stats, (G1 == nullptr || G1 == G2) ? nullptr : G1, G2, d_scales));
     CUDA_TRY(ctx, gpfq_record(ctx, 6, s));
     if (!(flags & GPFQ_Q_DEVICE)) {
         for (int a = 0; a < n_alph; ++a)
@@ -523,6 +566,21 @@ extern "C" int gpfq_dense_layer_from_gram(gpfq_ctx *ctx, const double *G1, const
     if (synced) CUDA_TRY(ctx, cudaStreamSynchronize(s));
     end_call(ctx, stats, synced);
     return GPFQ_OK;
+}
+
+extern "C" int gpfq_dense_layer_from_gram(gpfq_ctx *ctx, const double *G1, const double *G2, int64_t N0, const float *W,
+                                          int64_t ldw, int64_t N1, int64_t j0, int64_t j1, const double *alphabets,
+                                          const int32_t *K, int32_t n_alph, double *Q_out, int64_t ldq, uint32_t flags,
+                                          gpfq_stats *stats) {
+    return dense_layer_from_gram(ctx, G1, G2, N0, W, ldw, N1, j0, j1, alphabets, K, n_alph, Q_out, ldq, flags, stats, nullptr);
+}
+
+extern "C" int gpfq_dense_layer_from_gram_scaled(gpfq_ctx *ctx, const double *G1, const double *G2, int64_t N0, const float *W,
+                                                 int64_t ldw, int64_t N1, int64_t j0, int64_t j1, const double *alphabets,
+                                                 const int32_t *K, int32_t n_alph, double *Q_out, int64_t ldq, uint32_t flags,
+                                                 gpfq_stats *stats, const double *scales) {
+    if (ctx && !scales) return gpfq_fail(ctx, GPFQ_ERR_ARG, "NULL scales");
+    return dense_layer_from_gram(ctx, G1, G2, N0, W, ldw, N1, j0, j1, alphabets, K, n_alph, Q_out, ldq, flags, stats, scales);
 }
 
 // Diagnostics: the Gram stage alone (tests check it against an fp64 NumPy Gram).
@@ -610,9 +668,11 @@ static int conv_copy_q_grouped(gpfq_ctx *ctx, double *Q_out, const double *dQ, i
 }
 
 // W / Q_out: (kk, C / groups, F); channel c walks the F / groups filters of its group c / (C / groups).
+// d_scales (nullable): (n_alph, C / groups, F) per-unit scales on the device.
 static int conv_finish(gpfq_ctx *ctx, int kk, const double *partial, int n_ch, int n_chunks, bool same,
                        const float *W, int64_t C, int64_t F, int64_t c0, const Alphabets &al, int n_alph,
-                       double *Q_out, uint32_t flags, double *gram_ready = nullptr, int64_t groups = 1) {
+                       double *Q_out, uint32_t flags, double *gram_ready = nullptr, int64_t groups = 1,
+                       const double *d_scales = nullptr) {
     cudaStream_t s = ctx->stream;
     double *gram = gram_ready;  // per-channel [G1 | G2] already assembled (correlation form): no partials to sum
     if (!gram) {
@@ -638,7 +698,7 @@ static int conv_finish(gpfq_ctx *ctx, int kk, const double *partial, int n_ch, i
     }
     double *dQ = Q_out;
     if (!(flags & GPFQ_Q_DEVICE)) GPFQ_TRY(gpfq_ws(ctx, WS_Q, (size_t)n_alph * wcount * sizeof(double), (void **)&dQ));
-    GPFQ_TRY(conv_sweep_stage(ctx, kk, gram, dW, dQ, C, F, c0, n_ch, al.d_levels, al.d_koff, al.d_flags, n_alph, groups));
+    GPFQ_TRY(conv_sweep_stage(ctx, kk, gram, dW, dQ, C, F, c0, n_ch, al.d_levels, al.d_koff, al.d_flags, n_alph, groups, d_scales));
     CUDA_TRY(ctx, gpfq_record(ctx, 4, s));
     if (!(flags & GPFQ_Q_DEVICE) && groups > 1)
         return conv_copy_q_grouped(ctx, Q_out, dQ, kk, Cg, F, F / groups, c0, n_ch, n_alph, wcount);
@@ -663,10 +723,10 @@ static void conv_stats(gpfq_ctx *ctx, gpfq_stats *st, int kk, int64_t n, int64_t
     if (!conv_specialised_kk(kk)) st->flops_algorithmic = (same ? 1 : 2) * (int64_t)kk * (kk + 1) * n * n_ch;
 }
 
-extern "C" int gpfq_conv_channels(gpfq_ctx *ctx, const float *const *Xp, const float *const *Xqp, int64_t n,
-                                  int32_t kk, const float *W, int64_t C, int64_t F, int64_t c0, int64_t n_ch,
-                                  const double *alphabets, const int32_t *K, int32_t n_alph, double *Q_out,
-                                  uint32_t flags, gpfq_stats *stats) {
+// scales (nullable, host): (n_alph, C, F) per-unit scales.
+static int conv_channels(gpfq_ctx *ctx, const float *const *Xp, const float *const *Xqp, int64_t n, int32_t kk, const float *W,
+                         int64_t C, int64_t F, int64_t c0, int64_t n_ch, const double *alphabets, const int32_t *K,
+                         int32_t n_alph, double *Q_out, uint32_t flags, gpfq_stats *stats, const double *scales) {
     if (!ctx) return GPFQ_ERR_ARG;
     ctx->err.clear();
     if (stats) memset(stats, 0, sizeof(*stats));
@@ -676,6 +736,7 @@ extern "C" int gpfq_conv_channels(gpfq_ctx *ctx, const float *const *Xp, const f
                          (long long)C, (long long)F, (long long)c0, (long long)n_ch);
     if ((flags & GPFQ_NO_SYNC) && (flags & GPFQ_ALL_DEVICE) != GPFQ_ALL_DEVICE)
         return gpfq_fail(ctx, GPFQ_ERR_ARG, "GPFQ_NO_SYNC needs all-device pointers");
+    if (scales && n_alph >= 1) GPFQ_TRY(check_scales(ctx, scales, n_alph, C * F, C * F));
     ctx->conv_part_bytes = 0;
     if (n_ch == 0) return GPFQ_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
@@ -693,8 +754,9 @@ extern "C" int gpfq_conv_channels(gpfq_ctx *ctx, const float *const *Xp, const f
         for (int64_t i = 0; i < n_ch; ++i) {
             const int64_t c = c0 + i;
             // per-alphabet outputs are kk*C*F apart, which is exactly N0*ldq for N0=kk, ldq=C*F
-            GPFQ_TRY(gpfq_dense_layer(ctx, Xp[i], same ? Xp[i] : Xqp[i], n, kk, n, W + c * F, C * F, F, 0, F, alphabets, K,
-                                      n_alph, Q_out + c * F, C * F, (flags & ~GPFQ_NO_SYNC) | GPFQ_METHOD_GRAM, stats));
+            GPFQ_TRY(dense_layer(ctx, Xp[i], same ? Xp[i] : Xqp[i], n, kk, n, W + c * F, C * F, F, 0, F, alphabets, K, n_alph,
+                                 Q_out + c * F, C * F, (flags & ~GPFQ_NO_SYNC) | GPFQ_METHOD_GRAM, stats,
+                                 scales ? scales + c * F : nullptr, C * F));
             launches += stats ? stats->kernel_launches : 0;
         }
         if (stats) { stats->kernel_launches = (int)launches; stats->weights = (int64_t)kk * n_ch * F * n_alph; }
@@ -706,6 +768,8 @@ extern "C" int gpfq_conv_channels(gpfq_ctx *ctx, const float *const *Xp, const f
     CUDA_TRY(ctx, gpfq_record(ctx, 0, s));
     Alphabets al;
     GPFQ_TRY(upload_alphabets(ctx, alphabets, K, n_alph, &al));
+    const double *d_scales = nullptr;
+    if (scales) GPFQ_TRY(upload_scales(ctx, scales, n_alph, C * F, C * F, &d_scales));
 
     bool vec_ok = n % 4 == 0;  // float4 / bulk-copy paths: every row of every patch matrix 16-byte aligned
     if (flags & GPFQ_X_DEVICE)
@@ -772,7 +836,7 @@ extern "C" int gpfq_conv_channels(gpfq_ctx *ctx, const float *const *Xp, const f
         }
     }
     CUDA_TRY(ctx, gpfq_record(ctx, 3, s));
-    GPFQ_TRY(conv_finish(ctx, kk, partial, (int)n_ch, n_chunks, same, W, C, F, c0, al, n_alph, Q_out, flags));
+    GPFQ_TRY(conv_finish(ctx, kk, partial, (int)n_ch, n_chunks, same, W, C, F, c0, al, n_alph, Q_out, flags, nullptr, 1, d_scales));
     CUDA_TRY(ctx, gpfq_record(ctx, 1, s));
     gpfq_stats local = {};
     conv_stats(ctx, stats ? stats : &local, kk, n, n_ch, F, same, n_alph);
@@ -782,11 +846,27 @@ extern "C" int gpfq_conv_channels(gpfq_ctx *ctx, const float *const *Xp, const f
     return GPFQ_OK;
 }
 
+extern "C" int gpfq_conv_channels(gpfq_ctx *ctx, const float *const *Xp, const float *const *Xqp, int64_t n,
+                                  int32_t kk, const float *W, int64_t C, int64_t F, int64_t c0, int64_t n_ch,
+                                  const double *alphabets, const int32_t *K, int32_t n_alph, double *Q_out,
+                                  uint32_t flags, gpfq_stats *stats) {
+    return conv_channels(ctx, Xp, Xqp, n, kk, W, C, F, c0, n_ch, alphabets, K, n_alph, Q_out, flags, stats, nullptr);
+}
+
+extern "C" int gpfq_conv_channels_scaled(gpfq_ctx *ctx, const float *const *Xp, const float *const *Xqp, int64_t n,
+                                         int32_t kk, const float *W, int64_t C, int64_t F, int64_t c0, int64_t n_ch,
+                                         const double *alphabets, const int32_t *K, int32_t n_alph, double *Q_out,
+                                         uint32_t flags, gpfq_stats *stats, const double *scales) {
+    if (ctx && !scales) return gpfq_fail(ctx, GPFQ_ERR_ARG, "NULL scales");
+    return conv_channels(ctx, Xp, Xqp, n, kk, W, C, F, c0, n_ch, alphabets, K, n_alph, Q_out, flags, stats, scales);
+}
+
 // gpfq_conv_layer_nhwc(_grouped): W / Q_out (kh, kw, C / groups, F).
 static int conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float *actq, int64_t n_img, int64_t H, int64_t Wd, int64_t C,
                            int32_t kh, int32_t kw, int32_t sh, int32_t sw, int32_t rh, int32_t rw, int32_t padding_same,
                            const float *W, int64_t F, int64_t c0, int64_t n_ch, const double *alphabets, const int32_t *K,
-                           int32_t n_alph, double *Q_out, uint32_t flags, gpfq_stats *stats, int64_t groups) {
+                           int32_t n_alph, double *Q_out, uint32_t flags, gpfq_stats *stats, int64_t groups,
+                           const double *scales) {
     if (!ctx) return GPFQ_ERR_ARG;
     ctx->err.clear();
     if (stats) memset(stats, 0, sizeof(*stats));
@@ -798,6 +878,7 @@ static int conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float *actq, i
         return gpfq_fail(ctx, GPFQ_ERR_ARG, "bad groups=%lld for C=%lld, F=%lld", (long long)groups, (long long)C, (long long)F);
     const int64_t Cg = C / groups, Fg = F / groups;
     const int kk = kh * kw;
+    if (scales && n_alph >= 1) GPFQ_TRY(check_scales(ctx, scales, n_alph, Cg * F, Cg * F));
     ctx->conv_part_bytes = 0;
     if (n_ch == 0) return GPFQ_OK;
     // TensorFlow extract_patches geometry (quantized_network.py:158-172)
@@ -850,8 +931,9 @@ static int conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float *actq, i
             // channel c against the Fg filters of its group (all F when ungrouped); per-alphabet outputs are kk*Cg*F apart, which is
             // exactly N0*ldq for N0 = kk, ldq = Cg*F
             const int64_t off = (c % Cg) * F + (c / Cg) * Fg;
-            GPFQ_TRY(gpfq_dense_layer(ctx, pa, same ? pa : pq, n, kk, n, W + off, Cg * F, Fg, 0, Fg, alphabets, K, n_alph, Q_out + off,
-                                      Cg * F, ((flags & ~GPFQ_NO_SYNC) | GPFQ_X_DEVICE | GPFQ_METHOD_GRAM), stats));
+            GPFQ_TRY(dense_layer(ctx, pa, same ? pa : pq, n, kk, n, W + off, Cg * F, Fg, 0, Fg, alphabets, K, n_alph, Q_out + off,
+                                 Cg * F, ((flags & ~GPFQ_NO_SYNC) | GPFQ_X_DEVICE | GPFQ_METHOD_GRAM), stats,
+                                 scales ? scales + off : nullptr, Cg * F));
             launches += (stats ? stats->kernel_launches : 0) + (same ? 1 : 2);
         }
         if (stats) { stats->kernel_launches = (int)launches; stats->weights = (int64_t)kk * n_ch * Fg * n_alph; }
@@ -861,6 +943,8 @@ static int conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float *actq, i
     CUDA_TRY(ctx, gpfq_record(ctx, 0, s));
     Alphabets al;
     GPFQ_TRY(upload_alphabets(ctx, alphabets, K, n_alph, &al));
+    const double *d_scales = nullptr;
+    if (scales) GPFQ_TRY(upload_scales(ctx, scales, n_alph, Cg * F, Cg * F, &d_scales));
     const float *dA = act, *dAq = same ? act : actq;
     const size_t img_elems = (size_t)H * Wd * C;
     const size_t abytes = (size_t)n_img * img_elems * sizeof(float);
@@ -977,7 +1061,7 @@ static int conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float *actq, i
         }
         GPFQ_TRY(conv_corr9_assemble_stage(ctx, partial, slots, bpartial, bslots, same, (int)n_ch, pack ? corr_G : 1, gram));
         CUDA_TRY(ctx, gpfq_record(ctx, 3, s));
-        GPFQ_TRY(conv_finish(ctx, kk, nullptr, (int)n_ch, 0, same, W, C, F, c0, al, n_alph, Q_out, flags, gram, groups));
+        GPFQ_TRY(conv_finish(ctx, kk, nullptr, (int)n_ch, 0, same, W, C, F, c0, al, n_alph, Q_out, flags, gram, groups, d_scales));
         CUDA_TRY(ctx, gpfq_record(ctx, 1, s));
         gpfq_stats local = {};
         gpfq_stats *st = stats ? stats : &local;
@@ -1022,7 +1106,7 @@ static int conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float *actq, i
                                            planeP, bandR, (int)per_ic, partial + (size_t)ic * per_ic * 2 * kk * kk, slots));
         }
         CUDA_TRY(ctx, gpfq_record(ctx, 3, s));
-        GPFQ_TRY(conv_finish(ctx, kk, partial, (int)n_ch, slots, same, W, C, F, c0, al, n_alph, Q_out, flags, nullptr, groups));
+        GPFQ_TRY(conv_finish(ctx, kk, partial, (int)n_ch, slots, same, W, C, F, c0, al, n_alph, Q_out, flags, nullptr, groups, d_scales));
         CUDA_TRY(ctx, gpfq_record(ctx, 1, s));
         gpfq_stats local = {};
         gpfq_stats *st = stats ? stats : &local;
@@ -1094,7 +1178,7 @@ static int conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float *actq, i
         }
     }
     CUDA_TRY(ctx, gpfq_record(ctx, 3, s));
-    GPFQ_TRY(conv_finish(ctx, kk, partial, (int)n_ch, slots, same, W, C, F, c0, al, n_alph, Q_out, flags, nullptr, groups));
+    GPFQ_TRY(conv_finish(ctx, kk, partial, (int)n_ch, slots, same, W, C, F, c0, al, n_alph, Q_out, flags, nullptr, groups, d_scales));
     CUDA_TRY(ctx, gpfq_record(ctx, 1, s));
     gpfq_stats local = {};
     conv_stats(ctx, stats ? stats : &local, kk, n, n_ch, Fg, same, n_alph);
@@ -1110,7 +1194,7 @@ extern "C" int gpfq_conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float
                                     int64_t n_ch, const double *alphabets, const int32_t *K, int32_t n_alph,
                                     double *Q_out, uint32_t flags, gpfq_stats *stats) {
     return conv_layer_nhwc(ctx, act, actq, n_img, H, Wd, C, kh, kw, sh, sw, rh, rw, padding_same, W, F, c0, n_ch, alphabets, K,
-                           n_alph, Q_out, flags, stats, 1);
+                           n_alph, Q_out, flags, stats, 1, nullptr);
 }
 
 extern "C" int gpfq_conv_layer_nhwc_grouped(gpfq_ctx *ctx, const float *act, const float *actq, int64_t n_img, int64_t H,
@@ -1119,7 +1203,18 @@ extern "C" int gpfq_conv_layer_nhwc_grouped(gpfq_ctx *ctx, const float *act, con
                                             int64_t n_ch, const double *alphabets, const int32_t *K, int32_t n_alph,
                                             double *Q_out, uint32_t flags, gpfq_stats *stats, int32_t groups) {
     return conv_layer_nhwc(ctx, act, actq, n_img, H, Wd, C, kh, kw, sh, sw, rh, rw, padding_same, W, F, c0, n_ch, alphabets, K,
-                           n_alph, Q_out, flags, stats, groups);
+                           n_alph, Q_out, flags, stats, groups, nullptr);
+}
+
+extern "C" int gpfq_conv_layer_nhwc_scaled(gpfq_ctx *ctx, const float *act, const float *actq, int64_t n_img, int64_t H,
+                                           int64_t Wd, int64_t C, int32_t kh, int32_t kw, int32_t sh, int32_t sw, int32_t rh,
+                                           int32_t rw, int32_t padding_same, const float *W, int64_t F, int64_t c0,
+                                           int64_t n_ch, const double *alphabets, const int32_t *K, int32_t n_alph,
+                                           double *Q_out, uint32_t flags, gpfq_stats *stats, int32_t groups,
+                                           const double *scales) {
+    if (ctx && !scales) return gpfq_fail(ctx, GPFQ_ERR_ARG, "NULL scales");
+    return conv_layer_nhwc(ctx, act, actq, n_img, H, Wd, C, kh, kw, sh, sw, rh, rw, padding_same, W, F, c0, n_ch, alphabets, K,
+                           n_alph, Q_out, flags, stats, groups, scales);
 }
 
 // Gram stage of a conv layer alone (see include/gpfq.h): the same planner and kernels as gpfq_conv_layer_nhwc, stopped
@@ -1146,7 +1241,7 @@ extern "C" int gpfq_conv_gram_nhwc(gpfq_ctx *ctx, const float *act, const float 
 // Walk stage of a conv layer from per-channel Gram matrices on the device (see include/gpfq.h); W / Q_out (kk, C / groups, F).
 static int conv_layer_from_gram(gpfq_ctx *ctx, const double *gram, int32_t kk, const float *W, int64_t C, int64_t F, int64_t c0,
                                 int64_t n_ch, const double *alphabets, const int32_t *K, int32_t n_alph, double *Q_out,
-                                uint32_t flags, gpfq_stats *stats, int64_t groups) {
+                                uint32_t flags, gpfq_stats *stats, int64_t groups, const double *scales) {
     if (!ctx) return GPFQ_ERR_ARG;
     ctx->err.clear();
     if (stats) memset(stats, 0, sizeof(*stats));
@@ -1156,6 +1251,7 @@ static int conv_layer_from_gram(gpfq_ctx *ctx, const double *gram, int32_t kk, c
     if (groups < 1 || C % groups || F % groups)
         return gpfq_fail(ctx, GPFQ_ERR_ARG, "bad groups=%lld for C=%lld, F=%lld", (long long)groups, (long long)C, (long long)F);
     if (!conv_supported_kk(kk)) return gpfq_fail(ctx, GPFQ_ERR_UNSUPPORTED, "kernel size kk=%d has no walk kernel", kk);
+    if (scales && n_alph >= 1) GPFQ_TRY(check_scales(ctx, scales, n_alph, C / groups * F, C / groups * F));
     if (n_ch == 0) return GPFQ_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     cudaStream_t s = ctx->stream;
@@ -1163,11 +1259,13 @@ static int conv_layer_from_gram(gpfq_ctx *ctx, const double *gram, int32_t kk, c
     CUDA_TRY(ctx, gpfq_record(ctx, 0, s));
     Alphabets al;
     GPFQ_TRY(upload_alphabets(ctx, alphabets, K, n_alph, &al));
+    const double *d_scales = nullptr;
+    if (scales) GPFQ_TRY(upload_scales(ctx, scales, n_alph, C / groups * F, C / groups * F, &d_scales));
     CUDA_TRY(ctx, gpfq_record(ctx, 5, s));
     CUDA_TRY(ctx, gpfq_record(ctx, 2, s));
     CUDA_TRY(ctx, gpfq_record(ctx, 3, s));
     GPFQ_TRY(conv_finish(ctx, kk, nullptr, (int)n_ch, 0, false, W, C, F, c0, al, n_alph, Q_out, flags, const_cast<double *>(gram),
-                         groups));
+                         groups, d_scales));
     CUDA_TRY(ctx, gpfq_record(ctx, 1, s));
     gpfq_stats local = {};
     gpfq_stats *st = stats ? stats : &local;
@@ -1182,27 +1280,42 @@ static int conv_layer_from_gram(gpfq_ctx *ctx, const double *gram, int32_t kk, c
 extern "C" int gpfq_conv_layer_from_gram(gpfq_ctx *ctx, const double *gram, int32_t kk, const float *W, int64_t C, int64_t F,
                                          int64_t c0, int64_t n_ch, const double *alphabets, const int32_t *K, int32_t n_alph,
                                          double *Q_out, uint32_t flags, gpfq_stats *stats) {
-    return conv_layer_from_gram(ctx, gram, kk, W, C, F, c0, n_ch, alphabets, K, n_alph, Q_out, flags, stats, 1);
+    return conv_layer_from_gram(ctx, gram, kk, W, C, F, c0, n_ch, alphabets, K, n_alph, Q_out, flags, stats, 1, nullptr);
 }
 
 extern "C" int gpfq_conv_layer_from_gram_grouped(gpfq_ctx *ctx, const double *gram, int32_t kk, const float *W, int64_t C,
                                                  int64_t F, int64_t c0, int64_t n_ch, const double *alphabets, const int32_t *K,
                                                  int32_t n_alph, double *Q_out, uint32_t flags, gpfq_stats *stats,
                                                  int32_t groups) {
-    return conv_layer_from_gram(ctx, gram, kk, W, C, F, c0, n_ch, alphabets, K, n_alph, Q_out, flags, stats, groups);
+    return conv_layer_from_gram(ctx, gram, kk, W, C, F, c0, n_ch, alphabets, K, n_alph, Q_out, flags, stats, groups, nullptr);
 }
 
+extern "C" int gpfq_conv_layer_from_gram_scaled(gpfq_ctx *ctx, const double *gram, int32_t kk, const float *W, int64_t C,
+                                                int64_t F, int64_t c0, int64_t n_ch, const double *alphabets, const int32_t *K,
+                                                int32_t n_alph, double *Q_out, uint32_t flags, gpfq_stats *stats,
+                                                int32_t groups, const double *scales) {
+    if (ctx && !scales) return gpfq_fail(ctx, GPFQ_ERR_ARG, "NULL scales");
+    return conv_layer_from_gram(ctx, gram, kk, W, C, F, c0, n_ch, alphabets, K, n_alph, Q_out, flags, stats, groups, scales);
+}
+
+// scales (nullable, float32 W): element i rounds to the levels scales[i % n_units] * alphabet.
 static int round_elements(gpfq_ctx *ctx, const void *W, int is_f64, int64_t n, const double *alphabet, int32_t K,
-                          double *Q_out, uint32_t flags) {
+                          double *Q_out, uint32_t flags, const double *scales = nullptr, int64_t n_units = 0) {
     if (!ctx) return GPFQ_ERR_ARG;
     ctx->err.clear();
     if (!W || !Q_out || n < 0) return gpfq_fail(ctx, GPFQ_ERR_ARG, "bad arguments");
+    if (scales) {
+        if (n_units < 1) return gpfq_fail(ctx, GPFQ_ERR_ARG, "n_units must be >= 1");
+        GPFQ_TRY(check_scales(ctx, scales, 1, n_units, n_units));
+    }
     if (n == 0) return GPFQ_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     begin_call(ctx, 2);
     cudaStream_t s = ctx->stream;
     Alphabets al;
     GPFQ_TRY(upload_alphabets(ctx, alphabet, &K, 1, &al));
+    const double *d_scales = nullptr;
+    if (scales) GPFQ_TRY(upload_scales(ctx, scales, 1, n_units, n_units, &d_scales));
     const size_t esz = is_f64 ? sizeof(double) : sizeof(float);
     const void *dW = W;
     if (!(flags & GPFQ_W_DEVICE)) {
@@ -1213,7 +1326,7 @@ static int round_elements(gpfq_ctx *ctx, const void *W, int is_f64, int64_t n, c
     }
     double *dQ = Q_out;
     if (!(flags & GPFQ_Q_DEVICE)) GPFQ_TRY(gpfq_ws(ctx, WS_Q, (size_t)n * sizeof(double), (void **)&dQ));
-    GPFQ_TRY(msq_stage(ctx, dW, is_f64, n, al.d_levels, K, al.h_flags[0], dQ));
+    GPFQ_TRY(msq_stage(ctx, dW, is_f64, n, al.d_levels, K, al.h_flags[0], dQ, d_scales, n_units));
     if (!(flags & GPFQ_Q_DEVICE))
         CUDA_TRY(ctx, cudaMemcpyAsync(Q_out, dQ, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, s));
     if (!(flags & GPFQ_NO_SYNC) || !(flags & GPFQ_Q_DEVICE)) CUDA_TRY(ctx, cudaStreamSynchronize(s));
@@ -1223,6 +1336,12 @@ static int round_elements(gpfq_ctx *ctx, const void *W, int is_f64, int64_t n, c
 extern "C" int gpfq_msq(gpfq_ctx *ctx, const float *W, int64_t n, const double *alphabet, int32_t K, double *Q_out,
                         uint32_t flags) {
     return round_elements(ctx, W, 0, n, alphabet, K, Q_out, flags);
+}
+
+extern "C" int gpfq_msq_scaled(gpfq_ctx *ctx, const float *W, int64_t n, const double *alphabet, int32_t K, const double *scales,
+                               int64_t n_units, double *Q_out, uint32_t flags) {
+    if (ctx && !scales) return gpfq_fail(ctx, GPFQ_ERR_ARG, "NULL scales");
+    return round_elements(ctx, W, 0, n, alphabet, K, Q_out, flags, scales, n_units);
 }
 
 extern "C" int gpfq_bit_round(gpfq_ctx *ctx, const double *t, int64_t n, const double *alphabet, int32_t K,

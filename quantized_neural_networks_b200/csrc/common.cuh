@@ -88,7 +88,7 @@ enum WsSlot {
     WS_U, WS_PTRS, WS_CG, WS_CPART, WS_PATCH_A, WS_PATCH_B, WS_ACT_A, WS_ACT_B, WS_QIDX, WS_MISC,
     WS_I8_SQ, WS_I8_SX, WS_I8_E, WS_I8_TILES, WS_LR_XD, WS_LR_XT, WS_LR_U, WS_CORR_B,
     WS_SL_W, WS_SL_XT, WS_SL_XQT, WS_SL_XQ, WS_SL_U, WS_SL_KQ, WS_SL_E,
-    WS_TC_TAB, WS_TC_G2S, WS_TC_G1S, WS_TC_E, WS_TC_P, WS_TC_W, WS_TC_G1M
+    WS_TC_TAB, WS_TC_G2S, WS_TC_G1S, WS_TC_E, WS_TC_P, WS_TC_W, WS_TC_G1M, WS_SCALES, WS_UNIT_H
 };
 
 int gpfq_fail(gpfq_ctx *ctx, int code, const char *fmt, ...);
@@ -213,6 +213,64 @@ static __device__ __noinline__ double gpfq_decide_rcp(double nrm, double rinv, d
         v = fma(e, rinv, q0);
     }
     return gpfq_bit_round_eq(v, alph, K, inv_step);
+}
+
+// ---------------------------------------------------------------------------------------------
+// Per-unit (per-channel) alphabets: a unit with scale s uses the levels fl64(s * alph[k]), formed on the fly with one
+// correctly rounded product per level (what NumPy's `rad_u * alphabet` gives for a scalar rad_u), so no level table per
+// unit is staged.  s = 0 gives the all-zero alphabet; its inv_step is 0, so the literal scan decides and no division by
+// the zero span happens.  The window of gpfq_bit_round_eq carries over: the scaled levels are ascending and as nearly
+// equispaced as the base levels, and the three candidates are compared with the same tests in ascending order.
+// ---------------------------------------------------------------------------------------------
+__device__ __forceinline__ double gpfq_bit_round_s(double v, const double *__restrict__ alph, int K, double s) {
+    double best = __dmul_rn(s, alph[0]);
+    double bd = fabs(__dsub_rn(best, v));
+#pragma unroll 4
+    for (int k = 1; k < K; ++k) {
+        const double a = __dmul_rn(s, alph[k]);
+        const double d = fabs(__dsub_rn(a, v));
+        if (d < bd) { bd = d; best = a; }
+    }
+    return best;
+}
+
+static __device__ __noinline__ double gpfq_bit_round_s_slow(double v, const double *__restrict__ alph, int K, double s) {
+    return gpfq_bit_round_s(v, alph, K, s);
+}
+
+__device__ __forceinline__ double gpfq_bit_round_eq_s(double v, const double *__restrict__ alph, int K, double inv_step, double s) {
+    const double gpos = (v - __dmul_rn(s, alph[0])) * inv_step;
+    if (!(inv_step > 0.0) || !(fabs(gpos) < 1e9)) return gpfq_bit_round_s_slow(v, alph, K, s);
+    const int kr = __double2int_rn(gpos), hi = K - 1;
+    const int i1 = min(max(kr, 0), hi), i0 = max(i1 - 1, 0), i2 = min(i1 + 1, hi);
+    const double a0 = __dmul_rn(s, alph[i0]), a1 = __dmul_rn(s, alph[i1]), a2 = __dmul_rn(s, alph[i2]);
+    const double d0 = fabs(__dsub_rn(a0, v)), d1 = fabs(__dsub_rn(a1, v)), d2 = fabs(__dsub_rn(a2, v));
+    double best = a0, bd = d0;
+    if (d1 < bd) { bd = d1; best = a1; }
+    if (d2 < bd) best = a2;
+    return best;
+}
+
+// inv_step of the scaled levels of an equispaced base alphabet (0: literal scan), computed once per unit
+__device__ __forceinline__ double gpfq_inv_step_s(const double *alph, int K, int equispaced, double s) {
+    if (!equispaced || K < 2) return 0.0;
+    const double span = __dsub_rn(__dmul_rn(s, alph[K - 1]), __dmul_rn(s, alph[0]));
+    return (span > 0.0 && span < 1e300) ? (double)(K - 1) / span : 0.0;
+}
+
+// The scalar quantizer with the unit's own levels: SCALED = false is the base alphabet, unchanged
+template <bool SCALED>
+__device__ __forceinline__ double gpfq_round_unit(double v, const double *__restrict__ alph, int K, double inv_step, double s) {
+    if (SCALED) return gpfq_bit_round_eq_s(v, alph, K, inv_step, s);
+    return gpfq_bit_round_eq(v, alph, K, inv_step);
+}
+
+template <bool SCALED>
+__device__ __forceinline__ double gpfq_decide_unit(double nrm, double d, double num, double w, const double *__restrict__ alph,
+                                                   int K, double inv_step, double s) {
+    if (nrm < GPFQ_DEAD_NORM) return 0.0;
+    if (fabs(d) < GPFQ_PERP_DOT) return gpfq_round_unit<SCALED>(w, alph, K, inv_step, s);
+    return gpfq_round_unit<SCALED>(num / (nrm * nrm), alph, K, inv_step, s);
 }
 
 __device__ __forceinline__ double warp_sum(double v) {

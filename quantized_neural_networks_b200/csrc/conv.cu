@@ -731,11 +731,13 @@ __device__ __forceinline__ int64_t conv_wq_offset(int64_t c, int64_t f, int64_t 
     return GROUPED ? (c % Cg) * F + (c / Cg) * Fg + f : c * F + f;
 }
 
-template <int KK, bool GROUPED>
+// SCALED: the (channel, filter) unit walks with the levels scales[a * Cg * F + (c % Cg) * F + filter] * alphabet (common.cuh).
+template <int KK, bool GROUPED, bool SCALED = false>
 __global__ void __launch_bounds__(128)
 conv_sweep_kernel(const double *__restrict__ gram, const float *__restrict__ W, double *__restrict__ Q,
                   int64_t CF, int64_t F, int64_t c0, const double *__restrict__ alphabets,
-                  const int *__restrict__ Koff, const int *__restrict__ Flags, int64_t q_alph_stride, int64_t Cg, int64_t Fg) {
+                  const int *__restrict__ Koff, const int *__restrict__ Flags, int64_t q_alph_stride, int64_t Cg, int64_t Fg,
+                  const double *__restrict__ scales = nullptr) {
     __shared__ double g1[KK * KK], g2[KK * KK], nrm[KK], alph[GPFQ_MAX_K];
     const int ch = blockIdx.y, a = blockIdx.z;
     const int K = Koff[a + 1] - Koff[a];
@@ -747,10 +749,12 @@ conv_sweep_kernel(const double *__restrict__ gram, const float *__restrict__ W, 
     __syncthreads();
     if (threadIdx.x < KK) nrm[threadIdx.x] = (double)(float)sqrt(g2[threadIdx.x * KK + threadIdx.x]);
     __syncthreads();
-    const double inv_step = gpfq_inv_step(alph, K, Flags[a]);
+    const double inv_step_base = SCALED ? 0.0 : gpfq_inv_step(alph, K, Flags[a]);
     const int64_t f = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (f >= (GROUPED ? Fg : F)) return;
     const int64_t base = conv_wq_offset<GROUPED>(c0 + ch, f, F, Cg, Fg);
+    const double sc = SCALED ? scales[(int64_t)a * CF + base] : 1.0;
+    const double inv_step = SCALED ? gpfq_inv_step_s(alph, K, Flags[a], sc) : inv_step_base;
     double w[KK], q[KK];
 #pragma unroll
     for (int t = 0; t < KK; ++t) w[t] = (double)W[(int64_t)t * CF + base];
@@ -761,7 +765,7 @@ conv_sweep_kernel(const double *__restrict__ gram, const float *__restrict__ W, 
         for (int s = 0; s < KK; ++s)
             if (s < t) d += w[s] * g1[t * KK + s] - q[s] * g2[t * KK + s];
         const double num = fma(w[t], g1[t * KK + t], d);
-        q[t] = gpfq_decide(nrm[t], d, num, w[t], alph, K, inv_step);
+        q[t] = gpfq_decide_unit<SCALED>(nrm[t], d, num, w[t], alph, K, inv_step, sc);
         Q[(int64_t)a * q_alph_stride + (int64_t)t * CF + base] = q[t];
     }
 }
@@ -776,11 +780,12 @@ constexpr int MAXW = 16;  // warps (filters) per CTA
 __host__ __device__ constexpr int col_off(int s, int kk) { return s * kk - s * (s - 1) / 2; }
 }  // namespace walkx
 
-template <bool GROUPED>
+template <bool GROUPED, bool SCALED = false>
 __global__ void __launch_bounds__(walkx::MAXW * 32)
 conv_walkx_kernel(const double *__restrict__ gram, int kk, const float *__restrict__ W, double *__restrict__ Q, int64_t CF,
                   int64_t F, int64_t c0, const double *__restrict__ alphabets, const int *__restrict__ Koff,
-                  const int *__restrict__ Flags, int64_t q_alph_stride, int64_t Cg, int64_t Fg) {
+                  const int *__restrict__ Flags, int64_t q_alph_stride, int64_t Cg, int64_t Fg,
+                  const double *__restrict__ scales = nullptr) {
     extern __shared__ double walkx_smem[];
     const int tri = kk * (kk + 1) / 2;
     double *g1 = walkx_smem, *g2 = g1 + tri, *nrm = g2 + tri, *alph = nrm + kk;
@@ -798,11 +803,13 @@ conv_walkx_kernel(const double *__restrict__ gram, int kk, const float *__restri
     __syncthreads();
     for (int t = threadIdx.x; t < kk; t += blockDim.x) nrm[t] = (double)(float)sqrt(g2[walkx::col_off(t, kk)]);
     __syncthreads();
-    const double inv_step = gpfq_inv_step(alph, K, Flags[a]);
+    const double inv_step_base = SCALED ? 0.0 : gpfq_inv_step(alph, K, Flags[a]);
     const int lane = threadIdx.x & 31;
     const int64_t f = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (f >= (GROUPED ? Fg : F)) return;
     const int64_t base = conv_wq_offset<GROUPED>(c0 + ch, f, F, Cg, Fg);
+    const double sc = SCALED ? scales[(int64_t)a * CF + base] : 1.0;
+    const double inv_step = SCALED ? gpfq_inv_step_s(alph, K, Flags[a], sc) : inv_step_base;
     double *q_out = Q + (int64_t)a * q_alph_stride + base;
     double w[4], d[4];
 #pragma unroll
@@ -821,7 +828,7 @@ conv_walkx_kernel(const double *__restrict__ gram, int kk, const float *__restri
             double qt = 0.0;
             if (lane == o) {
                 const double num = fma(w[j], g1[off + t], d[j]);
-                qt = gpfq_decide(nrm[t], d[j], num, w[j], alph, K, inv_step);
+                qt = gpfq_decide_unit<SCALED>(nrm[t], d[j], num, w[j], alph, K, inv_step, sc);
                 q_out[(int64_t)t * CF] = qt;
             }
             qt = __shfl_sync(0xffffffffu, qt, o);
@@ -866,6 +873,19 @@ __global__ void msq_kernel(const T *__restrict__ W, int64_t n, const double *__r
     const double inv_step = gpfq_inv_step(alph, K, equispaced);
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
         Q[i] = gpfq_bit_round_eq((double)W[i], alph, K, inv_step);
+}
+
+// Per-unit MSQ: element i rounds to the levels scales[i % n_units] * alphabet (the unit is the last axis of a Dense or conv
+// kernel, flattened C-order).
+__global__ void msq_scaled_kernel(const float *__restrict__ W, int64_t n, const double *__restrict__ alphabet, int K, int equispaced,
+                                  const double *__restrict__ scales, int64_t n_units, double *__restrict__ Q) {
+    __shared__ double alph[GPFQ_MAX_K];
+    for (int e = threadIdx.x; e < K; e += blockDim.x) alph[e] = alphabet[e];
+    __syncthreads();
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        const double s = scales[i % n_units];
+        Q[i] = gpfq_bit_round_eq_s((double)W[i], alph, K, gpfq_inv_step_s(alph, K, equispaced, s), s);
+    }
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -983,19 +1003,20 @@ int conv_finalize_stage(gpfq_ctx *ctx, const double *partial, int n_ch, int n_ch
 }
 
 // W / Q: (kk, C / groups, F); channels c0 .. c0+n_ch-1 walk the F / groups filters of their group (groups = 1: all F).
+// scales (device, nullable): (n_alph, C / groups, F) per-unit scales, indexed like W.
 int conv_sweep_stage(gpfq_ctx *ctx, int kk, const double *gram, const float *W, double *Q, int64_t C,
                      int64_t F, int64_t c0, int n_ch, const double *d_alph, const int *d_koff, const int *d_flags,
-                     int n_alph, int64_t groups) {
+                     int n_alph, int64_t groups, const double *scales) {
     const int64_t Cg = C / groups, Fg = F / groups;
     const bool grouped = groups > 1;
     dim3 grid((unsigned)ceil_div64(Fg, 128), (unsigned)n_ch, (unsigned)n_alph);
     const int64_t CF = Cg * F, qs = (int64_t)kk * CF;
+#define SWEEP_LAUNCH(KKV, G, S) \
+    conv_sweep_kernel<KKV, G, S><<<grid, 128, 0, ctx->stream>>>(gram, W, Q, CF, F, c0, d_alph, d_koff, d_flags, qs, Cg, Fg, scales)
 #define SWEEP_CASE(KKV)                                                                                                 \
     case KKV:                                                                                                           \
-        if (grouped)                                                                                                    \
-            conv_sweep_kernel<KKV, true><<<grid, 128, 0, ctx->stream>>>(gram, W, Q, CF, F, c0, d_alph, d_koff, d_flags, qs, Cg, Fg); \
-        else                                                                                                            \
-            conv_sweep_kernel<KKV, false><<<grid, 128, 0, ctx->stream>>>(gram, W, Q, CF, F, c0, d_alph, d_koff, d_flags, qs, Cg, Fg); \
+        if (scales) { if (grouped) SWEEP_LAUNCH(KKV, true, true); else SWEEP_LAUNCH(KKV, false, true); }                \
+        else { if (grouped) SWEEP_LAUNCH(KKV, true, false); else SWEEP_LAUNCH(KKV, false, false); }                     \
         break;
     switch (kk) {
         SWEEP_CASE(1) SWEEP_CASE(2) SWEEP_CASE(3) SWEEP_CASE(4) SWEEP_CASE(6) SWEEP_CASE(9)
@@ -1005,18 +1026,14 @@ int conv_sweep_stage(gpfq_ctx *ctx, int kk, const double *gram, const float *W, 
             const int warps = Fg < MAXW ? (int)Fg : MAXW;
             const size_t smem = ((size_t)kk * (kk + 1) + kk + GPFQ_MAX_K) * sizeof(double);
             dim3 wgrid((unsigned)ceil_div64(Fg, warps), (unsigned)n_ch, (unsigned)n_alph);
-            if (grouped) {
-                CUDA_TRY(ctx, cudaFuncSetAttribute(conv_walkx_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                conv_walkx_kernel<true><<<wgrid, warps * 32, smem, ctx->stream>>>(gram, kk, W, Q, CF, F, c0, d_alph, d_koff, d_flags,
-                                                                                 qs, Cg, Fg);
-            } else {
-                CUDA_TRY(ctx, cudaFuncSetAttribute(conv_walkx_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-                conv_walkx_kernel<false><<<wgrid, warps * 32, smem, ctx->stream>>>(gram, kk, W, Q, CF, F, c0, d_alph, d_koff, d_flags,
-                                                                                  qs, Cg, Fg);
-            }
+            auto k = grouped ? (scales ? conv_walkx_kernel<true, true> : conv_walkx_kernel<true, false>)
+                             : (scales ? conv_walkx_kernel<false, true> : conv_walkx_kernel<false, false>);
+            CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            k<<<wgrid, warps * 32, smem, ctx->stream>>>(gram, kk, W, Q, CF, F, c0, d_alph, d_koff, d_flags, qs, Cg, Fg, scales);
         }
     }
 #undef SWEEP_CASE
+#undef SWEEP_LAUNCH
     KERNEL_CHECK(ctx);
     return GPFQ_OK;
 }
@@ -1072,10 +1089,14 @@ int conv_gram9_nhwc_stage(gpfq_ctx *ctx, const float *act, const float *actq, bo
     return GPFQ_OK;
 }
 
-int msq_stage(gpfq_ctx *ctx, const void *W, int is_f64, int64_t n, const double *d_alph, int K, int equispaced, double *Q) {
+// d_scales (nullable, float32 W only): per-unit scales, element i uses d_scales[i % n_units]
+int msq_stage(gpfq_ctx *ctx, const void *W, int is_f64, int64_t n, const double *d_alph, int K, int equispaced, double *Q,
+              const double *d_scales, int64_t n_units) {
     int bx = (int)(ceil_div64(n, 256) < 1184 ? ceil_div64(n, 256) : 1184);
     if (bx < 1) bx = 1;
-    if (is_f64) msq_kernel<double><<<bx, 256, 0, ctx->stream>>>((const double *)W, n, d_alph, K, equispaced, Q);
+    if (d_scales)
+        msq_scaled_kernel<<<bx, 256, 0, ctx->stream>>>((const float *)W, n, d_alph, K, equispaced, d_scales, n_units, Q);
+    else if (is_f64) msq_kernel<double><<<bx, 256, 0, ctx->stream>>>((const double *)W, n, d_alph, K, equispaced, Q);
     else msq_kernel<float><<<bx, 256, 0, ctx->stream>>>((const float *)W, n, d_alph, K, equispaced, Q);
     KERNEL_CHECK(ctx);
     return GPFQ_OK;

@@ -78,6 +78,37 @@ __device__ __forceinline__ double gpfq_decide_rcp_inl(double nrm, double rinv, d
     return gpfq_bit_round_eq(v, alph, K, inv_step);
 }
 
+// The same decision with the neuron's own levels fl64(s * alph[k]) (per-channel alphabets, common.cuh): inv_step and tern are
+// the neuron's (tern = fl64(s * a) of a ternary base alphabet {-a, 0, a}, 0 otherwise).
+template <bool SCALED>
+__device__ __forceinline__ double gpfq_decide_rcp_unit(double nrm, double rinv, double d, double num, double w,
+                                                       const double *__restrict__ alph, int K, double inv_step, double tern,
+                                                       double s) {
+    if (!SCALED) return gpfq_decide_rcp_inl(nrm, rinv, d, num, w, alph, K, inv_step, tern);
+    if (nrm < GPFQ_DEAD_NORM) return 0.0;
+    double v = w;
+    if (!(fabs(d) < GPFQ_PERP_DOT)) {
+        const double den = nrm * nrm;
+        const double q0 = num * rinv;
+        const double e = fma(-q0, den, num);
+        v = fma(e, rinv, q0);
+    }
+    if (tern > 0.0) return gpfq_bit_round_ternary(v, tern);
+    return gpfq_bit_round_eq_s(v, alph, K, inv_step, s);
+}
+
+// Per-neuron scale, inv_step and ternary radius of neuron jt + j (SCALED; else the alphabet's own)
+template <bool SCALED>
+__device__ __forceinline__ void sweep_unit_levels(const double *__restrict__ scales, int64_t idx, bool live,
+                                                  const double *alph, int K, int flag, double inv_step, double tern,
+                                                  double *sc, double *inv_u, double *tern_u) {
+    if (!SCALED) { *sc = 1.0; *inv_u = inv_step; *tern_u = tern; return; }
+    const double s = live ? scales[idx] : 0.0;
+    *sc = s;
+    *inv_u = gpfq_inv_step_s(alph, K, flag, s);
+    *tern_u = __dmul_rn(s, tern);
+}
+
 template <int NT>
 struct SweepCfg {
     // K chunk per pipeline stage: 64 earlier directions (one barrier per chunk: fewer, fatter steps on the latency-bound
@@ -89,13 +120,14 @@ struct SweepCfg {
     //  step, whatever the step)
 };
 
-template <int NT, bool ALIGNED>
+// SCALED: neuron j of alphabet a walks with the levels scales[a * nj + j] * alphabet (per-channel alphabets).
+template <int NT, bool ALIGNED, bool SCALED = false>
 __global__ void __launch_bounds__(256, 2)
 sweep_tile_kernel(const double *__restrict__ G1, const double *__restrict__ G2, int64_t ldg, int64_t N0,
                   const double *__restrict__ Wt, double *__restrict__ Qt, int64_t nj,
                   const double *__restrict__ alphabets, const int *__restrict__ Koff,
                   const int *__restrict__ Flags, int64_t t_begin, int64_t t_end, const double *__restrict__ Dt,
-                  int64_t ldd) {
+                  int64_t ldd, const double *__restrict__ scales = nullptr) {
     // Directions [t_begin, t_end) (t_begin a multiple of 32).  Dt (nullable): (n_alph, nj, ldd) contributions of the
     // directions before t_begin, from one large NT contraction on the host side (two-level blocking).
     using Cfg = SweepCfg<NT>;
@@ -127,6 +159,10 @@ sweep_tile_kernel(const double *__restrict__ G1, const double *__restrict__ G2, 
     __syncthreads();
     const double inv_step = gpfq_inv_step(alph, K, Flags[a]);
     const double tern = gpfq_ternary_radius(alph, K);
+    // the walker lanes' neuron levels (once per neuron, not per block)
+    double sc, inv_u, tern_u;
+    sweep_unit_levels<SCALED>(scales, (int64_t)a * nj + jt + (tid >> 2), tid < 4 * NT && jt + (tid >> 2) < nj, alph, K, Flags[a], inv_step,
+                              tern, &sc, &inv_u, &tern_u);
 
     // this thread's 16-byte chunks of every W / Q tile (fixed for the whole walk)
     int w_off[WCH];
@@ -289,7 +325,7 @@ sweep_tile_kernel(const double *__restrict__ G1, const double *__restrict__ G2, 
                     const double d0 = __shfl_sync(0xffffffffu, d[0], (lane & ~3) + rr);
                     const double wv = wrow[tt];
                     const double num = fma(wv, g1dd[tt], d0);
-                    double q = gpfq_decide_rcp_inl(nrm[tt], rinv[tt], d0, num, wv, alph, K, inv_step, tern);
+                    double q = gpfq_decide_rcp_unit<SCALED>(nrm[tt], rinv[tt], d0, num, wv, alph, K, inv_u, tern_u, sc);
                     if (tt >= nb) q = 0.0;  // past the end of a partial block: no decision, no update
                     if (r == rr && tt < nb) qrow[tt] = q;
                     if (rr < 3) {
@@ -337,12 +373,12 @@ struct PipeCfg {
     static constexpr size_t SMEM = sizeof(double) * ((size_t)STAGES * (B + NT) * LD + 2 * SET + GPFQ_MAX_K);
 };
 
-template <int NT>
+template <int NT, bool SCALED = false>
 __global__ void __launch_bounds__(256, 1)
 sweep_pipe_kernel(const double *__restrict__ G1, const double *__restrict__ G2, int64_t ldg, int64_t N0,
                   const double *__restrict__ Wt, double *__restrict__ Qt, int64_t nj, const double *__restrict__ alphabets,
                   const int *__restrict__ Koff, const int *__restrict__ Flags, int64_t t_begin, int64_t t_end,
-                  const double *__restrict__ Dt, int64_t ldd) {
+                  const double *__restrict__ Dt, int64_t ldd, const double *__restrict__ scales = nullptr) {
     using Cfg = PipeCfg<NT>;
     constexpr int B = Cfg::B, KC = Cfg::KC, LD = Cfg::LD, STAGES = Cfg::STAGES, CT = Cfg::CT, NA = NT / 8, NW = 4 * NT;
     constexpr int BAR_C = 1, BAR_READY = 2, BAR_WALK_DONE = 4, BAR_Q_STORED = 6, HANDOVER = NW + CT;
@@ -526,6 +562,9 @@ sweep_pipe_kernel(const double *__restrict__ G1, const double *__restrict__ G2, 
     } else if (tid < NW) {
         // =============================== walkers: FOUR lanes per neuron (lane = 4 j + r) ===============================
         const int j = tid >> 2, r = tid & 3;
+        double sc, inv_u, tern_u;
+        sweep_unit_levels<SCALED>(scales, (int64_t)a * nj + jt + j, jt + j < nj, alph, K, Flags[a], inv_step, tern, &sc, &inv_u,
+                                  &tern_u);
         for (int b = 0; b < nblk; ++b) {
             const int s = b & 1;
             const int64_t t0 = t_begin + (int64_t)b * B;
@@ -550,7 +589,7 @@ sweep_pipe_kernel(const double *__restrict__ G1, const double *__restrict__ G2, 
                     const double d0 = __shfl_sync(0xffffffffu, d[0], (lane & ~3) + rr);
                     const double wv = wrow[tt];
                     const double num = fma(wv, g1dd[tt], d0);
-                    double q = gpfq_decide_rcp_inl(nrm[tt], rinv[tt], d0, num, wv, alph, K, inv_step, tern);
+                    double q = gpfq_decide_rcp_unit<SCALED>(nrm[tt], rinv[tt], d0, num, wv, alph, K, inv_u, tern_u, sc);
                     if (tt >= nb) q = 0.0;  // past the end of a partial block: no decision, no update
                     if (r == rr && tt < nb) qrow[tt] = q;
                     if (rr < 3) {
@@ -585,12 +624,12 @@ sweep_pipe_kernel(const double *__restrict__ G1, const double *__restrict__ G2, 
 template <int NT>
 static int launch_sweep_pipe(gpfq_ctx *ctx, const double *G1, const double *G2, int64_t ldg, int64_t N0, const double *Wt,
                              double *Qt, int64_t nj, const double *d_alph, const int *d_koff, const int *d_flags,
-                             int n_alph, int64_t t_begin, int64_t t_end, const double *Dt, int64_t ldd) {
+                             int n_alph, int64_t t_begin, int64_t t_end, const double *Dt, int64_t ldd, const double *scales) {
     const size_t smem = PipeCfg<NT>::SMEM;
     dim3 grid((unsigned)ceil_div64(nj, NT), (unsigned)n_alph);
-    auto k = sweep_pipe_kernel<NT>;
+    auto k = scales ? sweep_pipe_kernel<NT, true> : sweep_pipe_kernel<NT, false>;
     CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    k<<<grid, 256, smem, ctx->stream>>>(G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, t_begin, t_end, Dt, ldd);
+    k<<<grid, 256, smem, ctx->stream>>>(G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, t_begin, t_end, Dt, ldd, scales);
     KERNEL_CHECK(ctx);
     return GPFQ_OK;
 }
@@ -598,20 +637,15 @@ static int launch_sweep_pipe(gpfq_ctx *ctx, const double *G1, const double *G2, 
 template <int NT>
 static int launch_sweep_tile(gpfq_ctx *ctx, const double *G1, const double *G2, int64_t ldg, int64_t N0, const double *Wt,
                              double *Qt, int64_t nj, const double *d_alph, const int *d_koff, const int *d_flags,
-                             int n_alph, int64_t t_begin, int64_t t_end, const double *Dt, int64_t ldd) {
+                             int n_alph, int64_t t_begin, int64_t t_end, const double *Dt, int64_t ldd, const double *scales) {
     const size_t smem = SweepCfg<NT>::SMEM;
     dim3 grid((unsigned)ceil_div64(nj, NT), (unsigned)n_alph);
     const bool aligned = (N0 % 2 == 0) && (ldg % 2 == 0) && ((uintptr_t)G1 % 16 == 0) && ((uintptr_t)G2 % 16 == 0) &&
                          ((uintptr_t)Wt % 16 == 0) && ((uintptr_t)Qt % 16 == 0) && ((nj * N0) % 2 == 0);
-    if (aligned) {
-        auto k = sweep_tile_kernel<NT, true>;
-        CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k<<<grid, 256, smem, ctx->stream>>>(G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, t_begin, t_end, Dt, ldd);
-    } else {
-        auto k = sweep_tile_kernel<NT, false>;
-        CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        k<<<grid, 256, smem, ctx->stream>>>(G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, t_begin, t_end, Dt, ldd);
-    }
+    auto k = aligned ? (scales ? sweep_tile_kernel<NT, true, true> : sweep_tile_kernel<NT, true, false>)
+                     : (scales ? sweep_tile_kernel<NT, false, true> : sweep_tile_kernel<NT, false, false>);
+    CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    k<<<grid, 256, smem, ctx->stream>>>(G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, t_begin, t_end, Dt, ldd, scales);
     KERNEL_CHECK(ctx);
     return GPFQ_OK;
 }
@@ -760,7 +794,8 @@ static int64_t pick_range_length(gpfq_ctx *ctx, int64_t nj, int n_alph) {
 
 static int dispatch_sweep_tile(gpfq_ctx *ctx, int NT, const double *G1, const double *G2, int64_t ldg, int64_t N0,
                                const double *Wt, double *Qt, int64_t nj, const double *d_alph, const int *d_koff,
-                               const int *d_flags, int n_alph, int64_t tb, int64_t te, const double *Dp, int64_t R) {
+                               const int *d_flags, int n_alph, int64_t tb, int64_t te, const double *Dp, int64_t R,
+                               const double *scales) {
     // The pipelined walk (one CTA per SM) when its 16-byte copies are possible and every CTA of the launch is resident at
     // once; the narrowest neuron tile that allows it.
     const bool aligned = (N0 % 2 == 0) && (ldg % 2 == 0) && ((uintptr_t)G1 % 16 == 0) && ((uintptr_t)G2 % 16 == 0) &&
@@ -768,21 +803,22 @@ static int dispatch_sweep_tile(gpfq_ctx *ctx, int NT, const double *G1, const do
     if (aligned) {
         const int64_t sms = ctx->sm_count;
         if (ceil_div64(nj, 8) * n_alph <= sms)
-            return launch_sweep_pipe<8>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R);
+            return launch_sweep_pipe<8>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R, scales);
         if (ceil_div64(nj, 16) * n_alph <= sms)
-            return launch_sweep_pipe<16>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R);
+            return launch_sweep_pipe<16>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R, scales);
         if (ceil_div64(nj, 32) * n_alph <= sms)
-            return launch_sweep_pipe<32>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R);
+            return launch_sweep_pipe<32>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R, scales);
     }
-    if (NT == 32) return launch_sweep_tile<32>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R);
-    if (NT == 16) return launch_sweep_tile<16>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R);
-    return launch_sweep_tile<8>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R);
+    if (NT == 32) return launch_sweep_tile<32>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R, scales);
+    if (NT == 16) return launch_sweep_tile<16>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R, scales);
+    return launch_sweep_tile<8>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R, scales);
 }
 
-// Sweep with the low-rank outer level.  Wt (nj, N0) is ready; Qt (n_alph, nj, N0) receives the result.
+// Sweep with the low-rank outer level.  Wt (nj, N0) is ready; Qt (n_alph, nj, N0) receives the result.  scales (nullable):
+// (n_alph, nj) per-neuron scales.
 static int dense_lowrank_sweep(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ldx, int64_t N0, int64_t m,
                                const double *Wt, double *Qt, int64_t nj, const double *d_alph, const int *d_koff,
-                               const int *d_flags, int n_alph, int NT) {
+                               const int *d_flags, int n_alph, int NT, const double *scales) {
     const bool same = (Xq == X);
     cudaStream_t st = ctx->stream;
     const int64_t R = pick_range_length(ctx, nj, n_alph);
@@ -901,7 +937,7 @@ static int dense_lowrank_sweep(gpfq_ctx *ctx, const float *X, const float *Xq, i
                     }
                 }
                 rc = dispatch_sweep_tile(ctx, NT, Gc1 - tb, Gc2 - tb, R, N0, Wt + j_lo * N0, Qt + j_lo * N0, njh, d_alph, d_koff,
-                                         d_flags, 1, tb, te, tb > 0 ? Do + j_lo * R : nullptr, R);
+                                         d_flags, 1, tb, te, tb > 0 ? Do + j_lo * R : nullptr, R, scales ? scales + j_lo : nullptr);
             }
             ctx->stream = keep;
             return rc;
@@ -982,7 +1018,7 @@ static int dense_lowrank_sweep(gpfq_ctx *ctx, const float *X, const float *Xq, i
         }
         // the compact tiles are addressed like the full matrices: column s of row t lives at Gc[t * R + (s - tb)]
         GPFQ_TRY(dispatch_sweep_tile(ctx, NT, Gc1 - tb, Gc2 - tb, R, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te,
-                                     tb > 0 ? Do : nullptr, R));
+                                     tb > 0 ? Do : nullptr, R, scales));
     }
     return GPFQ_OK;
 }
@@ -1009,9 +1045,17 @@ static bool dense_lowrank_uses_i8(gpfq_ctx *ctx, int64_t N0, int64_t m, int64_t 
     return alphabet_symmetric_equispaced(ctx->h_alph + ctx->h_koff[0], ctx->h_koff[1] - ctx->h_koff[0], ctx->h_flags[0], h);
 }
 
+// h_j = fl(s_j a) / (K - 1): the level step of neuron j with per-channel alphabets, computed as sweep_tc_kernel computes it
+__global__ void unit_steps_kernel(const double *__restrict__ scales, int64_t nj, int64_t njP, double a, int K, double *__restrict__ hrow) {
+    const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j < njP) hrow[j] = j < nj ? __dmul_rn(scales[j], a) / (double)(K - 1) : 0.0;
+}
+
+// d_scales (nullable): (nj) per-neuron scales (per-channel alphabets): the walk applies each neuron's own step, and the Q part of the
+// residual update becomes -diag(h) K'_r X~_r (a per-row multiplier in the slgemm_i8_kernel epilogue); the W part and D_r are unchanged.
 static int dense_lowrank_sweep_i8(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ldx, int64_t N0, int64_t m,
                                   const double *Wt, int64_t nj, const double *d_alph, double h, gpfq_stats *stats, const float *W,
-                                  int64_t ldw, int64_t j0, double *Qd, int64_t ldq, int64_t col0) {
+                                  int64_t ldw, int64_t j0, double *Qd, int64_t ldq, int64_t col0, const double *d_scales) {
     const bool same = (Xq == X);
     cudaStream_t st = ctx->stream, side = ctx->copy_stream;
     int64_t R = pick_range_length(ctx, nj, 1);
@@ -1038,6 +1082,13 @@ static int dense_lowrank_sweep_i8(gpfq_ctx *ctx, const float *X, const float *Xq
     int32_t *eW = e, *eU = eW + njP, *eXq = eU + njP, *eXT = eXq + N0P;   // X^T and X~^T share their per-sample exponents
     int *scratch = eXT + mP;
     GPFQ_TRY(gpfq_ws(ctx, WS_LR_U, (size_t)nj * m * sizeof(double), (void **)&Ut));
+    double *hrow = nullptr;   // per-neuron steps (per-channel alphabets), padded to njP rows
+    if (d_scales) {
+        GPFQ_TRY(gpfq_ws(ctx, WS_UNIT_H, (size_t)njP * sizeof(double), (void **)&hrow));
+        unit_steps_kernel<<<(unsigned)ceil_div64(njP, 256), 256, 0, st>>>(d_scales, nj, njP, a_top, K_levels, hrow);
+        KERNEL_CHECK(ctx);
+    }
+    const double h_q = d_scales ? 1.0 : h;   // the walk's tables and the Q part: h itself, or 1 with the steps applied per neuron
     const size_t gc_bytes = (size_t)ceil_div64(N0, R) * R * R * sizeof(double);
     GPFQ_TRY(gpfq_ws(ctx, WS_G2, gc_bytes, (void **)&Gc2));
     if (same) Gc1 = Gc2;
@@ -1089,7 +1140,7 @@ static int dense_lowrank_sweep_i8(gpfq_ctx *ctx, const float *X, const float *Xq
         GPFQ_TRY(gpfq_ws(ctx, WS_TC_G1S, (size_t)S * N0P * R, (void **)&sG1));
         GPFQ_TRY(gpfq_ws(ctx, WS_TC_E, (size_t)N0P * sizeof(int32_t), (void **)&eG1));
         GPFQ_TRY(gpfq_ws(ctx, WS_TC_P, (size_t)njP * N0P * sizeof(double), (void **)&Pd));
-        GPFQ_TRY(sweep_tc_prepare(ctx, Gc1, Gc2, R, true, N0, N0P, R, h, &tct));
+        GPFQ_TRY(sweep_tc_prepare(ctx, Gc1, Gc2, R, true, N0, N0P, R, h_q, &tct));
         GPFQ_TRY(sweep_tc_bind(ctx, &tct, Pd, Wn, njP, N0P));
         GPFQ_TRY(sweep_tc_slice_g1_lower(ctx, Gc1, R, true, N0, N0P, R, eG1, sG1));
         SlOperand oG1;
@@ -1133,11 +1184,11 @@ static int dense_lowrank_sweep_i8(gpfq_ctx *ctx, const float *X, const float *Xq
             if (tb > 0) {
                 const int64_t Kp = ceil_div64(tb - pb, 128) * 128;   // the walk of [pb, tb) left its level indices in sKq
                 if (merged) {   // U += W_r X_r - h K'_r X~_r as ONE launch of two products (same B-row exponents)
-                    SlProduct up[2] = {{&oW, &oXT, j_lo, 0, pb, Kp, D_UPDATE, 1.0}, {&oKq, &oXqT, j_lo, 0, pb, Kp, 6, -h}};
+                    SlProduct up[2] = {{&oW, &oXT, j_lo, 0, pb, Kp, D_UPDATE, 1.0}, {&oKq, &oXqT, j_lo, 0, pb, Kp, 6, -h_q, -1, hrow}};
                     rc = slgemm_i8(ctx, up, 2, Ut + j_lo * m, m, njh, m, true);
                 } else {
                     cu(cudaStreamWaitEvent(on, ev_wpart, 0));
-                    SlProduct qp = {&oKq, &oXqT, j_lo, 0, pb, Kp, 6, -h};
+                    SlProduct qp = {&oKq, &oXqT, j_lo, 0, pb, Kp, 6, -h_q, -1, hrow};
                     rc = slgemm_i8(ctx, &qp, 1, Ut + j_lo * m, m, njh, m, true);          // U -= h K'_r X~_r
                 }
                 if (rc != GPFQ_OK) break;
@@ -1175,7 +1226,8 @@ static int dense_lowrank_sweep_i8(gpfq_ctx *ctx, const float *X, const float *Xq
                 ctx->stream = on;
                 if (rc != GPFQ_OK) break;
             }
-            rc = sweep_tc_range(ctx, tct, tb, te, j_lo, njh, sKq, njP, j_lo, a_top, d_levels, K_levels);   // {-a, 0, a}: h = a / 2
+            rc = sweep_tc_range(ctx, tct, tb, te, j_lo, njh, sKq, njP, j_lo, a_top, d_levels, K_levels,   // {-a, 0, a}: h = a / 2
+                                d_scales ? d_scales + j_lo : nullptr);
         }
         ctx->stream = keep;
         return rc;
@@ -1209,16 +1261,18 @@ static int dense_lowrank_sweep_i8(gpfq_ctx *ctx, const float *X, const float *Xq
         GPFQ_TRY(chain(0, st, 0, nj));
     }
     // the tensor-core walk leaves level indices only: the layer's fp64 values are made from them here
-    GPFQ_TRY(sweep_tc_q_from_kq(ctx, sKq, njP, N0, nj, d_levels, K_levels, Qd, ldq, col0));
+    GPFQ_TRY(sweep_tc_q_from_kq(ctx, sKq, njP, N0, nj, d_levels, K_levels, Qd, ldq, col0, d_scales));
     return GPFQ_OK;
 }
 
 // Dense layer by Gram + sweep.  All pointers are device pointers.
 //   Qd: (n_alph, N0, ldq) fp64 device output, columns col0..col0+nj-1 written.
+//   d_scales (nullable): (n_alph, nj) per-neuron scales of the shard (per-channel alphabets): every walk applies each neuron's own
+//   levels, the same kernels run as for the per-layer call (DESIGN.md 5.5).
 int dense_gram_path(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ldx, int64_t N0, int64_t m,
                     const float *W, int64_t ldw, int64_t j0, int64_t nj, const double *d_alph,
                     const int *d_koff, const int *d_flags, int n_alph, double *Qd, int64_t ldq, int64_t col0,
-                    gpfq_stats *st, const double *G1_pre, const double *G2_pre) {
+                    gpfq_stats *st, const double *G1_pre, const double *G2_pre, const double *d_scales) {
     // G2_pre != NULL: the Gram stage already ran elsewhere (sample-split over the ranks of a job and all-reduced,
     // gpfq_dense_layer_from_gram); X / Xq / m are then unused and the sweep starts from the given (N0, N0) matrices.
     const bool pre = (G2_pre != nullptr);
@@ -1241,9 +1295,9 @@ int dense_gram_path(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ldx,
     }
     if (lowrank) {
         if (i8_sweep) {   // writes Qd itself
-            GPFQ_TRY(dense_lowrank_sweep_i8(ctx, X, Xq, ldx, N0, m, Wt, nj, d_alph, h_step, st, W, ldw, j0, Qd, ldq, col0));
+            GPFQ_TRY(dense_lowrank_sweep_i8(ctx, X, Xq, ldx, N0, m, Wt, nj, d_alph, h_step, st, W, ldw, j0, Qd, ldq, col0, d_scales));
         } else {
-            GPFQ_TRY(dense_lowrank_sweep(ctx, X, Xq, ldx, N0, m, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, NT));
+            GPFQ_TRY(dense_lowrank_sweep(ctx, X, Xq, ldx, N0, m, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, NT, d_scales));
             for (int a = 0; a < n_alph; ++a) {
                 dim3 grid((unsigned)ceil_div64(N0, 32), (unsigned)ceil_div64(nj, 32));
                 transpose_q_kernel<<<grid, dim3(32, 8), 0, ctx->stream>>>(Qt + (int64_t)a * nj * N0, N0, nj,
@@ -1304,7 +1358,7 @@ int dense_gram_path(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ldx,
         GPFQ_TRY(gpfq_ws(ctx, WS_SL_KQ, (size_t)njP * N0P, (void **)&sKq));
         CUDA_TRY(ctx, cudaMemsetAsync(Pd, 0, (size_t)njP * N0P * sizeof(double), ctx->stream));
         GPFQ_TRY(sweep_tc_weights(ctx, W, ldw, j0, N0, N0P, nj, Wn));
-        GPFQ_TRY(sweep_tc_prepare(ctx, G1, G2, N0, false, N0, N0P, R, h_tc, &tct));
+        GPFQ_TRY(sweep_tc_prepare(ctx, G1, G2, N0, false, N0, N0P, R, d_scales ? 1.0 : h_tc, &tct));   // scaled: steps per walker
         GPFQ_TRY(sweep_tc_bind(ctx, &tct, Pd, Wn, njP, N0P));
         GPFQ_TRY(sweep_tc_mask_g1_lower(ctx, G1, N0, N0, N0P, R, G1m));
         const int64_t nfull = N0 / R;
@@ -1370,11 +1424,11 @@ int dense_gram_path(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ldx,
         }
         if (use_tc) {
             if (tb > 0) GPFQ_TRY(sweep_tc_add_outer(ctx, Pd + tb, N0P, Do, R, nj, te - tb));
-            GPFQ_TRY(sweep_tc_range(ctx, tct, tb, te, 0, nj, sKq, njP, 0, a_top, d_alph, K_levels));
-            GPFQ_TRY(sweep_tc_qt_from_kq(ctx, sKq, njP, tb, te, nj, d_alph, K_levels, Qt, N0));
+            GPFQ_TRY(sweep_tc_range(ctx, tct, tb, te, 0, nj, sKq, njP, 0, a_top, d_alph, K_levels, d_scales));
+            GPFQ_TRY(sweep_tc_qt_from_kq(ctx, sKq, njP, tb, te, nj, d_alph, K_levels, Qt, N0, d_scales));
         } else {
             GPFQ_TRY(dispatch_sweep_tile(ctx, NT, G1, G2, N0, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te,
-                                         tb > 0 ? Do : nullptr, R));
+                                         tb > 0 ? Do : nullptr, R, d_scales));
         }
     }
     for (int a = 0; a < n_alph; ++a) {

@@ -38,13 +38,14 @@ __global__ void __launch_bounds__(256) row_norms_kernel(const float *__restrict_
     }
 }
 
-template <int J>
+// SCALED: neuron jb + j of the shard walks with the levels scales[jb + j] * alphabet (common.cuh)
+template <int J, bool SCALED = false>
 __global__ void __launch_bounds__(STREAM_T)
 dense_stream_kernel(const float *__restrict__ X, const float *__restrict__ Xq, int64_t ldx, int64_t N0,
                     int64_t m, const float *__restrict__ W, int64_t ldw, int64_t j0, int64_t nj,
                     const double *__restrict__ nrm, const double *__restrict__ alphabet, int K,
                     double *__restrict__ Q, int64_t ldq, int64_t col0, double *__restrict__ u_scratch,
-                    int u_in_smem) {
+                    int u_in_smem, const double *__restrict__ scales = nullptr) {
     extern __shared__ __align__(16) unsigned char stream_smem[];
     constexpr int NW = STREAM_T / 32;
     __shared__ double red[NW][2 * J];
@@ -59,6 +60,7 @@ dense_stream_kernel(const float *__restrict__ X, const float *__restrict__ Xq, i
     for (int e = tid; e < K; e += STREAM_T) alph[e] = alphabet[e];
     for (int64_t e = tid; e < (int64_t)J * m; e += STREAM_T) u[e] = 0.0;
     __syncthreads();
+    const double sc = (SCALED && tid < J && jb + tid < nj) ? scales[jb + tid] : 0.0;
 
     float wprev[J];
     double qprev[J];
@@ -109,7 +111,8 @@ dense_stream_kernel(const float *__restrict__ X, const float *__restrict__ Xq, i
         if (tid < J) {
             double dd = 0.0, ss = 0.0;
             for (int wv = 0; wv < NW; ++wv) { dd += red[wv][tid]; ss += red[wv][J + tid]; }
-            const double q = gpfq_decide(nrm[t], dd, ss, (double)w[tid], alph, K);
+            const double q = SCALED ? gpfq_decide_unit<true>(nrm[t], dd, ss, (double)w[tid], alph, K, 0.0, sc)
+                                    : gpfq_decide(nrm[t], dd, ss, (double)w[tid], alph, K);
             qsh[tid] = q;
             if (jb + tid < nj) Q[t * ldq + col0 + jb + tid] = q;
         }
@@ -164,21 +167,27 @@ __device__ __forceinline__ int warp_reduce_index(int lane) {
     return idx;
 }
 
-template <int EPV, int J, bool LITERAL, bool VEC>
+template <int EPV, int J, bool LITERAL, bool VEC, bool SCALED = false>
 __global__ void __launch_bounds__(STREAM_T)
 dense_stream_reg_kernel(const float *__restrict__ X, const float *__restrict__ Xq, int64_t ldx, int64_t N0,
                         int64_t m, const float *__restrict__ W, int64_t ldw, int64_t j0, int64_t nj,
                         const double *__restrict__ nrm, const double *__restrict__ g1d,
                         const double *__restrict__ alphabet, int K, int equispaced,
-                        double *__restrict__ Q, int64_t ldq, int64_t col0) {
+                        double *__restrict__ Q, int64_t ldq, int64_t col0, const double *__restrict__ scales = nullptr) {
     constexpr int NW = STREAM_T / 32, EPT = 4 * EPV;
     constexpr int V = LITERAL ? 2 * J : J;  // values reduced per step
     __shared__ double red[NW][V];
     __shared__ double qsh[J];
     __shared__ double alph[GPFQ_MAX_K];
+    __shared__ double unit_s[SCALED ? 2 * J : 1];  // per neuron: scale, inv_step of its levels
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int64_t jb = (int64_t)blockIdx.x * J;
     for (int e = tid; e < K; e += STREAM_T) alph[e] = alphabet[e];
+    if (SCALED && tid < J) {
+        const double sc = jb + tid < nj ? scales[jb + tid] : 0.0;
+        unit_s[tid] = sc;
+        unit_s[J + tid] = gpfq_inv_step_s(alphabet, K, equispaced, sc);
+    }
 
     double u[J][EPT];
 #pragma unroll
@@ -278,7 +287,8 @@ dense_stream_reg_kernel(const float *__restrict__ X, const float *__restrict__ X
 #pragma unroll
                     for (int jj = 1; jj < J; ++jj) wj = (j == jj) ? w[jj] : wj;
                     const double num = LITERAL ? ss : fma((double)wj, g1_t, dd);
-                    const double q = gpfq_decide(nrm_t, dd, num, (double)wj, alph, K, inv_step);
+                    const double q = SCALED ? gpfq_decide_unit<true>(nrm_t, dd, num, (double)wj, alph, K, unit_s[J + j], unit_s[j])
+                                            : gpfq_decide(nrm_t, dd, num, (double)wj, alph, K, inv_step);
                     qsh[j] = q;
                     if (jb + j < nj) Q[t * ldq + col0 + jb + j] = q;
                 }
@@ -311,13 +321,18 @@ template <int EPV, int J>
 static int launch_stream_reg(gpfq_ctx *ctx, bool literal, bool vec, const float *X, const float *Xq, int64_t ldx,
                              int64_t N0, int64_t m, const float *W, int64_t ldw, int64_t j0, int64_t nj,
                              const double *nrm, const double *g1d, const double *d_alph, int K, int eq, double *Qd,
-                             int64_t ldq, int64_t col0) {
+                             int64_t ldq, int64_t col0, const double *scales) {
     const unsigned nblk = (unsigned)ceil_div64(nj, J);
-#define LAUNCH(LIT, VEC) \
-    dense_stream_reg_kernel<EPV, J, LIT, VEC><<<nblk, STREAM_T, 0, ctx->stream>>>(X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm, \
-                                                                               g1d, d_alph, K, eq, Qd, ldq, col0)
-    if (literal) { if (vec) LAUNCH(true, true); else LAUNCH(true, false); }
-    else { if (vec) LAUNCH(false, true); else LAUNCH(false, false); }
+#define LAUNCH(LIT, VEC, S) \
+    dense_stream_reg_kernel<EPV, J, LIT, VEC, S><<<nblk, STREAM_T, 0, ctx->stream>>>(X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm, \
+                                                                                  g1d, d_alph, K, eq, Qd, ldq, col0, scales)
+    if (scales) {
+        if (literal) { if (vec) LAUNCH(true, true, true); else LAUNCH(true, false, true); }
+        else { if (vec) LAUNCH(false, true, true); else LAUNCH(false, false, true); }
+    } else {
+        if (literal) { if (vec) LAUNCH(true, true, false); else LAUNCH(true, false, false); }
+        else { if (vec) LAUNCH(false, true, false); else LAUNCH(false, false, false); }
+    }
 #undef LAUNCH
     KERNEL_CHECK(ctx);
     return GPFQ_OK;
@@ -327,11 +342,11 @@ static int launch_stream_reg(gpfq_ctx *ctx, bool literal, bool vec, const float 
 static int dispatch_stream_reg(gpfq_ctx *ctx, int epv, int J, bool literal, bool vec, const float *X, const float *Xq,
                                int64_t ldx, int64_t N0, int64_t m, const float *W, int64_t ldw, int64_t j0, int64_t nj,
                                const double *nrm, const double *g1d, const double *d_alph, int K, int eq, double *Qd,
-                               int64_t ldq, int64_t col0) {
+                               int64_t ldq, int64_t col0, const double *scales) {
 #define SR(E, JJ) \
     if (epv == E && J == JJ) \
         return launch_stream_reg<E, JJ>(ctx, literal, vec, X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm, g1d, d_alph, K, eq, Qd, \
-                                        ldq, col0);
+                                        ldq, col0, scales);
     SR(1, 1) SR(1, 2) SR(1, 4)
     SR(2, 1) SR(2, 2)
     SR(3, 1) SR(3, 2)
@@ -343,29 +358,29 @@ static int dispatch_stream_reg(gpfq_ctx *ctx, int epv, int J, bool literal, bool
 template <int J>
 static int launch_stream(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ldx, int64_t N0, int64_t m,
                          const float *W, int64_t ldw, int64_t j0, int64_t nj, const double *nrm,
-                         const double *d_alph, int K, double *Qd, int64_t ldq, int64_t col0) {
+                         const double *d_alph, int K, double *Qd, int64_t ldq, int64_t col0, const double *scales) {
     const int64_t nblk = ceil_div64(nj, J);
     const size_t need = (size_t)J * m * sizeof(double);
     const size_t static_smem = 8192;  // red/qsh/alph, generous
     const bool in_smem = need + static_smem <= ctx->smem_optin;
     double *scratch = nullptr;
     if (!in_smem) GPFQ_TRY(gpfq_ws(ctx, WS_U, (size_t)nblk * need, (void **)&scratch));
-    auto k = dense_stream_kernel<J>;
+    auto k = scales ? dense_stream_kernel<J, true> : dense_stream_kernel<J, false>;
     if (in_smem)
         CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)need));
     k<<<(unsigned)nblk, STREAM_T, in_smem ? need : 0, ctx->stream>>>(X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm,
                                                                    d_alph, K, Qd, ldq, col0, scratch,
-                                                                   in_smem ? 1 : 0);
+                                                                   in_smem ? 1 : 0, scales);
     KERNEL_CHECK(ctx);
     return GPFQ_OK;
 }
 
 // Dense layer by the streaming walk.  Device pointers.  Alphabets are walked one after another
-// (each needs its own residual); Qd: (n_alph, N0, ldq).
+// (each needs its own residual); Qd: (n_alph, N0, ldq).  d_scales (nullable): (n_alph, nj) per-neuron scales of the shard.
 int dense_stream_path(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ldx, int64_t N0, int64_t m,
                       const float *W, int64_t ldw, int64_t j0, int64_t nj, const double *d_alph,
                       const int *h_koff, const int *h_flags, int n_alph, double *Qd, int64_t ldq, int64_t col0,
-                      gpfq_stats *st) {
+                      gpfq_stats *st, const double *d_scales) {
     double *nrm = nullptr;
     GPFQ_TRY(gpfq_ws(ctx, WS_NRM, (size_t)2 * N0 * sizeof(double), (void **)&nrm));
     double *g1d = nrm + N0;
@@ -384,7 +399,7 @@ int dense_stream_path(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ld
             const double *al = d_alph + h_koff[a];
             const int K = h_koff[a + 1] - h_koff[a];
             GPFQ_TRY(dispatch_stream_reg(ctx, epv, J, literal, vec, X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm, g1d, al, K,
-                                         h_flags[a], Qd + (int64_t)a * N0 * ldq, ldq, col0));
+                                         h_flags[a], Qd + (int64_t)a * N0 * ldq, ldq, col0, d_scales ? d_scales + a * nj : nullptr));
         }
     } else {
         // long sample axis: residual in shared memory (or an L2-resident scratch), literal arithmetic
@@ -396,9 +411,10 @@ int dense_stream_path(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ld
             const double *al = d_alph + h_koff[a];
             const int K = h_koff[a + 1] - h_koff[a];
             double *Qa = Qd + (int64_t)a * N0 * ldq;
-            if (J == 4) GPFQ_TRY(launch_stream<4>(ctx, X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm, al, K, Qa, ldq, col0));
-            else if (J == 2) GPFQ_TRY(launch_stream<2>(ctx, X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm, al, K, Qa, ldq, col0));
-            else GPFQ_TRY(launch_stream<1>(ctx, X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm, al, K, Qa, ldq, col0));
+            const double *sa = d_scales ? d_scales + a * nj : nullptr;
+            if (J == 4) GPFQ_TRY(launch_stream<4>(ctx, X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm, al, K, Qa, ldq, col0, sa));
+            else if (J == 2) GPFQ_TRY(launch_stream<2>(ctx, X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm, al, K, Qa, ldq, col0, sa));
+            else GPFQ_TRY(launch_stream<1>(ctx, X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm, al, K, Qa, ldq, col0, sa));
         }
     }
     CUDA_TRY(ctx, gpfq_record(ctx, 3, ctx->stream));

@@ -44,6 +44,7 @@ struct SlSeg {
     int a_row0, b_row0;     // first row of this product inside the A / B slice tensors (the tile offset is added)
     int k0, k0b, kblocks;   // first K byte of A / of B and K blocks of 64 bytes
     double alpha;
+    const double *row_mul;  // per-row multiplier of alpha, indexed like the slice rows (nullptr: none; ROWMUL kernels only)
     const int32_t *eA;      // row exponents, indexed like the slice rows (nullptr: eA_const)
     int eA_const;
     const int8_t *A, *B;    // slice tensors (K-block tiled, pre-swizzled: sl_offset)
@@ -91,6 +92,9 @@ __device__ __forceinline__ void sl_issue_kblock(uint32_t tmem_base, uint64_t da,
     }
 }
 
+// ROWMUL: a segment with row_mul scales its rows by alpha * row_mul[row] (the per-neuron level step of the residual form's Q part
+// with per-channel alphabets); the kernel without it is the one every other product uses.
+template <bool ROWMUL>
 __global__ void __launch_bounds__(slg::THREADS, 1)
 slgemm_i8_kernel(const SlArgs args) {
     using namespace i8g;
@@ -212,11 +216,12 @@ slgemm_i8_kernel(const SlArgs args) {
         for (int sg = 0; sg < args.nseg; ++sg) {
             const SlSeg &g = args.seg[sg];
             const int ea = g.eA ? g.eA[g.a_row0 + brow_a + ti * TM + row_t] : g.eA_const;
+            const double alpha = (ROWMUL && g.row_mul) ? g.alpha * g.row_mul[g.a_row0 + brow_a + ti * TM + row_t] : g.alpha;
             mbar_wait(seg_full, sg & 1);
             asm volatile("tcgen05.fence::after_thread_sync;\n" ::: "memory");
 #pragma unroll 1
             for (int d = 2; d <= g.D; ++d) {
-                const double rs = ldexp(g.alpha, 4 - 8 * d + ea);
+                const double rs = ldexp(alpha, 4 - 8 * d + ea);
 #pragma unroll
                 for (int hf = 0; hf < TN / 32; ++hf) {
                     uint32_t v[32];
@@ -485,6 +490,7 @@ int slgemm_i8_ex(gpfq_ctx *ctx, const SlProduct *prod, int nprod, double *C, int
         g.k0b = (int)k0b;
         g.kblocks = (int)(p.K / BK);
         g.alpha = p.alpha;
+        g.row_mul = p.row_mul;
         g.eA = p.A->e;
         g.eA_const = p.A->e_const;
         g.A = p.A->slices;
@@ -510,9 +516,11 @@ int slgemm_i8_ex(gpfq_ctx *ctx, const SlProduct *prod, int nprod, double *C, int
     a.lower_only = batch.lower_only ? 1 : 0;
     a.ktri = batch.ktri ? 1 : 0;
     if (nbatch < 1 || nbatch > 65535) return gpfq_fail(ctx, GPFQ_ERR_ARG, "slgemm_i8: 1..65535 batches");
-    CUDA_TRY(ctx, cudaFuncSetAttribute(slgemm_i8_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM));
+    const bool rowmul = a.seg[0].row_mul || (nprod > 1 && a.seg[1].row_mul);
+    auto k = rowmul ? slgemm_i8_kernel<true> : slgemm_i8_kernel<false>;
+    CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM));
     const dim3 grid((unsigned)(ceil_div64(M, TM) * a.tiles_n), (unsigned)nbatch);
-    slgemm_i8_kernel<<<grid, THREADS, SMEM, ctx->stream>>>(a);
+    k<<<grid, THREADS, SMEM, ctx->stream>>>(a);
     KERNEL_CHECK(ctx);
     return GPFQ_OK;
 }

@@ -27,6 +27,7 @@ struct SlProduct {          // one segment: alpha * A[a_row0 : a_row0 + M, k0 : 
     int D;
     double alpha;
     int64_t k0b = -1;       // first K byte of the B operand when it differs from A's (-1: k0)
+    const double *row_mul = nullptr;   // optional fp64 multiplier per A row (indexed like the A rows): alpha * row_mul[row]
 };
 
 struct SlBatch {            // blockIdx.y batches: per batch the A rows advance by a_rows, the B rows (and the exponents of both) by

@@ -94,10 +94,15 @@ __device__ __forceinline__ void tmem_ld_5x16(uint32_t taddr, uint32_t (&v)[S][16
 
 // The literal walk of one block from the saved residual dots (own shared-memory column), for a warp that raised a flag:
 // gpfq_decide_rcp_inl of dense_gram.cu with the ternary scan.  Rolled loops; decisions go out as level indices.
+// SCALED: the neuron's levels are fl(s alph[k]) (per-channel alphabets; a = fl(s alph[K - 1]), `alph` the base alphabet); a neuron
+// with s = 0 decides the literal 0 everywhere (its levels are all zero) and never reaches the divisions by a.
+template <bool SCALED>
 static __device__ __noinline__ void replay_block(unsigned char *dset, const unsigned char *wset, int j, const TabA *tab, double a,
-                                                 int8_t *qcol, const double *alph, int K) {
+                                                 int8_t *qcol, const double *alph, int K, double s) {
     // K == 3: the ternary scan with the levels in registers; else the windowed scan of the equispaced levels (common.cuh)
-    const double inv_step = 0.5 * (double)(K - 1) / a, inv_h = (double)(K - 1) / a;
+    const bool zero = SCALED && !(a > 0.0);
+    const double inv_step = zero ? 0.0 : (SCALED ? gpfq_inv_step_s(alph, K, 1, s) : 0.5 * (double)(K - 1) / a);
+    const double inv_h = zero ? 0.0 : (double)(K - 1) / a;
     auto dptr = [&](int t) { return reinterpret_cast<double *>(dset + (t >> 4) * (D_BYTES / 2) + sw128(j, (t & 15) >> 1)) + (t & 1); };
     for (int t = 0; t < NB; ++t) {
         const double d0 = *dptr(t);
@@ -112,7 +117,9 @@ static __device__ __noinline__ void replay_block(unsigned char *dset, const unsi
                 const double e = fma(-q0, tab->den[t], num);
                 v = fma(e, rinv, q0);
             }
-            q = K == 3 ? gpfq_bit_round_ternary(v, a) : gpfq_bit_round_eq(v, alph, K, inv_step);
+            if (zero) q = 0.0;
+            else if (K == 3) q = gpfq_bit_round_ternary(v, a);
+            else q = SCALED ? gpfq_bit_round_eq_s(v, alph, K, inv_step, s) : gpfq_bit_round_eq(v, alph, K, inv_step);
         }
         qcol[t * NT] = (int8_t)__double2int_rn(q * inv_h);   // level index k' = q / h, h = a / (K - 1); the literal 0 of a dead direction is 0
         for (int u = t + 1; u < NB; ++u) {
@@ -122,11 +129,17 @@ static __device__ __noinline__ void replay_block(unsigned char *dset, const unsi
     }
 }
 
-template <bool TERN>
+// SCALED (per-channel alphabets): neuron jg walks with its own levels fl(scales[jg] levels[k]) -- a = fl(s levels[K - 1]) and the step
+// h = a / (K - 1) per walker, from tables prepared with h = 1 (TabA::sc = 2^(e - 38), TabA::ris = rinv / 2); `levels` is the base
+// alphabet.  Applying h per walker adds one rounding to the grid position (ris / h: RN(RN(rinv / 2) * RN(1 / h)) against RN(rinv / 2h),
+// at most 2 ulp of kr < 2^7), far inside the 2^-30 band that flags a tie; the Q-term scale h 2^(e - 38) stays exact.  The ternary
+// thresholds +- a / 2 and their flag window are per walker.
+template <bool TERN, bool SCALED = false>
 __global__ void __launch_bounds__(THREADS, 1)
 sweep_tc_kernel(const __grid_constant__ CUtensorMap mapP, const __grid_constant__ CUtensorMap mapW, const TabA *__restrict__ tabs,
                 const int8_t *__restrict__ g2s, int kbr, int64_t tb, int64_t te, int row0, int64_t nj, int8_t *__restrict__ Kq,
-                int64_t krows, int64_t krow0, double a, const double *__restrict__ levels, int K) {
+                int64_t krows, int64_t krow0, double a_base, const double *__restrict__ levels, int K,
+                const double *__restrict__ scales = nullptr) {
     using namespace i8g;
     extern __shared__ unsigned char stc_smem_raw[];
     // (offset arithmetic on the array itself: the compiler keeps the shared address space, LDS / STS instead of generic accesses)
@@ -167,6 +180,10 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap mapP, const __grid_constant_
         const int j = tid;
         const int64_t jg = (int64_t)blockIdx.x * NT + j;
         const bool valid = jg < nj;   // (rows beyond nj exist in P / Wn -- allocation padding -- and hold whatever they hold)
+        const double s_u = SCALED ? (valid ? scales[jg] : 0.0) : 1.0;
+        const double a = SCALED ? __dmul_rn(s_u, a_base) : a_base;
+        const bool zero = SCALED && !(a > 0.0);                     // s = 0: every decision is the literal 0, no replay
+        const double h_u = SCALED ? (zero ? 0.0 : a / (double)(K - 1)) : 1.0, inv_hu = SCALED ? (zero ? 0.0 : 1.0 / h_u) : 1.0;
         const double hh = 0.5 * a;
         // flags of the ternary walk, compared as high words: [hi(a / 2) - 1, hi(a / 2) + 1] around the thresholds (a window of ~2^-20
         // relative: one warp-block in ~300 replays), a * 2^40 and above (NaN / Inf included), 1e-10 and below (:86)
@@ -204,7 +221,8 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap mapP, const __grid_constant_
                         long long I = (long long)(int)v[0][i];
 #pragma unroll
                         for (int s = 1; s < S; ++s) I = I * 256 + (long long)(int)v[s][i];
-                        d[hf * 16 + i] = fma(-tab->sc[hf * 16 + i], (double)I, d[hf * 16 + i]);
+                        const double sc = SCALED ? h_u * tab->sc[hf * 16 + i] : tab->sc[hf * 16 + i];   // exact: sc = 2^(e - 38)
+                        d[hf * 16 + i] = fma(-sc, (double)I, d[hf * 16 + i]);
                     }
                 }
                 asm volatile("tcgen05.fence::before_thread_sync;\n" ::: "memory");
@@ -241,7 +259,7 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap mapP, const __grid_constant_
                     m_perp = min(m_perp, ((uint32_t)__double2hiint(d[t]) & 0x7fffffffu) | (uint32_t)tab->deadm[t]);
                     pk[t >> 2] |= (up ? 2u : (dn ? 0xfeu : 0u)) << (8 * (t & 3));   // level index k' = q / h = +-2 (h = a / 2)
                 } else {
-                    const double kr = fma(num, tab->ris[t], cmid);          // ris = rinv / s
+                    const double kr = fma(num, SCALED ? tab->ris[t] * inv_hu : tab->ris[t], cmid);   // ris = rinv / s
                     const double r0 = (kr + magic) - magic;                  // rint(kr)
                     const double r = fmin(fmax(r0, 0.0), km1);
                     const bool live = ri != 0.0;
@@ -263,9 +281,14 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap mapP, const __grid_constant_
                 if (kbr == -1 - t) asm volatile("trap;\n");
             }
             if (TERN) flag = (int)(m_near <= 2u) | (int)(m_big >= big_hi) | (int)(m_perp <= perp_hi);
+            if (SCALED && zero) {
+                flag = 0;
+#pragma unroll
+                for (int i = 0; i < NB / 4; ++i) pk[i] = 0u;
+            }
             if (__any_sync(0xffffffffu, flag != 0 && valid)) {   // (rows beyond nj hold zeros: they would trip the :86 guard at every step)
                 int8_t *qcol = reinterpret_cast<int8_t *>(smem + OFF_Q) + j;
-                replay_block(dset, wset, j, tab, a, qcol, alph, K);
+                replay_block<SCALED>(dset, wset, j, tab, a, qcol, alph, K, s_u);
 #pragma unroll
                 for (int i = 0; i < NB / 4; ++i) {
                     uint32_t w4 = 0u;
@@ -511,12 +534,17 @@ __global__ void stc_add_partials_kernel(double *__restrict__ P, int64_t ldp, con
 
 // Qt[j][t] = the level of index Kq[j][t] for the directions [tb, te): the neuron-major fp64 decisions the Gram-row contraction of the
 // later ranges reads
+// (scales, per-channel alphabets: neuron j's levels are fl(scales[j] levels[k]))
+template <bool SCALED>
 __global__ void stc_qt_from_kq_kernel(const int8_t *__restrict__ Kq, int64_t krows, int64_t tb, int64_t te, int64_t nj,
-                                      const double *__restrict__ levels, int K, double *__restrict__ Qt, int64_t ldq) {
+                                      const double *__restrict__ levels, int K, double *__restrict__ Qt, int64_t ldq,
+                                      const double *__restrict__ scales) {
     const int64_t j = blockIdx.x;
+    const double s = SCALED ? scales[j] : 1.0;
     for (int64_t t = tb + threadIdx.x; t < te; t += blockDim.x) {
         const int k = Kq[sl_offset(t, 0, j, krows, 1)];
-        Qt[j * ldq + t] = k == 0 ? 0.0 : levels[(k + K - 1) >> 1];
+        const double lv = SCALED ? __dmul_rn(s, levels[(k + K - 1) >> 1]) : levels[(k + K - 1) >> 1];
+        Qt[j * ldq + t] = k == 0 ? 0.0 : lv;
     }
 }
 
@@ -538,8 +566,9 @@ __global__ void stc_weights_kernel(const float *__restrict__ W, int64_t ldw, int
 
 // Q[t * ldq + col0 + j] = level of index Kq[j][t] (k' = 2 k - (K - 1); the literal 0 for k' = 0): the layer's quantized weights from
 // the level indices of the walk -- the stored levels themselves, bit for bit
+template <bool SCALED>
 __global__ void stc_q_from_kq_kernel(const int8_t *__restrict__ Kq, int64_t krows, int64_t N0, int64_t nj, const double *__restrict__ levels,
-                                     int K, double *__restrict__ Q, int64_t ldq, int64_t col0) {
+                                     int K, double *__restrict__ Q, int64_t ldq, int64_t col0, const double *__restrict__ scales) {
     __shared__ int8_t tile[32][33];
     const int64_t tb = (int64_t)blockIdx.x * 32, jb = (int64_t)blockIdx.y * 32;
     for (int r = threadIdx.y; r < 32; r += blockDim.y) {
@@ -551,7 +580,8 @@ __global__ void stc_q_from_kq_kernel(const int8_t *__restrict__ Kq, int64_t krow
         const int64_t t = tb + r, j = jb + threadIdx.x;
         if (t < N0 && j < nj) {
             const int k = tile[threadIdx.x][r];
-            Q[t * ldq + col0 + j] = k == 0 ? 0.0 : levels[(k + K - 1) >> 1];
+            const double lv = SCALED ? __dmul_rn(scales[j], levels[(k + K - 1) >> 1]) : levels[(k + K - 1) >> 1];
+            Q[t * ldq + col0 + j] = k == 0 ? 0.0 : lv;
         }
     }
 }
@@ -609,16 +639,18 @@ int sweep_tc_add_partials(gpfq_ctx *ctx, double *P, int64_t ldp, const double *p
 }
 
 int sweep_tc_qt_from_kq(gpfq_ctx *ctx, const int8_t *Kq, int64_t krows, int64_t tb, int64_t te, int64_t nj, const double *levels, int K,
-                        double *Qt, int64_t ldq) {
-    stc::stc_qt_from_kq_kernel<<<(unsigned)nj, 128, 0, ctx->stream>>>(Kq, krows, tb, te, nj, levels, K, Qt, ldq);
+                        double *Qt, int64_t ldq, const double *scales) {
+    if (scales) stc::stc_qt_from_kq_kernel<true><<<(unsigned)nj, 128, 0, ctx->stream>>>(Kq, krows, tb, te, nj, levels, K, Qt, ldq, scales);
+    else stc::stc_qt_from_kq_kernel<false><<<(unsigned)nj, 128, 0, ctx->stream>>>(Kq, krows, tb, te, nj, levels, K, Qt, ldq, nullptr);
     KERNEL_CHECK(ctx);
     return GPFQ_OK;
 }
 
 int sweep_tc_q_from_kq(gpfq_ctx *ctx, const int8_t *Kq, int64_t krows, int64_t N0, int64_t nj, const double *levels, int K, double *Q,
-                       int64_t ldq, int64_t col0) {
+                       int64_t ldq, int64_t col0, const double *scales) {
     dim3 grid((unsigned)ceil_div64(N0, 32), (unsigned)ceil_div64(nj, 32));
-    stc::stc_q_from_kq_kernel<<<grid, dim3(32, 8), 0, ctx->stream>>>(Kq, krows, N0, nj, levels, K, Q, ldq, col0);
+    if (scales) stc::stc_q_from_kq_kernel<true><<<grid, dim3(32, 8), 0, ctx->stream>>>(Kq, krows, N0, nj, levels, K, Q, ldq, col0, scales);
+    else stc::stc_q_from_kq_kernel<false><<<grid, dim3(32, 8), 0, ctx->stream>>>(Kq, krows, N0, nj, levels, K, Q, ldq, col0, nullptr);
     KERNEL_CHECK(ctx);
     return GPFQ_OK;
 }
@@ -652,12 +684,17 @@ int sweep_tc_bind(gpfq_ctx *ctx, TcTables *tab, const double *P, const float *Wn
 }
 
 int sweep_tc_range(gpfq_ctx *ctx, const TcTables &tab, int64_t tb, int64_t te, int64_t row0, int64_t nj, int8_t *Kq, int64_t krows,
-                   int64_t krow0, double a, const double *levels, int K) {
+                   int64_t krow0, double a, const double *levels, int K, const double *scales) {
     using namespace stc;
     if (tb % tab.R || te - tb > tab.R || te <= tb || row0 % NT || row0 + ceil_div64(nj, NT) * NT > tab.rowsP || !Kq || K < 2 || K > 128)
         return gpfq_fail(ctx, GPFQ_ERR_ARG, "sweep_tc: a range starts at a multiple of %lld directions", (long long)tab.R);
     const dim3 grid((unsigned)ceil_div64(nj, NT));
-    if (K == 3) {
+    if (scales) {
+        auto k = K == 3 ? sweep_tc_kernel<true, true> : sweep_tc_kernel<false, true>;
+        CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM));
+        k<<<grid, THREADS, SMEM, ctx->stream>>>(tab.mapP, tab.mapW, tab.tabs, tab.g2s, (int)(tab.R / KB), tb, te, (int)row0, nj, Kq, krows, krow0,
+                                                a, levels, K, scales);
+    } else if (K == 3) {
         CUDA_TRY(ctx, cudaFuncSetAttribute(sweep_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM));
         sweep_tc_kernel<true><<<grid, THREADS, SMEM, ctx->stream>>>(tab.mapP, tab.mapW, tab.tabs, tab.g2s, (int)(tab.R / KB), tb, te, (int)row0, nj,
                                                                     Kq, krows, krow0, a, levels, K);

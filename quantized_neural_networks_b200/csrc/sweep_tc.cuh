@@ -52,19 +52,21 @@ int sweep_tc_slice_g1_lower(gpfq_ctx *ctx, const double *G1, int64_t ldg, bool c
 //   Kq  out: the decisions as int8 level indices k' = q / (a / 2) (sl_offset layout, krows rows, neuron 0 at row krow0)
 int sweep_tc_bind(gpfq_ctx *ctx, TcTables *tab, const double *P, const float *Wn, int64_t rowsP, int64_t ldp);
 //   a, levels, K: the symmetric equispaced alphabet (device levels, a = levels[K - 1]); K == 3 runs the ternary specialisation
+//   scales (nullable, device, this launch's nj neurons): per-channel alphabets -- neuron j walks with fl(scales[j] levels[k]); the
+//       tables must then be prepared with h = 1
 int sweep_tc_range(gpfq_ctx *ctx, const TcTables &tab, int64_t tb, int64_t te, int64_t row0, int64_t nj, int8_t *Kq, int64_t krows,
-                   int64_t krow0, double a, const double *levels, int K);
+                   int64_t krow0, double a, const double *levels, int K, const double *scales = nullptr);
 // Wn[j][t] = W[t * ldw + wcol0 + j], (nj, N0P) fp32, zeros beyond N0
 int sweep_tc_weights(gpfq_ctx *ctx, const float *W, int64_t ldw, int64_t wcol0, int64_t N0, int64_t N0P, int64_t nj, float *Wn);
 // Q[t * ldq + col0 + j] = the level of index Kq[j][t] for t < N0, j < nj
 int sweep_tc_q_from_kq(gpfq_ctx *ctx, const int8_t *Kq, int64_t krows, int64_t N0, int64_t nj, const double *levels, int K, double *Q,
-                       int64_t ldq, int64_t col0);
+                       int64_t ldq, int64_t col0, const double *scales = nullptr);
 // Gram-row form of the sweep (full G1 / G2 in HBM): the strictly lower part of every range's G1 tile as a compact fp64 matrix
 // (N0P, R) for the in-range W terms on the fp64 pipe; P[:, tb : tb + n] += Do; Qt[:, tb : te] from the level indices
 int sweep_tc_mask_g1_lower(gpfq_ctx *ctx, const double *G1, int64_t ldg, int64_t N0, int64_t N0P, int64_t R, double *G1m);
 int sweep_tc_add_outer(gpfq_ctx *ctx, double *P, int64_t ldp, const double *Do, int64_t ldd, int64_t nj, int64_t n);
 int sweep_tc_qt_from_kq(gpfq_ctx *ctx, const int8_t *Kq, int64_t krows, int64_t tb, int64_t te, int64_t nj, const double *levels, int K,
-                        double *Qt, int64_t ldq);
+                        double *Qt, int64_t ldq, const double *scales = nullptr);
 // P[:, 0 : n] += part[0] + ... + part[ns - 1] (partials `stride` elements apart, row stride ldd): the K-split residual dots
 int sweep_tc_add_partials(gpfq_ctx *ctx, double *P, int64_t ldp, const double *part, int ns, int64_t stride, int64_t ldd, int64_t nj,
                           int64_t n);

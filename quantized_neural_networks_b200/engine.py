@@ -37,6 +37,28 @@ def _alph_args(alphabets):
     return flat, K, len(als), als
 
 
+def _scale_args(scales, n_alph, unit_shape, name="scales"):
+    """Per-unit scales (per-channel alphabets) -> a contiguous float64 host array of n_alph x prod(unit_shape), or None.
+    Accepts one table of unit_shape (used by every alphabet) or n_alph of them, as a NumPy array or a tensor."""
+    if scales is None:
+        return None
+    if _is_torch(scales):
+        scales = scales.detach().cpu().numpy()
+    s = np.asarray(scales, dtype=np.float64)
+    unit_shape = tuple(int(v) for v in unit_shape)
+    if s.shape == unit_shape:
+        s = np.broadcast_to(s, (n_alph,) + unit_shape)
+    elif s.shape != (n_alph,) + unit_shape:
+        raise ValueError(f"{name}: shape {s.shape}, expected {unit_shape} or {(n_alph,) + unit_shape}")
+    if not np.all(np.isfinite(s)) or np.any(s < 0):
+        raise ValueError(f"{name}: every scale must be finite and >= 0")
+    return np.ascontiguousarray(s)
+
+
+def _dptr(a):
+    return a.ctypes.data_as(POINTER(c_double))
+
+
 class GpfqEngine:
     """Owns a `gpfq_ctx` (include/gpfq.h).  Fails loudly when the library or an sm_100 GPU is absent."""
 
@@ -125,10 +147,12 @@ class GpfqEngine:
         return x.ctypes.data, (x.strides[0] // x.itemsize if x.shape[0] > 1 else x.shape[1])
 
     # -- Dense ----------------------------------------------------------------------------------
-    def dense_layer(self, X, Xq, W, alphabets, j0=0, j1=None, method="auto", out=None, sync=True):
+    def dense_layer(self, X, Xq, W, alphabets, j0=0, j1=None, method="auto", out=None, sync=True, scales=None):
         """Quantize neurons j0..j1-1 of a Dense layer.  X, Xq: (N0, m) fp32 feature-major (Xq may be
         None or X itself for the first layer); W: (N0, N1) fp32.  Returns Q fp64 (N0, N1) -- or
-        (n_alphabets, N0, N1) when a list of alphabets is given -- with only the shard's columns written."""
+        (n_alphabets, N0, N1) when a list of alphabets is given -- with only the shard's columns written.
+        `scales` (per-channel alphabets): (N1,) or (n_alphabets, N1), finite and >= 0; neuron j then walks with the levels
+        fl64(scales[j] * alphabet[k])."""
         flat, K, n_alph, als = _alph_args(alphabets)
         single = isinstance(alphabets, np.ndarray) and alphabets.ndim == 1
         X = self._f32(X, "X")
@@ -168,11 +192,12 @@ class GpfqEngine:
             if out is None:
                 out = np.zeros((n_alph, N0, N1), dtype=np.float64)
             pout = out.ctypes.data
+        sc = _scale_args(scales, n_alph, (N1,))
         st = _lib.GpfqStats()
-        rc = self._lib.gpfq_dense_layer(self._ctx, c_void_p(px), c_void_p(pq), ldx, N0, m, c_void_p(pw), ldw, N1,
-                                        int(j0), j1, flat.ctypes.data_as(POINTER(c_double)),
-                                        K.ctypes.data_as(POINTER(c_int32)), n_alph, c_void_p(pout), N1, flags,
-                                        byref(st))
+        args = (self._ctx, c_void_p(px), c_void_p(pq), ldx, N0, m, c_void_p(pw), ldw, N1, int(j0), j1,
+                flat.ctypes.data_as(POINTER(c_double)), K.ctypes.data_as(POINTER(c_int32)), n_alph, c_void_p(pout), N1, flags,
+                byref(st))
+        rc = self._lib.gpfq_dense_layer(*args) if sc is None else self._lib.gpfq_dense_layer_scaled(*args, _dptr(sc))
         self._check(rc)
         self.last_stats = st.as_dict()
         return out[0] if single else out
@@ -217,10 +242,10 @@ class GpfqEngine:
         self._check(rc)
         return G1, G2
 
-    def dense_layer_from_gram(self, G1, G2, W, alphabets, j0=0, j1=None, out=None, sync=True):
+    def dense_layer_from_gram(self, G1, G2, W, alphabets, j0=0, j1=None, out=None, sync=True, scales=None):
         """Sweep stage of a Dense layer from (N0, N0) fp64 Gram matrices on the device (CUDA tensors; G1 None or G2
         itself for the first layer): what every rank of a sample-split job runs after the all-reduce of the partial
-        Grams.  W: (N0, N1) fp32 NumPy array or CUDA tensor; the result follows W's kind."""
+        Grams.  W: (N0, N1) fp32 NumPy array or CUDA tensor; the result follows W's kind.  `scales` as in `dense_layer`."""
         flat, K, n_alph, als = _alph_args(alphabets)
         single = isinstance(alphabets, np.ndarray) and alphabets.ndim == 1
         if not _is_torch(G2) or G2.dtype != torch.float64 or not G2.is_cuda or not G2.is_contiguous():
@@ -254,21 +279,23 @@ class GpfqEngine:
             if out is None:
                 out = np.zeros((n_alph, N0, N1), dtype=np.float64)
             pout = out.ctypes.data
+        sc = _scale_args(scales, n_alph, (N1,))
         st = _lib.GpfqStats()
-        rc = self._lib.gpfq_dense_layer_from_gram(self._ctx, c_void_p(None if same else G1.data_ptr()),
-                                                  c_void_p(G2.data_ptr()), N0, c_void_p(pw), ldw, N1, int(j0), j1,
-                                                  flat.ctypes.data_as(POINTER(c_double)),
-                                                  K.ctypes.data_as(POINTER(c_int32)), n_alph, c_void_p(pout), N1, flags,
-                                                  byref(st))
+        args = (self._ctx, c_void_p(None if same else G1.data_ptr()), c_void_p(G2.data_ptr()), N0, c_void_p(pw), ldw, N1,
+                int(j0), j1, flat.ctypes.data_as(POINTER(c_double)), K.ctypes.data_as(POINTER(c_int32)), n_alph,
+                c_void_p(pout), N1, flags, byref(st))
+        rc = (self._lib.gpfq_dense_layer_from_gram(*args) if sc is None
+              else self._lib.gpfq_dense_layer_from_gram_scaled(*args, _dptr(sc)))
         self._check(rc)
         self.last_stats = st.as_dict()
         return out[0] if single else out
 
     # -- Conv -----------------------------------------------------------------------------------
-    def conv_channels(self, Xp, Xqp, W, alphabets, c0=0, n_channels=None, out=None, sync=True):
+    def conv_channels(self, Xp, Xqp, W, alphabets, c0=0, n_channels=None, out=None, sync=True, scales=None):
         """Quantize channels c0..c0+n_channels-1 of a (kh, kw, C, F) kernel from per-channel patch
         matrices.  Xp/Xqp: sequences (len n_channels) of (kh*kw, n_patches) fp32 arrays/tensors, or one
-        (n_channels, kh*kw, n_patches) array; Xqp None => first conv layer (X == Xq)."""
+        (n_channels, kh*kw, n_patches) array; Xqp None => first conv layer (X == Xq).  `scales` (per-channel alphabets):
+        (C, F) or (n_alphabets, C, F), finite and >= 0; the slice W[:, :, c, f] walks with fl64(scales[c, f] * alphabet[k])."""
         flat, K, n_alph, als = _alph_args(alphabets)
         single = isinstance(alphabets, np.ndarray) and alphabets.ndim == 1
         W = self._f32(W, "W")
@@ -308,10 +335,11 @@ class GpfqEngine:
             if out is None:
                 out = np.zeros((n_alph, kh, kw, C, F), dtype=np.float64)
             pout = out.ctypes.data
+        sc = _scale_args(scales, n_alph, (C, F))
         st = _lib.GpfqStats()
-        rc = self._lib.gpfq_conv_channels(self._ctx, PX, PQ, n, kk, c_void_p(ptr(W)), C, F, int(c0), n_channels,
-                                          flat.ctypes.data_as(POINTER(c_double)), K.ctypes.data_as(POINTER(c_int32)),
-                                          n_alph, c_void_p(pout), flags, byref(st))
+        args = (self._ctx, PX, PQ, n, kk, c_void_p(ptr(W)), C, F, int(c0), n_channels, flat.ctypes.data_as(POINTER(c_double)),
+                K.ctypes.data_as(POINTER(c_int32)), n_alph, c_void_p(pout), flags, byref(st))
+        rc = self._lib.gpfq_conv_channels(*args) if sc is None else self._lib.gpfq_conv_channels_scaled(*args, _dptr(sc))
         self._check(rc)
         self.last_stats = st.as_dict()
         return out[0] if single else out
@@ -326,10 +354,11 @@ class GpfqEngine:
         return groups
 
     def conv_layer_nhwc(self, act, actq, W, alphabets, strides=(1, 1), padding="SAME", rate=(1, 1), c0=0,
-                        n_channels=None, out=None, sync=True, groups=1):
+                        n_channels=None, out=None, sync=True, groups=1, scales=None):
         """Quantize a Conv2D kernel straight from the NHWC activations (on-device patch extraction).  With `groups` > 1, W is the
         (kh, kw, C / groups, F) kernel of a grouped Conv2D: input channel c is walked against the F / groups filters of its group
-        c // (C / groups); c0 / n_channels index input channels.  The result has W's shape."""
+        c // (C / groups); c0 / n_channels index input channels.  The result has W's shape.  `scales` (per-channel alphabets):
+        (C / groups, F) or (n_alphabets, C / groups, F), indexed like W's last two axes."""
         flat, K, n_alph, als = _alph_args(alphabets)
         single = isinstance(alphabets, np.ndarray) and alphabets.ndim == 1
         W = self._f32(W, "W")
@@ -368,12 +397,16 @@ class GpfqEngine:
             if out is None:
                 out = np.zeros((n_alph, kh, kw, Cg, F), dtype=np.float64)
             pout = out.ctypes.data
+        sc = _scale_args(scales, n_alph, (Cg, F))
         st = _lib.GpfqStats()
         args = (self._ctx, c_void_p(ptr(act)), c_void_p(ptr(actq)), n_img, H, Wd, C, kh, kw, int(strides[0]), int(strides[1]),
                 int(rate[0]), int(rate[1]), 1 if str(padding).upper() == "SAME" else 0, c_void_p(ptr(W)), F, int(c0), n_channels,
                 flat.ctypes.data_as(POINTER(c_double)), K.ctypes.data_as(POINTER(c_int32)), n_alph, c_void_p(pout), flags,
                 byref(st))
-        rc = (self._lib.gpfq_conv_layer_nhwc_grouped(*args, groups) if groups > 1 else self._lib.gpfq_conv_layer_nhwc(*args))
+        if sc is not None:
+            rc = self._lib.gpfq_conv_layer_nhwc_scaled(*args, groups, _dptr(sc))
+        else:
+            rc = (self._lib.gpfq_conv_layer_nhwc_grouped(*args, groups) if groups > 1 else self._lib.gpfq_conv_layer_nhwc(*args))
         self._check(rc)
         self.last_stats = st.as_dict()
         return out[0] if single else out
@@ -414,11 +447,11 @@ class GpfqEngine:
         self.last_stats = self.query_stats(0)
         return gram
 
-    def conv_layer_from_gram(self, gram, W, alphabets, c0=0, n_channels=None, out=None, sync=True, groups=1):
+    def conv_layer_from_gram(self, gram, W, alphabets, c0=0, n_channels=None, out=None, sync=True, groups=1, scales=None):
         """Walks of every filter of channels c0..c0+n_channels-1 from per-channel Gram matrices on the device
         (`conv_gram_nhwc`, summed over the ranks of an image-split job).  W: (kh, kw, C, F) NumPy array or CUDA tensor; with
         `groups` > 1 the (kh, kw, C / groups, F) kernel of a grouped Conv2D, each input channel walked against the F / groups
-        filters of its group (c0 / n_channels index input channels, as in the Gram stage)."""
+        filters of its group (c0 / n_channels index input channels, as in the Gram stage).  `scales` as in `conv_layer_nhwc`."""
         flat, K, n_alph, als = _alph_args(alphabets)
         single = isinstance(alphabets, np.ndarray) and alphabets.ndim == 1
         W = self._f32(W, "W")
@@ -445,11 +478,15 @@ class GpfqEngine:
             if out is None:
                 out = np.zeros((n_alph, kh, kw, Cg, F), dtype=np.float64)
             pout, pw = out.ctypes.data, W.ctypes.data
+        sc = _scale_args(scales, n_alph, (Cg, F))
         st = _lib.GpfqStats()
         args = (self._ctx, c_void_p(gram.data_ptr()), kk, c_void_p(pw), C, F, int(c0), n_channels,
                 flat.ctypes.data_as(POINTER(c_double)), K.ctypes.data_as(POINTER(c_int32)), n_alph, c_void_p(pout), flags, byref(st))
-        rc = (self._lib.gpfq_conv_layer_from_gram_grouped(*args, groups) if groups > 1
-              else self._lib.gpfq_conv_layer_from_gram(*args))
+        if sc is not None:
+            rc = self._lib.gpfq_conv_layer_from_gram_scaled(*args, groups, _dptr(sc))
+        else:
+            rc = (self._lib.gpfq_conv_layer_from_gram_grouped(*args, groups) if groups > 1
+                  else self._lib.gpfq_conv_layer_from_gram(*args))
         self._check(rc)
         self.last_stats = st.as_dict()
         return out[0] if single else out
@@ -469,12 +506,25 @@ class GpfqEngine:
                                                 1 if transposed_b else 0, c_void_p(C.ctypes.data)))
         return C
 
-    def msq(self, W, alphabet):
-        """Plain nearest-level rounding of every weight (the MSQ baseline of the reference's drivers)."""
+    def msq(self, W, alphabet, scales=None):
+        """Plain nearest-level rounding of every weight (the MSQ baseline of the reference's drivers).  `scales` (per-channel
+        alphabets): one scale per unit of W's last axis (a Dense neuron or a conv filter), shape (W.shape[-1],) or W.shape[-2:]
+        for a conv kernel's (C, F) table; weight W[..., u] rounds to the levels fl64(scales[u] * alphabet[k])."""
         W = np.ascontiguousarray(W, dtype=np.float32)
         A = np.ascontiguousarray(alphabet, dtype=np.float64)
         out = np.zeros(W.shape, dtype=np.float64)
         self._bind_stream(False)
+        if scales is not None:
+            s = np.asarray(scales.detach().cpu().numpy() if _is_torch(scales) else scales, dtype=np.float64)
+            if W.ndim < 1 or s.shape not in (W.shape[-1:], W.shape[-2:]):
+                raise ValueError(f"scales: shape {s.shape}, expected {W.shape[-1:]} or {W.shape[-2:]}")
+            if not np.all(np.isfinite(s)) or np.any(s < 0):
+                raise ValueError("scales: every scale must be finite and >= 0")
+            s = np.ascontiguousarray(s).reshape(-1)
+            rc = self._lib.gpfq_msq_scaled(self._ctx, c_void_p(W.ctypes.data), W.size, A.ctypes.data_as(POINTER(c_double)),
+                                           len(A), _dptr(s), s.size, c_void_p(out.ctypes.data), 0)
+            self._check(rc)
+            return out
         rc = self._lib.gpfq_msq(self._ctx, c_void_p(W.ctypes.data), W.size, A.ctypes.data_as(POINTER(c_double)), len(A),
                                 c_void_p(out.ctypes.data), 0)
         self._check(rc)

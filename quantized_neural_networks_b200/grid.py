@@ -28,31 +28,48 @@ from .quantized_network import QuantizedCNN
 LAYER_KINDS = ("Dense", "Conv2D", "DepthwiseConv2D")
 
 
-def pack_levels(Q: np.ndarray, alphabet: np.ndarray):
-    """Quantized kernel -> (int8 level indices, alphabet).  Index -1 marks the literal 0.0 a dead direction produces
-    (quantized_network.py:83-84), which need not be a level of an even-sized alphabet."""
+def _unit_levels(alphabet, scales, shape):
+    """Levels per entry of a kernel of `shape`: the alphabet itself, or with per-unit `scales` (shaped like the kernel's trailing
+    axes: (N1,) for a Dense kernel, (C, F) for a conv kernel) the per-channel levels fl64(scales[u] * alphabet[k])."""
     A = np.asarray(alphabet, dtype=np.float64)
-    idx = np.abs(Q[..., None] - A).argmin(-1).astype(np.int8)
-    exact = A[idx] == Q
+    if scales is None:
+        return A
+    s = np.asarray(scales, dtype=np.float64)
+    if s.ndim > len(shape) or s.shape != tuple(shape[len(shape) - s.ndim:]):
+        raise ValueError(f"scales of shape {s.shape} do not match the trailing axes of a kernel of shape {tuple(shape)}")
+    return s[..., None] * A
+
+
+def pack_levels(Q: np.ndarray, alphabet: np.ndarray, scales=None):
+    """Quantized kernel -> (int8 level indices, alphabet).  Index -1 marks the literal 0.0 a dead direction produces
+    (quantized_network.py:83-84), which need not be a level of an even-sized alphabet.  With per-channel alphabets, `alphabet` is
+    the base alphabet and `scales` the per-unit scales (see `_unit_levels`); the indices then refer to each unit's own levels."""
+    L = _unit_levels(alphabet, scales, Q.shape)
+    idx = np.abs(Q[..., None] - L).argmin(-1).astype(np.int8)
+    exact = np.take_along_axis(np.broadcast_to(L, Q.shape + L.shape[-1:]), idx[..., None].astype(np.int64), -1)[..., 0] == Q
     if not np.all(exact | (Q == 0.0)):
         raise ValueError("Q holds values that are neither alphabet levels nor 0.0")
     idx[~exact] = -1
-    return idx, A
+    return idx, np.asarray(alphabet, dtype=np.float64)
 
 
-def unpack_levels(idx: np.ndarray, alphabet: np.ndarray) -> np.ndarray:
-    A = np.asarray(alphabet, dtype=np.float64)
-    return np.where(idx < 0, 0.0, A[np.maximum(idx, 0)])
+def unpack_levels(idx: np.ndarray, alphabet: np.ndarray, scales=None) -> np.ndarray:
+    L = np.broadcast_to(_unit_levels(alphabet, scales, idx.shape), idx.shape + (np.asarray(alphabet).shape[-1],))
+    vals = np.take_along_axis(L, np.maximum(idx, 0)[..., None].astype(np.int64), -1)[..., 0]
+    return np.where(idx < 0, 0.0, vals)
 
 
 class QuantizedCNNGrid:
     """All (bits, alphabet_scalar) grid points of one network, quantized layer by layer in lock-step."""
 
     def __init__(self, network, batch_size, get_data, bits_list, alphabet_scalars, logger=None, is_quantize_conv2d=True,
-                 device: int = 0, data_set: str = "synthetic", q_train_size=None):
+                 device: int = 0, data_set: str = "synthetic", q_train_size=None, *, alphabet_scope: str = "layer"):
+        """`alphabet_scope` ("layer" | "channel") as in `QuantizedCNN`: with "channel" every grid point quantizes each output
+        channel against its own radius, and `msq_networks()` rounds with the same per-channel levels."""
         self.grid = list(product(bits_list, alphabet_scalars))          # the order of itertools.product in the driver
         self.points = [QuantizedCNN(network, batch_size, get_data, logger=logger, bits=b, alphabet_scalar=c,
-                                    is_quantize_conv2d=is_quantize_conv2d, device=device) for b, c in self.grid]
+                                    is_quantize_conv2d=is_quantize_conv2d, device=device, alphabet_scope=alphabet_scope)
+                       for b, c in self.grid]
         self.trained_net, self.logger, self.device = network, logger, device
         self.is_quantize_conv2d = is_quantize_conv2d
         self.data_set = data_set
@@ -66,10 +83,6 @@ class QuantizedCNNGrid:
 
     def _log(self, msg):
         (self.logger.info if self.logger else print)(msg)
-
-    def _alphabets(self, W):
-        """Per grid point `rad * alphabet` with `rad = alphabet_scalar * median(|W|)` (quantized_network.py:544-545)."""
-        return [np.asarray(p._layer_alphabet(W), dtype=np.float64) for p in self.points]
 
     def _groups(self, qXs, wX):
         """Grid points with identical quantized inputs share a call.  Returns [(qX or None when it equals wX, [point ids])]."""
@@ -96,7 +109,7 @@ class QuantizedCNNGrid:
             dense = kind == "Dense"
             tic = time()
             W = layer.get_weights()[0]
-            alphabets = self._alphabets(W)
+            levels = [p._levels(W, kind) for p in self.points]        # (alphabet, per-channel scales or None) per grid point
             datas = [p._get_layer_data_generator(layer_idx, transpose=True) if dense else p._get_layer_data_generator(layer_idx)
                      for p in self.points]
             wX = datas[0].wX                                      # the analog inputs do not depend on the grid point
@@ -105,14 +118,15 @@ class QuantizedCNNGrid:
             Qs = [None] * len(self.points)
             for qX, members in self._groups([d.wX if d.same else d.qX for d in datas], wX):
                 Xqd = None if qX is None else torch.from_numpy(np.ascontiguousarray(qX)).to(dev)
-                A = [alphabets[g] for g in members]
+                A = [levels[g][0] for g in members]
+                scaled = {} if levels[0][1] is None else {"scales": np.stack([levels[g][1] for g in members])}
                 if dense:
-                    Q = eng.dense_layer(Xd, Xqd, Wd, A)
+                    Q = eng.dense_layer(Xd, Xqd, Wd, A, **scaled)
                 else:
                     rate = getattr(layer, "dilation_rate", None)
                     groups = int(getattr(layer, "groups", 1)) if kind == "Conv2D" else 1
                     Q = eng.conv_layer_nhwc(Xd, Xqd, Wd, A, strides=layer.strides, padding=layer.padding.upper(), rate=rate,
-                                            **({"groups": groups} if groups > 1 else {}))
+                                            **({"groups": groups} if groups > 1 else {}), **scaled)
                 Q = Q.cpu().numpy()
                 for a, g in enumerate(members):
                     Qs[g] = Q[a]
@@ -128,7 +142,7 @@ class QuantizedCNNGrid:
 
     def msq_networks(self):
         """MSQ baselines (quantize_pretrained_cnn.py:97-117): every Dense / Conv2D kernel rounded to the layer alphabet of the
-        corresponding grid point, biases and all other layers untouched."""
+        corresponding grid point (per-channel levels with `alphabet_scope="channel"`), biases and all other layers untouched."""
         from .quantized_network import _clone
         eng = self.points[0].engine
         nets = []
@@ -138,7 +152,8 @@ class QuantizedCNNGrid:
             for layer_idx, layer in enumerate(self.trained_net.layers):
                 if layer.__class__.__name__ in ("Dense", "Conv2D"):
                     ws = layer.get_weights()
-                    Q = eng.msq(ws[0], np.asarray(p._layer_alphabet(ws[0]), dtype=np.float64))
+                    A, scales = p._levels(ws[0], layer.__class__.__name__)
+                    Q = eng.msq(ws[0], A, **({} if scales is None else {"scales": scales}))
                     net.layers[layer_idx].set_weights([Q] + list(ws[1:]))
             nets.append(net)
         return nets

@@ -104,6 +104,7 @@ class QuantizedNeuralNetwork:
         method: str = "auto",
         shard=None,
         gram_split: str = "auto",
+        alphabet_scope: str = "layer",
     ):
         """Wrapper of a Keras-style model that quantizes the weights of its Dense layers with GPFQ.
 
@@ -114,7 +115,9 @@ class QuantizedNeuralNetwork:
         over the ranks of a torch.distributed job (Q blocks are all-gathered after each layer), and
         `gram_split` ("auto" | "samples" | "replicate"): how a multi-GPU job feeds a Dense layer -- "samples" contracts
         m / world samples per rank and all-reduces the Gram matrices, "replicate" all-gathers the inputs; "auto" picks
-        by bytes moved (`replicate.prefer_sample_split`).
+        by bytes moved (`replicate.prefer_sample_split`).  `alphabet_scope` ("layer" | "channel"): "layer" (the reference)
+        quantizes every layer against `alphabet_scalar * median(|W|) * linspace(-1, 1, K)`; "channel" gives every output
+        channel its own radius `alphabet_scalar * median(|w_u|)` (`_unit_scales`), as per-channel weight scales do.
         """
         self.get_data = get_data
         self.trained_net = network
@@ -130,14 +133,17 @@ class QuantizedNeuralNetwork:
         self.alphabet = linspace(-1, 1, num=int(round(2 ** (bits))))
         self.logger = logger
         self.ignore_layers = ignore_layers
-        self._init_device(device, method, shard, gram_split)
+        self._init_device(device, method, shard, gram_split, alphabet_scope)
 
-    def _init_device(self, device, method, shard, gram_split="auto"):
+    def _init_device(self, device, method, shard, gram_split="auto", alphabet_scope="layer"):
         if int(round(2 ** self.bits)) > 64:   # GPFQ_MAX_K of include/gpfq.h: the kernels keep an alphabet in shared memory
             raise ValueError(f"bits={self.bits}: the CUDA path supports alphabets of up to 64 levels (bits <= 6); the reference "
                              "accepts any `bits`, see INTEGRATION.md")
         if gram_split not in ("auto", "samples", "replicate"):
             raise ValueError(f"gram_split must be 'auto', 'samples' or 'replicate', not {gram_split!r}")
+        if alphabet_scope not in ("layer", "channel"):
+            raise ValueError(f"alphabet_scope must be 'layer' or 'channel', not {alphabet_scope!r}")
+        self.alphabet_scope = alphabet_scope
         self.device, self.method, self.gram_split = device, method, gram_split
         self.shard = tuple(shard) if shard else (0, 1)
         self.layer_stats = {}
@@ -212,6 +218,25 @@ class QuantizedNeuralNetwork:
         rad = self.alphabet_scalar * median(abs(W.flatten()))
         return rad * self.alphabet
 
+    def _unit_scales(self, W, kind="Dense"):
+        """Per-output-channel radii `alphabet_scalar * median(|w_u|)`, the expression (and dtype) of `_layer_alphabet` applied to
+        each output channel: a Dense neuron (column j: shape (N1,)), a Conv2D filter f over W[..., f] (broadcast over the kernel's
+        input channels: (Cw, F)), a DepthwiseConv2D output channel (c, d) over W[:, :, c, d] (shape (C, d)).  Unit u then walks
+        with the levels fl64(rad_u * linspace(-1, 1, K)), exactly `rad_u * self.alphabet`."""
+        A = abs(W)
+        if kind == "Dense":
+            return np.asarray(self.alphabet_scalar * median(A, axis=0), dtype=np.float64)
+        if kind == "DepthwiseConv2D":
+            return np.asarray(self.alphabet_scalar * median(A, axis=(0, 1)), dtype=np.float64)
+        rad = np.asarray(self.alphabet_scalar * median(A, axis=(0, 1, 2)), dtype=np.float64)
+        return np.ascontiguousarray(np.broadcast_to(rad, W.shape[2:]))
+
+    def _levels(self, W, kind="Dense"):
+        """(alphabet, scales) of a layer: the layer alphabet and None, or the base alphabet and the per-channel radii."""
+        if self.alphabet_scope == "channel":
+            return np.asarray(self.alphabet, dtype=np.float64), self._unit_scales(W, kind)
+        return np.asarray(self._layer_alphabet(W), dtype=np.float64), None
+
     def _nccl_job(self):
         """True when this object is one rank of a torch.distributed job on GPUs (NCCL): layer inputs are then replicated
         through `replicate_leading_axis` (1 / world of the bytes over each rank's host link + one NVLink all-gather)."""
@@ -274,7 +299,8 @@ class QuantizedNeuralNetwork:
         data = self._get_layer_data_generator(layer_idx, transpose=True)
         self._log(f"\tdone. {time()-tic:2f} seconds.")
 
-        layer_alphabet = self._layer_alphabet(W)
+        layer_alphabet, scales = self._levels(W)
+        scaled = {"scales": scales} if scales is not None else {}   # the per-layer call keeps its signature
 
         self._log("\tQuantizing neurons (on the GPU)...")
         tic = time()
@@ -285,16 +311,17 @@ class QuantizedNeuralNetwork:
                 dev = torch.device("cuda", self.device)
                 G1, G2 = sample_split_gram(self.engine, data.wX, None if data.same else data.qX, *self.shard, device=dev)
                 Q = self.engine.dense_layer_from_gram(G1, G2, np.ascontiguousarray(W),
-                                                      np.asarray(layer_alphabet, dtype=np.float64), j0=lo, j1=hi)
+                                                      np.asarray(layer_alphabet, dtype=np.float64), j0=lo, j1=hi, **scaled)
             elif self._nccl_job():
                 import torch
                 Xd, Xqd = self._replicated(data.wX, None if data.same else data.qX)
                 Wd = torch.from_numpy(np.ascontiguousarray(W)).to(Xd.device)
                 Q = self.engine.dense_layer(Xd, Xqd, Wd, np.asarray(layer_alphabet, dtype=np.float64), j0=lo, j1=hi,
-                                            method=self.method).cpu().numpy()
+                                            method=self.method, **scaled).cpu().numpy()
             else:
                 Q = self.engine.dense_layer(data.wX, None if data.same else data.qX, np.ascontiguousarray(W),
-                                            np.asarray(layer_alphabet, dtype=np.float64), j0=lo, j1=hi, method=self.method)
+                                            np.asarray(layer_alphabet, dtype=np.float64), j0=lo, j1=hi, method=self.method,
+                                            **scaled)
         except Exception as exc:
             self._log(f"\t\tNeurons {lo}:{hi} generated an exception: {exc}")
             raise exc
@@ -333,11 +360,12 @@ class QuantizedCNN(QuantizedNeuralNetwork):
         shard=None,
         conv_path: str = "nhwc",
         gram_split: str = "auto",
+        alphabet_scope: str = "layer",
     ):
         """Dense + Conv2D / DepthwiseConv2D quantization (quantized_network.py:594-650).  Like the reference this
         constructor does not take `ignore_layers`.  `conv_path="nhwc"` hands the layer's activation tensors to
         CUDA (patches are extracted on the device); `"patches"` builds the per-channel patch matrices on the host
-        exactly as `_build_patch_array` does and hands those over."""
+        exactly as `_build_patch_array` does and hands those over.  `alphabet_scope` as in `QuantizedNeuralNetwork`."""
         self.get_data = get_data
         self.trained_net = network
         self.quantized_net = _clone(network)
@@ -350,7 +378,7 @@ class QuantizedCNN(QuantizedNeuralNetwork):
         self.logger = logger
         self.ignore_layers = []
         self.conv_path = conv_path
-        self._init_device(device, method, shard, gram_split)
+        self._init_device(device, method, shard, gram_split, alphabet_scope)
 
     def _build_patch_array(self, channel_idx: int, kernel_size: tuple, strides: tuple, padding: str, rate: tuple,
                            data, mini_batch_size: int):
@@ -370,7 +398,7 @@ class QuantizedCNN(QuantizedNeuralNetwork):
 
     def _quantize_channel_parallel_jit(self, channel_idx: int, channel_filters: array, hidden_activations,
                                        strides: tuple, padding: str, rate: tuple, alphabet: array,
-                                       patch_mini_batch_size=5000) -> array:
+                                       patch_mini_batch_size=5000, scales=None) -> array:
         """All filters of one input channel (quantized_network.py:652-727): host patches + one C-ABI call."""
         filter_shape = channel_filters.shape[0:2]
         patches = self._build_patch_array(channel_idx, filter_shape, strides, padding, rate, hidden_activations,
@@ -379,7 +407,8 @@ class QuantizedCNN(QuantizedNeuralNetwork):
         Wc = np.ascontiguousarray(channel_filters.reshape(*channel_filters.shape[:2], 1, channel_filters.shape[-1]),
                                   dtype=np.float32)
         try:
-            Qc = self.engine.conv_channels([Xp], None if Xqp is Xp else [Xqp], Wc, np.asarray(alphabet, dtype=np.float64))
+            scaled = {} if scales is None else {"scales": np.reshape(scales, (1, -1))}
+            Qc = self.engine.conv_channels([Xp], None if Xqp is Xp else [Xqp], Wc, np.asarray(alphabet, dtype=np.float64), **scaled)
         except Exception as exc:
             self._log(f"\t\t\tChannel {channel_idx} generated an exception: {exc}")
             raise Exception
@@ -397,7 +426,8 @@ class QuantizedCNN(QuantizedNeuralNetwork):
         layer = self.trained_net.layers[layer_idx]
         rate = getattr(layer, "dilation_rate", None)
         W = layer.get_weights()[0]
-        alphabet = self._layer_alphabet(W)
+        alphabet, scales = self._levels(W, layer.__class__.__name__)
+        scaled = {"scales": scales} if scales is not None else {}
         # a grouped Conv2D has a (kh, kw, C / groups, F) kernel: input channel c meets only the Fg filters of its group c // Cg,
         # so ranks take whole groups and gather their filters (groups == 1: channels, all filters)
         groups = int(getattr(layer, "groups", 1)) if layer.__class__.__name__ == "Conv2D" else 1
@@ -417,7 +447,7 @@ class QuantizedCNN(QuantizedNeuralNetwork):
                                                  layer.strides, layer.padding.upper(), rate, *self.shard)
                     self.layer_stats[layer_idx] = dict(self.engine.last_stats)
                     Q = self.engine.conv_layer_from_gram(gram, np.ascontiguousarray(W), np.asarray(alphabet, dtype=np.float64),
-                                                         **grouped)
+                                                         **grouped, **scaled)
                     lo, hi = 0, num_channels
                 elif self._nccl_job():
                     import torch
@@ -425,12 +455,12 @@ class QuantizedCNN(QuantizedNeuralNetwork):
                     Wd = torch.from_numpy(np.ascontiguousarray(W)).to(Ad.device)
                     Q = self.engine.conv_layer_nhwc(Ad, Aqd, Wd, np.asarray(alphabet, dtype=np.float64), strides=layer.strides,
                                                     padding=layer.padding.upper(), rate=rate, c0=lo,
-                                                    n_channels=hi - lo, **grouped).cpu().numpy()
+                                                    n_channels=hi - lo, **grouped, **scaled).cpu().numpy()
                 else:
                     Q = self.engine.conv_layer_nhwc(data.wX, None if data.same else data.qX, np.ascontiguousarray(W),
                                                     np.asarray(alphabet, dtype=np.float64), strides=layer.strides,
                                                     padding=layer.padding.upper(), rate=rate, c0=lo, n_channels=hi - lo,
-                                                    **grouped)
+                                                    **grouped, **scaled)
             except Exception as exc:
                 self._log(f"\t\tChannels {lo}:{hi} generated an exception: {exc}")
                 raise exc
@@ -441,7 +471,8 @@ class QuantizedCNN(QuantizedNeuralNetwork):
                 ci, f0 = channel_idx % Cg, (channel_idx // Cg) * Fg   # the channel's kernel slice and its group's filters
                 Q[:, :, ci, f0:f0 + Fg] = self._quantize_channel_parallel_jit(
                     channel_idx, W[:, :, ci, f0:f0 + Fg], data, strides=layer.strides, padding=layer.padding.upper(),
-                    rate=rate, alphabet=alphabet, patch_mini_batch_size=self.patch_mini_batch_size)
+                    rate=rate, alphabet=alphabet, patch_mini_batch_size=self.patch_mini_batch_size,
+                    scales=None if scales is None else scales[ci, f0:f0 + Fg])
         if (lo, hi) != (0, num_channels) and groups > 1:
             # this rank wrote the filters of groups lo / Cg .. hi / Cg: gather along the group axis of (kh, kw, Cg, groups, Fg)
             Q = self._gather_columns(Q.reshape(*Q.shape[:3], groups, Fg), lo // Cg, hi // Cg, axis=3).reshape(W.shape)

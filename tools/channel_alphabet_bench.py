@@ -1,0 +1,122 @@
+"""Per-layer against per-channel alphabets at realistic sizes, through the public engine API.
+
+    python tools/channel_alphabet_bench.py [--reps 3] [--warmup 1] [--only NAME ...]
+
+Layers (hidden-layer form, X != Xq, seeded device-resident inputs, ternary alphabets):
+  * vgg16_fc1        Dense 25088 -> 4096, m = 1504 (the residual form of the sweep, contractions on tcgen05)
+  * vgg16_fc2        Dense 4096 -> 4096, m = 1504
+  * dense_4096_25k   Dense 4096 -> 4096, m = 25000 (tcgen05 Gram + Gram-row sweep walked by the tensor-core walk)
+  * cifar_conv2      Conv2D 3 x 3, 32 -> 32 channels, 32 x 32 images, 5008 images
+  * dw3x3_14_512     DepthwiseConv2D 3 x 3 on 14 x 14 x 512 (groups = C), 1504 images
+  * convnext_t_dw7   ConvNeXt-T stage-1 depthwise 7 x 7 on 56 x 56 x 96, 256 images
+Per layer: median ms over --reps synchronised calls after --warmup of the per-layer call (alphabet rad * linspace, rad from the median
+of the whole kernel) and of the per-channel call (base alphabet linspace, one radius per output channel), the kernels each ran
+(`gram_kernel`, `reserved`: bit 0 int8 residual form, bit 1 tensor-core walk) and the per-channel / per-layer time ratio.  The GPU
+name and power limit come from the same run.
+"""
+import argparse
+import json
+import os
+import subprocess
+import sys
+import time
+
+import numpy as np
+
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+
+# name: ("dense", N0, N1, m) | ("conv", kernel, C, F, groups, H, n_img)
+LAYERS = {
+    "vgg16_fc1": ("dense", 25088, 4096, 1504),
+    "vgg16_fc2": ("dense", 4096, 4096, 1504),
+    "dense_4096_25k": ("dense", 4096, 4096, 25000),
+    "cifar_conv2": ("conv", (3, 3), 32, 32, 1, 32, 5008),
+    "dw3x3_14_512": ("conv", (3, 3), 512, 512, 512, 14, 1504),
+    "convnext_t_dw7": ("conv", (7, 7), 96, 96, 96, 56, 256),
+}
+
+
+def gpu_info():
+    import torch
+    name = torch.cuda.get_device_name(0)
+    try:
+        power = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader", "-i", "0"],
+                               capture_output=True, text=True, timeout=30).stdout.strip()
+    except (OSError, subprocess.SubprocessError):
+        power = "unknown"
+    return name, power
+
+
+def timed(fn, reps, warmup):
+    import torch
+    for _ in range(warmup):
+        fn()
+    times = []
+    for _ in range(reps):
+        torch.cuda.synchronize()
+        t0 = time.perf_counter()
+        fn()
+        torch.cuda.synchronize()
+        times.append(time.perf_counter() - t0)
+    return float(np.median(times)) * 1e3
+
+
+def main():
+    ap = argparse.ArgumentParser(description=__doc__.split("\n")[0])
+    ap.add_argument("--reps", type=int, default=3)
+    ap.add_argument("--warmup", type=int, default=1)
+    ap.add_argument("--only", nargs="*", default=None)
+    args = ap.parse_args()
+    import torch
+    from quantized_neural_networks_b200 import get_engine
+    if not torch.cuda.is_available():
+        sys.exit("channel_alphabet_bench: no CUDA device")
+    eng = get_engine(0)
+    name, power = gpu_info()
+    print(json.dumps({"gpu": name, "power_limit": power}), flush=True)
+    base = np.linspace(-1, 1, 3)
+    for li, (lname, spec) in enumerate(LAYERS.items()):
+        if args.only and lname not in args.only:
+            continue
+        g = torch.Generator(device="cuda").manual_seed(3000 + li)
+        if spec[0] == "dense":
+            _, N0, N1, m = spec
+            X = torch.relu(torch.randn((N0, m), generator=g, device="cuda"))
+            Xq = torch.relu(X + 0.05 * torch.randn((N0, m), generator=g, device="cuda"))
+            # columns of spread scale, as per-channel alphabets are meant for
+            col = torch.logspace(-1, 1, N1, device="cuda")
+            W = ((torch.rand((N0, N1), generator=g, device="cuda") * 2 - 1) * np.sqrt(6.0 / (N0 + N1)) * col).contiguous()
+            Wh = W.cpu().numpy()
+            A = np.float32(3) * np.median(np.abs(Wh.flatten())) * base
+            s = (np.float32(3) * np.median(np.abs(Wh), axis=0)).astype(np.float64)
+            layer_call = lambda: eng.dense_layer(X, Xq, W, A)
+            chan_call = lambda: eng.dense_layer(X, Xq, W, base, scales=s)
+            shape = {"N0": N0, "N1": N1, "m": m}
+        else:
+            _, ks, C, F, groups, H, n_img = spec
+            act = torch.relu(torch.randn((n_img, H, H, C), generator=g, device="cuda"))
+            actq = torch.relu(act + 0.05 * torch.randn(act.shape, generator=g, device="cuda"))
+            Cg = C // groups
+            W = ((torch.rand((*ks, Cg, F), generator=g, device="cuda") * 2 - 1) * 0.2
+                 * torch.logspace(-1, 1, F, device="cuda")).contiguous()
+            Wh = W.cpu().numpy()
+            A = np.float32(3) * np.median(np.abs(Wh.flatten())) * base
+            s = np.ascontiguousarray(np.broadcast_to((np.float32(3) * np.median(np.abs(Wh), axis=(0, 1, 2))).astype(np.float64),
+                                                     (Cg, F)))
+            gk = {"groups": groups} if groups > 1 else {}
+            layer_call = lambda: eng.conv_layer_nhwc(act, actq, W, A, **gk)
+            chan_call = lambda: eng.conv_layer_nhwc(act, actq, W, base, scales=s, **gk)
+            shape = {"kernel": list(ks), "C": C, "F": F, "groups": groups, "H": H, "n_img": n_img}
+        ms_l = timed(layer_call, args.reps, args.warmup)
+        st_l = dict(eng.last_stats)
+        ms_c = timed(chan_call, args.reps, args.warmup)
+        st_c = dict(eng.last_stats)
+        print(json.dumps({"layer": lname, **shape, "per_layer_ms": round(ms_l, 3), "per_channel_ms": round(ms_c, 3),
+                          "ratio": round(ms_c / ms_l, 3), "gram_kernel": [st_l["gram_kernel"], st_c["gram_kernel"]],
+                          "reserved": [st_l["reserved"], st_c["reserved"]]}), flush=True)
+        del W
+        torch.cuda.empty_cache()
+
+
+if __name__ == "__main__":
+    main()

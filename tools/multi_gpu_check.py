@@ -87,12 +87,18 @@ def main():
     c_one = run_cnn()
     c_img = run_cnn(shard=(rank, world))
     c_rep = run_cnn(shard=(rank, world), gram_split="replicate")
-    pc = c_one.quantized_net.predict(xi_eval).argmax(-1)
-    for name, q, exact in (("image split", c_img, False), ("replicate", c_rep, True)):
-        for idx, layer in enumerate(c_one.trained_net.layers):
+    # the same CNN with per-channel alphabets (alphabet_scope="channel"): image split and channel / group shards against one GPU
+    p_one = run_cnn(alphabet_scope="channel")
+    p_img = run_cnn(shard=(rank, world), alphabet_scope="channel")
+    p_rep = run_cnn(shard=(rank, world), gram_split="replicate", alphabet_scope="channel")
+    for (name, q, exact), ref in zip((("image split", c_img, False), ("replicate", c_rep, True),
+                                      ("per-channel image split", p_img, False), ("per-channel replicate", p_rep, True)),
+                                     (c_one, c_one, p_one, p_one)):
+        pc = ref.quantized_net.predict(xi_eval).argmax(-1)
+        for idx, layer in enumerate(ref.trained_net.layers):
             if layer.__class__.__name__ not in ("Conv2D", "Dense"):
                 continue
-            a = c_one.quantized_net.layers[idx].get_weights()[0]
+            a = ref.quantized_net.layers[idx].get_weights()[0]
             b = q.quantized_net.layers[idx].get_weights()[0]
             agree = float(np.mean(a == b))
             good = agree == 1.0 if exact else agree >= 0.9999
