@@ -257,6 +257,28 @@ int gpfq_conv_layer_from_gram_scaled(gpfq_ctx *ctx, const double *gram, int32_t 
 int gpfq_msq_scaled(gpfq_ctx *ctx, const float *W, int64_t n, const double *alphabet, int32_t K, const double *scales,
                     int64_t n_units, double *Q_out, uint32_t flags);
 
+/* ---- stochastic rounding (SPFQ) --------------------------------------------------------------------------------------------
+ * Context state, like gpfq_set_stream: every later call that quantizes (the Dense, conv, _grouped, _scaled, MSQ and bit_round
+ * entry points) rounds with this mode; Gram-only calls ignore it.  GPFQ_ROUND_NEAREST (the default) is the reference's nearest-
+ * level rounding, bit for bit.  GPFQ_ROUND_STOCHASTIC runs the same path-following walk with the nearest quantizer replaced by
+ * unbiased stochastic rounding between the two bracketing levels (Zhang & Saab, SPFQ, 2023):
+ *   splitmix64(x)    = the SplitMix64 finaliser of x + 0x9E3779B97F4A7C15 (mod 2^64)
+ *   draw(seed, u, t) = (splitmix64(splitmix64(seed ^ splitmix64(u)) ^ t) >> 11) * 2^-53               exact fp64 in [0, 1)
+ *   stoc_round(v, A, r) = A[0] unless v > A[0] (NaN included); A[K-1] if v >= A[K-1]; else, with k = max{i : A[i] <= v} and
+ *                         p = (v - A[k]) / (A[k+1] - A[k]) in fp64, A[k+1] if r < p else A[k]
+ * A greedy step keeps the reference's guards: the literal 0 for a dead direction, stoc_round(w_t) when |d| < 1e-10, else
+ * stoc_round(num / nrm^2), with A the alphabet or the unit's levels fl(s_u * A[k]) and r = draw(seeds[a], u, t) for alphabet a.
+ * Unit and step ids are global, so results do not depend on shards, channel ranges, conv paths or the Gram split:
+ *   Dense: u = neuron (column) j, t = direction;   Conv: u = ci * F + f (ci < C / groups, f the filter), t = tap r * kw + col;
+ *   MSQ / bit_round: u = flat element index, t = 0.
+ * `seeds` (n_seeds >= 1, host) are copied into the context; a call with more alphabets than seeds, or with an alphabet that is
+ * not non-decreasing and finite, returns GPFQ_ERR_ARG before any work.  A stochastic call runs the kernels of its nearest
+ * counterpart (the tensor-core walk and the int8 residual form included), with equal stats.method, gram_kernel, reserved and launch
+ * count; every option applies as for nearest rounding. */
+#define GPFQ_ROUND_NEAREST 0
+#define GPFQ_ROUND_STOCHASTIC 1
+int gpfq_set_rounding(gpfq_ctx *ctx, int32_t mode, const uint64_t *seeds, int32_t n_seeds);
+
 /* ---- MSQ baseline ---------------------------------------------------------------------------
  * Plain nearest-level rounding of every weight (_bit_round_parallel :40-57 applied elementwise,
  * as in quantize_pretrained_mlp.py:97-117).  n elements, contiguous. */

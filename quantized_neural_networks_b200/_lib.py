@@ -5,7 +5,7 @@ from __future__ import annotations
 import ctypes
 import os
 import subprocess
-from ctypes import POINTER, c_char_p, c_double, c_float, c_int, c_int32, c_int64, c_uint32, c_void_p
+from ctypes import POINTER, c_char_p, c_double, c_float, c_int, c_int32, c_int64, c_uint32, c_uint64, c_void_p
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libgpfq.so")
@@ -17,6 +17,7 @@ ALL_DEVICE = 7
 METHOD_AUTO, METHOD_STREAM, METHOD_GRAM, METHOD_STREAM_FAST = 0 << 4, 1 << 4, 2 << 4, 3 << 4
 NO_SYNC = 1 << 8
 MAX_K = 64
+ROUND_NEAREST, ROUND_STOCHASTIC = 0, 1
 
 ERRORS = {1: "GPFQ_ERR_ARG", 2: "GPFQ_ERR_CUDA", 3: "GPFQ_ERR_OOM", 4: "GPFQ_ERR_UNSUPPORTED"}
 
@@ -48,6 +49,7 @@ EXPORTS = {
     "gpfq_last_error": (c_char_p, [c_void_p]),
     "gpfq_set_stream": (c_int, [c_void_p, c_void_p]),
     "gpfq_set_option": (c_int, [c_void_p, c_char_p, c_int64]),
+    "gpfq_set_rounding": (c_int, [c_void_p, c_int32, POINTER(c_uint64), c_int32]),
     "gpfq_trim": (c_int, [c_void_p]),
     "gpfq_conv_partial_bytes": (c_int64, [c_void_p]),
     "gpfq_query_stats": (c_int, [c_void_p, c_int32, POINTER(GpfqStats)]),

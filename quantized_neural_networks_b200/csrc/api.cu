@@ -11,10 +11,11 @@
 // kernels / stages implemented in the other translation units
 int dense_gram_path(gpfq_ctx *, const float *, const float *, int64_t, int64_t, int64_t, const float *, int64_t,
                     int64_t, int64_t, const double *, const int *, const int *, int, double *, int64_t, int64_t,
-                    gpfq_stats *, const double *G1_pre = nullptr, const double *G2_pre = nullptr, const double *d_scales = nullptr);
+                    gpfq_stats *, const double *G1_pre = nullptr, const double *G2_pre = nullptr, const double *d_scales = nullptr,
+                    int64_t u0 = 0);
 int dense_stream_path(gpfq_ctx *, const float *, const float *, int64_t, int64_t, int64_t, const float *, int64_t,
                       int64_t, int64_t, const double *, const int *, const int *, int, double *, int64_t, int64_t,
-                      gpfq_stats *, const double *d_scales);
+                      gpfq_stats *, const double *d_scales, int64_t u0);
 int dense_gram_only(gpfq_ctx *, const float *, const float *, int64_t, int64_t, int64_t, double *, double *);
 bool dense_gram_uses_i8(gpfq_ctx *, int64_t, int64_t, bool);
 int conv_supported_kk(int kk);
@@ -26,7 +27,7 @@ int conv_sweep_stage(gpfq_ctx *, int, const double *, const float *, double *, i
                      const double *, const int *, const int *, int, int64_t, const double *);
 int im2col_stage(gpfq_ctx *, const float *, int64_t, int, int, int64_t, int64_t, int, int, int, int, int, int, int,
                  int, int, int, int, float *, int64_t);
-int msq_stage(gpfq_ctx *, const void *, int, int64_t, const double *, int, int, double *, const double *, int64_t);
+int msq_stage(gpfq_ctx *, const void *, int, int64_t, const double *, int, int, double *, const double *, int64_t);  // ctx->d_seeds
 int nhwc9_plan(int, int, int, int, int, int, int, int, int *, int *);
 int corr9_plan(int, int, int, int, int, int, int, int, int, int);
 int corr9_pack_stage(gpfq_ctx *, const float *, int64_t, int, int, int64_t, int64_t, int, int, int64_t, int64_t, float *);
@@ -214,6 +215,21 @@ extern "C" int gpfq_set_option(gpfq_ctx *ctx, const char *key, int64_t value) {
     return GPFQ_OK;
 }
 
+extern "C" int gpfq_set_rounding(gpfq_ctx *ctx, int32_t mode, const uint64_t *seeds, int32_t n_seeds) {
+    if (!ctx) return GPFQ_ERR_ARG;
+    ctx->err.clear();
+    if (mode == GPFQ_ROUND_NEAREST) {
+        ctx->rounding = mode;
+        ctx->seeds.clear();
+        return GPFQ_OK;
+    }
+    if (mode != GPFQ_ROUND_STOCHASTIC) return gpfq_fail(ctx, GPFQ_ERR_ARG, "unknown rounding mode %d", mode);
+    if (!seeds || n_seeds < 1) return gpfq_fail(ctx, GPFQ_ERR_ARG, "stochastic rounding needs n_seeds >= 1 seeds");
+    ctx->rounding = mode;
+    ctx->seeds.assign(seeds, seeds + n_seeds);
+    return GPFQ_OK;
+}
+
 extern "C" int gpfq_set_stream(gpfq_ctx *ctx, void *cuda_stream) {
     if (!ctx) return GPFQ_ERR_ARG;
     cudaStream_t next = cuda_stream ? (cudaStream_t)cuda_stream : ctx->own_stream;
@@ -317,6 +333,37 @@ static int upload_scales(gpfq_ctx *ctx, const double *scales, int n_alph, int64_
     return GPFQ_OK;
 }
 
+// Stochastic rounding: a seed for every alphabet of the call, and levels the bracketing search can rely on (non-decreasing and
+// finite).  Nothing to check for nearest rounding.
+static int check_rounding(gpfq_ctx *ctx, const double *alphabets, const int32_t *K, int n_alph) {
+    if (ctx->rounding != GPFQ_ROUND_STOCHASTIC || !alphabets || !K) return GPFQ_OK;
+    if ((size_t)n_alph > ctx->seeds.size())
+        return gpfq_fail(ctx, GPFQ_ERR_ARG, "%d alphabets but %zu stochastic-rounding seeds", n_alph, ctx->seeds.size());
+    int64_t off = 0;
+    for (int a = 0; a < n_alph; ++a) {
+        if (K[a] < 1 || K[a] > GPFQ_MAX_K) return GPFQ_OK;   // upload_alphabets reports it
+        for (int k = 0; k < K[a]; ++k) {
+            const double v = alphabets[off + k];
+            if (!std::isfinite(v) || (k > 0 && !(alphabets[off + k - 1] <= v)))
+                return gpfq_fail(ctx, GPFQ_ERR_ARG, "stochastic rounding: alphabet %d must be non-decreasing and finite", a);
+        }
+        off += K[a];
+    }
+    return GPFQ_OK;
+}
+
+// The seeds of this call on the device (one per alphabet, read by the walks in stream order; pageable source: staged before the
+// call returns, so GPFQ_NO_SYNC calls stay asynchronous), or nullptr for nearest rounding and for Gram-only calls.
+static int stage_seeds(gpfq_ctx *ctx, int n_alph) {
+    ctx->d_seeds = nullptr;
+    if (ctx->rounding != GPFQ_ROUND_STOCHASTIC || ctx->gram_only_out) return GPFQ_OK;
+    uint64_t *d = nullptr;
+    GPFQ_TRY(gpfq_ws(ctx, WS_SEEDS, (size_t)n_alph * sizeof(uint64_t), (void **)&d));
+    CUDA_TRY(ctx, cudaMemcpyAsync(d, ctx->seeds.data(), (size_t)n_alph * sizeof(uint64_t), cudaMemcpyHostToDevice, ctx->stream));
+    ctx->d_seeds = d;
+    return GPFQ_OK;
+}
+
 cudaError_t gpfq_record(gpfq_ctx *ctx, int which, cudaStream_t s) {
     ctx->cur->rec[which] = true;
     return cudaEventRecord(ctx->cur->e[which], s);
@@ -405,7 +452,8 @@ static int choose_dense_method(gpfq_ctx *ctx, uint32_t flags, int64_t N0, int64_
 // scales (nullable, host): per-neuron scales, neuron j of alphabet a at scales[a * lds + j].
 static int dense_layer(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ldx, int64_t N0, int64_t m, const float *W,
                        int64_t ldw, int64_t N1, int64_t j0, int64_t j1, const double *alphabets, const int32_t *K, int32_t n_alph,
-                       double *Q_out, int64_t ldq, uint32_t flags, gpfq_stats *stats, const double *scales, int64_t lds) {
+                       double *Q_out, int64_t ldq, uint32_t flags, gpfq_stats *stats, const double *scales, int64_t lds,
+                       int64_t ubase = 0) {
     if (!ctx) return GPFQ_ERR_ARG;
     ctx->err.clear();
     if (stats) memset(stats, 0, sizeof(*stats));
@@ -419,6 +467,7 @@ static int dense_layer(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t l
         return gpfq_fail(ctx, GPFQ_ERR_ARG, "GPFQ_NO_SYNC needs all-device pointers");
     const int64_t nj = j1 - j0;
     if (scales && n_alph >= 1) GPFQ_TRY(check_scales(ctx, scales + j0, n_alph, nj, lds));
+    GPFQ_TRY(check_rounding(ctx, alphabets, K, n_alph));
     if (nj == 0) return GPFQ_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     const bool same = (Xq == nullptr || Xq == X);
@@ -429,6 +478,7 @@ static int dense_layer(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t l
 
     Alphabets al;
     GPFQ_TRY(upload_alphabets(ctx, alphabets, K, n_alph, &al));
+    GPFQ_TRY(stage_seeds(ctx, n_alph));
     const double *d_scales = nullptr;
     if (scales) GPFQ_TRY(upload_scales(ctx, scales + j0, n_alph, nj, lds, &d_scales));
 
@@ -468,11 +518,11 @@ static int dense_layer(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t l
 
     if (method == GPFQ_METHOD_GRAM)
         GPFQ_TRY(dense_gram_path(ctx, dX, dXq, dldx, N0, m, dW, dldw, dj0, nj, al.d_levels, al.d_koff, al.d_flags, n_alph, dQ,
-                                 dldq, col0, stats, nullptr, nullptr, d_scales));
+                                 dldq, col0, stats, nullptr, nullptr, d_scales, ubase + j0));
     else {
         ctx->stream_literal = (method == GPFQ_METHOD_STREAM);
         GPFQ_TRY(dense_stream_path(ctx, dX, dXq, dldx, N0, m, dW, dldw, dj0, nj, al.d_levels, al.h_koff.data(),
-                                   al.h_flags.data(), n_alph, dQ, dldq, col0, stats, d_scales));
+                                   al.h_flags.data(), n_alph, dQ, dldq, col0, stats, d_scales, ubase + j0));
         if (stats) stats->method = method >> 4;
     }
     CUDA_TRY(ctx, gpfq_record(ctx, 6, s));
@@ -523,6 +573,7 @@ static int dense_layer_from_gram(gpfq_ctx *ctx, const double *G1, const double *
         return gpfq_fail(ctx, GPFQ_ERR_ARG, "GPFQ_NO_SYNC needs all-device pointers");
     const int64_t nj = j1 - j0;
     if (scales && n_alph >= 1) GPFQ_TRY(check_scales(ctx, scales + j0, n_alph, nj, N1));
+    GPFQ_TRY(check_rounding(ctx, alphabets, K, n_alph));
     if (nj == 0) return GPFQ_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     cudaStream_t s = ctx->stream;
@@ -530,6 +581,7 @@ static int dense_layer_from_gram(gpfq_ctx *ctx, const double *G1, const double *
     CUDA_TRY(ctx, gpfq_record(ctx, 0, s));
     Alphabets al;
     GPFQ_TRY(upload_alphabets(ctx, alphabets, K, n_alph, &al));
+    GPFQ_TRY(stage_seeds(ctx, n_alph));
     const double *d_scales = nullptr;
     if (scales) GPFQ_TRY(upload_scales(ctx, scales + j0, n_alph, nj, N1, &d_scales));
     const float *dW = W;
@@ -552,7 +604,7 @@ static int dense_layer_from_gram(gpfq_ctx *ctx, const double *G1, const double *
     }
     CUDA_TRY(ctx, gpfq_record(ctx, 5, s));
     GPFQ_TRY(dense_gram_path(ctx, nullptr, nullptr, 0, N0, 0, dW, dldw, dj0, nj, al.d_levels, al.d_koff, al.d_flags, n_alph,
-                             dQ, dldq, col0, stats, (G1 == nullptr || G1 == G2) ? nullptr : G1, G2, d_scales));
+                             dQ, dldq, col0, stats, (G1 == nullptr || G1 == G2) ? nullptr : G1, G2, d_scales, j0));
     CUDA_TRY(ctx, gpfq_record(ctx, 6, s));
     if (!(flags & GPFQ_Q_DEVICE)) {
         for (int a = 0; a < n_alph; ++a)
@@ -737,6 +789,7 @@ static int conv_channels(gpfq_ctx *ctx, const float *const *Xp, const float *con
     if ((flags & GPFQ_NO_SYNC) && (flags & GPFQ_ALL_DEVICE) != GPFQ_ALL_DEVICE)
         return gpfq_fail(ctx, GPFQ_ERR_ARG, "GPFQ_NO_SYNC needs all-device pointers");
     if (scales && n_alph >= 1) GPFQ_TRY(check_scales(ctx, scales, n_alph, C * F, C * F));
+    GPFQ_TRY(check_rounding(ctx, alphabets, K, n_alph));
     ctx->conv_part_bytes = 0;
     if (n_ch == 0) return GPFQ_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
@@ -756,7 +809,7 @@ static int conv_channels(gpfq_ctx *ctx, const float *const *Xp, const float *con
             // per-alphabet outputs are kk*C*F apart, which is exactly N0*ldq for N0=kk, ldq=C*F
             GPFQ_TRY(dense_layer(ctx, Xp[i], same ? Xp[i] : Xqp[i], n, kk, n, W + c * F, C * F, F, 0, F, alphabets, K, n_alph,
                                  Q_out + c * F, C * F, (flags & ~GPFQ_NO_SYNC) | GPFQ_METHOD_GRAM, stats,
-                                 scales ? scales + c * F : nullptr, C * F));
+                                 scales ? scales + c * F : nullptr, C * F, c * F));   // unit ids c * F + f
             launches += stats ? stats->kernel_launches : 0;
         }
         if (stats) { stats->kernel_launches = (int)launches; stats->weights = (int64_t)kk * n_ch * F * n_alph; }
@@ -768,6 +821,7 @@ static int conv_channels(gpfq_ctx *ctx, const float *const *Xp, const float *con
     CUDA_TRY(ctx, gpfq_record(ctx, 0, s));
     Alphabets al;
     GPFQ_TRY(upload_alphabets(ctx, alphabets, K, n_alph, &al));
+    GPFQ_TRY(stage_seeds(ctx, n_alph));
     const double *d_scales = nullptr;
     if (scales) GPFQ_TRY(upload_scales(ctx, scales, n_alph, C * F, C * F, &d_scales));
 
@@ -879,6 +933,7 @@ static int conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float *actq, i
     const int64_t Cg = C / groups, Fg = F / groups;
     const int kk = kh * kw;
     if (scales && n_alph >= 1) GPFQ_TRY(check_scales(ctx, scales, n_alph, Cg * F, Cg * F));
+    if (!ctx->gram_only_out) GPFQ_TRY(check_rounding(ctx, alphabets, K, n_alph));
     ctx->conv_part_bytes = 0;
     if (n_ch == 0) return GPFQ_OK;
     // TensorFlow extract_patches geometry (quantized_network.py:158-172)
@@ -933,7 +988,7 @@ static int conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float *actq, i
             const int64_t off = (c % Cg) * F + (c / Cg) * Fg;
             GPFQ_TRY(dense_layer(ctx, pa, same ? pa : pq, n, kk, n, W + off, Cg * F, Fg, 0, Fg, alphabets, K, n_alph, Q_out + off,
                                  Cg * F, ((flags & ~GPFQ_NO_SYNC) | GPFQ_X_DEVICE | GPFQ_METHOD_GRAM), stats,
-                                 scales ? scales + off : nullptr, Cg * F));
+                                 scales ? scales + off : nullptr, Cg * F, off));   // unit ids (c % Cg) * F + g * Fg + f
             launches += (stats ? stats->kernel_launches : 0) + (same ? 1 : 2);
         }
         if (stats) { stats->kernel_launches = (int)launches; stats->weights = (int64_t)kk * n_ch * Fg * n_alph; }
@@ -943,6 +998,7 @@ static int conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float *actq, i
     CUDA_TRY(ctx, gpfq_record(ctx, 0, s));
     Alphabets al;
     GPFQ_TRY(upload_alphabets(ctx, alphabets, K, n_alph, &al));
+    GPFQ_TRY(stage_seeds(ctx, n_alph));
     const double *d_scales = nullptr;
     if (scales) GPFQ_TRY(upload_scales(ctx, scales, n_alph, Cg * F, Cg * F, &d_scales));
     const float *dA = act, *dAq = same ? act : actq;
@@ -1252,6 +1308,7 @@ static int conv_layer_from_gram(gpfq_ctx *ctx, const double *gram, int32_t kk, c
         return gpfq_fail(ctx, GPFQ_ERR_ARG, "bad groups=%lld for C=%lld, F=%lld", (long long)groups, (long long)C, (long long)F);
     if (!conv_supported_kk(kk)) return gpfq_fail(ctx, GPFQ_ERR_UNSUPPORTED, "kernel size kk=%d has no walk kernel", kk);
     if (scales && n_alph >= 1) GPFQ_TRY(check_scales(ctx, scales, n_alph, C / groups * F, C / groups * F));
+    GPFQ_TRY(check_rounding(ctx, alphabets, K, n_alph));
     if (n_ch == 0) return GPFQ_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     cudaStream_t s = ctx->stream;
@@ -1259,6 +1316,7 @@ static int conv_layer_from_gram(gpfq_ctx *ctx, const double *gram, int32_t kk, c
     CUDA_TRY(ctx, gpfq_record(ctx, 0, s));
     Alphabets al;
     GPFQ_TRY(upload_alphabets(ctx, alphabets, K, n_alph, &al));
+    GPFQ_TRY(stage_seeds(ctx, n_alph));
     const double *d_scales = nullptr;
     if (scales) GPFQ_TRY(upload_scales(ctx, scales, n_alph, C / groups * F, C / groups * F, &d_scales));
     CUDA_TRY(ctx, gpfq_record(ctx, 5, s));
@@ -1308,12 +1366,14 @@ static int round_elements(gpfq_ctx *ctx, const void *W, int is_f64, int64_t n, c
         if (n_units < 1) return gpfq_fail(ctx, GPFQ_ERR_ARG, "n_units must be >= 1");
         GPFQ_TRY(check_scales(ctx, scales, 1, n_units, n_units));
     }
+    GPFQ_TRY(check_rounding(ctx, alphabet, &K, 1));
     if (n == 0) return GPFQ_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     begin_call(ctx, 2);
     cudaStream_t s = ctx->stream;
     Alphabets al;
     GPFQ_TRY(upload_alphabets(ctx, alphabet, &K, 1, &al));
+    GPFQ_TRY(stage_seeds(ctx, 1));
     const double *d_scales = nullptr;
     if (scales) GPFQ_TRY(upload_scales(ctx, scales, 1, n_units, n_units, &d_scales));
     const size_t esz = is_f64 ? sizeof(double) : sizeof(float);

@@ -75,6 +75,9 @@ struct gpfq_ctx {
     double *gram_only_out = nullptr;  // set for the duration of gpfq_conv_gram_nhwc: conv_finish hands the Grams out, no walk
     int last_gram_kernel = 0;     // what the last Dense Gram stage ran (1 DMMA, 2 int8 tcgen05)
     size_t i8_oom_bytes = 0;      // smallest int8-Gram workspace that failed to allocate (0: none yet)
+    int rounding = GPFQ_ROUND_NEAREST;  // gpfq_set_rounding: the mode and its seeds (one per alphabet of a call)
+    std::vector<uint64_t> seeds;
+    const uint64_t *d_seeds = nullptr;  // the seeds of the call in progress on the device; nullptr: nearest rounding
     // grow-only named workspaces
     DevBuf ws[48];
     DevBuf pinned[4];
@@ -88,7 +91,7 @@ enum WsSlot {
     WS_U, WS_PTRS, WS_CG, WS_CPART, WS_PATCH_A, WS_PATCH_B, WS_ACT_A, WS_ACT_B, WS_QIDX, WS_MISC,
     WS_I8_SQ, WS_I8_SX, WS_I8_E, WS_I8_TILES, WS_LR_XD, WS_LR_XT, WS_LR_U, WS_CORR_B,
     WS_SL_W, WS_SL_XT, WS_SL_XQT, WS_SL_XQ, WS_SL_U, WS_SL_KQ, WS_SL_E,
-    WS_TC_TAB, WS_TC_G2S, WS_TC_G1S, WS_TC_E, WS_TC_P, WS_TC_W, WS_TC_G1M, WS_SCALES, WS_UNIT_H
+    WS_TC_TAB, WS_TC_G2S, WS_TC_G1S, WS_TC_E, WS_TC_P, WS_TC_W, WS_TC_G1M, WS_SCALES, WS_UNIT_H, WS_SEEDS
 };
 
 int gpfq_fail(gpfq_ctx *ctx, int code, const char *fmt, ...);
@@ -271,6 +274,90 @@ __device__ __forceinline__ double gpfq_decide_unit(double nrm, double d, double 
     if (nrm < GPFQ_DEAD_NORM) return 0.0;
     if (fabs(d) < GPFQ_PERP_DOT) return gpfq_round_unit<SCALED>(w, alph, K, inv_step, s);
     return gpfq_round_unit<SCALED>(num / (nrm * nrm), alph, K, inv_step, s);
+}
+
+// ---------------------------------------------------------------------------------------------
+// Stochastic rounding (SPFQ, gpfq_set_rounding): unbiased rounding between the two levels that bracket the argument, with
+// counter-based draws, so a decision depends only on (seed, unit, step) -- not on the shard, launch geometry or device.
+//   draw(seed, u, t) = (splitmix64(splitmix64(seed ^ splitmix64(u)) ^ t) >> 11) * 2^-53      exact fp64 in [0, 1)
+// A walk forms the unit key splitmix64(seed ^ splitmix64(u)) once; each step then costs one splitmix64, off the chain.
+//   stoc_round(v, A, r): A[0] unless v > A[0] (NaN included); A[K-1] when v >= A[K-1]; else with k = max{i : A[i] <= v},
+//                        p = (v - A[k]) / (A[k+1] - A[k]) (correctly rounded fp64), A[k+1] if r < p else A[k].
+// A unit with a scale s uses the levels fl64(s * A[k]), as the nearest quantizer does.
+// ---------------------------------------------------------------------------------------------
+__host__ __device__ __forceinline__ uint64_t gpfq_splitmix64(uint64_t x) {
+    uint64_t z = x + 0x9E3779B97F4A7C15ull;
+    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+    return z ^ (z >> 31);
+}
+__device__ __forceinline__ uint64_t gpfq_unit_key(uint64_t seed, int64_t u) { return gpfq_splitmix64(seed ^ gpfq_splitmix64((uint64_t)u)); }
+__device__ __forceinline__ double gpfq_draw(uint64_t key, int64_t t) {
+    return (double)(gpfq_splitmix64(key ^ (uint64_t)t) >> 11) * 0x1p-53;
+}
+
+template <bool SCALED>
+__device__ __forceinline__ double gpfq_level(const double *__restrict__ alph, int k, double s) {
+    return SCALED ? __dmul_rn(s, alph[k]) : alph[k];
+}
+__device__ __forceinline__ double gpfq_stoc_pick(double v, double lo, double hi, double r) {
+    return r < __ddiv_rn(__dsub_rn(v, lo), __dsub_rn(hi, lo)) ? hi : lo;
+}
+
+// the literal form: the bracketing interval by a downward scan (levels non-decreasing, checked by the host)
+template <bool SCALED>
+static __device__ __noinline__ double gpfq_stoc_round_scan(double v, const double *__restrict__ alph, int K, double s, double r) {
+    const double a0 = gpfq_level<SCALED>(alph, 0, s);
+    if (!(v > a0)) return a0;
+    const double top = gpfq_level<SCALED>(alph, K - 1, s);
+    if (v >= top) return top;
+    int k = K - 2;
+    while (gpfq_level<SCALED>(alph, k, s) > v) --k;   // stops at k = 0 at the latest: A[0] < v
+    return gpfq_stoc_pick(v, gpfq_level<SCALED>(alph, k, s), gpfq_level<SCALED>(alph, k + 1, s), r);
+}
+
+// The same quantizer for an equispaced alphabet (inv_step > 0, as for gpfq_bit_round_eq): the grid position's integer part
+// guesses k, and the guess is moved until A[k] <= v < A[k+1] holds, so k is the literal scan's (the guess is off by at most one
+// for levels within 1 % of a step of the grid).  inv_step <= 0, a non-finite or huge argument: the scan.
+template <bool SCALED>
+__device__ __forceinline__ double gpfq_stoc_round_eq(double v, const double *__restrict__ alph, int K, double inv_step, double s,
+                                                     double r) {
+    const double a0 = gpfq_level<SCALED>(alph, 0, s);
+    const double gpos = (v - a0) * inv_step;
+    if (!(inv_step > 0.0) || !(fabs(gpos) < 1e9)) return gpfq_stoc_round_scan<SCALED>(v, alph, K, s, r);
+    if (!(v > a0)) return a0;
+    const double top = gpfq_level<SCALED>(alph, K - 1, s);
+    if (v >= top) return top;
+    int k = min(max((int)floor(gpos), 0), K - 2);
+    while (k > 0 && gpfq_level<SCALED>(alph, k, s) > v) --k;
+    while (k < K - 2 && gpfq_level<SCALED>(alph, k + 1, s) <= v) ++k;
+    return gpfq_stoc_pick(v, gpfq_level<SCALED>(alph, k, s), gpfq_level<SCALED>(alph, k + 1, s), r);
+}
+
+// ... for the ternary alphabet {-a, 0, a} with the levels in registers: p = (v - (-a)) / (0 - (-a)) on (-a, 0), (v - 0) / (a - 0)
+// on [0, a) -- the literal expressions, since v - (-a) = v + a and 0 - (-a) = a, v - 0 = v exactly
+__device__ __forceinline__ double gpfq_stoc_round_ternary(double v, double a, double r) {
+    if (!(v > -a)) return -a;
+    if (v >= a) return a;
+    if (v >= 0.0) return r < __ddiv_rn(v, a) ? a : 0.0;
+    return r < __ddiv_rn(__dadd_rn(v, a), a) ? 0.0 : -a;
+}
+
+// One greedy step with stochastic rounding: the reference's guards, then stoc_round of w (:86 guard) or num / nrm^2
+template <bool SCALED>
+__device__ __forceinline__ double gpfq_decide_stoch(double nrm, double d, double num, double w, const double *__restrict__ alph,
+                                                    int K, double inv_step, double s, double r) {
+    if (nrm < GPFQ_DEAD_NORM) return 0.0;
+    const double v = fabs(d) < GPFQ_PERP_DOT ? w : __ddiv_rn(num, nrm * nrm);
+    return gpfq_stoc_round_eq<SCALED>(v, alph, K, inv_step, s, r);
+}
+
+// The step of a walk: nearest rounding (STOCH = false: gpfq_decide_unit, unchanged) or stochastic with the draw r
+template <bool SCALED, bool STOCH>
+__device__ __forceinline__ double gpfq_decide_any(double nrm, double d, double num, double w, const double *__restrict__ alph, int K,
+                                                  double inv_step, double s, double r) {
+    if (STOCH) return gpfq_decide_stoch<SCALED>(nrm, d, num, w, alph, K, inv_step, s, r);
+    return gpfq_decide_unit<SCALED>(nrm, d, num, w, alph, K, inv_step, s);
 }
 
 __device__ __forceinline__ double warp_sum(double v) {

@@ -732,12 +732,13 @@ __device__ __forceinline__ int64_t conv_wq_offset(int64_t c, int64_t f, int64_t 
 }
 
 // SCALED: the (channel, filter) unit walks with the levels scales[a * Cg * F + (c % Cg) * F + filter] * alphabet (common.cuh).
-template <int KK, bool GROUPED, bool SCALED = false>
+// STOCH: stochastic rounding, unit id = that same scale index, step id = tap, seed seeds[a].
+template <int KK, bool GROUPED, bool SCALED = false, bool STOCH = false>
 __global__ void __launch_bounds__(128)
 conv_sweep_kernel(const double *__restrict__ gram, const float *__restrict__ W, double *__restrict__ Q,
                   int64_t CF, int64_t F, int64_t c0, const double *__restrict__ alphabets,
                   const int *__restrict__ Koff, const int *__restrict__ Flags, int64_t q_alph_stride, int64_t Cg, int64_t Fg,
-                  const double *__restrict__ scales = nullptr) {
+                  const double *__restrict__ scales = nullptr, const uint64_t *__restrict__ seeds = nullptr) {
     __shared__ double g1[KK * KK], g2[KK * KK], nrm[KK], alph[GPFQ_MAX_K];
     const int ch = blockIdx.y, a = blockIdx.z;
     const int K = Koff[a + 1] - Koff[a];
@@ -755,6 +756,7 @@ conv_sweep_kernel(const double *__restrict__ gram, const float *__restrict__ W, 
     const int64_t base = conv_wq_offset<GROUPED>(c0 + ch, f, F, Cg, Fg);
     const double sc = SCALED ? scales[(int64_t)a * CF + base] : 1.0;
     const double inv_step = SCALED ? gpfq_inv_step_s(alph, K, Flags[a], sc) : inv_step_base;
+    const uint64_t key = STOCH ? gpfq_unit_key(seeds[a], base) : 0;
     double w[KK], q[KK];
 #pragma unroll
     for (int t = 0; t < KK; ++t) w[t] = (double)W[(int64_t)t * CF + base];
@@ -765,7 +767,7 @@ conv_sweep_kernel(const double *__restrict__ gram, const float *__restrict__ W, 
         for (int s = 0; s < KK; ++s)
             if (s < t) d += w[s] * g1[t * KK + s] - q[s] * g2[t * KK + s];
         const double num = fma(w[t], g1[t * KK + t], d);
-        q[t] = gpfq_decide_unit<SCALED>(nrm[t], d, num, w[t], alph, K, inv_step, sc);
+        q[t] = gpfq_decide_any<SCALED, STOCH>(nrm[t], d, num, w[t], alph, K, inv_step, sc, STOCH ? gpfq_draw(key, t) : 0.0);
         Q[(int64_t)a * q_alph_stride + (int64_t)t * CF + base] = q[t];
     }
 }
@@ -780,12 +782,12 @@ constexpr int MAXW = 16;  // warps (filters) per CTA
 __host__ __device__ constexpr int col_off(int s, int kk) { return s * kk - s * (s - 1) / 2; }
 }  // namespace walkx
 
-template <bool GROUPED, bool SCALED = false>
+template <bool GROUPED, bool SCALED = false, bool STOCH = false>
 __global__ void __launch_bounds__(walkx::MAXW * 32)
 conv_walkx_kernel(const double *__restrict__ gram, int kk, const float *__restrict__ W, double *__restrict__ Q, int64_t CF,
                   int64_t F, int64_t c0, const double *__restrict__ alphabets, const int *__restrict__ Koff,
                   const int *__restrict__ Flags, int64_t q_alph_stride, int64_t Cg, int64_t Fg,
-                  const double *__restrict__ scales = nullptr) {
+                  const double *__restrict__ scales = nullptr, const uint64_t *__restrict__ seeds = nullptr) {
     extern __shared__ double walkx_smem[];
     const int tri = kk * (kk + 1) / 2;
     double *g1 = walkx_smem, *g2 = g1 + tri, *nrm = g2 + tri, *alph = nrm + kk;
@@ -810,6 +812,7 @@ conv_walkx_kernel(const double *__restrict__ gram, int kk, const float *__restri
     const int64_t base = conv_wq_offset<GROUPED>(c0 + ch, f, F, Cg, Fg);
     const double sc = SCALED ? scales[(int64_t)a * CF + base] : 1.0;
     const double inv_step = SCALED ? gpfq_inv_step_s(alph, K, Flags[a], sc) : inv_step_base;
+    const uint64_t key = STOCH ? gpfq_unit_key(seeds[a], base) : 0;
     double *q_out = Q + (int64_t)a * q_alph_stride + base;
     double w[4], d[4];
 #pragma unroll
@@ -828,7 +831,7 @@ conv_walkx_kernel(const double *__restrict__ gram, int kk, const float *__restri
             double qt = 0.0;
             if (lane == o) {
                 const double num = fma(w[j], g1[off + t], d[j]);
-                qt = gpfq_decide_unit<SCALED>(nrm[t], d[j], num, w[j], alph, K, inv_step, sc);
+                qt = gpfq_decide_any<SCALED, STOCH>(nrm[t], d[j], num, w[j], alph, K, inv_step, sc, STOCH ? gpfq_draw(key, t) : 0.0);
                 q_out[(int64_t)t * CF] = qt;
             }
             qt = __shfl_sync(0xffffffffu, qt, o);
@@ -864,27 +867,34 @@ __global__ void im2col_kernel(const float *__restrict__ act, int64_t n_img, int 
 }
 
 // ---- MSQ -------------------------------------------------------------------------------------
-template <typename T>
+// STOCH: stochastic rounding of element i with r = draw(seeds[0], i, 0)
+template <typename T, bool STOCH = false>
 __global__ void msq_kernel(const T *__restrict__ W, int64_t n, const double *__restrict__ alphabet, int K, int equispaced,
-                           double *__restrict__ Q) {
+                           double *__restrict__ Q, const uint64_t *__restrict__ seeds = nullptr) {
     __shared__ double alph[GPFQ_MAX_K];
     for (int e = threadIdx.x; e < K; e += blockDim.x) alph[e] = alphabet[e];
     __syncthreads();
     const double inv_step = gpfq_inv_step(alph, K, equispaced);
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
-        Q[i] = gpfq_bit_round_eq((double)W[i], alph, K, inv_step);
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        if (STOCH) Q[i] = gpfq_stoc_round_eq<false>((double)W[i], alph, K, inv_step, 1.0, gpfq_draw(gpfq_unit_key(seeds[0], i), 0));
+        else Q[i] = gpfq_bit_round_eq((double)W[i], alph, K, inv_step);
+    }
 }
 
 // Per-unit MSQ: element i rounds to the levels scales[i % n_units] * alphabet (the unit is the last axis of a Dense or conv
 // kernel, flattened C-order).
+template <bool STOCH = false>
 __global__ void msq_scaled_kernel(const float *__restrict__ W, int64_t n, const double *__restrict__ alphabet, int K, int equispaced,
-                                  const double *__restrict__ scales, int64_t n_units, double *__restrict__ Q) {
+                                  const double *__restrict__ scales, int64_t n_units, double *__restrict__ Q,
+                                  const uint64_t *__restrict__ seeds = nullptr) {
     __shared__ double alph[GPFQ_MAX_K];
     for (int e = threadIdx.x; e < K; e += blockDim.x) alph[e] = alphabet[e];
     __syncthreads();
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
         const double s = scales[i % n_units];
-        Q[i] = gpfq_bit_round_eq_s((double)W[i], alph, K, gpfq_inv_step_s(alph, K, equispaced, s), s);
+        const double inv_step = gpfq_inv_step_s(alph, K, equispaced, s);
+        if (STOCH) Q[i] = gpfq_stoc_round_eq<true>((double)W[i], alph, K, inv_step, s, gpfq_draw(gpfq_unit_key(seeds[0], i), 0));
+        else Q[i] = gpfq_bit_round_eq_s((double)W[i], alph, K, inv_step, s);
     }
 }
 
@@ -1011,12 +1021,15 @@ int conv_sweep_stage(gpfq_ctx *ctx, int kk, const double *gram, const float *W, 
     const bool grouped = groups > 1;
     dim3 grid((unsigned)ceil_div64(Fg, 128), (unsigned)n_ch, (unsigned)n_alph);
     const int64_t CF = Cg * F, qs = (int64_t)kk * CF;
-#define SWEEP_LAUNCH(KKV, G, S) \
-    conv_sweep_kernel<KKV, G, S><<<grid, 128, 0, ctx->stream>>>(gram, W, Q, CF, F, c0, d_alph, d_koff, d_flags, qs, Cg, Fg, scales)
+    const uint64_t *seeds = ctx->d_seeds;
+#define SWEEP_LAUNCH(KKV, G, S, R) \
+    conv_sweep_kernel<KKV, G, S, R><<<grid, 128, 0, ctx->stream>>>(gram, W, Q, CF, F, c0, d_alph, d_koff, d_flags, qs, Cg, Fg, scales, seeds)
+#define SWEEP_SCALED(KKV, R)                                                                                            \
+    if (scales) { if (grouped) SWEEP_LAUNCH(KKV, true, true, R); else SWEEP_LAUNCH(KKV, false, true, R); }              \
+    else { if (grouped) SWEEP_LAUNCH(KKV, true, false, R); else SWEEP_LAUNCH(KKV, false, false, R); }
 #define SWEEP_CASE(KKV)                                                                                                 \
     case KKV:                                                                                                           \
-        if (scales) { if (grouped) SWEEP_LAUNCH(KKV, true, true); else SWEEP_LAUNCH(KKV, false, true); }                \
-        else { if (grouped) SWEEP_LAUNCH(KKV, true, false); else SWEEP_LAUNCH(KKV, false, false); }                     \
+        if (seeds) { SWEEP_SCALED(KKV, true) } else { SWEEP_SCALED(KKV, false) }                                        \
         break;
     switch (kk) {
         SWEEP_CASE(1) SWEEP_CASE(2) SWEEP_CASE(3) SWEEP_CASE(4) SWEEP_CASE(6) SWEEP_CASE(9)
@@ -1026,13 +1039,16 @@ int conv_sweep_stage(gpfq_ctx *ctx, int kk, const double *gram, const float *W, 
             const int warps = Fg < MAXW ? (int)Fg : MAXW;
             const size_t smem = ((size_t)kk * (kk + 1) + kk + GPFQ_MAX_K) * sizeof(double);
             dim3 wgrid((unsigned)ceil_div64(Fg, warps), (unsigned)n_ch, (unsigned)n_alph);
-            auto k = grouped ? (scales ? conv_walkx_kernel<true, true> : conv_walkx_kernel<true, false>)
-                             : (scales ? conv_walkx_kernel<false, true> : conv_walkx_kernel<false, false>);
+            auto k = seeds ? (grouped ? (scales ? conv_walkx_kernel<true, true, true> : conv_walkx_kernel<true, false, true>)
+                                      : (scales ? conv_walkx_kernel<false, true, true> : conv_walkx_kernel<false, false, true>))
+                           : (grouped ? (scales ? conv_walkx_kernel<true, true> : conv_walkx_kernel<true, false>)
+                                      : (scales ? conv_walkx_kernel<false, true> : conv_walkx_kernel<false, false>));
             CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            k<<<wgrid, warps * 32, smem, ctx->stream>>>(gram, kk, W, Q, CF, F, c0, d_alph, d_koff, d_flags, qs, Cg, Fg, scales);
+            k<<<wgrid, warps * 32, smem, ctx->stream>>>(gram, kk, W, Q, CF, F, c0, d_alph, d_koff, d_flags, qs, Cg, Fg, scales, seeds);
         }
     }
 #undef SWEEP_CASE
+#undef SWEEP_SCALED
 #undef SWEEP_LAUNCH
     KERNEL_CHECK(ctx);
     return GPFQ_OK;
@@ -1094,9 +1110,14 @@ int msq_stage(gpfq_ctx *ctx, const void *W, int is_f64, int64_t n, const double 
               const double *d_scales, int64_t n_units) {
     int bx = (int)(ceil_div64(n, 256) < 1184 ? ceil_div64(n, 256) : 1184);
     if (bx < 1) bx = 1;
-    if (d_scales)
+    const uint64_t *seeds = ctx->d_seeds;   // stochastic rounding (nullptr: nearest)
+    if (d_scales && seeds)
+        msq_scaled_kernel<true><<<bx, 256, 0, ctx->stream>>>((const float *)W, n, d_alph, K, equispaced, d_scales, n_units, Q, seeds);
+    else if (d_scales)
         msq_scaled_kernel<<<bx, 256, 0, ctx->stream>>>((const float *)W, n, d_alph, K, equispaced, d_scales, n_units, Q);
+    else if (is_f64 && seeds) msq_kernel<double, true><<<bx, 256, 0, ctx->stream>>>((const double *)W, n, d_alph, K, equispaced, Q, seeds);
     else if (is_f64) msq_kernel<double><<<bx, 256, 0, ctx->stream>>>((const double *)W, n, d_alph, K, equispaced, Q);
+    else if (seeds) msq_kernel<float, true><<<bx, 256, 0, ctx->stream>>>((const float *)W, n, d_alph, K, equispaced, Q, seeds);
     else msq_kernel<float><<<bx, 256, 0, ctx->stream>>>((const float *)W, n, d_alph, K, equispaced, Q);
     KERNEL_CHECK(ctx);
     return GPFQ_OK;

@@ -97,6 +97,24 @@ __device__ __forceinline__ double gpfq_decide_rcp_unit(double nrm, double rinv, 
     return gpfq_bit_round_eq_s(v, alph, K, inv_step, s);
 }
 
+// The same step with stochastic rounding (r = the step's draw): the argument is formed exactly as above (the Markstein quotient is
+// the correctly rounded num / nrm^2), then stoc_round between the bracketing levels (common.cuh)
+template <bool SCALED>
+__device__ __forceinline__ double gpfq_decide_rcp_stoch(double nrm, double rinv, double d, double num, double w,
+                                                        const double *__restrict__ alph, int K, double inv_step, double tern,
+                                                        double s, double r) {
+    if (nrm < GPFQ_DEAD_NORM) return 0.0;
+    double v = w;
+    if (!(fabs(d) < GPFQ_PERP_DOT)) {
+        const double den = nrm * nrm;
+        const double q0 = num * rinv;
+        const double e = fma(-q0, den, num);
+        v = fma(e, rinv, q0);
+    }
+    if (tern > 0.0) return gpfq_stoc_round_ternary(v, tern, r);
+    return gpfq_stoc_round_eq<SCALED>(v, alph, K, inv_step, s, r);
+}
+
 // Per-neuron scale, inv_step and ternary radius of neuron jt + j (SCALED; else the alphabet's own)
 template <bool SCALED>
 __device__ __forceinline__ void sweep_unit_levels(const double *__restrict__ scales, int64_t idx, bool live,
@@ -121,13 +139,15 @@ struct SweepCfg {
 };
 
 // SCALED: neuron j of alphabet a walks with the levels scales[a * nj + j] * alphabet (per-channel alphabets).
-template <int NT, bool ALIGNED, bool SCALED = false>
+// STOCH: stochastic rounding, neuron j with unit id u0 + j and seed seeds[a], direction t with step id t.
+template <int NT, bool ALIGNED, bool SCALED = false, bool STOCH = false>
 __global__ void __launch_bounds__(256, 2)
 sweep_tile_kernel(const double *__restrict__ G1, const double *__restrict__ G2, int64_t ldg, int64_t N0,
                   const double *__restrict__ Wt, double *__restrict__ Qt, int64_t nj,
                   const double *__restrict__ alphabets, const int *__restrict__ Koff,
                   const int *__restrict__ Flags, int64_t t_begin, int64_t t_end, const double *__restrict__ Dt,
-                  int64_t ldd, const double *__restrict__ scales = nullptr) {
+                  int64_t ldd, const double *__restrict__ scales = nullptr, const uint64_t *__restrict__ seeds = nullptr,
+                  int64_t u0 = 0) {
     // Directions [t_begin, t_end) (t_begin a multiple of 32).  Dt (nullable): (n_alph, nj, ldd) contributions of the
     // directions before t_begin, from one large NT contraction on the host side (two-level blocking).
     using Cfg = SweepCfg<NT>;
@@ -163,6 +183,7 @@ sweep_tile_kernel(const double *__restrict__ G1, const double *__restrict__ G2, 
     double sc, inv_u, tern_u;
     sweep_unit_levels<SCALED>(scales, (int64_t)a * nj + jt + (tid >> 2), tid < 4 * NT && jt + (tid >> 2) < nj, alph, K, Flags[a], inv_step,
                               tern, &sc, &inv_u, &tern_u);
+    const uint64_t key = STOCH ? gpfq_unit_key(seeds[a], u0 + jt + (tid >> 2)) : 0;
 
     // this thread's 16-byte chunks of every W / Q tile (fixed for the whole walk)
     int w_off[WCH];
@@ -325,7 +346,9 @@ sweep_tile_kernel(const double *__restrict__ G1, const double *__restrict__ G2, 
                     const double d0 = __shfl_sync(0xffffffffu, d[0], (lane & ~3) + rr);
                     const double wv = wrow[tt];
                     const double num = fma(wv, g1dd[tt], d0);
-                    double q = gpfq_decide_rcp_unit<SCALED>(nrm[tt], rinv[tt], d0, num, wv, alph, K, inv_u, tern_u, sc);
+                    double q = STOCH ? gpfq_decide_rcp_stoch<SCALED>(nrm[tt], rinv[tt], d0, num, wv, alph, K, inv_u, tern_u, sc,
+                                                                     gpfq_draw(key, t0 + tt))
+                                     : gpfq_decide_rcp_unit<SCALED>(nrm[tt], rinv[tt], d0, num, wv, alph, K, inv_u, tern_u, sc);
                     if (tt >= nb) q = 0.0;  // past the end of a partial block: no decision, no update
                     if (r == rr && tt < nb) qrow[tt] = q;
                     if (rr < 3) {
@@ -373,12 +396,13 @@ struct PipeCfg {
     static constexpr size_t SMEM = sizeof(double) * ((size_t)STAGES * (B + NT) * LD + 2 * SET + GPFQ_MAX_K);
 };
 
-template <int NT, bool SCALED = false>
+template <int NT, bool SCALED = false, bool STOCH = false>
 __global__ void __launch_bounds__(256, 1)
 sweep_pipe_kernel(const double *__restrict__ G1, const double *__restrict__ G2, int64_t ldg, int64_t N0,
                   const double *__restrict__ Wt, double *__restrict__ Qt, int64_t nj, const double *__restrict__ alphabets,
                   const int *__restrict__ Koff, const int *__restrict__ Flags, int64_t t_begin, int64_t t_end,
-                  const double *__restrict__ Dt, int64_t ldd, const double *__restrict__ scales = nullptr) {
+                  const double *__restrict__ Dt, int64_t ldd, const double *__restrict__ scales = nullptr,
+                  const uint64_t *__restrict__ seeds = nullptr, int64_t u0 = 0) {
     using Cfg = PipeCfg<NT>;
     constexpr int B = Cfg::B, KC = Cfg::KC, LD = Cfg::LD, STAGES = Cfg::STAGES, CT = Cfg::CT, NA = NT / 8, NW = 4 * NT;
     constexpr int BAR_C = 1, BAR_READY = 2, BAR_WALK_DONE = 4, BAR_Q_STORED = 6, HANDOVER = NW + CT;
@@ -565,6 +589,7 @@ sweep_pipe_kernel(const double *__restrict__ G1, const double *__restrict__ G2, 
         double sc, inv_u, tern_u;
         sweep_unit_levels<SCALED>(scales, (int64_t)a * nj + jt + j, jt + j < nj, alph, K, Flags[a], inv_step, tern, &sc, &inv_u,
                                   &tern_u);
+        const uint64_t key = STOCH ? gpfq_unit_key(seeds[a], u0 + jt + j) : 0;
         for (int b = 0; b < nblk; ++b) {
             const int s = b & 1;
             const int64_t t0 = t_begin + (int64_t)b * B;
@@ -589,7 +614,9 @@ sweep_pipe_kernel(const double *__restrict__ G1, const double *__restrict__ G2, 
                     const double d0 = __shfl_sync(0xffffffffu, d[0], (lane & ~3) + rr);
                     const double wv = wrow[tt];
                     const double num = fma(wv, g1dd[tt], d0);
-                    double q = gpfq_decide_rcp_unit<SCALED>(nrm[tt], rinv[tt], d0, num, wv, alph, K, inv_u, tern_u, sc);
+                    double q = STOCH ? gpfq_decide_rcp_stoch<SCALED>(nrm[tt], rinv[tt], d0, num, wv, alph, K, inv_u, tern_u, sc,
+                                                                     gpfq_draw(key, t0 + tt))
+                                     : gpfq_decide_rcp_unit<SCALED>(nrm[tt], rinv[tt], d0, num, wv, alph, K, inv_u, tern_u, sc);
                     if (tt >= nb) q = 0.0;  // past the end of a partial block: no decision, no update
                     if (r == rr && tt < nb) qrow[tt] = q;
                     if (rr < 3) {
@@ -624,12 +651,15 @@ sweep_pipe_kernel(const double *__restrict__ G1, const double *__restrict__ G2, 
 template <int NT>
 static int launch_sweep_pipe(gpfq_ctx *ctx, const double *G1, const double *G2, int64_t ldg, int64_t N0, const double *Wt,
                              double *Qt, int64_t nj, const double *d_alph, const int *d_koff, const int *d_flags,
-                             int n_alph, int64_t t_begin, int64_t t_end, const double *Dt, int64_t ldd, const double *scales) {
+                             int n_alph, int64_t t_begin, int64_t t_end, const double *Dt, int64_t ldd, const double *scales,
+                             int64_t u0) {
     const size_t smem = PipeCfg<NT>::SMEM;
     dim3 grid((unsigned)ceil_div64(nj, NT), (unsigned)n_alph);
-    auto k = scales ? sweep_pipe_kernel<NT, true> : sweep_pipe_kernel<NT, false>;
+    const uint64_t *seeds = ctx->d_seeds;
+    auto k = seeds ? (scales ? sweep_pipe_kernel<NT, true, true> : sweep_pipe_kernel<NT, false, true>)
+                   : (scales ? sweep_pipe_kernel<NT, true> : sweep_pipe_kernel<NT, false>);
     CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    k<<<grid, 256, smem, ctx->stream>>>(G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, t_begin, t_end, Dt, ldd, scales);
+    k<<<grid, 256, smem, ctx->stream>>>(G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, t_begin, t_end, Dt, ldd, scales, seeds, u0);
     KERNEL_CHECK(ctx);
     return GPFQ_OK;
 }
@@ -637,15 +667,19 @@ static int launch_sweep_pipe(gpfq_ctx *ctx, const double *G1, const double *G2, 
 template <int NT>
 static int launch_sweep_tile(gpfq_ctx *ctx, const double *G1, const double *G2, int64_t ldg, int64_t N0, const double *Wt,
                              double *Qt, int64_t nj, const double *d_alph, const int *d_koff, const int *d_flags,
-                             int n_alph, int64_t t_begin, int64_t t_end, const double *Dt, int64_t ldd, const double *scales) {
+                             int n_alph, int64_t t_begin, int64_t t_end, const double *Dt, int64_t ldd, const double *scales,
+                             int64_t u0) {
     const size_t smem = SweepCfg<NT>::SMEM;
     dim3 grid((unsigned)ceil_div64(nj, NT), (unsigned)n_alph);
     const bool aligned = (N0 % 2 == 0) && (ldg % 2 == 0) && ((uintptr_t)G1 % 16 == 0) && ((uintptr_t)G2 % 16 == 0) &&
                          ((uintptr_t)Wt % 16 == 0) && ((uintptr_t)Qt % 16 == 0) && ((nj * N0) % 2 == 0);
-    auto k = aligned ? (scales ? sweep_tile_kernel<NT, true, true> : sweep_tile_kernel<NT, true, false>)
-                     : (scales ? sweep_tile_kernel<NT, false, true> : sweep_tile_kernel<NT, false, false>);
+    const uint64_t *seeds = ctx->d_seeds;
+    auto k = seeds ? (aligned ? (scales ? sweep_tile_kernel<NT, true, true, true> : sweep_tile_kernel<NT, true, false, true>)
+                              : (scales ? sweep_tile_kernel<NT, false, true, true> : sweep_tile_kernel<NT, false, false, true>))
+                   : (aligned ? (scales ? sweep_tile_kernel<NT, true, true> : sweep_tile_kernel<NT, true, false>)
+                              : (scales ? sweep_tile_kernel<NT, false, true> : sweep_tile_kernel<NT, false, false>));
     CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    k<<<grid, 256, smem, ctx->stream>>>(G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, t_begin, t_end, Dt, ldd, scales);
+    k<<<grid, 256, smem, ctx->stream>>>(G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, t_begin, t_end, Dt, ldd, scales, seeds, u0);
     KERNEL_CHECK(ctx);
     return GPFQ_OK;
 }
@@ -795,7 +829,7 @@ static int64_t pick_range_length(gpfq_ctx *ctx, int64_t nj, int n_alph) {
 static int dispatch_sweep_tile(gpfq_ctx *ctx, int NT, const double *G1, const double *G2, int64_t ldg, int64_t N0,
                                const double *Wt, double *Qt, int64_t nj, const double *d_alph, const int *d_koff,
                                const int *d_flags, int n_alph, int64_t tb, int64_t te, const double *Dp, int64_t R,
-                               const double *scales) {
+                               const double *scales, int64_t u0) {
     // The pipelined walk (one CTA per SM) when its 16-byte copies are possible and every CTA of the launch is resident at
     // once; the narrowest neuron tile that allows it.
     const bool aligned = (N0 % 2 == 0) && (ldg % 2 == 0) && ((uintptr_t)G1 % 16 == 0) && ((uintptr_t)G2 % 16 == 0) &&
@@ -803,22 +837,22 @@ static int dispatch_sweep_tile(gpfq_ctx *ctx, int NT, const double *G1, const do
     if (aligned) {
         const int64_t sms = ctx->sm_count;
         if (ceil_div64(nj, 8) * n_alph <= sms)
-            return launch_sweep_pipe<8>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R, scales);
+            return launch_sweep_pipe<8>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R, scales, u0);
         if (ceil_div64(nj, 16) * n_alph <= sms)
-            return launch_sweep_pipe<16>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R, scales);
+            return launch_sweep_pipe<16>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R, scales, u0);
         if (ceil_div64(nj, 32) * n_alph <= sms)
-            return launch_sweep_pipe<32>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R, scales);
+            return launch_sweep_pipe<32>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R, scales, u0);
     }
-    if (NT == 32) return launch_sweep_tile<32>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R, scales);
-    if (NT == 16) return launch_sweep_tile<16>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R, scales);
-    return launch_sweep_tile<8>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R, scales);
+    if (NT == 32) return launch_sweep_tile<32>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R, scales, u0);
+    if (NT == 16) return launch_sweep_tile<16>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R, scales, u0);
+    return launch_sweep_tile<8>(ctx, G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te, Dp, R, scales, u0);
 }
 
 // Sweep with the low-rank outer level.  Wt (nj, N0) is ready; Qt (n_alph, nj, N0) receives the result.  scales (nullable):
 // (n_alph, nj) per-neuron scales.
 static int dense_lowrank_sweep(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ldx, int64_t N0, int64_t m,
                                const double *Wt, double *Qt, int64_t nj, const double *d_alph, const int *d_koff,
-                               const int *d_flags, int n_alph, int NT, const double *scales) {
+                               const int *d_flags, int n_alph, int NT, const double *scales, int64_t u0) {
     const bool same = (Xq == X);
     cudaStream_t st = ctx->stream;
     const int64_t R = pick_range_length(ctx, nj, n_alph);
@@ -937,7 +971,8 @@ static int dense_lowrank_sweep(gpfq_ctx *ctx, const float *X, const float *Xq, i
                     }
                 }
                 rc = dispatch_sweep_tile(ctx, NT, Gc1 - tb, Gc2 - tb, R, N0, Wt + j_lo * N0, Qt + j_lo * N0, njh, d_alph, d_koff,
-                                         d_flags, 1, tb, te, tb > 0 ? Do + j_lo * R : nullptr, R, scales ? scales + j_lo : nullptr);
+                                         d_flags, 1, tb, te, tb > 0 ? Do + j_lo * R : nullptr, R, scales ? scales + j_lo : nullptr,
+                                         u0 + j_lo);
             }
             ctx->stream = keep;
             return rc;
@@ -1018,7 +1053,7 @@ static int dense_lowrank_sweep(gpfq_ctx *ctx, const float *X, const float *Xq, i
         }
         // the compact tiles are addressed like the full matrices: column s of row t lives at Gc[t * R + (s - tb)]
         GPFQ_TRY(dispatch_sweep_tile(ctx, NT, Gc1 - tb, Gc2 - tb, R, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te,
-                                     tb > 0 ? Do : nullptr, R, scales));
+                                     tb > 0 ? Do : nullptr, R, scales, u0));
     }
     return GPFQ_OK;
 }
@@ -1055,7 +1090,7 @@ __global__ void unit_steps_kernel(const double *__restrict__ scales, int64_t nj,
 // residual update becomes -diag(h) K'_r X~_r (a per-row multiplier in the slgemm_i8_kernel epilogue); the W part and D_r are unchanged.
 static int dense_lowrank_sweep_i8(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ldx, int64_t N0, int64_t m,
                                   const double *Wt, int64_t nj, const double *d_alph, double h, gpfq_stats *stats, const float *W,
-                                  int64_t ldw, int64_t j0, double *Qd, int64_t ldq, int64_t col0, const double *d_scales) {
+                                  int64_t ldw, int64_t j0, double *Qd, int64_t ldq, int64_t col0, const double *d_scales, int64_t u0) {
     const bool same = (Xq == X);
     cudaStream_t st = ctx->stream, side = ctx->copy_stream;
     int64_t R = pick_range_length(ctx, nj, 1);
@@ -1227,7 +1262,7 @@ static int dense_lowrank_sweep_i8(gpfq_ctx *ctx, const float *X, const float *Xq
                 if (rc != GPFQ_OK) break;
             }
             rc = sweep_tc_range(ctx, tct, tb, te, j_lo, njh, sKq, njP, j_lo, a_top, d_levels, K_levels,   // {-a, 0, a}: h = a / 2
-                                d_scales ? d_scales + j_lo : nullptr);
+                                d_scales ? d_scales + j_lo : nullptr, u0 + j_lo);
         }
         ctx->stream = keep;
         return rc;
@@ -1272,13 +1307,14 @@ static int dense_lowrank_sweep_i8(gpfq_ctx *ctx, const float *X, const float *Xq
 int dense_gram_path(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ldx, int64_t N0, int64_t m,
                     const float *W, int64_t ldw, int64_t j0, int64_t nj, const double *d_alph,
                     const int *d_koff, const int *d_flags, int n_alph, double *Qd, int64_t ldq, int64_t col0,
-                    gpfq_stats *st, const double *G1_pre, const double *G2_pre, const double *d_scales) {
+                    gpfq_stats *st, const double *G1_pre, const double *G2_pre, const double *d_scales, int64_t u0) {
     // G2_pre != NULL: the Gram stage already ran elsewhere (sample-split over the ranks of a job and all-reduced,
     // gpfq_dense_layer_from_gram); X / Xq / m are then unused and the sweep starts from the given (N0, N0) matrices.
     const bool pre = (G2_pre != nullptr);
     const bool same = pre ? (G1_pre == nullptr || G1_pre == G2_pre) : (Xq == X);
     double *G1 = nullptr, *G2 = nullptr, *Wt = nullptr, *Qt = nullptr;
     double h_step = 0.0;
+    // Stochastic rounding (ctx->d_seeds): every walk below takes it; the shard's first neuron has unit id u0
     const bool i8_sweep = !pre && dense_lowrank_uses_i8(ctx, N0, m, nj, n_alph, &h_step);
     const bool lowrank = !pre && dense_uses_lowrank(ctx, N0, m, nj, n_alph, same, i8_sweep);
     // Neurons per CTA of the range walk: the narrowest tile that still fits every CTA on the chip at once (two per SM, so
@@ -1295,9 +1331,9 @@ int dense_gram_path(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ldx,
     }
     if (lowrank) {
         if (i8_sweep) {   // writes Qd itself
-            GPFQ_TRY(dense_lowrank_sweep_i8(ctx, X, Xq, ldx, N0, m, Wt, nj, d_alph, h_step, st, W, ldw, j0, Qd, ldq, col0, d_scales));
+            GPFQ_TRY(dense_lowrank_sweep_i8(ctx, X, Xq, ldx, N0, m, Wt, nj, d_alph, h_step, st, W, ldw, j0, Qd, ldq, col0, d_scales, u0));
         } else {
-            GPFQ_TRY(dense_lowrank_sweep(ctx, X, Xq, ldx, N0, m, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, NT, d_scales));
+            GPFQ_TRY(dense_lowrank_sweep(ctx, X, Xq, ldx, N0, m, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, NT, d_scales, u0));
             for (int a = 0; a < n_alph; ++a) {
                 dim3 grid((unsigned)ceil_div64(N0, 32), (unsigned)ceil_div64(nj, 32));
                 transpose_q_kernel<<<grid, dim3(32, 8), 0, ctx->stream>>>(Qt + (int64_t)a * nj * N0, N0, nj,
@@ -1424,11 +1460,11 @@ int dense_gram_path(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ldx,
         }
         if (use_tc) {
             if (tb > 0) GPFQ_TRY(sweep_tc_add_outer(ctx, Pd + tb, N0P, Do, R, nj, te - tb));
-            GPFQ_TRY(sweep_tc_range(ctx, tct, tb, te, 0, nj, sKq, njP, 0, a_top, d_alph, K_levels, d_scales));
+            GPFQ_TRY(sweep_tc_range(ctx, tct, tb, te, 0, nj, sKq, njP, 0, a_top, d_alph, K_levels, d_scales, u0));
             GPFQ_TRY(sweep_tc_qt_from_kq(ctx, sKq, njP, tb, te, nj, d_alph, K_levels, Qt, N0, d_scales));
         } else {
             GPFQ_TRY(dispatch_sweep_tile(ctx, NT, G1, G2, N0, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, n_alph, tb, te,
-                                         tb > 0 ? Do : nullptr, R, d_scales));
+                                         tb > 0 ? Do : nullptr, R, d_scales, u0));
         }
     }
     for (int a = 0; a < n_alph; ++a) {

@@ -39,13 +39,15 @@ __global__ void __launch_bounds__(256) row_norms_kernel(const float *__restrict_
 }
 
 // SCALED: neuron jb + j of the shard walks with the levels scales[jb + j] * alphabet (common.cuh)
-template <int J, bool SCALED = false>
+// STOCH: stochastic rounding with the seed *seed, unit id u0 + jb + j (the global neuron), step id t
+template <int J, bool SCALED = false, bool STOCH = false>
 __global__ void __launch_bounds__(STREAM_T)
 dense_stream_kernel(const float *__restrict__ X, const float *__restrict__ Xq, int64_t ldx, int64_t N0,
                     int64_t m, const float *__restrict__ W, int64_t ldw, int64_t j0, int64_t nj,
                     const double *__restrict__ nrm, const double *__restrict__ alphabet, int K,
                     double *__restrict__ Q, int64_t ldq, int64_t col0, double *__restrict__ u_scratch,
-                    int u_in_smem, const double *__restrict__ scales = nullptr) {
+                    int u_in_smem, const double *__restrict__ scales = nullptr, const uint64_t *__restrict__ seed = nullptr,
+                    int64_t u0 = 0) {
     extern __shared__ __align__(16) unsigned char stream_smem[];
     constexpr int NW = STREAM_T / 32;
     __shared__ double red[NW][2 * J];
@@ -61,6 +63,7 @@ dense_stream_kernel(const float *__restrict__ X, const float *__restrict__ Xq, i
     for (int64_t e = tid; e < (int64_t)J * m; e += STREAM_T) u[e] = 0.0;
     __syncthreads();
     const double sc = (SCALED && tid < J && jb + tid < nj) ? scales[jb + tid] : 0.0;
+    const uint64_t key = (STOCH && tid < J) ? gpfq_unit_key(*seed, u0 + jb + tid) : 0;
 
     float wprev[J];
     double qprev[J];
@@ -111,7 +114,8 @@ dense_stream_kernel(const float *__restrict__ X, const float *__restrict__ Xq, i
         if (tid < J) {
             double dd = 0.0, ss = 0.0;
             for (int wv = 0; wv < NW; ++wv) { dd += red[wv][tid]; ss += red[wv][J + tid]; }
-            const double q = SCALED ? gpfq_decide_unit<true>(nrm[t], dd, ss, (double)w[tid], alph, K, 0.0, sc)
+            const double q = STOCH    ? gpfq_decide_stoch<SCALED>(nrm[t], dd, ss, (double)w[tid], alph, K, 0.0, sc, gpfq_draw(key, t))
+                           : SCALED ? gpfq_decide_unit<true>(nrm[t], dd, ss, (double)w[tid], alph, K, 0.0, sc)
                                     : gpfq_decide(nrm[t], dd, ss, (double)w[tid], alph, K);
             qsh[tid] = q;
             if (jb + tid < nj) Q[t * ldq + col0 + jb + tid] = q;
@@ -167,22 +171,25 @@ __device__ __forceinline__ int warp_reduce_index(int lane) {
     return idx;
 }
 
-template <int EPV, int J, bool LITERAL, bool VEC, bool SCALED = false>
+template <int EPV, int J, bool LITERAL, bool VEC, bool SCALED = false, bool STOCH = false>
 __global__ void __launch_bounds__(STREAM_T)
 dense_stream_reg_kernel(const float *__restrict__ X, const float *__restrict__ Xq, int64_t ldx, int64_t N0,
                         int64_t m, const float *__restrict__ W, int64_t ldw, int64_t j0, int64_t nj,
                         const double *__restrict__ nrm, const double *__restrict__ g1d,
                         const double *__restrict__ alphabet, int K, int equispaced,
-                        double *__restrict__ Q, int64_t ldq, int64_t col0, const double *__restrict__ scales = nullptr) {
+                        double *__restrict__ Q, int64_t ldq, int64_t col0, const double *__restrict__ scales = nullptr,
+                        const uint64_t *__restrict__ seed = nullptr, int64_t u0 = 0) {
     constexpr int NW = STREAM_T / 32, EPT = 4 * EPV;
     constexpr int V = LITERAL ? 2 * J : J;  // values reduced per step
     __shared__ double red[NW][V];
     __shared__ double qsh[J];
     __shared__ double alph[GPFQ_MAX_K];
     __shared__ double unit_s[SCALED ? 2 * J : 1];  // per neuron: scale, inv_step of its levels
+    __shared__ uint64_t unit_key[STOCH ? J : 1];    // per neuron: the stochastic-rounding unit key (one per unit, not per step)
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int64_t jb = (int64_t)blockIdx.x * J;
     for (int e = tid; e < K; e += STREAM_T) alph[e] = alphabet[e];
+    if (STOCH && tid < J) unit_key[tid] = gpfq_unit_key(*seed, u0 + jb + tid);
     if (SCALED && tid < J) {
         const double sc = jb + tid < nj ? scales[jb + tid] : 0.0;
         unit_s[tid] = sc;
@@ -287,8 +294,11 @@ dense_stream_reg_kernel(const float *__restrict__ X, const float *__restrict__ X
 #pragma unroll
                     for (int jj = 1; jj < J; ++jj) wj = (j == jj) ? w[jj] : wj;
                     const double num = LITERAL ? ss : fma((double)wj, g1_t, dd);
-                    const double q = SCALED ? gpfq_decide_unit<true>(nrm_t, dd, num, (double)wj, alph, K, unit_s[J + j], unit_s[j])
-                                            : gpfq_decide(nrm_t, dd, num, (double)wj, alph, K, inv_step);
+                    const double q =
+                        STOCH    ? gpfq_decide_stoch<SCALED>(nrm_t, dd, num, (double)wj, alph, K, SCALED ? unit_s[J + j] : inv_step,
+                                                             SCALED ? unit_s[j] : 1.0, gpfq_draw(unit_key[j], t))
+                      : SCALED ? gpfq_decide_unit<true>(nrm_t, dd, num, (double)wj, alph, K, unit_s[J + j], unit_s[j])
+                               : gpfq_decide(nrm_t, dd, num, (double)wj, alph, K, inv_step);
                     qsh[j] = q;
                     if (jb + j < nj) Q[t * ldq + col0 + jb + j] = q;
                 }
@@ -321,18 +331,21 @@ template <int EPV, int J>
 static int launch_stream_reg(gpfq_ctx *ctx, bool literal, bool vec, const float *X, const float *Xq, int64_t ldx,
                              int64_t N0, int64_t m, const float *W, int64_t ldw, int64_t j0, int64_t nj,
                              const double *nrm, const double *g1d, const double *d_alph, int K, int eq, double *Qd,
-                             int64_t ldq, int64_t col0, const double *scales) {
+                             int64_t ldq, int64_t col0, const double *scales, const uint64_t *seed, int64_t u0) {
     const unsigned nblk = (unsigned)ceil_div64(nj, J);
-#define LAUNCH(LIT, VEC, S) \
-    dense_stream_reg_kernel<EPV, J, LIT, VEC, S><<<nblk, STREAM_T, 0, ctx->stream>>>(X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm, \
-                                                                                  g1d, d_alph, K, eq, Qd, ldq, col0, scales)
-    if (scales) {
-        if (literal) { if (vec) LAUNCH(true, true, true); else LAUNCH(true, false, true); }
-        else { if (vec) LAUNCH(false, true, true); else LAUNCH(false, false, true); }
-    } else {
-        if (literal) { if (vec) LAUNCH(true, true, false); else LAUNCH(true, false, false); }
-        else { if (vec) LAUNCH(false, true, false); else LAUNCH(false, false, false); }
+#define LAUNCH(LIT, VEC, S, R) \
+    dense_stream_reg_kernel<EPV, J, LIT, VEC, S, R><<<nblk, STREAM_T, 0, ctx->stream>>>(X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm, \
+                                                                                     g1d, d_alph, K, eq, Qd, ldq, col0, scales, seed, u0)
+#define LAUNCH_S(R)                                                                           \
+    if (scales) {                                                                             \
+        if (literal) { if (vec) LAUNCH(true, true, true, R); else LAUNCH(true, false, true, R); }  \
+        else { if (vec) LAUNCH(false, true, true, R); else LAUNCH(false, false, true, R); }        \
+    } else {                                                                                  \
+        if (literal) { if (vec) LAUNCH(true, true, false, R); else LAUNCH(true, false, false, R); } \
+        else { if (vec) LAUNCH(false, true, false, R); else LAUNCH(false, false, false, R); }      \
     }
+    if (seed) { LAUNCH_S(true) } else { LAUNCH_S(false) }
+#undef LAUNCH_S
 #undef LAUNCH
     KERNEL_CHECK(ctx);
     return GPFQ_OK;
@@ -342,11 +355,11 @@ static int launch_stream_reg(gpfq_ctx *ctx, bool literal, bool vec, const float 
 static int dispatch_stream_reg(gpfq_ctx *ctx, int epv, int J, bool literal, bool vec, const float *X, const float *Xq,
                                int64_t ldx, int64_t N0, int64_t m, const float *W, int64_t ldw, int64_t j0, int64_t nj,
                                const double *nrm, const double *g1d, const double *d_alph, int K, int eq, double *Qd,
-                               int64_t ldq, int64_t col0, const double *scales) {
+                               int64_t ldq, int64_t col0, const double *scales, const uint64_t *seed, int64_t u0) {
 #define SR(E, JJ) \
     if (epv == E && J == JJ) \
         return launch_stream_reg<E, JJ>(ctx, literal, vec, X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm, g1d, d_alph, K, eq, Qd, \
-                                        ldq, col0, scales);
+                                        ldq, col0, scales, seed, u0);
     SR(1, 1) SR(1, 2) SR(1, 4)
     SR(2, 1) SR(2, 2)
     SR(3, 1) SR(3, 2)
@@ -358,29 +371,32 @@ static int dispatch_stream_reg(gpfq_ctx *ctx, int epv, int J, bool literal, bool
 template <int J>
 static int launch_stream(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ldx, int64_t N0, int64_t m,
                          const float *W, int64_t ldw, int64_t j0, int64_t nj, const double *nrm,
-                         const double *d_alph, int K, double *Qd, int64_t ldq, int64_t col0, const double *scales) {
+                         const double *d_alph, int K, double *Qd, int64_t ldq, int64_t col0, const double *scales,
+                         const uint64_t *seed, int64_t u0) {
     const int64_t nblk = ceil_div64(nj, J);
     const size_t need = (size_t)J * m * sizeof(double);
     const size_t static_smem = 8192;  // red/qsh/alph, generous
     const bool in_smem = need + static_smem <= ctx->smem_optin;
     double *scratch = nullptr;
     if (!in_smem) GPFQ_TRY(gpfq_ws(ctx, WS_U, (size_t)nblk * need, (void **)&scratch));
-    auto k = scales ? dense_stream_kernel<J, true> : dense_stream_kernel<J, false>;
+    auto k = seed ? (scales ? dense_stream_kernel<J, true, true> : dense_stream_kernel<J, false, true>)
+                  : (scales ? dense_stream_kernel<J, true> : dense_stream_kernel<J, false>);
     if (in_smem)
         CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)need));
     k<<<(unsigned)nblk, STREAM_T, in_smem ? need : 0, ctx->stream>>>(X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm,
                                                                    d_alph, K, Qd, ldq, col0, scratch,
-                                                                   in_smem ? 1 : 0, scales);
+                                                                   in_smem ? 1 : 0, scales, seed, u0);
     KERNEL_CHECK(ctx);
     return GPFQ_OK;
 }
 
 // Dense layer by the streaming walk.  Device pointers.  Alphabets are walked one after another
 // (each needs its own residual); Qd: (n_alph, N0, ldq).  d_scales (nullable): (n_alph, nj) per-neuron scales of the shard.
+// Stochastic rounding (ctx->d_seeds): the shard's first neuron has unit id u0.
 int dense_stream_path(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ldx, int64_t N0, int64_t m,
                       const float *W, int64_t ldw, int64_t j0, int64_t nj, const double *d_alph,
                       const int *h_koff, const int *h_flags, int n_alph, double *Qd, int64_t ldq, int64_t col0,
-                      gpfq_stats *st, const double *d_scales) {
+                      gpfq_stats *st, const double *d_scales, int64_t u0) {
     double *nrm = nullptr;
     GPFQ_TRY(gpfq_ws(ctx, WS_NRM, (size_t)2 * N0 * sizeof(double), (void **)&nrm));
     double *g1d = nrm + N0;
@@ -399,7 +415,8 @@ int dense_stream_path(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ld
             const double *al = d_alph + h_koff[a];
             const int K = h_koff[a + 1] - h_koff[a];
             GPFQ_TRY(dispatch_stream_reg(ctx, epv, J, literal, vec, X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm, g1d, al, K,
-                                         h_flags[a], Qd + (int64_t)a * N0 * ldq, ldq, col0, d_scales ? d_scales + a * nj : nullptr));
+                                         h_flags[a], Qd + (int64_t)a * N0 * ldq, ldq, col0, d_scales ? d_scales + a * nj : nullptr,
+                                         ctx->d_seeds ? ctx->d_seeds + a : nullptr, u0));
         }
     } else {
         // long sample axis: residual in shared memory (or an L2-resident scratch), literal arithmetic
@@ -412,9 +429,10 @@ int dense_stream_path(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ld
             const int K = h_koff[a + 1] - h_koff[a];
             double *Qa = Qd + (int64_t)a * N0 * ldq;
             const double *sa = d_scales ? d_scales + a * nj : nullptr;
-            if (J == 4) GPFQ_TRY(launch_stream<4>(ctx, X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm, al, K, Qa, ldq, col0, sa));
-            else if (J == 2) GPFQ_TRY(launch_stream<2>(ctx, X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm, al, K, Qa, ldq, col0, sa));
-            else GPFQ_TRY(launch_stream<1>(ctx, X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm, al, K, Qa, ldq, col0, sa));
+            const uint64_t *sd = ctx->d_seeds ? ctx->d_seeds + a : nullptr;
+            if (J == 4) GPFQ_TRY(launch_stream<4>(ctx, X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm, al, K, Qa, ldq, col0, sa, sd, u0));
+            else if (J == 2) GPFQ_TRY(launch_stream<2>(ctx, X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm, al, K, Qa, ldq, col0, sa, sd, u0));
+            else GPFQ_TRY(launch_stream<1>(ctx, X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm, al, K, Qa, ldq, col0, sa, sd, u0));
         }
     }
     CUDA_TRY(ctx, gpfq_record(ctx, 3, ctx->stream));

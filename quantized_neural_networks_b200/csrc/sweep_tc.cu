@@ -96,9 +96,10 @@ __device__ __forceinline__ void tmem_ld_5x16(uint32_t taddr, uint32_t (&v)[S][16
 // gpfq_decide_rcp_inl of dense_gram.cu with the ternary scan.  Rolled loops; decisions go out as level indices.
 // SCALED: the neuron's levels are fl(s alph[k]) (per-channel alphabets; a = fl(s alph[K - 1]), `alph` the base alphabet); a neuron
 // with s = 0 decides the literal 0 everywhere (its levels are all zero) and never reaches the divisions by a.
-template <bool SCALED>
+// STOCH: stochastic rounding (common.cuh) with the draw of step t0 + t from the neuron's unit key.
+template <bool SCALED, bool STOCH = false>
 static __device__ __noinline__ void replay_block(unsigned char *dset, const unsigned char *wset, int j, const TabA *tab, double a,
-                                                 int8_t *qcol, const double *alph, int K, double s) {
+                                                 int8_t *qcol, const double *alph, int K, double s, uint64_t key = 0, int64_t t0 = 0) {
     // K == 3: the ternary scan with the levels in registers; else the windowed scan of the equispaced levels (common.cuh)
     const bool zero = SCALED && !(a > 0.0);
     const double inv_step = zero ? 0.0 : (SCALED ? gpfq_inv_step_s(alph, K, 1, s) : 0.5 * (double)(K - 1) / a);
@@ -118,6 +119,8 @@ static __device__ __noinline__ void replay_block(unsigned char *dset, const unsi
                 v = fma(e, rinv, q0);
             }
             if (zero) q = 0.0;
+            else if (STOCH && K == 3) q = gpfq_stoc_round_ternary(v, a, gpfq_draw(key, t0 + t));
+            else if (STOCH) q = gpfq_stoc_round_eq<SCALED>(v, alph, K, inv_step, s, gpfq_draw(key, t0 + t));
             else if (K == 3) q = gpfq_bit_round_ternary(v, a);
             else q = SCALED ? gpfq_bit_round_eq_s(v, alph, K, inv_step, s) : gpfq_bit_round_eq(v, alph, K, inv_step);
         }
@@ -134,12 +137,19 @@ static __device__ __noinline__ void replay_block(unsigned char *dset, const unsi
 // alphabet.  Applying h per walker adds one rounding to the grid position (ris / h: RN(RN(rinv / 2) * RN(1 / h)) against RN(rinv / 2h),
 // at most 2 ulp of kr < 2^7), far inside the 2^-30 band that flags a tie; the Q-term scale h 2^(e - 38) stays exact.  The ternary
 // thresholds +- a / 2 and their flag window are per walker.
-template <bool TERN, bool SCALED = false>
+//
+// STOCH (stochastic rounding, DESIGN.md 5.6): step t of neuron jg draws r = draw(seed, u0 + jg, t) -- the unit key once per walker, one
+// splitmix64 per step, on the integer pipe beside the chain.  Ternary: q = a if p > r a, -a if p <= (r - 1) a, else 0 (on [0, a) the
+// literal rule is r < v / a, on (-a, 0) it is r < (v + a) / a); a step is flagged when p lies within 2^-30 a of either threshold.  More
+// levels: the grid position kr = (p + a) / step splits into the interval k = floor(kr) and the fraction f = kr - k; the upper level is
+// taken when r < f, and a step is flagged when f lies within 2^-30 of 0, 1 or r.  The non-finite / huge and :86 flags are those of
+// the nearest walk; a flagged warp replays its block with the literal stoc_round.
+template <bool TERN, bool SCALED = false, bool STOCH = false>
 __global__ void __launch_bounds__(THREADS, 1)
 sweep_tc_kernel(const __grid_constant__ CUtensorMap mapP, const __grid_constant__ CUtensorMap mapW, const TabA *__restrict__ tabs,
                 const int8_t *__restrict__ g2s, int kbr, int64_t tb, int64_t te, int row0, int64_t nj, int8_t *__restrict__ Kq,
                 int64_t krows, int64_t krow0, double a_base, const double *__restrict__ levels, int K,
-                const double *__restrict__ scales = nullptr) {
+                const double *__restrict__ scales = nullptr, const uint64_t *__restrict__ seeds = nullptr, int64_t u0 = 0) {
     using namespace i8g;
     extern __shared__ unsigned char stc_smem_raw[];
     // (offset arithmetic on the array itself: the compiler keeps the shared address space, LDS / STS instead of generic accesses)
@@ -192,6 +202,7 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap mapP, const __grid_constant_
         // more than three levels a_k = -a + k s, s = 2 a / (K - 1): grid position kr = (p + a) / s, nearest level by the 1.5 * 2^52 trick
         const double km1 = (double)(K - 1), step = 2.0 * a / km1, cmid = 0.5 * km1, magic = 6755399441055744.0;
         const uint32_t lane_field = (uint32_t)(warp * 32) << 16;
+        const uint64_t key = STOCH ? gpfq_unit_key(seeds[0], u0 + jg) : 0;
         for (int b = 0; b < nblk; ++b) {
             const int buf = b & 1;
             const int64_t t0 = tb + (int64_t)b * NB;
@@ -239,6 +250,7 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap mapP, const __grid_constant_
             for (int i = 0; i < NB / 4; ++i) pk[i] = 0u;
             int flag = 0;
             uint32_t m_near = 0xffffffffu, m_big = 0u, m_perp = 0xffffffffu;
+            double m_thr = 1e300;   // STOCH ternary: the least |p - threshold| / a of the block
 #pragma unroll
             for (int t = 0; t < NB; ++t) {
                 float4 w4;
@@ -247,7 +259,18 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap mapP, const __grid_constant_
                 const double ri = tab->rinv[t];
                 const double num = fma(wv, tab->g1dd[t], d[t]);
                 double q;
-                if (TERN) {
+                if (TERN && STOCH) {
+                    const double p = num * ri;
+                    const double rr = gpfq_draw(key, t0 + t);
+                    const double ra = rr * a, rm = (rr - 1.0) * a;       // the thresholds of this step, off the chain
+                    const bool up = p > ra, dn = p <= rm;
+                    q = up ? a : (dn ? -a : 0.0);
+                    m_thr = fmin(m_thr, fmin(fabs(p - ra), fabs(p - rm)));
+                    const uint32_t hp = (uint32_t)__double2hiint(p) & 0x7fffffffu;
+                    m_big = max(m_big, hp);
+                    m_perp = min(m_perp, ((uint32_t)__double2hiint(d[t]) & 0x7fffffffu) | (uint32_t)tab->deadm[t]);
+                    pk[t >> 2] |= (up ? 2u : (dn ? 0xfeu : 0u)) << (8 * (t & 3));
+                } else if (TERN) {
                     const double p = num * ri;
                     const bool up = p > hh, dn = p <= -hh;
                     q = up ? a : (dn ? -a : 0.0);
@@ -258,6 +281,19 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap mapP, const __grid_constant_
                     m_big = max(m_big, hp);
                     m_perp = min(m_perp, ((uint32_t)__double2hiint(d[t]) & 0x7fffffffu) | (uint32_t)tab->deadm[t]);
                     pk[t >> 2] |= (up ? 2u : (dn ? 0xfeu : 0u)) << (8 * (t & 3));   // level index k' = q / h = +-2 (h = a / 2)
+                } else if (STOCH) {
+                    // grid position kr = (p + a) / step: interval k = floor(kr) (clamped to the K - 1 intervals), fraction f against r
+                    const double kr = fma(num, SCALED ? tab->ris[t] * inv_hu : tab->ris[t], cmid);
+                    const double rr = gpfq_draw(key, t0 + t);
+                    const double k0 = fmin(fmax(floor(kr), 0.0), km1 - 1.0);
+                    const double f = kr - k0;
+                    const double r = rr < f ? k0 + 1.0 : k0;
+                    const bool live = ri != 0.0;
+                    q = live ? fma(r, step, -a) : 0.0;
+                    flag |= ((int)!(fabs(f) > 0x1p-30) | (int)!(fabs(f - 1.0) > 0x1p-30) | (int)!(fabs(f - rr) > 0x1p-30) |
+                             (int)!(fabs(kr) < 0x1p40) | (int)(fabs(d[t]) < GPFQ_PERP_DOT)) & (int)live;
+                    const int kq = live ? __double2int_rn(fma(r, 2.0, -km1)) : 0;
+                    pk[t >> 2] |= ((uint32_t)kq & 0xffu) << (8 * (t & 3));
                 } else {
                     const double kr = fma(num, SCALED ? tab->ris[t] * inv_hu : tab->ris[t], cmid);   // ris = rinv / s
                     const double r0 = (kr + magic) - magic;                  // rint(kr)
@@ -280,7 +316,8 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap mapP, const __grid_constant_
                 // late steps, 2.4 us per block instead of ~1.)
                 if (kbr == -1 - t) asm volatile("trap;\n");
             }
-            if (TERN) flag = (int)(m_near <= 2u) | (int)(m_big >= big_hi) | (int)(m_perp <= perp_hi);
+            if (TERN && STOCH) flag = (int)!(m_thr > 0x1p-30 * a) | (int)(m_big >= big_hi) | (int)(m_perp <= perp_hi);
+            else if (TERN) flag = (int)(m_near <= 2u) | (int)(m_big >= big_hi) | (int)(m_perp <= perp_hi);
             if (SCALED && zero) {
                 flag = 0;
 #pragma unroll
@@ -288,7 +325,7 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap mapP, const __grid_constant_
             }
             if (__any_sync(0xffffffffu, flag != 0 && valid)) {   // (rows beyond nj hold zeros: they would trip the :86 guard at every step)
                 int8_t *qcol = reinterpret_cast<int8_t *>(smem + OFF_Q) + j;
-                replay_block<SCALED>(dset, wset, j, tab, a, qcol, alph, K, s_u);
+                replay_block<SCALED, STOCH>(dset, wset, j, tab, a, qcol, alph, K, s_u, key, t0);
 #pragma unroll
                 for (int i = 0; i < NB / 4; ++i) {
                     uint32_t w4 = 0u;
@@ -684,16 +721,22 @@ int sweep_tc_bind(gpfq_ctx *ctx, TcTables *tab, const double *P, const float *Wn
 }
 
 int sweep_tc_range(gpfq_ctx *ctx, const TcTables &tab, int64_t tb, int64_t te, int64_t row0, int64_t nj, int8_t *Kq, int64_t krows,
-                   int64_t krow0, double a, const double *levels, int K, const double *scales) {
+                   int64_t krow0, double a, const double *levels, int K, const double *scales, int64_t u0) {
     using namespace stc;
     if (tb % tab.R || te - tb > tab.R || te <= tb || row0 % NT || row0 + ceil_div64(nj, NT) * NT > tab.rowsP || !Kq || K < 2 || K > 128)
         return gpfq_fail(ctx, GPFQ_ERR_ARG, "sweep_tc: a range starts at a multiple of %lld directions", (long long)tab.R);
     const dim3 grid((unsigned)ceil_div64(nj, NT));
-    if (scales) {
+    if (const uint64_t *seeds = ctx->d_seeds) {   // stochastic rounding: one alphabet on this path, seeds[0]
+        auto k = K == 3 ? (scales ? sweep_tc_kernel<true, true, true> : sweep_tc_kernel<true, false, true>)
+                        : (scales ? sweep_tc_kernel<false, true, true> : sweep_tc_kernel<false, false, true>);
+        CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM));
+        k<<<grid, THREADS, SMEM, ctx->stream>>>(tab.mapP, tab.mapW, tab.tabs, tab.g2s, (int)(tab.R / KB), tb, te, (int)row0, nj, Kq, krows, krow0,
+                                                a, levels, K, scales, seeds, u0);
+    } else if (scales) {
         auto k = K == 3 ? sweep_tc_kernel<true, true> : sweep_tc_kernel<false, true>;
         CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM));
         k<<<grid, THREADS, SMEM, ctx->stream>>>(tab.mapP, tab.mapW, tab.tabs, tab.g2s, (int)(tab.R / KB), tb, te, (int)row0, nj, Kq, krows, krow0,
-                                                a, levels, K, scales);
+                                                a, levels, K, scales, nullptr, 0);
     } else if (K == 3) {
         CUDA_TRY(ctx, cudaFuncSetAttribute(sweep_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM));
         sweep_tc_kernel<true><<<grid, THREADS, SMEM, ctx->stream>>>(tab.mapP, tab.mapW, tab.tabs, tab.g2s, (int)(tab.R / KB), tb, te, (int)row0, nj,

@@ -54,8 +54,9 @@ int sweep_tc_bind(gpfq_ctx *ctx, TcTables *tab, const double *P, const float *Wn
 //   a, levels, K: the symmetric equispaced alphabet (device levels, a = levels[K - 1]); K == 3 runs the ternary specialisation
 //   scales (nullable, device, this launch's nj neurons): per-channel alphabets -- neuron j walks with fl(scales[j] levels[k]); the
 //       tables must then be prepared with h = 1
+//   u0: stochastic rounding (ctx->d_seeds set): this launch's neuron j draws as unit u0 + j
 int sweep_tc_range(gpfq_ctx *ctx, const TcTables &tab, int64_t tb, int64_t te, int64_t row0, int64_t nj, int8_t *Kq, int64_t krows,
-                   int64_t krow0, double a, const double *levels, int K, const double *scales = nullptr);
+                   int64_t krow0, double a, const double *levels, int K, const double *scales = nullptr, int64_t u0 = 0);
 // Wn[j][t] = W[t * ldw + wcol0 + j], (nj, N0P) fp32, zeros beyond N0
 int sweep_tc_weights(gpfq_ctx *ctx, const float *W, int64_t ldw, int64_t wcol0, int64_t N0, int64_t N0P, int64_t nj, float *Wn);
 // Q[t * ldq + col0 + j] = the level of index Kq[j][t] for t < N0, j < nj

@@ -2,8 +2,10 @@
 happen inside the library call) or CUDA torch tensors (device pointers; torch is only the buffer)."""
 from __future__ import annotations
 
+import contextlib
 import ctypes
-from ctypes import POINTER, byref, c_double, c_int32, c_void_p
+import numbers
+from ctypes import POINTER, byref, c_double, c_int32, c_uint64, c_void_p
 
 import numpy as np
 
@@ -53,6 +55,27 @@ def _scale_args(scales, n_alph, unit_shape, name="scales"):
     if not np.all(np.isfinite(s)) or np.any(s < 0):
         raise ValueError(f"{name}: every scale must be finite and >= 0")
     return np.ascontiguousarray(s)
+
+
+def _seed_args(seeds, n_alph):
+    """Stochastic-rounding seeds -> None (nearest rounding) or a list of n_alph ints in [0, 2^64).  Accepts None, one int (used by
+    every alphabet) or a sequence of n_alph ints."""
+    if seeds is None:
+        return None
+    if isinstance(seeds, numbers.Integral) and not isinstance(seeds, bool):
+        seeds = [seeds] * n_alph
+    elif isinstance(seeds, (list, tuple, np.ndarray)):
+        seeds = list(np.asarray(seeds, dtype=object).reshape(-1)) if isinstance(seeds, np.ndarray) else list(seeds)
+        if len(seeds) != n_alph:
+            raise ValueError(f"seeds: {len(seeds)} seeds for {n_alph} alphabets")
+    else:
+        raise ValueError(f"seeds: expected None, an int or a sequence of {n_alph} ints, got {type(seeds).__name__}")
+    out = []
+    for v in seeds:
+        if not isinstance(v, numbers.Integral) or isinstance(v, bool) or not 0 <= int(v) < 1 << 64:
+            raise ValueError(f"seeds: {v!r} is not an int in [0, 2^64)")
+        out.append(int(v))
+    return out
 
 
 def _dptr(a):
@@ -108,6 +131,20 @@ class GpfqEngine:
         `sweep_i8`)."""
         self._check(self._lib.gpfq_set_option(self._ctx, key.encode(), int(value)))
 
+    @contextlib.contextmanager
+    def _rounding(self, seeds, n_alph):
+        """Stochastic rounding with these seeds for the calls inside (seeds None: nearest rounding); nearest again afterwards."""
+        sd = _seed_args(seeds, n_alph)
+        if sd is None:
+            yield
+            return
+        arr = (c_uint64 * len(sd))(*sd)
+        self._check(self._lib.gpfq_set_rounding(self._ctx, _lib.ROUND_STOCHASTIC, arr, len(sd)))
+        try:
+            yield
+        finally:
+            self._lib.gpfq_set_rounding(self._ctx, _lib.ROUND_NEAREST, None, 0)
+
     def _bind_stream(self, dev):
         """Device-tensor calls launch on torch's CURRENT stream: the tensors were produced there, so this is what
         orders our kernels after their producers (and lets torch.cuda.Event brackets time them).  Host-array
@@ -147,12 +184,13 @@ class GpfqEngine:
         return x.ctypes.data, (x.strides[0] // x.itemsize if x.shape[0] > 1 else x.shape[1])
 
     # -- Dense ----------------------------------------------------------------------------------
-    def dense_layer(self, X, Xq, W, alphabets, j0=0, j1=None, method="auto", out=None, sync=True, scales=None):
+    def dense_layer(self, X, Xq, W, alphabets, j0=0, j1=None, method="auto", out=None, sync=True, scales=None, seeds=None):
         """Quantize neurons j0..j1-1 of a Dense layer.  X, Xq: (N0, m) fp32 feature-major (Xq may be
         None or X itself for the first layer); W: (N0, N1) fp32.  Returns Q fp64 (N0, N1) -- or
         (n_alphabets, N0, N1) when a list of alphabets is given -- with only the shard's columns written.
         `scales` (per-channel alphabets): (N1,) or (n_alphabets, N1), finite and >= 0; neuron j then walks with the levels
-        fl64(scales[j] * alphabet[k])."""
+        fl64(scales[j] * alphabet[k]).  `seeds`: None rounds to the nearest level (the reference); an int or one int per alphabet in
+        [0, 2^64) rounds stochastically (SPFQ, include/gpfq.h), neuron j drawing as unit j whatever the shard."""
         flat, K, n_alph, als = _alph_args(alphabets)
         single = isinstance(alphabets, np.ndarray) and alphabets.ndim == 1
         X = self._f32(X, "X")
@@ -197,7 +235,8 @@ class GpfqEngine:
         args = (self._ctx, c_void_p(px), c_void_p(pq), ldx, N0, m, c_void_p(pw), ldw, N1, int(j0), j1,
                 flat.ctypes.data_as(POINTER(c_double)), K.ctypes.data_as(POINTER(c_int32)), n_alph, c_void_p(pout), N1, flags,
                 byref(st))
-        rc = self._lib.gpfq_dense_layer(*args) if sc is None else self._lib.gpfq_dense_layer_scaled(*args, _dptr(sc))
+        with self._rounding(seeds, n_alph):
+            rc = self._lib.gpfq_dense_layer(*args) if sc is None else self._lib.gpfq_dense_layer_scaled(*args, _dptr(sc))
         self._check(rc)
         self.last_stats = st.as_dict()
         return out[0] if single else out
@@ -242,10 +281,11 @@ class GpfqEngine:
         self._check(rc)
         return G1, G2
 
-    def dense_layer_from_gram(self, G1, G2, W, alphabets, j0=0, j1=None, out=None, sync=True, scales=None):
+    def dense_layer_from_gram(self, G1, G2, W, alphabets, j0=0, j1=None, out=None, sync=True, scales=None, seeds=None):
         """Sweep stage of a Dense layer from (N0, N0) fp64 Gram matrices on the device (CUDA tensors; G1 None or G2
         itself for the first layer): what every rank of a sample-split job runs after the all-reduce of the partial
-        Grams.  W: (N0, N1) fp32 NumPy array or CUDA tensor; the result follows W's kind.  `scales` as in `dense_layer`."""
+        Grams.  W: (N0, N1) fp32 NumPy array or CUDA tensor; the result follows W's kind.  `scales` and `seeds` as in
+        `dense_layer`."""
         flat, K, n_alph, als = _alph_args(alphabets)
         single = isinstance(alphabets, np.ndarray) and alphabets.ndim == 1
         if not _is_torch(G2) or G2.dtype != torch.float64 or not G2.is_cuda or not G2.is_contiguous():
@@ -284,18 +324,20 @@ class GpfqEngine:
         args = (self._ctx, c_void_p(None if same else G1.data_ptr()), c_void_p(G2.data_ptr()), N0, c_void_p(pw), ldw, N1,
                 int(j0), j1, flat.ctypes.data_as(POINTER(c_double)), K.ctypes.data_as(POINTER(c_int32)), n_alph,
                 c_void_p(pout), N1, flags, byref(st))
-        rc = (self._lib.gpfq_dense_layer_from_gram(*args) if sc is None
-              else self._lib.gpfq_dense_layer_from_gram_scaled(*args, _dptr(sc)))
+        with self._rounding(seeds, n_alph):
+            rc = (self._lib.gpfq_dense_layer_from_gram(*args) if sc is None
+                  else self._lib.gpfq_dense_layer_from_gram_scaled(*args, _dptr(sc)))
         self._check(rc)
         self.last_stats = st.as_dict()
         return out[0] if single else out
 
     # -- Conv -----------------------------------------------------------------------------------
-    def conv_channels(self, Xp, Xqp, W, alphabets, c0=0, n_channels=None, out=None, sync=True, scales=None):
+    def conv_channels(self, Xp, Xqp, W, alphabets, c0=0, n_channels=None, out=None, sync=True, scales=None, seeds=None):
         """Quantize channels c0..c0+n_channels-1 of a (kh, kw, C, F) kernel from per-channel patch
         matrices.  Xp/Xqp: sequences (len n_channels) of (kh*kw, n_patches) fp32 arrays/tensors, or one
         (n_channels, kh*kw, n_patches) array; Xqp None => first conv layer (X == Xq).  `scales` (per-channel alphabets):
-        (C, F) or (n_alphabets, C, F), finite and >= 0; the slice W[:, :, c, f] walks with fl64(scales[c, f] * alphabet[k])."""
+        (C, F) or (n_alphabets, C, F), finite and >= 0; the slice W[:, :, c, f] walks with fl64(scales[c, f] * alphabet[k]).
+        `seeds` as in `dense_layer`; the slice W[:, :, c, f] draws as unit c * F + f, tap r * kw + col as step."""
         flat, K, n_alph, als = _alph_args(alphabets)
         single = isinstance(alphabets, np.ndarray) and alphabets.ndim == 1
         W = self._f32(W, "W")
@@ -339,7 +381,8 @@ class GpfqEngine:
         st = _lib.GpfqStats()
         args = (self._ctx, PX, PQ, n, kk, c_void_p(ptr(W)), C, F, int(c0), n_channels, flat.ctypes.data_as(POINTER(c_double)),
                 K.ctypes.data_as(POINTER(c_int32)), n_alph, c_void_p(pout), flags, byref(st))
-        rc = self._lib.gpfq_conv_channels(*args) if sc is None else self._lib.gpfq_conv_channels_scaled(*args, _dptr(sc))
+        with self._rounding(seeds, n_alph):
+            rc = self._lib.gpfq_conv_channels(*args) if sc is None else self._lib.gpfq_conv_channels_scaled(*args, _dptr(sc))
         self._check(rc)
         self.last_stats = st.as_dict()
         return out[0] if single else out
@@ -354,11 +397,12 @@ class GpfqEngine:
         return groups
 
     def conv_layer_nhwc(self, act, actq, W, alphabets, strides=(1, 1), padding="SAME", rate=(1, 1), c0=0,
-                        n_channels=None, out=None, sync=True, groups=1, scales=None):
+                        n_channels=None, out=None, sync=True, groups=1, scales=None, seeds=None):
         """Quantize a Conv2D kernel straight from the NHWC activations (on-device patch extraction).  With `groups` > 1, W is the
         (kh, kw, C / groups, F) kernel of a grouped Conv2D: input channel c is walked against the F / groups filters of its group
         c // (C / groups); c0 / n_channels index input channels.  The result has W's shape.  `scales` (per-channel alphabets):
-        (C / groups, F) or (n_alphabets, C / groups, F), indexed like W's last two axes."""
+        (C / groups, F) or (n_alphabets, C / groups, F), indexed like W's last two axes.  `seeds` as in `dense_layer`; the slice
+        W[:, :, ci, f] draws as unit ci * F + f."""
         flat, K, n_alph, als = _alph_args(alphabets)
         single = isinstance(alphabets, np.ndarray) and alphabets.ndim == 1
         W = self._f32(W, "W")
@@ -403,10 +447,11 @@ class GpfqEngine:
                 int(rate[0]), int(rate[1]), 1 if str(padding).upper() == "SAME" else 0, c_void_p(ptr(W)), F, int(c0), n_channels,
                 flat.ctypes.data_as(POINTER(c_double)), K.ctypes.data_as(POINTER(c_int32)), n_alph, c_void_p(pout), flags,
                 byref(st))
-        if sc is not None:
-            rc = self._lib.gpfq_conv_layer_nhwc_scaled(*args, groups, _dptr(sc))
-        else:
-            rc = (self._lib.gpfq_conv_layer_nhwc_grouped(*args, groups) if groups > 1 else self._lib.gpfq_conv_layer_nhwc(*args))
+        with self._rounding(seeds, n_alph):
+            if sc is not None:
+                rc = self._lib.gpfq_conv_layer_nhwc_scaled(*args, groups, _dptr(sc))
+            else:
+                rc = (self._lib.gpfq_conv_layer_nhwc_grouped(*args, groups) if groups > 1 else self._lib.gpfq_conv_layer_nhwc(*args))
         self._check(rc)
         self.last_stats = st.as_dict()
         return out[0] if single else out
@@ -447,11 +492,13 @@ class GpfqEngine:
         self.last_stats = self.query_stats(0)
         return gram
 
-    def conv_layer_from_gram(self, gram, W, alphabets, c0=0, n_channels=None, out=None, sync=True, groups=1, scales=None):
+    def conv_layer_from_gram(self, gram, W, alphabets, c0=0, n_channels=None, out=None, sync=True, groups=1, scales=None,
+                             seeds=None):
         """Walks of every filter of channels c0..c0+n_channels-1 from per-channel Gram matrices on the device
         (`conv_gram_nhwc`, summed over the ranks of an image-split job).  W: (kh, kw, C, F) NumPy array or CUDA tensor; with
         `groups` > 1 the (kh, kw, C / groups, F) kernel of a grouped Conv2D, each input channel walked against the F / groups
-        filters of its group (c0 / n_channels index input channels, as in the Gram stage).  `scales` as in `conv_layer_nhwc`."""
+        filters of its group (c0 / n_channels index input channels, as in the Gram stage).  `scales` and `seeds` as in
+        `conv_layer_nhwc`."""
         flat, K, n_alph, als = _alph_args(alphabets)
         single = isinstance(alphabets, np.ndarray) and alphabets.ndim == 1
         W = self._f32(W, "W")
@@ -482,11 +529,12 @@ class GpfqEngine:
         st = _lib.GpfqStats()
         args = (self._ctx, c_void_p(gram.data_ptr()), kk, c_void_p(pw), C, F, int(c0), n_channels,
                 flat.ctypes.data_as(POINTER(c_double)), K.ctypes.data_as(POINTER(c_int32)), n_alph, c_void_p(pout), flags, byref(st))
-        if sc is not None:
-            rc = self._lib.gpfq_conv_layer_from_gram_scaled(*args, groups, _dptr(sc))
-        else:
-            rc = (self._lib.gpfq_conv_layer_from_gram_grouped(*args, groups) if groups > 1
-                  else self._lib.gpfq_conv_layer_from_gram(*args))
+        with self._rounding(seeds, n_alph):
+            if sc is not None:
+                rc = self._lib.gpfq_conv_layer_from_gram_scaled(*args, groups, _dptr(sc))
+            else:
+                rc = (self._lib.gpfq_conv_layer_from_gram_grouped(*args, groups) if groups > 1
+                      else self._lib.gpfq_conv_layer_from_gram(*args))
         self._check(rc)
         self.last_stats = st.as_dict()
         return out[0] if single else out
@@ -506,10 +554,11 @@ class GpfqEngine:
                                                 1 if transposed_b else 0, c_void_p(C.ctypes.data)))
         return C
 
-    def msq(self, W, alphabet, scales=None):
+    def msq(self, W, alphabet, scales=None, seeds=None):
         """Plain nearest-level rounding of every weight (the MSQ baseline of the reference's drivers).  `scales` (per-channel
         alphabets): one scale per unit of W's last axis (a Dense neuron or a conv filter), shape (W.shape[-1],) or W.shape[-2:]
-        for a conv kernel's (C, F) table; weight W[..., u] rounds to the levels fl64(scales[u] * alphabet[k])."""
+        for a conv kernel's (C, F) table; weight W[..., u] rounds to the levels fl64(scales[u] * alphabet[k]).  `seeds` (one int):
+        stochastic rounding, the flat element index as unit id."""
         W = np.ascontiguousarray(W, dtype=np.float32)
         A = np.ascontiguousarray(alphabet, dtype=np.float64)
         out = np.zeros(W.shape, dtype=np.float64)
@@ -521,23 +570,27 @@ class GpfqEngine:
             if not np.all(np.isfinite(s)) or np.any(s < 0):
                 raise ValueError("scales: every scale must be finite and >= 0")
             s = np.ascontiguousarray(s).reshape(-1)
-            rc = self._lib.gpfq_msq_scaled(self._ctx, c_void_p(W.ctypes.data), W.size, A.ctypes.data_as(POINTER(c_double)),
-                                           len(A), _dptr(s), s.size, c_void_p(out.ctypes.data), 0)
+            with self._rounding(seeds, 1):
+                rc = self._lib.gpfq_msq_scaled(self._ctx, c_void_p(W.ctypes.data), W.size, A.ctypes.data_as(POINTER(c_double)),
+                                               len(A), _dptr(s), s.size, c_void_p(out.ctypes.data), 0)
             self._check(rc)
             return out
-        rc = self._lib.gpfq_msq(self._ctx, c_void_p(W.ctypes.data), W.size, A.ctypes.data_as(POINTER(c_double)), len(A),
-                                c_void_p(out.ctypes.data), 0)
+        with self._rounding(seeds, 1):
+            rc = self._lib.gpfq_msq(self._ctx, c_void_p(W.ctypes.data), W.size, A.ctypes.data_as(POINTER(c_double)), len(A),
+                                    c_void_p(out.ctypes.data), 0)
         self._check(rc)
         return out
 
 
-    def _bit_round(self, t, alphabet):
+    def _bit_round(self, t, alphabet, seeds=None):
+        """The scalar quantizer on fp64 values; `seeds` (one int): stochastic rounding, the flat index as unit id."""
         t = np.ascontiguousarray(t, dtype=np.float64)
         A = np.ascontiguousarray(alphabet, dtype=np.float64)
         out = np.zeros(t.shape, dtype=np.float64)
         self._bind_stream(False)
-        rc = self._lib.gpfq_bit_round(self._ctx, c_void_p(t.ctypes.data), t.size, A.ctypes.data_as(POINTER(c_double)),
-                                      len(A), c_void_p(out.ctypes.data), 0)
+        with self._rounding(seeds, 1):
+            rc = self._lib.gpfq_bit_round(self._ctx, c_void_p(t.ctypes.data), t.size, A.ctypes.data_as(POINTER(c_double)),
+                                          len(A), c_void_p(out.ctypes.data), 0)
         self._check(rc)
         return out
 

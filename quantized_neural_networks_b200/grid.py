@@ -23,7 +23,7 @@ from time import time
 import numpy as np
 from numpy import abs, linspace, median
 
-from .quantized_network import QuantizedCNN
+from .quantized_network import QuantizedCNN, layer_seed
 
 LAYER_KINDS = ("Dense", "Conv2D", "DepthwiseConv2D")
 
@@ -63,13 +63,17 @@ class QuantizedCNNGrid:
     """All (bits, alphabet_scalar) grid points of one network, quantized layer by layer in lock-step."""
 
     def __init__(self, network, batch_size, get_data, bits_list, alphabet_scalars, logger=None, is_quantize_conv2d=True,
-                 device: int = 0, data_set: str = "synthetic", q_train_size=None, *, alphabet_scope: str = "layer"):
+                 device: int = 0, data_set: str = "synthetic", q_train_size=None, *, alphabet_scope: str = "layer",
+                 rounding: str = "nearest", seed: int = 0):
         """`alphabet_scope` ("layer" | "channel") as in `QuantizedCNN`: with "channel" every grid point quantizes each output
-        channel against its own radius, and `msq_networks()` rounds with the same per-channel levels."""
+        channel against its own radius, and `msq_networks()` rounds with the same per-channel levels.  `rounding` as in
+        `QuantizedCNN`; with "stochastic", grid point g (in the order of `self.grid`) is the run of `QuantizedCNN(..., seed=seed + g)`,
+        and `msq_networks()` rounds stochastically with the same layer seeds."""
         self.grid = list(product(bits_list, alphabet_scalars))          # the order of itertools.product in the driver
         self.points = [QuantizedCNN(network, batch_size, get_data, logger=logger, bits=b, alphabet_scalar=c,
-                                    is_quantize_conv2d=is_quantize_conv2d, device=device, alphabet_scope=alphabet_scope)
-                       for b, c in self.grid]
+                                    is_quantize_conv2d=is_quantize_conv2d, device=device, alphabet_scope=alphabet_scope,
+                                    rounding=rounding, seed=(int(seed) + g) % (1 << 64) if rounding == "stochastic" else seed)
+                       for g, (b, c) in enumerate(self.grid)]
         self.trained_net, self.logger, self.device = network, logger, device
         self.is_quantize_conv2d = is_quantize_conv2d
         self.data_set = data_set
@@ -120,6 +124,8 @@ class QuantizedCNNGrid:
                 Xqd = None if qX is None else torch.from_numpy(np.ascontiguousarray(qX)).to(dev)
                 A = [levels[g][0] for g in members]
                 scaled = {} if levels[0][1] is None else {"scales": np.stack([levels[g][1] for g in members])}
+                if self.points[0].rounding == "stochastic":
+                    scaled["seeds"] = [layer_seed(self.points[g].seed, layer_idx) for g in members]
                 if dense:
                     Q = eng.dense_layer(Xd, Xqd, Wd, A, **scaled)
                 else:
@@ -153,7 +159,7 @@ class QuantizedCNNGrid:
                 if layer.__class__.__name__ in ("Dense", "Conv2D"):
                     ws = layer.get_weights()
                     A, scales = p._levels(ws[0], layer.__class__.__name__)
-                    Q = eng.msq(ws[0], A, **({} if scales is None else {"scales": scales}))
+                    Q = eng.msq(ws[0], A, **({} if scales is None else {"scales": scales}), **p._seeds(layer_idx))
                     net.layers[layer_idx].set_weights([Q] + list(ws[1:]))
             nets.append(net)
         return nets

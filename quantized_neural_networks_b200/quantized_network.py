@@ -16,6 +16,7 @@ There is no CPU fallback for the hot path: without libgpfq.so and an sm_100 GPU 
 """
 from __future__ import annotations
 
+import numbers
 from time import time
 from typing import List
 
@@ -88,6 +89,23 @@ class LayerData:
         self.same = qX is wX or np.array_equal(wX, qX)
 
 
+_MASK64 = (1 << 64) - 1
+
+
+def splitmix64(x: int) -> int:
+    """The SplitMix64 finaliser of x + 0x9E3779B97F4A7C15 (mod 2^64): the hash of the stochastic-rounding draws (include/gpfq.h)."""
+    z = (x + 0x9E3779B97F4A7C15) & _MASK64
+    z = ((z ^ (z >> 30)) * 0xBF58476D1CE4E5B9) & _MASK64
+    z = ((z ^ (z >> 27)) * 0x94D049BB133111EB) & _MASK64
+    return z ^ (z >> 31)
+
+
+def layer_seed(seed: int, layer_idx: int) -> int:
+    """The stochastic-rounding seed of layer `layer_idx` of a network quantized with `seed`: every layer draws its own stream,
+    and a layer's decisions do not depend on which other layers are quantized."""
+    return splitmix64(splitmix64(int(seed) & _MASK64) ^ int(layer_idx))
+
+
 class QuantizedNeuralNetwork:
     def __init__(
         self,
@@ -105,6 +123,8 @@ class QuantizedNeuralNetwork:
         shard=None,
         gram_split: str = "auto",
         alphabet_scope: str = "layer",
+        rounding: str = "nearest",
+        seed: int = 0,
     ):
         """Wrapper of a Keras-style model that quantizes the weights of its Dense layers with GPFQ.
 
@@ -118,6 +138,9 @@ class QuantizedNeuralNetwork:
         by bytes moved (`replicate.prefer_sample_split`).  `alphabet_scope` ("layer" | "channel"): "layer" (the reference)
         quantizes every layer against `alphabet_scalar * median(|W|) * linspace(-1, 1, K)`; "channel" gives every output
         channel its own radius `alphabet_scalar * median(|w_u|)` (`_unit_scales`), as per-channel weight scales do.
+        `rounding` ("nearest" | "stochastic"): "nearest" (the reference) rounds every greedy step to the nearest level;
+        "stochastic" is SPFQ, unbiased stochastic rounding between the two bracketing levels, reproducible from `seed` (layer
+        `layer_idx` draws with `layer_seed(seed, layer_idx)`, whatever the device count, shards or conv path).
         """
         self.get_data = get_data
         self.trained_net = network
@@ -133,9 +156,9 @@ class QuantizedNeuralNetwork:
         self.alphabet = linspace(-1, 1, num=int(round(2 ** (bits))))
         self.logger = logger
         self.ignore_layers = ignore_layers
-        self._init_device(device, method, shard, gram_split, alphabet_scope)
+        self._init_device(device, method, shard, gram_split, alphabet_scope, rounding, seed)
 
-    def _init_device(self, device, method, shard, gram_split="auto", alphabet_scope="layer"):
+    def _init_device(self, device, method, shard, gram_split="auto", alphabet_scope="layer", rounding="nearest", seed=0):
         if int(round(2 ** self.bits)) > 64:   # GPFQ_MAX_K of include/gpfq.h: the kernels keep an alphabet in shared memory
             raise ValueError(f"bits={self.bits}: the CUDA path supports alphabets of up to 64 levels (bits <= 6); the reference "
                              "accepts any `bits`, see INTEGRATION.md")
@@ -144,6 +167,11 @@ class QuantizedNeuralNetwork:
         if alphabet_scope not in ("layer", "channel"):
             raise ValueError(f"alphabet_scope must be 'layer' or 'channel', not {alphabet_scope!r}")
         self.alphabet_scope = alphabet_scope
+        if rounding not in ("nearest", "stochastic"):
+            raise ValueError(f"rounding must be 'nearest' or 'stochastic', not {rounding!r}")
+        if isinstance(seed, bool) or not isinstance(seed, numbers.Integral) or not 0 <= int(seed) < 1 << 64:
+            raise ValueError(f"seed must be an int in [0, 2^64), not {seed!r}")
+        self.rounding, self.seed = rounding, int(seed)
         self.device, self.method, self.gram_split = device, method, gram_split
         self.shard = tuple(shard) if shard else (0, 1)
         self.layer_stats = {}
@@ -237,6 +265,10 @@ class QuantizedNeuralNetwork:
             return np.asarray(self.alphabet, dtype=np.float64), self._unit_scales(W, kind)
         return np.asarray(self._layer_alphabet(W), dtype=np.float64), None
 
+    def _seeds(self, layer_idx):
+        """Engine keyword of layer `layer_idx`: nothing for nearest rounding (the call keeps its signature), else its seed."""
+        return {"seeds": layer_seed(self.seed, layer_idx)} if self.rounding == "stochastic" else {}
+
     def _nccl_job(self):
         """True when this object is one rank of a torch.distributed job on GPUs (NCCL): layer inputs are then replicated
         through `replicate_leading_axis` (1 / world of the bytes over each rank's host link + one NVLink all-gather)."""
@@ -301,6 +333,7 @@ class QuantizedNeuralNetwork:
 
         layer_alphabet, scales = self._levels(W)
         scaled = {"scales": scales} if scales is not None else {}   # the per-layer call keeps its signature
+        scaled.update(self._seeds(layer_idx))
 
         self._log("\tQuantizing neurons (on the GPU)...")
         tic = time()
@@ -361,11 +394,14 @@ class QuantizedCNN(QuantizedNeuralNetwork):
         conv_path: str = "nhwc",
         gram_split: str = "auto",
         alphabet_scope: str = "layer",
+        rounding: str = "nearest",
+        seed: int = 0,
     ):
         """Dense + Conv2D / DepthwiseConv2D quantization (quantized_network.py:594-650).  Like the reference this
         constructor does not take `ignore_layers`.  `conv_path="nhwc"` hands the layer's activation tensors to
         CUDA (patches are extracted on the device); `"patches"` builds the per-channel patch matrices on the host
-        exactly as `_build_patch_array` does and hands those over.  `alphabet_scope` as in `QuantizedNeuralNetwork`."""
+        exactly as `_build_patch_array` does and hands those over.  `alphabet_scope`, `rounding` and `seed` as in
+        `QuantizedNeuralNetwork`."""
         self.get_data = get_data
         self.trained_net = network
         self.quantized_net = _clone(network)
@@ -378,7 +414,7 @@ class QuantizedCNN(QuantizedNeuralNetwork):
         self.logger = logger
         self.ignore_layers = []
         self.conv_path = conv_path
-        self._init_device(device, method, shard, gram_split, alphabet_scope)
+        self._init_device(device, method, shard, gram_split, alphabet_scope, rounding, seed)
 
     def _build_patch_array(self, channel_idx: int, kernel_size: tuple, strides: tuple, padding: str, rate: tuple,
                            data, mini_batch_size: int):
@@ -398,8 +434,11 @@ class QuantizedCNN(QuantizedNeuralNetwork):
 
     def _quantize_channel_parallel_jit(self, channel_idx: int, channel_filters: array, hidden_activations,
                                        strides: tuple, padding: str, rate: tuple, alphabet: array,
-                                       patch_mini_batch_size=5000, scales=None) -> array:
-        """All filters of one input channel (quantized_network.py:652-727): host patches + one C-ABI call."""
+                                       patch_mini_batch_size=5000, scales=None, stochastic=None) -> array:
+        """All filters of one input channel (quantized_network.py:652-727): host patches + one C-ABI call.  `stochastic`
+        (stochastic rounding): (kernel, ci, f0, seed, scales) -- the whole (kh, kw, Cw, F) kernel, the channel's slice ci and its
+        first filter f0, so that the slice draws with its global unit ids ci * F + f; the call walks all F filters of slice ci and
+        the Fg of `channel_filters` are kept."""
         filter_shape = channel_filters.shape[0:2]
         patches = self._build_patch_array(channel_idx, filter_shape, strides, padding, rate, hidden_activations,
                                           patch_mini_batch_size)
@@ -407,6 +446,12 @@ class QuantizedCNN(QuantizedNeuralNetwork):
         Wc = np.ascontiguousarray(channel_filters.reshape(*channel_filters.shape[:2], 1, channel_filters.shape[-1]),
                                   dtype=np.float32)
         try:
+            if stochastic is not None:
+                Wk, ci, f0, seed, sk = stochastic
+                Qk = self.engine.conv_channels([Xp], None if Xqp is Xp else [Xqp], np.ascontiguousarray(Wk, dtype=np.float32),
+                                               np.asarray(alphabet, dtype=np.float64), c0=ci, n_channels=1, seeds=seed,
+                                               **({} if sk is None else {"scales": sk}))
+                return Qk[:, :, ci, f0:f0 + channel_filters.shape[-1]]
             scaled = {} if scales is None else {"scales": np.reshape(scales, (1, -1))}
             Qc = self.engine.conv_channels([Xp], None if Xqp is Xp else [Xqp], Wc, np.asarray(alphabet, dtype=np.float64), **scaled)
         except Exception as exc:
@@ -428,6 +473,7 @@ class QuantizedCNN(QuantizedNeuralNetwork):
         W = layer.get_weights()[0]
         alphabet, scales = self._levels(W, layer.__class__.__name__)
         scaled = {"scales": scales} if scales is not None else {}
+        scaled.update(self._seeds(layer_idx))
         # a grouped Conv2D has a (kh, kw, C / groups, F) kernel: input channel c meets only the Fg filters of its group c // Cg,
         # so ranks take whole groups and gather their filters (groups == 1: channels, all filters)
         groups = int(getattr(layer, "groups", 1)) if layer.__class__.__name__ == "Conv2D" else 1
@@ -469,10 +515,11 @@ class QuantizedCNN(QuantizedNeuralNetwork):
             Q = zeros(W.shape)
             for channel_idx in range(lo, hi):
                 ci, f0 = channel_idx % Cg, (channel_idx // Cg) * Fg   # the channel's kernel slice and its group's filters
+                stoch = (W, ci, f0, scaled["seeds"], scales) if "seeds" in scaled else None
                 Q[:, :, ci, f0:f0 + Fg] = self._quantize_channel_parallel_jit(
                     channel_idx, W[:, :, ci, f0:f0 + Fg], data, strides=layer.strides, padding=layer.padding.upper(),
                     rate=rate, alphabet=alphabet, patch_mini_batch_size=self.patch_mini_batch_size,
-                    scales=None if scales is None else scales[ci, f0:f0 + Fg])
+                    scales=None if scales is None else scales[ci, f0:f0 + Fg], stochastic=stoch)
         if (lo, hi) != (0, num_channels) and groups > 1:
             # this rank wrote the filters of groups lo / Cg .. hi / Cg: gather along the group axis of (kh, kw, Cg, groups, Fg)
             Q = self._gather_columns(Q.reshape(*Q.shape[:3], groups, Fg), lo // Cg, hi // Cg, axis=3).reshape(W.shape)
@@ -497,5 +544,6 @@ class QuantizedCNN(QuantizedNeuralNetwork):
                 self._log(f"done. {time() - tic:.2f} seconds.")
 
 
-__all__: List[str] = ["QuantizedNeuralNetwork", "QuantizedCNN", "LayerData", "shard_range", "_bit_round_parallel",
+__all__: List[str] = ["QuantizedNeuralNetwork", "QuantizedCNN", "LayerData", "shard_range", "layer_seed", "splitmix64",
+                      "_bit_round_parallel",
                       "_quantize_neuron_parallel", "_quantize_filter2D_parallel_jit"]
