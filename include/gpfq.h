@@ -279,6 +279,24 @@ int gpfq_msq_scaled(gpfq_ctx *ctx, const float *W, int64_t n, const double *alph
 #define GPFQ_ROUND_STOCHASTIC 1
 int gpfq_set_rounding(gpfq_ctx *ctx, int32_t mode, const uint64_t *seeds, int32_t n_seeds);
 
+/* ---- sparse GPFQ: an L1 penalty on every greedy step -----------------------------------------------------------------------
+ * Context state, like gpfq_set_rounding: every later Dense, conv, _grouped and _scaled call walks with the penalty lambdas[a] for
+ * alphabet a (n_lambdas = 0 turns it off, the default); Gram-only calls, gpfq_msq* and gpfq_bit_round ignore it.  One greedy step
+ * of unit u at step t (unit and step as for stochastic rounding), in fp64 with correct rounding:
+ *   q = 0                                                    if nrm < 1e-16 (dead direction)
+ *   den = fl(nrm * nrm);  v = w_t if |d| < 1e-10 else fl(num / den)           (the reference's value)
+ *   tau = fl(lambda / den)
+ *   v' = 0 if |v| <= tau, else fl(v - copysign(tau, v))                       (NaN: the comparison is false, v' = NaN)
+ *   q = Q(v')   with the call's quantizer: nearest (first level on ties) or stoc_round, levels A[k] or fl(s_u * A[k])
+ * In the main branch v' = s_lambda(num) / den with s_lambda(x) = sign(x) max(|x| - lambda, 0): the exact minimiser over real p of
+ * 1/2 |u_{t-1} + w_t X_t - p Xq_t|^2 + lambda |p|, then quantized; the shrink in value space also covers the :86 branch.
+ * lambda = 0 reproduces the call without the penalty bit for bit (tau = +0; only the sign of a zero v changes, which neither
+ * quantizer sees).  Zeros come from an alphabet with a 0 level (odd K of the symmetric alphabets).  Each lambda must be finite
+ * and >= 0 (else GPFQ_ERR_ARG from this call, the state unchanged); a quantizing call with more alphabets than lambdas returns
+ * GPFQ_ERR_ARG before any work.  The lambdas are staged like the seeds: GPFQ_NO_SYNC calls stay asynchronous.  A call with the
+ * penalty runs the kernels of its counterpart without it, with equal stats.method, gram_kernel, reserved and launch count. */
+int gpfq_set_l1_penalty(gpfq_ctx *ctx, const double *lambdas, int32_t n_lambdas);
+
 /* ---- MSQ baseline ---------------------------------------------------------------------------
  * Plain nearest-level rounding of every weight (_bit_round_parallel :40-57 applied elementwise,
  * as in quantize_pretrained_mlp.py:97-117).  n elements, contiguous. */

@@ -50,6 +50,7 @@ EXPORTS = {
     "gpfq_set_stream": (c_int, [c_void_p, c_void_p]),
     "gpfq_set_option": (c_int, [c_void_p, c_char_p, c_int64]),
     "gpfq_set_rounding": (c_int, [c_void_p, c_int32, POINTER(c_uint64), c_int32]),
+    "gpfq_set_l1_penalty": (c_int, [c_void_p, POINTER(c_double), c_int32]),
     "gpfq_trim": (c_int, [c_void_p]),
     "gpfq_conv_partial_bytes": (c_int64, [c_void_p]),
     "gpfq_query_stats": (c_int, [c_void_p, c_int32, POINTER(GpfqStats)]),

@@ -230,6 +230,17 @@ extern "C" int gpfq_set_rounding(gpfq_ctx *ctx, int32_t mode, const uint64_t *se
     return GPFQ_OK;
 }
 
+extern "C" int gpfq_set_l1_penalty(gpfq_ctx *ctx, const double *lambdas, int32_t n_lambdas) {
+    if (!ctx) return GPFQ_ERR_ARG;
+    ctx->err.clear();
+    if (n_lambdas < 0 || (n_lambdas > 0 && !lambdas)) return gpfq_fail(ctx, GPFQ_ERR_ARG, "bad n_lambdas=%d", n_lambdas);
+    for (int i = 0; i < n_lambdas; ++i)
+        if (!std::isfinite(lambdas[i]) || !(lambdas[i] >= 0.0))
+            return gpfq_fail(ctx, GPFQ_ERR_ARG, "L1 penalty %d must be finite and >= 0", i);
+    ctx->l1.assign(lambdas, lambdas + n_lambdas);
+    return GPFQ_OK;
+}
+
 extern "C" int gpfq_set_stream(gpfq_ctx *ctx, void *cuda_stream) {
     if (!ctx) return GPFQ_ERR_ARG;
     cudaStream_t next = cuda_stream ? (cudaStream_t)cuda_stream : ctx->own_stream;
@@ -364,6 +375,24 @@ static int stage_seeds(gpfq_ctx *ctx, int n_alph) {
     return GPFQ_OK;
 }
 
+// L1 penalty: one lambda for every alphabet of the call.  Nothing to check when it is off.
+static int check_l1(gpfq_ctx *ctx, int n_alph) {
+    if (ctx->l1.empty() || (size_t)n_alph <= ctx->l1.size()) return GPFQ_OK;
+    return gpfq_fail(ctx, GPFQ_ERR_ARG, "%d alphabets but %zu L1 penalties", n_alph, ctx->l1.size());
+}
+
+// The lambdas of this call on the device (one per alphabet, read by the walks in stream order; staged like the seeds, so
+// GPFQ_NO_SYNC calls stay asynchronous), or nullptr when the penalty is off and for Gram-only calls.
+static int stage_l1(gpfq_ctx *ctx, int n_alph) {
+    ctx->d_l1 = nullptr;
+    if (ctx->l1.empty() || ctx->gram_only_out) return GPFQ_OK;
+    double *d = nullptr;
+    GPFQ_TRY(gpfq_ws(ctx, WS_L1_LAMBDA, (size_t)n_alph * sizeof(double), (void **)&d));
+    CUDA_TRY(ctx, cudaMemcpyAsync(d, ctx->l1.data(), (size_t)n_alph * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+    ctx->d_l1 = d;
+    return GPFQ_OK;
+}
+
 cudaError_t gpfq_record(gpfq_ctx *ctx, int which, cudaStream_t s) {
     ctx->cur->rec[which] = true;
     return cudaEventRecord(ctx->cur->e[which], s);
@@ -468,6 +497,7 @@ static int dense_layer(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t l
     const int64_t nj = j1 - j0;
     if (scales && n_alph >= 1) GPFQ_TRY(check_scales(ctx, scales + j0, n_alph, nj, lds));
     GPFQ_TRY(check_rounding(ctx, alphabets, K, n_alph));
+    GPFQ_TRY(check_l1(ctx, n_alph));
     if (nj == 0) return GPFQ_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     const bool same = (Xq == nullptr || Xq == X);
@@ -479,6 +509,7 @@ static int dense_layer(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t l
     Alphabets al;
     GPFQ_TRY(upload_alphabets(ctx, alphabets, K, n_alph, &al));
     GPFQ_TRY(stage_seeds(ctx, n_alph));
+    GPFQ_TRY(stage_l1(ctx, n_alph));
     const double *d_scales = nullptr;
     if (scales) GPFQ_TRY(upload_scales(ctx, scales + j0, n_alph, nj, lds, &d_scales));
 
@@ -574,6 +605,7 @@ static int dense_layer_from_gram(gpfq_ctx *ctx, const double *G1, const double *
     const int64_t nj = j1 - j0;
     if (scales && n_alph >= 1) GPFQ_TRY(check_scales(ctx, scales + j0, n_alph, nj, N1));
     GPFQ_TRY(check_rounding(ctx, alphabets, K, n_alph));
+    GPFQ_TRY(check_l1(ctx, n_alph));
     if (nj == 0) return GPFQ_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     cudaStream_t s = ctx->stream;
@@ -582,6 +614,7 @@ static int dense_layer_from_gram(gpfq_ctx *ctx, const double *G1, const double *
     Alphabets al;
     GPFQ_TRY(upload_alphabets(ctx, alphabets, K, n_alph, &al));
     GPFQ_TRY(stage_seeds(ctx, n_alph));
+    GPFQ_TRY(stage_l1(ctx, n_alph));
     const double *d_scales = nullptr;
     if (scales) GPFQ_TRY(upload_scales(ctx, scales + j0, n_alph, nj, N1, &d_scales));
     const float *dW = W;
@@ -790,6 +823,7 @@ static int conv_channels(gpfq_ctx *ctx, const float *const *Xp, const float *con
         return gpfq_fail(ctx, GPFQ_ERR_ARG, "GPFQ_NO_SYNC needs all-device pointers");
     if (scales && n_alph >= 1) GPFQ_TRY(check_scales(ctx, scales, n_alph, C * F, C * F));
     GPFQ_TRY(check_rounding(ctx, alphabets, K, n_alph));
+    GPFQ_TRY(check_l1(ctx, n_alph));
     ctx->conv_part_bytes = 0;
     if (n_ch == 0) return GPFQ_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
@@ -822,6 +856,7 @@ static int conv_channels(gpfq_ctx *ctx, const float *const *Xp, const float *con
     Alphabets al;
     GPFQ_TRY(upload_alphabets(ctx, alphabets, K, n_alph, &al));
     GPFQ_TRY(stage_seeds(ctx, n_alph));
+    GPFQ_TRY(stage_l1(ctx, n_alph));
     const double *d_scales = nullptr;
     if (scales) GPFQ_TRY(upload_scales(ctx, scales, n_alph, C * F, C * F, &d_scales));
 
@@ -934,6 +969,7 @@ static int conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float *actq, i
     const int kk = kh * kw;
     if (scales && n_alph >= 1) GPFQ_TRY(check_scales(ctx, scales, n_alph, Cg * F, Cg * F));
     if (!ctx->gram_only_out) GPFQ_TRY(check_rounding(ctx, alphabets, K, n_alph));
+    if (!ctx->gram_only_out) GPFQ_TRY(check_l1(ctx, n_alph));
     ctx->conv_part_bytes = 0;
     if (n_ch == 0) return GPFQ_OK;
     // TensorFlow extract_patches geometry (quantized_network.py:158-172)
@@ -999,6 +1035,7 @@ static int conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float *actq, i
     Alphabets al;
     GPFQ_TRY(upload_alphabets(ctx, alphabets, K, n_alph, &al));
     GPFQ_TRY(stage_seeds(ctx, n_alph));
+    GPFQ_TRY(stage_l1(ctx, n_alph));
     const double *d_scales = nullptr;
     if (scales) GPFQ_TRY(upload_scales(ctx, scales, n_alph, Cg * F, Cg * F, &d_scales));
     const float *dA = act, *dAq = same ? act : actq;
@@ -1309,6 +1346,7 @@ static int conv_layer_from_gram(gpfq_ctx *ctx, const double *gram, int32_t kk, c
     if (!conv_supported_kk(kk)) return gpfq_fail(ctx, GPFQ_ERR_UNSUPPORTED, "kernel size kk=%d has no walk kernel", kk);
     if (scales && n_alph >= 1) GPFQ_TRY(check_scales(ctx, scales, n_alph, C / groups * F, C / groups * F));
     GPFQ_TRY(check_rounding(ctx, alphabets, K, n_alph));
+    GPFQ_TRY(check_l1(ctx, n_alph));
     if (n_ch == 0) return GPFQ_OK;
     CUDA_TRY(ctx, cudaSetDevice(ctx->device));
     cudaStream_t s = ctx->stream;
@@ -1317,6 +1355,7 @@ static int conv_layer_from_gram(gpfq_ctx *ctx, const double *gram, int32_t kk, c
     Alphabets al;
     GPFQ_TRY(upload_alphabets(ctx, alphabets, K, n_alph, &al));
     GPFQ_TRY(stage_seeds(ctx, n_alph));
+    GPFQ_TRY(stage_l1(ctx, n_alph));
     const double *d_scales = nullptr;
     if (scales) GPFQ_TRY(upload_scales(ctx, scales, n_alph, C / groups * F, C / groups * F, &d_scales));
     CUDA_TRY(ctx, gpfq_record(ctx, 5, s));
@@ -1374,6 +1413,7 @@ static int round_elements(gpfq_ctx *ctx, const void *W, int is_f64, int64_t n, c
     Alphabets al;
     GPFQ_TRY(upload_alphabets(ctx, alphabet, &K, 1, &al));
     GPFQ_TRY(stage_seeds(ctx, 1));
+    ctx->d_l1 = nullptr;   // MSQ and bit_round have no greedy step: the penalty does not apply
     const double *d_scales = nullptr;
     if (scales) GPFQ_TRY(upload_scales(ctx, scales, 1, n_units, n_units, &d_scales));
     const size_t esz = is_f64 ? sizeof(double) : sizeof(float);

@@ -78,8 +78,10 @@ struct gpfq_ctx {
     int rounding = GPFQ_ROUND_NEAREST;  // gpfq_set_rounding: the mode and its seeds (one per alphabet of a call)
     std::vector<uint64_t> seeds;
     const uint64_t *d_seeds = nullptr;  // the seeds of the call in progress on the device; nullptr: nearest rounding
+    std::vector<double> l1;             // gpfq_set_l1_penalty: one lambda per alphabet of a call (empty: no penalty)
+    const double *d_l1 = nullptr;       // the lambdas of the call in progress on the device; nullptr: no penalty
     // grow-only named workspaces
-    DevBuf ws[48];
+    DevBuf ws[50];
     DevBuf pinned[4];
     // alphabets already resident on the device (steady-state calls re-use them: no copy, no sync)
     std::vector<AlphEntry> alph_cache;
@@ -91,7 +93,7 @@ enum WsSlot {
     WS_U, WS_PTRS, WS_CG, WS_CPART, WS_PATCH_A, WS_PATCH_B, WS_ACT_A, WS_ACT_B, WS_QIDX, WS_MISC,
     WS_I8_SQ, WS_I8_SX, WS_I8_E, WS_I8_TILES, WS_LR_XD, WS_LR_XT, WS_LR_U, WS_CORR_B,
     WS_SL_W, WS_SL_XT, WS_SL_XQT, WS_SL_XQ, WS_SL_U, WS_SL_KQ, WS_SL_E,
-    WS_TC_TAB, WS_TC_G2S, WS_TC_G1S, WS_TC_E, WS_TC_P, WS_TC_W, WS_TC_G1M, WS_SCALES, WS_UNIT_H, WS_SEEDS
+    WS_TC_TAB, WS_TC_G2S, WS_TC_G1S, WS_TC_E, WS_TC_P, WS_TC_W, WS_TC_G1M, WS_SCALES, WS_UNIT_H, WS_SEEDS, WS_L1, WS_L1_LAMBDA
 };
 
 int gpfq_fail(gpfq_ctx *ctx, int code, const char *fmt, ...);
@@ -352,10 +354,35 @@ __device__ __forceinline__ double gpfq_decide_stoch(double nrm, double d, double
     return gpfq_stoc_round_eq<SCALED>(v, alph, K, inv_step, s, r);
 }
 
-// The step of a walk: nearest rounding (STOCH = false: gpfq_decide_unit, unchanged) or stochastic with the draw r
+// ---------------------------------------------------------------------------------------------
+// Sparse GPFQ (gpfq_set_l1_penalty): an L1 penalty lambda per alphabet soft-thresholds the value of every greedy step before it
+// is quantized.  tau = fl(lambda / fl(nrm^2)) depends only on the direction and the alphabet, so the walks form it off the chain
+// (per tap, per block of directions, or in a table); the step is then
+//   v' = 0 if |v| <= tau, else fl(v - copysign(tau, v))          (NaN stays NaN: the comparison is false)
+// with v the reference's value (w for the :86 guard, num / nrm^2 otherwise).  tau = +0 (lambda = 0) gives v' = v up to the
+// sign of a zero, which neither quantizer sees.
+// ---------------------------------------------------------------------------------------------
+__device__ __forceinline__ double gpfq_shrink(double v, double tau) {
+    return fabs(v) <= tau ? 0.0 : __dsub_rn(v, copysign(tau, v));
+}
+__device__ __forceinline__ double gpfq_l1_tau(double lambda, double nrm) { return __ddiv_rn(lambda, __dmul_rn(nrm, nrm)); }
+
+// One greedy step with the penalty: the reference's guards, the shrink, then nearest (STOCH = false) or stochastic rounding
 template <bool SCALED, bool STOCH>
+__device__ __forceinline__ double gpfq_decide_l1(double nrm, double d, double num, double w, const double *__restrict__ alph, int K,
+                                                 double inv_step, double s, double r, double tau) {
+    if (nrm < GPFQ_DEAD_NORM) return 0.0;
+    const double v = gpfq_shrink(fabs(d) < GPFQ_PERP_DOT ? w : __ddiv_rn(num, nrm * nrm), tau);
+    if (STOCH) return gpfq_stoc_round_eq<SCALED>(v, alph, K, inv_step, s, r);
+    return gpfq_round_unit<SCALED>(v, alph, K, inv_step, s);
+}
+
+// The step of a walk: nearest rounding (STOCH = false: gpfq_decide_unit, unchanged) or stochastic with the draw r
+// L1: the penalty's shrink with the step's tau
+template <bool SCALED, bool STOCH, bool L1 = false>
 __device__ __forceinline__ double gpfq_decide_any(double nrm, double d, double num, double w, const double *__restrict__ alph, int K,
-                                                  double inv_step, double s, double r) {
+                                                  double inv_step, double s, double r, double tau = 0.0) {
+    if (L1) return gpfq_decide_l1<SCALED, STOCH>(nrm, d, num, w, alph, K, inv_step, s, r, tau);
     if (STOCH) return gpfq_decide_stoch<SCALED>(nrm, d, num, w, alph, K, inv_step, s, r);
     return gpfq_decide_unit<SCALED>(nrm, d, num, w, alph, K, inv_step, s);
 }

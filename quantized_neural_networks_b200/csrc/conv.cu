@@ -733,13 +733,16 @@ __device__ __forceinline__ int64_t conv_wq_offset(int64_t c, int64_t f, int64_t 
 
 // SCALED: the (channel, filter) unit walks with the levels scales[a * Cg * F + (c % Cg) * F + filter] * alphabet (common.cuh).
 // STOCH: stochastic rounding, unit id = that same scale index, step id = tap, seed seeds[a].
-template <int KK, bool GROUPED, bool SCALED = false, bool STOCH = false>
+// L1: the penalty lambdas[a] (common.cuh), tau once per tap in shared memory.
+template <int KK, bool GROUPED, bool SCALED = false, bool STOCH = false, bool L1 = false>
 __global__ void __launch_bounds__(128)
 conv_sweep_kernel(const double *__restrict__ gram, const float *__restrict__ W, double *__restrict__ Q,
                   int64_t CF, int64_t F, int64_t c0, const double *__restrict__ alphabets,
                   const int *__restrict__ Koff, const int *__restrict__ Flags, int64_t q_alph_stride, int64_t Cg, int64_t Fg,
-                  const double *__restrict__ scales = nullptr, const uint64_t *__restrict__ seeds = nullptr) {
+                  const double *__restrict__ scales = nullptr, const uint64_t *__restrict__ seeds = nullptr,
+                  const double *__restrict__ lambdas = nullptr) {
     __shared__ double g1[KK * KK], g2[KK * KK], nrm[KK], alph[GPFQ_MAX_K];
+    __shared__ double tau[L1 ? KK : 1];
     const int ch = blockIdx.y, a = blockIdx.z;
     const int K = Koff[a + 1] - Koff[a];
     for (int e = threadIdx.x; e < KK * KK; e += blockDim.x) {
@@ -749,6 +752,7 @@ conv_sweep_kernel(const double *__restrict__ gram, const float *__restrict__ W, 
     for (int e = threadIdx.x; e < K; e += blockDim.x) alph[e] = alphabets[Koff[a] + e];
     __syncthreads();
     if (threadIdx.x < KK) nrm[threadIdx.x] = (double)(float)sqrt(g2[threadIdx.x * KK + threadIdx.x]);
+    if (L1 && threadIdx.x < KK) tau[threadIdx.x] = gpfq_l1_tau(lambdas[a], (double)(float)sqrt(g2[threadIdx.x * KK + threadIdx.x]));
     __syncthreads();
     const double inv_step_base = SCALED ? 0.0 : gpfq_inv_step(alph, K, Flags[a]);
     const int64_t f = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -767,7 +771,8 @@ conv_sweep_kernel(const double *__restrict__ gram, const float *__restrict__ W, 
         for (int s = 0; s < KK; ++s)
             if (s < t) d += w[s] * g1[t * KK + s] - q[s] * g2[t * KK + s];
         const double num = fma(w[t], g1[t * KK + t], d);
-        q[t] = gpfq_decide_any<SCALED, STOCH>(nrm[t], d, num, w[t], alph, K, inv_step, sc, STOCH ? gpfq_draw(key, t) : 0.0);
+        q[t] = gpfq_decide_any<SCALED, STOCH, L1>(nrm[t], d, num, w[t], alph, K, inv_step, sc, STOCH ? gpfq_draw(key, t) : 0.0,
+                                                  L1 ? tau[t] : 0.0);
         Q[(int64_t)a * q_alph_stride + (int64_t)t * CF + base] = q[t];
     }
 }
@@ -782,12 +787,13 @@ constexpr int MAXW = 16;  // warps (filters) per CTA
 __host__ __device__ constexpr int col_off(int s, int kk) { return s * kk - s * (s - 1) / 2; }
 }  // namespace walkx
 
-template <bool GROUPED, bool SCALED = false, bool STOCH = false>
+template <bool GROUPED, bool SCALED = false, bool STOCH = false, bool L1 = false>
 __global__ void __launch_bounds__(walkx::MAXW * 32)
 conv_walkx_kernel(const double *__restrict__ gram, int kk, const float *__restrict__ W, double *__restrict__ Q, int64_t CF,
                   int64_t F, int64_t c0, const double *__restrict__ alphabets, const int *__restrict__ Koff,
                   const int *__restrict__ Flags, int64_t q_alph_stride, int64_t Cg, int64_t Fg,
-                  const double *__restrict__ scales = nullptr, const uint64_t *__restrict__ seeds = nullptr) {
+                  const double *__restrict__ scales = nullptr, const uint64_t *__restrict__ seeds = nullptr,
+                  const double *__restrict__ lambdas = nullptr) {
     extern __shared__ double walkx_smem[];
     const int tri = kk * (kk + 1) / 2;
     double *g1 = walkx_smem, *g2 = g1 + tri, *nrm = g2 + tri, *alph = nrm + kk;
@@ -804,6 +810,9 @@ conv_walkx_kernel(const double *__restrict__ gram, int kk, const float *__restri
     for (int e = threadIdx.x; e < K; e += blockDim.x) alph[e] = alphabets[Koff[a] + e];
     __syncthreads();
     for (int t = threadIdx.x; t < kk; t += blockDim.x) nrm[t] = (double)(float)sqrt(g2[walkx::col_off(t, kk)]);
+    double *tau = alph + GPFQ_MAX_K;   // L1: kk more doubles of dynamic shared memory
+    if (L1)
+        for (int t = threadIdx.x; t < kk; t += blockDim.x) tau[t] = gpfq_l1_tau(lambdas[a], (double)(float)sqrt(g2[walkx::col_off(t, kk)]));
     __syncthreads();
     const double inv_step_base = SCALED ? 0.0 : gpfq_inv_step(alph, K, Flags[a]);
     const int lane = threadIdx.x & 31;
@@ -831,7 +840,8 @@ conv_walkx_kernel(const double *__restrict__ gram, int kk, const float *__restri
             double qt = 0.0;
             if (lane == o) {
                 const double num = fma(w[j], g1[off + t], d[j]);
-                qt = gpfq_decide_any<SCALED, STOCH>(nrm[t], d[j], num, w[j], alph, K, inv_step, sc, STOCH ? gpfq_draw(key, t) : 0.0);
+                qt = gpfq_decide_any<SCALED, STOCH, L1>(nrm[t], d[j], num, w[j], alph, K, inv_step, sc, STOCH ? gpfq_draw(key, t) : 0.0,
+                                                        L1 ? tau[t] : 0.0);
                 q_out[(int64_t)t * CF] = qt;
             }
             qt = __shfl_sync(0xffffffffu, qt, o);
@@ -1022,14 +1032,17 @@ int conv_sweep_stage(gpfq_ctx *ctx, int kk, const double *gram, const float *W, 
     dim3 grid((unsigned)ceil_div64(Fg, 128), (unsigned)n_ch, (unsigned)n_alph);
     const int64_t CF = Cg * F, qs = (int64_t)kk * CF;
     const uint64_t *seeds = ctx->d_seeds;
-#define SWEEP_LAUNCH(KKV, G, S, R) \
-    conv_sweep_kernel<KKV, G, S, R><<<grid, 128, 0, ctx->stream>>>(gram, W, Q, CF, F, c0, d_alph, d_koff, d_flags, qs, Cg, Fg, scales, seeds)
-#define SWEEP_SCALED(KKV, R)                                                                                            \
-    if (scales) { if (grouped) SWEEP_LAUNCH(KKV, true, true, R); else SWEEP_LAUNCH(KKV, false, true, R); }              \
-    else { if (grouped) SWEEP_LAUNCH(KKV, true, false, R); else SWEEP_LAUNCH(KKV, false, false, R); }
+    const double *lambdas = ctx->d_l1;   // the L1 penalty (nullptr: off)
+#define SWEEP_LAUNCH(KKV, G, S, R, L)                                                                                   \
+    conv_sweep_kernel<KKV, G, S, R, L><<<grid, 128, 0, ctx->stream>>>(gram, W, Q, CF, F, c0, d_alph, d_koff, d_flags, qs, Cg, Fg, \
+                                                                      scales, seeds, lambdas)
+#define SWEEP_SCALED(KKV, R, L)                                                                                         \
+    if (scales) { if (grouped) SWEEP_LAUNCH(KKV, true, true, R, L); else SWEEP_LAUNCH(KKV, false, true, R, L); }        \
+    else { if (grouped) SWEEP_LAUNCH(KKV, true, false, R, L); else SWEEP_LAUNCH(KKV, false, false, R, L); }
 #define SWEEP_CASE(KKV)                                                                                                 \
     case KKV:                                                                                                           \
-        if (seeds) { SWEEP_SCALED(KKV, true) } else { SWEEP_SCALED(KKV, false) }                                        \
+        if (lambdas) { if (seeds) { SWEEP_SCALED(KKV, true, true) } else { SWEEP_SCALED(KKV, false, true) } }           \
+        else if (seeds) { SWEEP_SCALED(KKV, true, false) } else { SWEEP_SCALED(KKV, false, false) }                     \
         break;
     switch (kk) {
         SWEEP_CASE(1) SWEEP_CASE(2) SWEEP_CASE(3) SWEEP_CASE(4) SWEEP_CASE(6) SWEEP_CASE(9)
@@ -1037,14 +1050,20 @@ int conv_sweep_stage(gpfq_ctx *ctx, int kk, const double *gram, const float *W, 
             if (!conv_supported_kk(kk)) return gpfq_fail(ctx, GPFQ_ERR_UNSUPPORTED, "conv kernel size kk=%d has no walk kernel", kk);
             using namespace walkx;
             const int warps = Fg < MAXW ? (int)Fg : MAXW;
-            const size_t smem = ((size_t)kk * (kk + 1) + kk + GPFQ_MAX_K) * sizeof(double);
+            const size_t smem = ((size_t)kk * (kk + 1) + kk + GPFQ_MAX_K + (lambdas ? kk : 0)) * sizeof(double);
             dim3 wgrid((unsigned)ceil_div64(Fg, warps), (unsigned)n_ch, (unsigned)n_alph);
             auto k = seeds ? (grouped ? (scales ? conv_walkx_kernel<true, true, true> : conv_walkx_kernel<true, false, true>)
                                       : (scales ? conv_walkx_kernel<false, true, true> : conv_walkx_kernel<false, false, true>))
                            : (grouped ? (scales ? conv_walkx_kernel<true, true> : conv_walkx_kernel<true, false>)
                                       : (scales ? conv_walkx_kernel<false, true> : conv_walkx_kernel<false, false>));
+            if (lambdas)
+                k = seeds ? (grouped ? (scales ? conv_walkx_kernel<true, true, true, true> : conv_walkx_kernel<true, false, true, true>)
+                                     : (scales ? conv_walkx_kernel<false, true, true, true> : conv_walkx_kernel<false, false, true, true>))
+                          : (grouped ? (scales ? conv_walkx_kernel<true, true, false, true> : conv_walkx_kernel<true, false, false, true>)
+                                     : (scales ? conv_walkx_kernel<false, true, false, true> : conv_walkx_kernel<false, false, false, true>));
             CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            k<<<wgrid, warps * 32, smem, ctx->stream>>>(gram, kk, W, Q, CF, F, c0, d_alph, d_koff, d_flags, qs, Cg, Fg, scales, seeds);
+            k<<<wgrid, warps * 32, smem, ctx->stream>>>(gram, kk, W, Q, CF, F, c0, d_alph, d_koff, d_flags, qs, Cg, Fg, scales, seeds,
+                                                        lambdas);
         }
     }
 #undef SWEEP_CASE

@@ -115,6 +115,29 @@ __device__ __forceinline__ double gpfq_decide_rcp_stoch(double nrm, double rinv,
     return gpfq_stoc_round_eq<SCALED>(v, alph, K, inv_step, s, r);
 }
 
+// The step with the L1 penalty (common.cuh): the same argument, shrunk by the direction's tau, then nearest (STOCH = false) or
+// stochastic rounding
+template <bool SCALED, bool STOCH>
+__device__ __forceinline__ double gpfq_decide_rcp_l1(double nrm, double rinv, double d, double num, double w,
+                                                     const double *__restrict__ alph, int K, double inv_step, double tern, double s,
+                                                     double r, double tau) {
+    if (nrm < GPFQ_DEAD_NORM) return 0.0;
+    double v = w;
+    if (!(fabs(d) < GPFQ_PERP_DOT)) {
+        const double den = nrm * nrm;
+        const double q0 = num * rinv;
+        const double e = fma(-q0, den, num);
+        v = fma(e, rinv, q0);
+    }
+    v = gpfq_shrink(v, tau);
+    if (STOCH) {
+        if (tern > 0.0) return gpfq_stoc_round_ternary(v, tern, r);
+        return gpfq_stoc_round_eq<SCALED>(v, alph, K, inv_step, s, r);
+    }
+    if (tern > 0.0) return gpfq_bit_round_ternary(v, tern);
+    return gpfq_round_unit<SCALED>(v, alph, K, inv_step, s);
+}
+
 // Per-neuron scale, inv_step and ternary radius of neuron jt + j (SCALED; else the alphabet's own)
 template <bool SCALED>
 __device__ __forceinline__ void sweep_unit_levels(const double *__restrict__ scales, int64_t idx, bool live,
@@ -140,14 +163,15 @@ struct SweepCfg {
 
 // SCALED: neuron j of alphabet a walks with the levels scales[a * nj + j] * alphabet (per-channel alphabets).
 // STOCH: stochastic rounding, neuron j with unit id u0 + j and seed seeds[a], direction t with step id t.
-template <int NT, bool ALIGNED, bool SCALED = false, bool STOCH = false>
+// L1: the penalty lambdas[a]; each walker lane forms tau of one direction of the block, broadcast by a shuffle at its step.
+template <int NT, bool ALIGNED, bool SCALED = false, bool STOCH = false, bool L1 = false>
 __global__ void __launch_bounds__(256, 2)
 sweep_tile_kernel(const double *__restrict__ G1, const double *__restrict__ G2, int64_t ldg, int64_t N0,
                   const double *__restrict__ Wt, double *__restrict__ Qt, int64_t nj,
                   const double *__restrict__ alphabets, const int *__restrict__ Koff,
                   const int *__restrict__ Flags, int64_t t_begin, int64_t t_end, const double *__restrict__ Dt,
                   int64_t ldd, const double *__restrict__ scales = nullptr, const uint64_t *__restrict__ seeds = nullptr,
-                  int64_t u0 = 0) {
+                  int64_t u0 = 0, const double *__restrict__ lambdas = nullptr) {
     // Directions [t_begin, t_end) (t_begin a multiple of 32).  Dt (nullable): (n_alph, nj, ldd) contributions of the
     // directions before t_begin, from one large NT contraction on the host side (two-level blocking).
     using Cfg = SweepCfg<NT>;
@@ -334,6 +358,7 @@ sweep_tile_kernel(const double *__restrict__ G1, const double *__restrict__ G2, 
                 d[i] = qblk[j * (B + 1) + t] + (dsm[t * (NT + 1) + j] + dsm[B * (NT + 1) + t * (NT + 1) + j]);
             }
             __syncwarp();  // every lane has read its prior-range values before the first q lands in qblk
+            const double tau_l = L1 ? gpfq_l1_tau(lambdas[a], nrm[lane]) : 0.0;   // tau of direction `lane` of the block
             const double *wrow = wblk + j * (B + 1);
             double *qrow = qblk + j * (B + 1);
             const int ngrp = (nb + 3) >> 2;
@@ -346,7 +371,10 @@ sweep_tile_kernel(const double *__restrict__ G1, const double *__restrict__ G2, 
                     const double d0 = __shfl_sync(0xffffffffu, d[0], (lane & ~3) + rr);
                     const double wv = wrow[tt];
                     const double num = fma(wv, g1dd[tt], d0);
-                    double q = STOCH ? gpfq_decide_rcp_stoch<SCALED>(nrm[tt], rinv[tt], d0, num, wv, alph, K, inv_u, tern_u, sc,
+                    double q = L1 ? gpfq_decide_rcp_l1<SCALED, STOCH>(nrm[tt], rinv[tt], d0, num, wv, alph, K, inv_u, tern_u, sc,
+                                                                      STOCH ? gpfq_draw(key, t0 + tt) : 0.0,
+                                                                      __shfl_sync(0xffffffffu, tau_l, tt))
+                             : STOCH ? gpfq_decide_rcp_stoch<SCALED>(nrm[tt], rinv[tt], d0, num, wv, alph, K, inv_u, tern_u, sc,
                                                                      gpfq_draw(key, t0 + tt))
                                      : gpfq_decide_rcp_unit<SCALED>(nrm[tt], rinv[tt], d0, num, wv, alph, K, inv_u, tern_u, sc);
                     if (tt >= nb) q = 0.0;  // past the end of a partial block: no decision, no update
@@ -396,13 +424,13 @@ struct PipeCfg {
     static constexpr size_t SMEM = sizeof(double) * ((size_t)STAGES * (B + NT) * LD + 2 * SET + GPFQ_MAX_K);
 };
 
-template <int NT, bool SCALED = false, bool STOCH = false>
+template <int NT, bool SCALED = false, bool STOCH = false, bool L1 = false>
 __global__ void __launch_bounds__(256, 1)
 sweep_pipe_kernel(const double *__restrict__ G1, const double *__restrict__ G2, int64_t ldg, int64_t N0,
                   const double *__restrict__ Wt, double *__restrict__ Qt, int64_t nj, const double *__restrict__ alphabets,
                   const int *__restrict__ Koff, const int *__restrict__ Flags, int64_t t_begin, int64_t t_end,
                   const double *__restrict__ Dt, int64_t ldd, const double *__restrict__ scales = nullptr,
-                  const uint64_t *__restrict__ seeds = nullptr, int64_t u0 = 0) {
+                  const uint64_t *__restrict__ seeds = nullptr, int64_t u0 = 0, const double *__restrict__ lambdas = nullptr) {
     using Cfg = PipeCfg<NT>;
     constexpr int B = Cfg::B, KC = Cfg::KC, LD = Cfg::LD, STAGES = Cfg::STAGES, CT = Cfg::CT, NA = NT / 8, NW = 4 * NT;
     constexpr int BAR_C = 1, BAR_READY = 2, BAR_WALK_DONE = 4, BAR_Q_STORED = 6, HANDOVER = NW + CT;
@@ -604,6 +632,7 @@ sweep_pipe_kernel(const double *__restrict__ G1, const double *__restrict__ G2, 
                 d[i] = qrow[t] + dsm[t * (NT + 1) + j];
             }
             __syncwarp();  // every lane has read its prior-range values before the first q lands in qblk
+            const double tau_l = L1 ? gpfq_l1_tau(lambdas[a], nrm[lane]) : 0.0;   // tau of direction `lane` of the block
             const int ngrp = (nb + 3) >> 2;
 #pragma unroll 1
             for (int g4 = 0; g4 < ngrp; ++g4) {
@@ -614,7 +643,10 @@ sweep_pipe_kernel(const double *__restrict__ G1, const double *__restrict__ G2, 
                     const double d0 = __shfl_sync(0xffffffffu, d[0], (lane & ~3) + rr);
                     const double wv = wrow[tt];
                     const double num = fma(wv, g1dd[tt], d0);
-                    double q = STOCH ? gpfq_decide_rcp_stoch<SCALED>(nrm[tt], rinv[tt], d0, num, wv, alph, K, inv_u, tern_u, sc,
+                    double q = L1 ? gpfq_decide_rcp_l1<SCALED, STOCH>(nrm[tt], rinv[tt], d0, num, wv, alph, K, inv_u, tern_u, sc,
+                                                                      STOCH ? gpfq_draw(key, t0 + tt) : 0.0,
+                                                                      __shfl_sync(0xffffffffu, tau_l, tt))
+                             : STOCH ? gpfq_decide_rcp_stoch<SCALED>(nrm[tt], rinv[tt], d0, num, wv, alph, K, inv_u, tern_u, sc,
                                                                      gpfq_draw(key, t0 + tt))
                                      : gpfq_decide_rcp_unit<SCALED>(nrm[tt], rinv[tt], d0, num, wv, alph, K, inv_u, tern_u, sc);
                     if (tt >= nb) q = 0.0;  // past the end of a partial block: no decision, no update
@@ -656,10 +688,15 @@ static int launch_sweep_pipe(gpfq_ctx *ctx, const double *G1, const double *G2, 
     const size_t smem = PipeCfg<NT>::SMEM;
     dim3 grid((unsigned)ceil_div64(nj, NT), (unsigned)n_alph);
     const uint64_t *seeds = ctx->d_seeds;
+    const double *lambdas = ctx->d_l1;
     auto k = seeds ? (scales ? sweep_pipe_kernel<NT, true, true> : sweep_pipe_kernel<NT, false, true>)
                    : (scales ? sweep_pipe_kernel<NT, true> : sweep_pipe_kernel<NT, false>);
+    if (lambdas)
+        k = seeds ? (scales ? sweep_pipe_kernel<NT, true, true, true> : sweep_pipe_kernel<NT, false, true, true>)
+                  : (scales ? sweep_pipe_kernel<NT, true, false, true> : sweep_pipe_kernel<NT, false, false, true>);
     CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    k<<<grid, 256, smem, ctx->stream>>>(G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, t_begin, t_end, Dt, ldd, scales, seeds, u0);
+    k<<<grid, 256, smem, ctx->stream>>>(G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, t_begin, t_end, Dt, ldd, scales, seeds, u0,
+                                        lambdas);
     KERNEL_CHECK(ctx);
     return GPFQ_OK;
 }
@@ -674,12 +711,19 @@ static int launch_sweep_tile(gpfq_ctx *ctx, const double *G1, const double *G2, 
     const bool aligned = (N0 % 2 == 0) && (ldg % 2 == 0) && ((uintptr_t)G1 % 16 == 0) && ((uintptr_t)G2 % 16 == 0) &&
                          ((uintptr_t)Wt % 16 == 0) && ((uintptr_t)Qt % 16 == 0) && ((nj * N0) % 2 == 0);
     const uint64_t *seeds = ctx->d_seeds;
+    const double *lambdas = ctx->d_l1;
     auto k = seeds ? (aligned ? (scales ? sweep_tile_kernel<NT, true, true, true> : sweep_tile_kernel<NT, true, false, true>)
                               : (scales ? sweep_tile_kernel<NT, false, true, true> : sweep_tile_kernel<NT, false, false, true>))
                    : (aligned ? (scales ? sweep_tile_kernel<NT, true, true> : sweep_tile_kernel<NT, true, false>)
                               : (scales ? sweep_tile_kernel<NT, false, true> : sweep_tile_kernel<NT, false, false>));
+    if (lambdas)
+        k = seeds ? (aligned ? (scales ? sweep_tile_kernel<NT, true, true, true, true> : sweep_tile_kernel<NT, true, false, true, true>)
+                             : (scales ? sweep_tile_kernel<NT, false, true, true, true> : sweep_tile_kernel<NT, false, false, true, true>))
+                  : (aligned ? (scales ? sweep_tile_kernel<NT, true, true, false, true> : sweep_tile_kernel<NT, true, false, false, true>)
+                             : (scales ? sweep_tile_kernel<NT, false, true, false, true> : sweep_tile_kernel<NT, false, false, false, true>));
     CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    k<<<grid, 256, smem, ctx->stream>>>(G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, t_begin, t_end, Dt, ldd, scales, seeds, u0);
+    k<<<grid, 256, smem, ctx->stream>>>(G1, G2, ldg, N0, Wt, Qt, nj, d_alph, d_koff, d_flags, t_begin, t_end, Dt, ldd, scales, seeds, u0,
+                                        lambdas);
     KERNEL_CHECK(ctx);
     return GPFQ_OK;
 }

@@ -40,14 +40,15 @@ __global__ void __launch_bounds__(256) row_norms_kernel(const float *__restrict_
 
 // SCALED: neuron jb + j of the shard walks with the levels scales[jb + j] * alphabet (common.cuh)
 // STOCH: stochastic rounding with the seed *seed, unit id u0 + jb + j (the global neuron), step id t
-template <int J, bool SCALED = false, bool STOCH = false>
+// L1: the penalty's shrink with tau[t] (row_norms_l1_kernel)
+template <int J, bool SCALED = false, bool STOCH = false, bool L1 = false>
 __global__ void __launch_bounds__(STREAM_T)
 dense_stream_kernel(const float *__restrict__ X, const float *__restrict__ Xq, int64_t ldx, int64_t N0,
                     int64_t m, const float *__restrict__ W, int64_t ldw, int64_t j0, int64_t nj,
                     const double *__restrict__ nrm, const double *__restrict__ alphabet, int K,
                     double *__restrict__ Q, int64_t ldq, int64_t col0, double *__restrict__ u_scratch,
                     int u_in_smem, const double *__restrict__ scales = nullptr, const uint64_t *__restrict__ seed = nullptr,
-                    int64_t u0 = 0) {
+                    int64_t u0 = 0, const double *__restrict__ tau = nullptr) {
     extern __shared__ __align__(16) unsigned char stream_smem[];
     constexpr int NW = STREAM_T / 32;
     __shared__ double red[NW][2 * J];
@@ -114,7 +115,9 @@ dense_stream_kernel(const float *__restrict__ X, const float *__restrict__ Xq, i
         if (tid < J) {
             double dd = 0.0, ss = 0.0;
             for (int wv = 0; wv < NW; ++wv) { dd += red[wv][tid]; ss += red[wv][J + tid]; }
-            const double q = STOCH    ? gpfq_decide_stoch<SCALED>(nrm[t], dd, ss, (double)w[tid], alph, K, 0.0, sc, gpfq_draw(key, t))
+            const double q = L1       ? gpfq_decide_l1<SCALED, STOCH>(nrm[t], dd, ss, (double)w[tid], alph, K, 0.0, sc,
+                                                                        STOCH ? gpfq_draw(key, t) : 0.0, tau[t])
+                           : STOCH    ? gpfq_decide_stoch<SCALED>(nrm[t], dd, ss, (double)w[tid], alph, K, 0.0, sc, gpfq_draw(key, t))
                            : SCALED ? gpfq_decide_unit<true>(nrm[t], dd, ss, (double)w[tid], alph, K, 0.0, sc)
                                     : gpfq_decide(nrm[t], dd, ss, (double)w[tid], alph, K);
             qsh[tid] = q;
@@ -171,14 +174,14 @@ __device__ __forceinline__ int warp_reduce_index(int lane) {
     return idx;
 }
 
-template <int EPV, int J, bool LITERAL, bool VEC, bool SCALED = false, bool STOCH = false>
+template <int EPV, int J, bool LITERAL, bool VEC, bool SCALED = false, bool STOCH = false, bool L1 = false>
 __global__ void __launch_bounds__(STREAM_T)
 dense_stream_reg_kernel(const float *__restrict__ X, const float *__restrict__ Xq, int64_t ldx, int64_t N0,
                         int64_t m, const float *__restrict__ W, int64_t ldw, int64_t j0, int64_t nj,
                         const double *__restrict__ nrm, const double *__restrict__ g1d,
                         const double *__restrict__ alphabet, int K, int equispaced,
                         double *__restrict__ Q, int64_t ldq, int64_t col0, const double *__restrict__ scales = nullptr,
-                        const uint64_t *__restrict__ seed = nullptr, int64_t u0 = 0) {
+                        const uint64_t *__restrict__ seed = nullptr, int64_t u0 = 0, const double *__restrict__ tau = nullptr) {
     constexpr int NW = STREAM_T / 32, EPT = 4 * EPV;
     constexpr int V = LITERAL ? 2 * J : J;  // values reduced per step
     __shared__ double red[NW][V];
@@ -295,7 +298,9 @@ dense_stream_reg_kernel(const float *__restrict__ X, const float *__restrict__ X
                     for (int jj = 1; jj < J; ++jj) wj = (j == jj) ? w[jj] : wj;
                     const double num = LITERAL ? ss : fma((double)wj, g1_t, dd);
                     const double q =
-                        STOCH    ? gpfq_decide_stoch<SCALED>(nrm_t, dd, num, (double)wj, alph, K, SCALED ? unit_s[J + j] : inv_step,
+                        L1       ? gpfq_decide_l1<SCALED, STOCH>(nrm_t, dd, num, (double)wj, alph, K, SCALED ? unit_s[J + j] : inv_step,
+                                                                 SCALED ? unit_s[j] : 1.0, STOCH ? gpfq_draw(unit_key[j], t) : 0.0, tau[t])
+                      : STOCH    ? gpfq_decide_stoch<SCALED>(nrm_t, dd, num, (double)wj, alph, K, SCALED ? unit_s[J + j] : inv_step,
                                                              SCALED ? unit_s[j] : 1.0, gpfq_draw(unit_key[j], t))
                       : SCALED ? gpfq_decide_unit<true>(nrm_t, dd, num, (double)wj, alph, K, unit_s[J + j], unit_s[j])
                                : gpfq_decide(nrm_t, dd, num, (double)wj, alph, K, inv_step);
@@ -331,20 +336,21 @@ template <int EPV, int J>
 static int launch_stream_reg(gpfq_ctx *ctx, bool literal, bool vec, const float *X, const float *Xq, int64_t ldx,
                              int64_t N0, int64_t m, const float *W, int64_t ldw, int64_t j0, int64_t nj,
                              const double *nrm, const double *g1d, const double *d_alph, int K, int eq, double *Qd,
-                             int64_t ldq, int64_t col0, const double *scales, const uint64_t *seed, int64_t u0) {
+                             int64_t ldq, int64_t col0, const double *scales, const uint64_t *seed, int64_t u0, const double *tau) {
     const unsigned nblk = (unsigned)ceil_div64(nj, J);
-#define LAUNCH(LIT, VEC, S, R) \
-    dense_stream_reg_kernel<EPV, J, LIT, VEC, S, R><<<nblk, STREAM_T, 0, ctx->stream>>>(X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm, \
-                                                                                     g1d, d_alph, K, eq, Qd, ldq, col0, scales, seed, u0)
-#define LAUNCH_S(R)                                                                           \
-    if (scales) {                                                                             \
-        if (literal) { if (vec) LAUNCH(true, true, true, R); else LAUNCH(true, false, true, R); }  \
-        else { if (vec) LAUNCH(false, true, true, R); else LAUNCH(false, false, true, R); }        \
-    } else {                                                                                  \
-        if (literal) { if (vec) LAUNCH(true, true, false, R); else LAUNCH(true, false, false, R); } \
-        else { if (vec) LAUNCH(false, true, false, R); else LAUNCH(false, false, false, R); }      \
+#define LAUNCH(LIT, VEC, S, R, L) \
+    dense_stream_reg_kernel<EPV, J, LIT, VEC, S, R, L><<<nblk, STREAM_T, 0, ctx->stream>>>(X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm, \
+                                                                                        g1d, d_alph, K, eq, Qd, ldq, col0, scales, seed, u0, tau)
+#define LAUNCH_S(R, L)                                                                                 \
+    if (scales) {                                                                                      \
+        if (literal) { if (vec) LAUNCH(true, true, true, R, L); else LAUNCH(true, false, true, R, L); }  \
+        else { if (vec) LAUNCH(false, true, true, R, L); else LAUNCH(false, false, true, R, L); }        \
+    } else {                                                                                           \
+        if (literal) { if (vec) LAUNCH(true, true, false, R, L); else LAUNCH(true, false, false, R, L); } \
+        else { if (vec) LAUNCH(false, true, false, R, L); else LAUNCH(false, false, false, R, L); }      \
     }
-    if (seed) { LAUNCH_S(true) } else { LAUNCH_S(false) }
+    if (tau) { if (seed) { LAUNCH_S(true, true) } else { LAUNCH_S(false, true) } }
+    else if (seed) { LAUNCH_S(true, false) } else { LAUNCH_S(false, false) }
 #undef LAUNCH_S
 #undef LAUNCH
     KERNEL_CHECK(ctx);
@@ -355,11 +361,11 @@ static int launch_stream_reg(gpfq_ctx *ctx, bool literal, bool vec, const float 
 static int dispatch_stream_reg(gpfq_ctx *ctx, int epv, int J, bool literal, bool vec, const float *X, const float *Xq,
                                int64_t ldx, int64_t N0, int64_t m, const float *W, int64_t ldw, int64_t j0, int64_t nj,
                                const double *nrm, const double *g1d, const double *d_alph, int K, int eq, double *Qd,
-                               int64_t ldq, int64_t col0, const double *scales, const uint64_t *seed, int64_t u0) {
+                               int64_t ldq, int64_t col0, const double *scales, const uint64_t *seed, int64_t u0, const double *tau) {
 #define SR(E, JJ) \
     if (epv == E && J == JJ) \
         return launch_stream_reg<E, JJ>(ctx, literal, vec, X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm, g1d, d_alph, K, eq, Qd, \
-                                        ldq, col0, scales, seed, u0);
+                                        ldq, col0, scales, seed, u0, tau);
     SR(1, 1) SR(1, 2) SR(1, 4)
     SR(2, 1) SR(2, 2)
     SR(3, 1) SR(3, 2)
@@ -372,7 +378,7 @@ template <int J>
 static int launch_stream(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ldx, int64_t N0, int64_t m,
                          const float *W, int64_t ldw, int64_t j0, int64_t nj, const double *nrm,
                          const double *d_alph, int K, double *Qd, int64_t ldq, int64_t col0, const double *scales,
-                         const uint64_t *seed, int64_t u0) {
+                         const uint64_t *seed, int64_t u0, const double *tau) {
     const int64_t nblk = ceil_div64(nj, J);
     const size_t need = (size_t)J * m * sizeof(double);
     const size_t static_smem = 8192;  // red/qsh/alph, generous
@@ -381,27 +387,60 @@ static int launch_stream(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t
     if (!in_smem) GPFQ_TRY(gpfq_ws(ctx, WS_U, (size_t)nblk * need, (void **)&scratch));
     auto k = seed ? (scales ? dense_stream_kernel<J, true, true> : dense_stream_kernel<J, false, true>)
                   : (scales ? dense_stream_kernel<J, true> : dense_stream_kernel<J, false>);
+    if (tau)
+        k = seed ? (scales ? dense_stream_kernel<J, true, true, true> : dense_stream_kernel<J, false, true, true>)
+                 : (scales ? dense_stream_kernel<J, true, false, true> : dense_stream_kernel<J, false, false, true>);
     if (in_smem)
         CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)need));
     k<<<(unsigned)nblk, STREAM_T, in_smem ? need : 0, ctx->stream>>>(X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm,
                                                                    d_alph, K, Qd, ldq, col0, scratch,
-                                                                   in_smem ? 1 : 0, scales, seed, u0);
+                                                                   in_smem ? 1 : 0, scales, seed, u0, tau);
     KERNEL_CHECK(ctx);
     return GPFQ_OK;
 }
 
 // Dense layer by the streaming walk.  Device pointers.  Alphabets are walked one after another
 // (each needs its own residual); Qd: (n_alph, N0, ldq).  d_scales (nullable): (n_alph, nj) per-neuron scales of the shard.
-// Stochastic rounding (ctx->d_seeds): the shard's first neuron has unit id u0.
+// The same norms and, for the L1 penalty (common.cuh), tau[a * N0 + t] = lambda_a / nrm_t^2 for each of the call's n_alph
+// penalties: one table per alphabet, built in the same pass so that the walks read tau instead of dividing per step
+__global__ void __launch_bounds__(256) row_norms_l1_kernel(const float *__restrict__ X, const float *__restrict__ Xq,
+                                                           int64_t ldx, int64_t m, double *__restrict__ nrm,
+                                                           double *__restrict__ g1d, const double *__restrict__ lambdas,
+                                                           int n_alph, int64_t N0, double *__restrict__ tau) {
+    __shared__ double red[2][8];
+    const float *rq = Xq + (int64_t)blockIdx.x * ldx, *rx = X + (int64_t)blockIdx.x * ldx;
+    double s = 0.0, g = 0.0;
+    for (int64_t i = threadIdx.x; i < m; i += 256) {
+        const double v = (double)rq[i];
+        s = fma(v, v, s);
+        g = fma(v, (double)rx[i], g);
+    }
+    s = warp_sum(s);
+    g = warp_sum(g);
+    if ((threadIdx.x & 31) == 0) { red[0][threadIdx.x >> 5] = s; red[1][threadIdx.x >> 5] = g; }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double tot = 0.0, gt = 0.0;
+        for (int w = 0; w < 8; ++w) { tot += red[0][w]; gt += red[1][w]; }
+        const double nv = (double)(float)sqrt(tot);
+        nrm[blockIdx.x] = nv;
+        g1d[blockIdx.x] = gt;
+        for (int a = 0; a < n_alph; ++a) tau[(int64_t)a * N0 + blockIdx.x] = gpfq_l1_tau(lambdas[a], nv);
+    }
+}
+
+// Stochastic rounding (ctx->d_seeds): the shard's first neuron has unit id u0.  L1 penalty (ctx->d_l1): tau from a table.
 int dense_stream_path(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ldx, int64_t N0, int64_t m,
                       const float *W, int64_t ldw, int64_t j0, int64_t nj, const double *d_alph,
                       const int *h_koff, const int *h_flags, int n_alph, double *Qd, int64_t ldq, int64_t col0,
                       gpfq_stats *st, const double *d_scales, int64_t u0) {
-    double *nrm = nullptr;
+    double *nrm = nullptr, *tau = nullptr;
     GPFQ_TRY(gpfq_ws(ctx, WS_NRM, (size_t)2 * N0 * sizeof(double), (void **)&nrm));
     double *g1d = nrm + N0;
+    if (ctx->d_l1) GPFQ_TRY(gpfq_ws(ctx, WS_L1, (size_t)n_alph * N0 * sizeof(double), (void **)&tau));
     CUDA_TRY(ctx, gpfq_record(ctx, 2, ctx->stream));
-    row_norms_kernel<<<(unsigned)N0, 256, 0, ctx->stream>>>(X, Xq, ldx, m, nrm, g1d);
+    if (tau) row_norms_l1_kernel<<<(unsigned)N0, 256, 0, ctx->stream>>>(X, Xq, ldx, m, nrm, g1d, ctx->d_l1, n_alph, N0, tau);
+    else row_norms_kernel<<<(unsigned)N0, 256, 0, ctx->stream>>>(X, Xq, ldx, m, nrm, g1d);
     KERNEL_CHECK(ctx);
     const bool literal = ctx->stream_literal;
     if (m <= (int64_t)STREAM_T * 16) {
@@ -416,7 +455,7 @@ int dense_stream_path(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ld
             const int K = h_koff[a + 1] - h_koff[a];
             GPFQ_TRY(dispatch_stream_reg(ctx, epv, J, literal, vec, X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm, g1d, al, K,
                                          h_flags[a], Qd + (int64_t)a * N0 * ldq, ldq, col0, d_scales ? d_scales + a * nj : nullptr,
-                                         ctx->d_seeds ? ctx->d_seeds + a : nullptr, u0));
+                                         ctx->d_seeds ? ctx->d_seeds + a : nullptr, u0, tau ? tau + a * N0 : nullptr));
         }
     } else {
         // long sample axis: residual in shared memory (or an L2-resident scratch), literal arithmetic
@@ -430,9 +469,10 @@ int dense_stream_path(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ld
             double *Qa = Qd + (int64_t)a * N0 * ldq;
             const double *sa = d_scales ? d_scales + a * nj : nullptr;
             const uint64_t *sd = ctx->d_seeds ? ctx->d_seeds + a : nullptr;
-            if (J == 4) GPFQ_TRY(launch_stream<4>(ctx, X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm, al, K, Qa, ldq, col0, sa, sd, u0));
-            else if (J == 2) GPFQ_TRY(launch_stream<2>(ctx, X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm, al, K, Qa, ldq, col0, sa, sd, u0));
-            else GPFQ_TRY(launch_stream<1>(ctx, X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm, al, K, Qa, ldq, col0, sa, sd, u0));
+            const double *ta = tau ? tau + a * N0 : nullptr;
+            if (J == 4) GPFQ_TRY(launch_stream<4>(ctx, X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm, al, K, Qa, ldq, col0, sa, sd, u0, ta));
+            else if (J == 2) GPFQ_TRY(launch_stream<2>(ctx, X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm, al, K, Qa, ldq, col0, sa, sd, u0, ta));
+            else GPFQ_TRY(launch_stream<1>(ctx, X, Xq, ldx, N0, m, W, ldw, j0, nj, nrm, al, K, Qa, ldq, col0, sa, sd, u0, ta));
         }
     }
     CUDA_TRY(ctx, gpfq_record(ctx, 3, ctx->stream));

@@ -33,6 +33,7 @@
 //   warp 6     producer of a block's inputs, one block ahead: the P rows and fp32 weights of the CTA's 128 neurons (three TMA boxes,
 //              128B swizzle: thread j reads row j conflict-free) and the per-block table (TabA), 2 stages
 #include <algorithm>
+#include <cfloat>
 
 #include "slgemm_i8.cuh"
 #include "sweep_tc.cuh"
@@ -97,9 +98,11 @@ __device__ __forceinline__ void tmem_ld_5x16(uint32_t taddr, uint32_t (&v)[S][16
 // SCALED: the neuron's levels are fl(s alph[k]) (per-channel alphabets; a = fl(s alph[K - 1]), `alph` the base alphabet); a neuron
 // with s = 0 decides the literal 0 everywhere (its levels are all zero) and never reaches the divisions by a.
 // STOCH: stochastic rounding (common.cuh) with the draw of step t0 + t from the neuron's unit key.
-template <bool SCALED, bool STOCH = false>
+// L1: the value of step t is shrunk by its tau (lane t's tau_l: the whole warp replays).
+template <bool SCALED, bool STOCH = false, bool L1 = false>
 static __device__ __noinline__ void replay_block(unsigned char *dset, const unsigned char *wset, int j, const TabA *tab, double a,
-                                                 int8_t *qcol, const double *alph, int K, double s, uint64_t key = 0, int64_t t0 = 0) {
+                                                 int8_t *qcol, const double *alph, int K, double s, uint64_t key = 0, int64_t t0 = 0,
+                                                 double tau_l = 0.0) {
     // K == 3: the ternary scan with the levels in registers; else the windowed scan of the equispaced levels (common.cuh)
     const bool zero = SCALED && !(a > 0.0);
     const double inv_step = zero ? 0.0 : (SCALED ? gpfq_inv_step_s(alph, K, 1, s) : 0.5 * (double)(K - 1) / a);
@@ -109,6 +112,7 @@ static __device__ __noinline__ void replay_block(unsigned char *dset, const unsi
         const double d0 = *dptr(t);
         const double wv = (double)reinterpret_cast<const float *>(wset + sw128(j, t >> 2))[t & 3];
         const double nrm = tab->nrm[t];
+        const double tau = L1 ? __shfl_sync(0xffffffffu, tau_l, t) : 0.0;
         double q = 0.0;
         if (!(nrm < GPFQ_DEAD_NORM)) {
             double v = wv;
@@ -118,6 +122,7 @@ static __device__ __noinline__ void replay_block(unsigned char *dset, const unsi
                 const double e = fma(-q0, tab->den[t], num);
                 v = fma(e, rinv, q0);
             }
+            if (L1) v = gpfq_shrink(v, tau);
             if (zero) q = 0.0;
             else if (STOCH && K == 3) q = gpfq_stoc_round_ternary(v, a, gpfq_draw(key, t0 + t));
             else if (STOCH) q = gpfq_stoc_round_eq<SCALED>(v, alph, K, inv_step, s, gpfq_draw(key, t0 + t));
@@ -144,12 +149,20 @@ static __device__ __noinline__ void replay_block(unsigned char *dset, const unsi
 // levels: the grid position kr = (p + a) / step splits into the interval k = floor(kr) and the fraction f = kr - k; the upper level is
 // taken when r < f, and a step is flagged when f lies within 2^-30 of 0, 1 or r.  The non-finite / huge and :86 flags are those of
 // the nearest walk; a flagged warp replays its block with the literal stoc_round.
-template <bool TERN, bool SCALED = false, bool STOCH = false>
+//
+// L1 (the penalty lambda = *lambdas, DESIGN.md 5.7): lane t of a walker warp forms tau of the block's direction t once per block
+// (one division per lane and block), and step t takes it by a shuffle, off the chain.  Ternary: the shrink moves the thresholds
+// out by tau -- q = a iff p > r a + tau, -a iff p <= (r - 1) a - tau, with r = 1/2 for nearest rounding -- and a step is flagged
+// when p lies within 2^-30 (a + tau) of either.  More levels: the grid position is taken from the shrunk p; the tie / fraction flags
+// are those above, and a step whose tau exceeds 2^16 steps is flagged unless |p| < tau (1 - 2^-40), where the shrink gives the
+// literal 0 either way (a huge tau would otherwise carry its rounding into the grid position).
+template <bool TERN, bool SCALED = false, bool STOCH = false, bool L1 = false>
 __global__ void __launch_bounds__(THREADS, 1)
 sweep_tc_kernel(const __grid_constant__ CUtensorMap mapP, const __grid_constant__ CUtensorMap mapW, const TabA *__restrict__ tabs,
                 const int8_t *__restrict__ g2s, int kbr, int64_t tb, int64_t te, int row0, int64_t nj, int8_t *__restrict__ Kq,
                 int64_t krows, int64_t krow0, double a_base, const double *__restrict__ levels, int K,
-                const double *__restrict__ scales = nullptr, const uint64_t *__restrict__ seeds = nullptr, int64_t u0 = 0) {
+                const double *__restrict__ scales = nullptr, const uint64_t *__restrict__ seeds = nullptr, int64_t u0 = 0,
+                const double *__restrict__ lambdas = nullptr) {
     using namespace i8g;
     extern __shared__ unsigned char stc_smem_raw[];
     // (offset arithmetic on the array itself: the compiler keeps the shared address space, LDS / STS instead of generic accesses)
@@ -203,6 +216,7 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap mapP, const __grid_constant_
         const double km1 = (double)(K - 1), step = 2.0 * a / km1, cmid = 0.5 * km1, magic = 6755399441055744.0;
         const uint32_t lane_field = (uint32_t)(warp * 32) << 16;
         const uint64_t key = STOCH ? gpfq_unit_key(seeds[0], u0 + jg) : 0;
+        const double lam = L1 ? lambdas[0] : 0.0, inv_st = SCALED ? 0.5 * inv_hu : cmid / a;   // (one step = 2 h)
         for (int b = 0; b < nblk; ++b) {
             const int buf = b & 1;
             const int64_t t0 = tb + (int64_t)b * NB;
@@ -251,6 +265,7 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap mapP, const __grid_constant_
             int flag = 0;
             uint32_t m_near = 0xffffffffu, m_big = 0u, m_perp = 0xffffffffu;
             double m_thr = 1e300;   // STOCH ternary: the least |p - threshold| / a of the block
+            const double tau_l = L1 ? gpfq_l1_tau(lam, tab->nrm[lane]) : 0.0;   // tau of the block's direction `lane`
 #pragma unroll
             for (int t = 0; t < NB; ++t) {
                 float4 w4;
@@ -259,7 +274,46 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap mapP, const __grid_constant_
                 const double ri = tab->rinv[t];
                 const double num = fma(wv, tab->g1dd[t], d[t]);
                 double q;
-                if (TERN && STOCH) {
+                if (TERN && L1) {
+                    const double p = num * ri;
+                    const double tau = __shfl_sync(0xffffffffu, tau_l, t);
+                    const double rr = STOCH ? gpfq_draw(key, t0 + t) : 0.5;
+                    // the step's thresholds and flag window, off the chain (clamped: tau = inf flags nothing, decides 0)
+                    const double up_t = fmin(fma(rr, a, tau), DBL_MAX), dn_t = fmax(fma(rr - 1.0, a, -tau), -DBL_MAX);
+                    const double band = 0x1p-30 * fmin(a + tau, DBL_MAX);
+                    const bool up = p > up_t, dn = p <= dn_t;
+                    q = up ? a : (dn ? -a : 0.0);
+                    flag |= (int)!(fmin(fabs(p - up_t), fabs(p - dn_t)) > band);
+                    const uint32_t hp = (uint32_t)__double2hiint(p) & 0x7fffffffu;
+                    m_big = max(m_big, hp);
+                    m_perp = min(m_perp, ((uint32_t)__double2hiint(d[t]) & 0x7fffffffu) | (uint32_t)tab->deadm[t]);
+                    pk[t >> 2] |= (up ? 2u : (dn ? 0xfeu : 0u)) << (8 * (t & 3));
+                } else if (L1) {
+                    const double p = num * ri;
+                    const double tau = __shfl_sync(0xffffffffu, tau_l, t);
+                    const double ps = fabs(p) <= tau ? 0.0 : p - copysign(tau, p);   // the shrink of p
+                    const double kr = fma(ps, inv_st, cmid);
+                    double r;
+                    int fl;
+                    if (STOCH) {
+                        const double rr = gpfq_draw(key, t0 + t);
+                        const double k0 = fmin(fmax(floor(kr), 0.0), km1 - 1.0);
+                        const double f = kr - k0;
+                        r = rr < f ? k0 + 1.0 : k0;
+                        fl = (int)!(fabs(f) > 0x1p-30) | (int)!(fabs(f - 1.0) > 0x1p-30) | (int)!(fabs(f - rr) > 0x1p-30);
+                    } else {
+                        const double r0 = (kr + magic) - magic;
+                        r = fmin(fmax(r0, 0.0), km1);
+                        fl = (int)!(fabs(kr - r0) < 0.5 - 0x1p-30);
+                    }
+                    const bool live = ri != 0.0;
+                    q = live ? fma(r, step, -a) : 0.0;
+                    fl |= (int)!(fabs(kr) < 0x1p40) | (int)(fabs(d[t]) < GPFQ_PERP_DOT) |
+                          ((int)(tau * inv_st >= 0x1p16) & (int)!(fabs(p) < tau * (1.0 - 0x1p-40)));
+                    flag |= fl & (int)live;
+                    const int kq = live ? __double2int_rn(fma(r, 2.0, -km1)) : 0;
+                    pk[t >> 2] |= ((uint32_t)kq & 0xffu) << (8 * (t & 3));
+                } else if (TERN && STOCH) {
                     const double p = num * ri;
                     const double rr = gpfq_draw(key, t0 + t);
                     const double ra = rr * a, rm = (rr - 1.0) * a;       // the thresholds of this step, off the chain
@@ -316,7 +370,8 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap mapP, const __grid_constant_
                 // late steps, 2.4 us per block instead of ~1.)
                 if (kbr == -1 - t) asm volatile("trap;\n");
             }
-            if (TERN && STOCH) flag = (int)!(m_thr > 0x1p-30 * a) | (int)(m_big >= big_hi) | (int)(m_perp <= perp_hi);
+            if (TERN && L1) flag |= (int)(m_big >= big_hi) | (int)(m_perp <= perp_hi);
+            else if (TERN && STOCH) flag = (int)!(m_thr > 0x1p-30 * a) | (int)(m_big >= big_hi) | (int)(m_perp <= perp_hi);
             else if (TERN) flag = (int)(m_near <= 2u) | (int)(m_big >= big_hi) | (int)(m_perp <= perp_hi);
             if (SCALED && zero) {
                 flag = 0;
@@ -325,7 +380,8 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap mapP, const __grid_constant_
             }
             if (__any_sync(0xffffffffu, flag != 0 && valid)) {   // (rows beyond nj hold zeros: they would trip the :86 guard at every step)
                 int8_t *qcol = reinterpret_cast<int8_t *>(smem + OFF_Q) + j;
-                replay_block<SCALED, STOCH>(dset, wset, j, tab, a, qcol, alph, K, s_u, key, t0);
+                if (L1) replay_block<SCALED, STOCH, true>(dset, wset, j, tab, a, qcol, alph, K, s_u, key, t0, tau_l);
+                else replay_block<SCALED, STOCH>(dset, wset, j, tab, a, qcol, alph, K, s_u, key, t0);
 #pragma unroll
                 for (int i = 0; i < NB / 4; ++i) {
                     uint32_t w4 = 0u;
@@ -726,17 +782,27 @@ int sweep_tc_range(gpfq_ctx *ctx, const TcTables &tab, int64_t tb, int64_t te, i
     if (tb % tab.R || te - tb > tab.R || te <= tb || row0 % NT || row0 + ceil_div64(nj, NT) * NT > tab.rowsP || !Kq || K < 2 || K > 128)
         return gpfq_fail(ctx, GPFQ_ERR_ARG, "sweep_tc: a range starts at a multiple of %lld directions", (long long)tab.R);
     const dim3 grid((unsigned)ceil_div64(nj, NT));
-    if (const uint64_t *seeds = ctx->d_seeds) {   // stochastic rounding: one alphabet on this path, seeds[0]
+    if (const double *lambdas = ctx->d_l1) {   // L1 penalty: one alphabet on this path, lambdas[0]
+        const uint64_t *seeds = ctx->d_seeds;
+        auto k = K == 3 ? (scales ? sweep_tc_kernel<true, true, false, true> : sweep_tc_kernel<true, false, false, true>)
+                        : (scales ? sweep_tc_kernel<false, true, false, true> : sweep_tc_kernel<false, false, false, true>);
+        if (seeds)
+            k = K == 3 ? (scales ? sweep_tc_kernel<true, true, true, true> : sweep_tc_kernel<true, false, true, true>)
+                       : (scales ? sweep_tc_kernel<false, true, true, true> : sweep_tc_kernel<false, false, true, true>);
+        CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM));
+        k<<<grid, THREADS, SMEM, ctx->stream>>>(tab.mapP, tab.mapW, tab.tabs, tab.g2s, (int)(tab.R / KB), tb, te, (int)row0, nj, Kq, krows, krow0,
+                                                a, levels, K, scales, seeds, u0, lambdas);
+    } else if (const uint64_t *seeds = ctx->d_seeds) {   // stochastic rounding: one alphabet on this path, seeds[0]
         auto k = K == 3 ? (scales ? sweep_tc_kernel<true, true, true> : sweep_tc_kernel<true, false, true>)
                         : (scales ? sweep_tc_kernel<false, true, true> : sweep_tc_kernel<false, false, true>);
         CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM));
         k<<<grid, THREADS, SMEM, ctx->stream>>>(tab.mapP, tab.mapW, tab.tabs, tab.g2s, (int)(tab.R / KB), tb, te, (int)row0, nj, Kq, krows, krow0,
-                                                a, levels, K, scales, seeds, u0);
+                                                a, levels, K, scales, seeds, u0, nullptr);
     } else if (scales) {
         auto k = K == 3 ? sweep_tc_kernel<true, true> : sweep_tc_kernel<false, true>;
         CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM));
         k<<<grid, THREADS, SMEM, ctx->stream>>>(tab.mapP, tab.mapW, tab.tabs, tab.g2s, (int)(tab.R / KB), tb, te, (int)row0, nj, Kq, krows, krow0,
-                                                a, levels, K, scales, nullptr, 0);
+                                                a, levels, K, scales, nullptr, 0, nullptr);
     } else if (K == 3) {
         CUDA_TRY(ctx, cudaFuncSetAttribute(sweep_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM));
         sweep_tc_kernel<true><<<grid, THREADS, SMEM, ctx->stream>>>(tab.mapP, tab.mapW, tab.tabs, tab.g2s, (int)(tab.R / KB), tb, te, (int)row0, nj,

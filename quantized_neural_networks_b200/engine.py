@@ -78,6 +78,27 @@ def _seed_args(seeds, n_alph):
     return out
 
 
+def _l1_args(l1_penalty, n_alph):
+    """L1 penalty -> None (off) or a list of n_alph floats, each finite and >= 0.  Accepts None, one number (used by every
+    alphabet) or a sequence of n_alph numbers."""
+    if l1_penalty is None:
+        return None
+    if isinstance(l1_penalty, numbers.Real) and not isinstance(l1_penalty, bool):
+        vals = [l1_penalty] * n_alph
+    elif isinstance(l1_penalty, (list, tuple, np.ndarray)):
+        vals = list(np.asarray(l1_penalty, dtype=object).reshape(-1)) if isinstance(l1_penalty, np.ndarray) else list(l1_penalty)
+        if len(vals) != n_alph:
+            raise ValueError(f"l1_penalty: {len(vals)} penalties for {n_alph} alphabets")
+    else:
+        raise ValueError(f"l1_penalty: expected None, a number or a sequence of {n_alph} numbers, got {type(l1_penalty).__name__}")
+    out = []
+    for v in vals:
+        if not isinstance(v, numbers.Real) or isinstance(v, bool) or not np.isfinite(float(v)) or float(v) < 0:
+            raise ValueError(f"l1_penalty: {v!r} is not a finite number >= 0")
+        out.append(float(v))
+    return out
+
+
 def _dptr(a):
     return a.ctypes.data_as(POINTER(c_double))
 
@@ -145,6 +166,20 @@ class GpfqEngine:
         finally:
             self._lib.gpfq_set_rounding(self._ctx, _lib.ROUND_NEAREST, None, 0)
 
+    @contextlib.contextmanager
+    def _penalty(self, l1_penalty, n_alph):
+        """The L1 penalty (sparse GPFQ) for the calls inside (None: off); off again afterwards."""
+        lam = _l1_args(l1_penalty, n_alph)
+        if lam is None:
+            yield
+            return
+        arr = (c_double * len(lam))(*lam)
+        self._check(self._lib.gpfq_set_l1_penalty(self._ctx, arr, len(lam)))
+        try:
+            yield
+        finally:
+            self._lib.gpfq_set_l1_penalty(self._ctx, None, 0)
+
     def _bind_stream(self, dev):
         """Device-tensor calls launch on torch's CURRENT stream: the tensors were produced there, so this is what
         orders our kernels after their producers (and lets torch.cuda.Event brackets time them).  Host-array
@@ -184,13 +219,17 @@ class GpfqEngine:
         return x.ctypes.data, (x.strides[0] // x.itemsize if x.shape[0] > 1 else x.shape[1])
 
     # -- Dense ----------------------------------------------------------------------------------
-    def dense_layer(self, X, Xq, W, alphabets, j0=0, j1=None, method="auto", out=None, sync=True, scales=None, seeds=None):
+    def dense_layer(self, X, Xq, W, alphabets, j0=0, j1=None, method="auto", out=None, sync=True, scales=None, seeds=None,
+                    l1_penalty=None):
         """Quantize neurons j0..j1-1 of a Dense layer.  X, Xq: (N0, m) fp32 feature-major (Xq may be
         None or X itself for the first layer); W: (N0, N1) fp32.  Returns Q fp64 (N0, N1) -- or
         (n_alphabets, N0, N1) when a list of alphabets is given -- with only the shard's columns written.
         `scales` (per-channel alphabets): (N1,) or (n_alphabets, N1), finite and >= 0; neuron j then walks with the levels
         fl64(scales[j] * alphabet[k]).  `seeds`: None rounds to the nearest level (the reference); an int or one int per alphabet in
-        [0, 2^64) rounds stochastically (SPFQ, include/gpfq.h), neuron j drawing as unit j whatever the shard."""
+        [0, 2^64) rounds stochastically (SPFQ, include/gpfq.h), neuron j drawing as unit j whatever the shard.  `l1_penalty`
+        (sparse GPFQ): None walks without it; a number or one number per alphabet, finite and >= 0, soft-thresholds the value of
+        every greedy step by lambda / nrm^2 before it is quantized (include/gpfq.h; 0.0 runs the penalty's kernels and gives the
+        weights of the call without it)."""
         flat, K, n_alph, als = _alph_args(alphabets)
         single = isinstance(alphabets, np.ndarray) and alphabets.ndim == 1
         X = self._f32(X, "X")
@@ -235,7 +274,7 @@ class GpfqEngine:
         args = (self._ctx, c_void_p(px), c_void_p(pq), ldx, N0, m, c_void_p(pw), ldw, N1, int(j0), j1,
                 flat.ctypes.data_as(POINTER(c_double)), K.ctypes.data_as(POINTER(c_int32)), n_alph, c_void_p(pout), N1, flags,
                 byref(st))
-        with self._rounding(seeds, n_alph):
+        with self._rounding(seeds, n_alph), self._penalty(l1_penalty, n_alph):
             rc = self._lib.gpfq_dense_layer(*args) if sc is None else self._lib.gpfq_dense_layer_scaled(*args, _dptr(sc))
         self._check(rc)
         self.last_stats = st.as_dict()
@@ -281,11 +320,12 @@ class GpfqEngine:
         self._check(rc)
         return G1, G2
 
-    def dense_layer_from_gram(self, G1, G2, W, alphabets, j0=0, j1=None, out=None, sync=True, scales=None, seeds=None):
+    def dense_layer_from_gram(self, G1, G2, W, alphabets, j0=0, j1=None, out=None, sync=True, scales=None, seeds=None,
+                              l1_penalty=None):
         """Sweep stage of a Dense layer from (N0, N0) fp64 Gram matrices on the device (CUDA tensors; G1 None or G2
         itself for the first layer): what every rank of a sample-split job runs after the all-reduce of the partial
-        Grams.  W: (N0, N1) fp32 NumPy array or CUDA tensor; the result follows W's kind.  `scales` and `seeds` as in
-        `dense_layer`."""
+        Grams.  W: (N0, N1) fp32 NumPy array or CUDA tensor; the result follows W's kind.  `scales`, `seeds` and `l1_penalty`
+        as in `dense_layer`."""
         flat, K, n_alph, als = _alph_args(alphabets)
         single = isinstance(alphabets, np.ndarray) and alphabets.ndim == 1
         if not _is_torch(G2) or G2.dtype != torch.float64 or not G2.is_cuda or not G2.is_contiguous():
@@ -324,7 +364,7 @@ class GpfqEngine:
         args = (self._ctx, c_void_p(None if same else G1.data_ptr()), c_void_p(G2.data_ptr()), N0, c_void_p(pw), ldw, N1,
                 int(j0), j1, flat.ctypes.data_as(POINTER(c_double)), K.ctypes.data_as(POINTER(c_int32)), n_alph,
                 c_void_p(pout), N1, flags, byref(st))
-        with self._rounding(seeds, n_alph):
+        with self._rounding(seeds, n_alph), self._penalty(l1_penalty, n_alph):
             rc = (self._lib.gpfq_dense_layer_from_gram(*args) if sc is None
                   else self._lib.gpfq_dense_layer_from_gram_scaled(*args, _dptr(sc)))
         self._check(rc)
@@ -332,12 +372,14 @@ class GpfqEngine:
         return out[0] if single else out
 
     # -- Conv -----------------------------------------------------------------------------------
-    def conv_channels(self, Xp, Xqp, W, alphabets, c0=0, n_channels=None, out=None, sync=True, scales=None, seeds=None):
+    def conv_channels(self, Xp, Xqp, W, alphabets, c0=0, n_channels=None, out=None, sync=True, scales=None, seeds=None,
+                      l1_penalty=None):
         """Quantize channels c0..c0+n_channels-1 of a (kh, kw, C, F) kernel from per-channel patch
         matrices.  Xp/Xqp: sequences (len n_channels) of (kh*kw, n_patches) fp32 arrays/tensors, or one
         (n_channels, kh*kw, n_patches) array; Xqp None => first conv layer (X == Xq).  `scales` (per-channel alphabets):
         (C, F) or (n_alphabets, C, F), finite and >= 0; the slice W[:, :, c, f] walks with fl64(scales[c, f] * alphabet[k]).
-        `seeds` as in `dense_layer`; the slice W[:, :, c, f] draws as unit c * F + f, tap r * kw + col as step."""
+        `seeds` as in `dense_layer`; the slice W[:, :, c, f] draws as unit c * F + f, tap r * kw + col as step.  `l1_penalty` as
+        in `dense_layer`."""
         flat, K, n_alph, als = _alph_args(alphabets)
         single = isinstance(alphabets, np.ndarray) and alphabets.ndim == 1
         W = self._f32(W, "W")
@@ -381,7 +423,7 @@ class GpfqEngine:
         st = _lib.GpfqStats()
         args = (self._ctx, PX, PQ, n, kk, c_void_p(ptr(W)), C, F, int(c0), n_channels, flat.ctypes.data_as(POINTER(c_double)),
                 K.ctypes.data_as(POINTER(c_int32)), n_alph, c_void_p(pout), flags, byref(st))
-        with self._rounding(seeds, n_alph):
+        with self._rounding(seeds, n_alph), self._penalty(l1_penalty, n_alph):
             rc = self._lib.gpfq_conv_channels(*args) if sc is None else self._lib.gpfq_conv_channels_scaled(*args, _dptr(sc))
         self._check(rc)
         self.last_stats = st.as_dict()
@@ -397,12 +439,12 @@ class GpfqEngine:
         return groups
 
     def conv_layer_nhwc(self, act, actq, W, alphabets, strides=(1, 1), padding="SAME", rate=(1, 1), c0=0,
-                        n_channels=None, out=None, sync=True, groups=1, scales=None, seeds=None):
+                        n_channels=None, out=None, sync=True, groups=1, scales=None, seeds=None, l1_penalty=None):
         """Quantize a Conv2D kernel straight from the NHWC activations (on-device patch extraction).  With `groups` > 1, W is the
         (kh, kw, C / groups, F) kernel of a grouped Conv2D: input channel c is walked against the F / groups filters of its group
         c // (C / groups); c0 / n_channels index input channels.  The result has W's shape.  `scales` (per-channel alphabets):
         (C / groups, F) or (n_alphabets, C / groups, F), indexed like W's last two axes.  `seeds` as in `dense_layer`; the slice
-        W[:, :, ci, f] draws as unit ci * F + f."""
+        W[:, :, ci, f] draws as unit ci * F + f.  `l1_penalty` as in `dense_layer`."""
         flat, K, n_alph, als = _alph_args(alphabets)
         single = isinstance(alphabets, np.ndarray) and alphabets.ndim == 1
         W = self._f32(W, "W")
@@ -447,7 +489,7 @@ class GpfqEngine:
                 int(rate[0]), int(rate[1]), 1 if str(padding).upper() == "SAME" else 0, c_void_p(ptr(W)), F, int(c0), n_channels,
                 flat.ctypes.data_as(POINTER(c_double)), K.ctypes.data_as(POINTER(c_int32)), n_alph, c_void_p(pout), flags,
                 byref(st))
-        with self._rounding(seeds, n_alph):
+        with self._rounding(seeds, n_alph), self._penalty(l1_penalty, n_alph):
             if sc is not None:
                 rc = self._lib.gpfq_conv_layer_nhwc_scaled(*args, groups, _dptr(sc))
             else:
@@ -493,12 +535,12 @@ class GpfqEngine:
         return gram
 
     def conv_layer_from_gram(self, gram, W, alphabets, c0=0, n_channels=None, out=None, sync=True, groups=1, scales=None,
-                             seeds=None):
+                             seeds=None, l1_penalty=None):
         """Walks of every filter of channels c0..c0+n_channels-1 from per-channel Gram matrices on the device
         (`conv_gram_nhwc`, summed over the ranks of an image-split job).  W: (kh, kw, C, F) NumPy array or CUDA tensor; with
         `groups` > 1 the (kh, kw, C / groups, F) kernel of a grouped Conv2D, each input channel walked against the F / groups
-        filters of its group (c0 / n_channels index input channels, as in the Gram stage).  `scales` and `seeds` as in
-        `conv_layer_nhwc`."""
+        filters of its group (c0 / n_channels index input channels, as in the Gram stage).  `scales`, `seeds` and `l1_penalty` as
+        in `conv_layer_nhwc`."""
         flat, K, n_alph, als = _alph_args(alphabets)
         single = isinstance(alphabets, np.ndarray) and alphabets.ndim == 1
         W = self._f32(W, "W")
@@ -529,7 +571,7 @@ class GpfqEngine:
         st = _lib.GpfqStats()
         args = (self._ctx, c_void_p(gram.data_ptr()), kk, c_void_p(pw), C, F, int(c0), n_channels,
                 flat.ctypes.data_as(POINTER(c_double)), K.ctypes.data_as(POINTER(c_int32)), n_alph, c_void_p(pout), flags, byref(st))
-        with self._rounding(seeds, n_alph):
+        with self._rounding(seeds, n_alph), self._penalty(l1_penalty, n_alph):
             if sc is not None:
                 rc = self._lib.gpfq_conv_layer_from_gram_scaled(*args, groups, _dptr(sc))
             else:

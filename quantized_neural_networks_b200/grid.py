@@ -64,15 +64,17 @@ class QuantizedCNNGrid:
 
     def __init__(self, network, batch_size, get_data, bits_list, alphabet_scalars, logger=None, is_quantize_conv2d=True,
                  device: int = 0, data_set: str = "synthetic", q_train_size=None, *, alphabet_scope: str = "layer",
-                 rounding: str = "nearest", seed: int = 0):
+                 rounding: str = "nearest", seed: int = 0, l1_penalty=None):
         """`alphabet_scope` ("layer" | "channel") as in `QuantizedCNN`: with "channel" every grid point quantizes each output
         channel against its own radius, and `msq_networks()` rounds with the same per-channel levels.  `rounding` as in
         `QuantizedCNN`; with "stochastic", grid point g (in the order of `self.grid`) is the run of `QuantizedCNN(..., seed=seed + g)`,
-        and `msq_networks()` rounds stochastically with the same layer seeds."""
+        and `msq_networks()` rounds stochastically with the same layer seeds.  `l1_penalty` as in `QuantizedCNN`, the same for every
+        grid point (each lock-step call passes one lambda per batched alphabet; the MSQ baselines have no penalty)."""
         self.grid = list(product(bits_list, alphabet_scalars))          # the order of itertools.product in the driver
         self.points = [QuantizedCNN(network, batch_size, get_data, logger=logger, bits=b, alphabet_scalar=c,
                                     is_quantize_conv2d=is_quantize_conv2d, device=device, alphabet_scope=alphabet_scope,
-                                    rounding=rounding, seed=(int(seed) + g) % (1 << 64) if rounding == "stochastic" else seed)
+                                    rounding=rounding, seed=(int(seed) + g) % (1 << 64) if rounding == "stochastic" else seed,
+                                    l1_penalty=l1_penalty)
                        for g, (b, c) in enumerate(self.grid)]
         self.trained_net, self.logger, self.device = network, logger, device
         self.is_quantize_conv2d = is_quantize_conv2d
@@ -126,6 +128,8 @@ class QuantizedCNNGrid:
                 scaled = {} if levels[0][1] is None else {"scales": np.stack([levels[g][1] for g in members])}
                 if self.points[0].rounding == "stochastic":
                     scaled["seeds"] = [layer_seed(self.points[g].seed, layer_idx) for g in members]
+                if self.points[0]._layer_l1(layer_idx) is not None:
+                    scaled["l1_penalty"] = [self.points[g]._layer_l1(layer_idx) for g in members]
                 if dense:
                     Q = eng.dense_layer(Xd, Xqd, Wd, A, **scaled)
                 else:

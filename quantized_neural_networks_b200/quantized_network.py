@@ -17,6 +17,7 @@ There is no CPU fallback for the hot path: without libgpfq.so and an sm_100 GPU 
 from __future__ import annotations
 
 import numbers
+from collections.abc import Mapping
 from time import time
 from typing import List
 
@@ -106,6 +107,31 @@ def layer_seed(seed: int, layer_idx: int) -> int:
     return splitmix64(splitmix64(int(seed) & _MASK64) ^ int(layer_idx))
 
 
+def _check_l1_penalty(l1_penalty, alphabet):
+    """The `l1_penalty` argument of the mirror classes, validated: None, a float, or a dict {layer_idx: float}."""
+    if l1_penalty is None:
+        return None
+
+    def one(v, what):
+        if isinstance(v, bool) or not isinstance(v, numbers.Real) or not np.isfinite(float(v)) or float(v) < 0:
+            raise ValueError(f"l1_penalty{what} must be a finite number >= 0, not {v!r}")
+        return float(v)
+
+    if isinstance(l1_penalty, Mapping):
+        out = {}
+        for k, v in l1_penalty.items():
+            if isinstance(k, bool) or not isinstance(k, numbers.Integral):
+                raise ValueError(f"l1_penalty: layer index {k!r} is not an int")
+            out[int(k)] = one(v, f"[{k}]")
+        lams = out
+    else:
+        lams = one(l1_penalty, "")
+    if not np.any(np.asarray(alphabet) == 0.0):
+        raise ValueError(f"l1_penalty needs an alphabet with a 0 level, and linspace(-1, 1, {len(alphabet)}) has none: soft "
+                         "thresholding only makes zeros with an odd number of levels K, bits = log2(2K + 1) (log2(3), log2(5), ...)")
+    return lams
+
+
 class QuantizedNeuralNetwork:
     def __init__(
         self,
@@ -125,6 +151,7 @@ class QuantizedNeuralNetwork:
         alphabet_scope: str = "layer",
         rounding: str = "nearest",
         seed: int = 0,
+        l1_penalty=None,
     ):
         """Wrapper of a Keras-style model that quantizes the weights of its Dense layers with GPFQ.
 
@@ -141,6 +168,10 @@ class QuantizedNeuralNetwork:
         `rounding` ("nearest" | "stochastic"): "nearest" (the reference) rounds every greedy step to the nearest level;
         "stochastic" is SPFQ, unbiased stochastic rounding between the two bracketing levels, reproducible from `seed` (layer
         `layer_idx` draws with `layer_seed(seed, layer_idx)`, whatever the device count, shards or conv path).
+        `l1_penalty` (sparse GPFQ): None (the reference) or a finite lambda >= 0 for every quantized layer, or a mapping
+        {layer_idx: lambda} (layers not in it walk without the penalty).  Every greedy step's value is then soft-thresholded by
+        lambda / nrm^2 before it is quantized (include/gpfq.h), so the layer is pruned and quantized in one pass; the alphabet
+        needs a 0 level (odd K: bits = log2(2K + 1)).
         """
         self.get_data = get_data
         self.trained_net = network
@@ -156,9 +187,10 @@ class QuantizedNeuralNetwork:
         self.alphabet = linspace(-1, 1, num=int(round(2 ** (bits))))
         self.logger = logger
         self.ignore_layers = ignore_layers
-        self._init_device(device, method, shard, gram_split, alphabet_scope, rounding, seed)
+        self._init_device(device, method, shard, gram_split, alphabet_scope, rounding, seed, l1_penalty)
 
-    def _init_device(self, device, method, shard, gram_split="auto", alphabet_scope="layer", rounding="nearest", seed=0):
+    def _init_device(self, device, method, shard, gram_split="auto", alphabet_scope="layer", rounding="nearest", seed=0,
+                     l1_penalty=None):
         if int(round(2 ** self.bits)) > 64:   # GPFQ_MAX_K of include/gpfq.h: the kernels keep an alphabet in shared memory
             raise ValueError(f"bits={self.bits}: the CUDA path supports alphabets of up to 64 levels (bits <= 6); the reference "
                              "accepts any `bits`, see INTEGRATION.md")
@@ -172,6 +204,7 @@ class QuantizedNeuralNetwork:
         if isinstance(seed, bool) or not isinstance(seed, numbers.Integral) or not 0 <= int(seed) < 1 << 64:
             raise ValueError(f"seed must be an int in [0, 2^64), not {seed!r}")
         self.rounding, self.seed = rounding, int(seed)
+        self.l1_penalty = _check_l1_penalty(l1_penalty, self.alphabet)
         self.device, self.method, self.gram_split = device, method, gram_split
         self.shard = tuple(shard) if shard else (0, 1)
         self.layer_stats = {}
@@ -269,6 +302,17 @@ class QuantizedNeuralNetwork:
         """Engine keyword of layer `layer_idx`: nothing for nearest rounding (the call keeps its signature), else its seed."""
         return {"seeds": layer_seed(self.seed, layer_idx)} if self.rounding == "stochastic" else {}
 
+    def _penalty(self, layer_idx):
+        """Engine keyword of layer `layer_idx`: nothing without a penalty (the call keeps its signature), else its lambda."""
+        lam = self._layer_l1(layer_idx)
+        return {} if lam is None else {"l1_penalty": lam}
+
+    def _layer_l1(self, layer_idx):
+        """The L1 penalty of layer `layer_idx`, or None."""
+        if isinstance(self.l1_penalty, dict):
+            return self.l1_penalty.get(layer_idx)
+        return self.l1_penalty
+
     def _nccl_job(self):
         """True when this object is one rank of a torch.distributed job on GPUs (NCCL): layer inputs are then replicated
         through `replicate_leading_axis` (1 / world of the bytes over each rank's host link + one NVLink all-gather)."""
@@ -334,6 +378,7 @@ class QuantizedNeuralNetwork:
         layer_alphabet, scales = self._levels(W)
         scaled = {"scales": scales} if scales is not None else {}   # the per-layer call keeps its signature
         scaled.update(self._seeds(layer_idx))
+        scaled.update(self._penalty(layer_idx))
 
         self._log("\tQuantizing neurons (on the GPU)...")
         tic = time()
@@ -396,12 +441,13 @@ class QuantizedCNN(QuantizedNeuralNetwork):
         alphabet_scope: str = "layer",
         rounding: str = "nearest",
         seed: int = 0,
+        l1_penalty=None,
     ):
         """Dense + Conv2D / DepthwiseConv2D quantization (quantized_network.py:594-650).  Like the reference this
         constructor does not take `ignore_layers`.  `conv_path="nhwc"` hands the layer's activation tensors to
         CUDA (patches are extracted on the device); `"patches"` builds the per-channel patch matrices on the host
-        exactly as `_build_patch_array` does and hands those over.  `alphabet_scope`, `rounding` and `seed` as in
-        `QuantizedNeuralNetwork`."""
+        exactly as `_build_patch_array` does and hands those over.  `alphabet_scope`, `rounding`, `seed` and `l1_penalty` as
+        in `QuantizedNeuralNetwork`."""
         self.get_data = get_data
         self.trained_net = network
         self.quantized_net = _clone(network)
@@ -414,7 +460,7 @@ class QuantizedCNN(QuantizedNeuralNetwork):
         self.logger = logger
         self.ignore_layers = []
         self.conv_path = conv_path
-        self._init_device(device, method, shard, gram_split, alphabet_scope, rounding, seed)
+        self._init_device(device, method, shard, gram_split, alphabet_scope, rounding, seed, l1_penalty)
 
     def _build_patch_array(self, channel_idx: int, kernel_size: tuple, strides: tuple, padding: str, rate: tuple,
                            data, mini_batch_size: int):
@@ -434,11 +480,12 @@ class QuantizedCNN(QuantizedNeuralNetwork):
 
     def _quantize_channel_parallel_jit(self, channel_idx: int, channel_filters: array, hidden_activations,
                                        strides: tuple, padding: str, rate: tuple, alphabet: array,
-                                       patch_mini_batch_size=5000, scales=None, stochastic=None) -> array:
+                                       patch_mini_batch_size=5000, scales=None, stochastic=None, l1_penalty=None) -> array:
         """All filters of one input channel (quantized_network.py:652-727): host patches + one C-ABI call.  `stochastic`
         (stochastic rounding): (kernel, ci, f0, seed, scales) -- the whole (kh, kw, Cw, F) kernel, the channel's slice ci and its
         first filter f0, so that the slice draws with its global unit ids ci * F + f; the call walks all F filters of slice ci and
-        the Fg of `channel_filters` are kept."""
+        the Fg of `channel_filters` are kept.  `l1_penalty`: the layer's lambda, or None."""
+        pen = {} if l1_penalty is None else {"l1_penalty": l1_penalty}
         filter_shape = channel_filters.shape[0:2]
         patches = self._build_patch_array(channel_idx, filter_shape, strides, padding, rate, hidden_activations,
                                           patch_mini_batch_size)
@@ -450,10 +497,11 @@ class QuantizedCNN(QuantizedNeuralNetwork):
                 Wk, ci, f0, seed, sk = stochastic
                 Qk = self.engine.conv_channels([Xp], None if Xqp is Xp else [Xqp], np.ascontiguousarray(Wk, dtype=np.float32),
                                                np.asarray(alphabet, dtype=np.float64), c0=ci, n_channels=1, seeds=seed,
-                                               **({} if sk is None else {"scales": sk}))
+                                               **({} if sk is None else {"scales": sk}), **pen)
                 return Qk[:, :, ci, f0:f0 + channel_filters.shape[-1]]
             scaled = {} if scales is None else {"scales": np.reshape(scales, (1, -1))}
-            Qc = self.engine.conv_channels([Xp], None if Xqp is Xp else [Xqp], Wc, np.asarray(alphabet, dtype=np.float64), **scaled)
+            Qc = self.engine.conv_channels([Xp], None if Xqp is Xp else [Xqp], Wc, np.asarray(alphabet, dtype=np.float64), **scaled,
+                                           **pen)
         except Exception as exc:
             self._log(f"\t\t\tChannel {channel_idx} generated an exception: {exc}")
             raise Exception
@@ -474,6 +522,7 @@ class QuantizedCNN(QuantizedNeuralNetwork):
         alphabet, scales = self._levels(W, layer.__class__.__name__)
         scaled = {"scales": scales} if scales is not None else {}
         scaled.update(self._seeds(layer_idx))
+        scaled.update(self._penalty(layer_idx))
         # a grouped Conv2D has a (kh, kw, C / groups, F) kernel: input channel c meets only the Fg filters of its group c // Cg,
         # so ranks take whole groups and gather their filters (groups == 1: channels, all filters)
         groups = int(getattr(layer, "groups", 1)) if layer.__class__.__name__ == "Conv2D" else 1
@@ -519,7 +568,8 @@ class QuantizedCNN(QuantizedNeuralNetwork):
                 Q[:, :, ci, f0:f0 + Fg] = self._quantize_channel_parallel_jit(
                     channel_idx, W[:, :, ci, f0:f0 + Fg], data, strides=layer.strides, padding=layer.padding.upper(),
                     rate=rate, alphabet=alphabet, patch_mini_batch_size=self.patch_mini_batch_size,
-                    scales=None if scales is None else scales[ci, f0:f0 + Fg], stochastic=stoch)
+                    scales=None if scales is None else scales[ci, f0:f0 + Fg], stochastic=stoch,
+                    l1_penalty=scaled.get("l1_penalty"))
         if (lo, hi) != (0, num_channels) and groups > 1:
             # this rank wrote the filters of groups lo / Cg .. hi / Cg: gather along the group axis of (kh, kw, Cg, groups, Fg)
             Q = self._gather_columns(Q.reshape(*Q.shape[:3], groups, Fg), lo // Cg, hi // Cg, axis=3).reshape(W.shape)
