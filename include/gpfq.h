@@ -91,7 +91,8 @@ int gpfq_set_stream(gpfq_ctx *ctx, void *cuda_stream);
  *   "corr_pack"    correlation form, images packed side by side as virtual channels: 0 when the channel count cannot be
  *                  mapped (C < 32 or C % 4 != 0) and the images are large, 1 always, 2 never
  *   "corr_small"   1: correlation form also on images below 128 pixels (default: the planes kernel is faster there)
- *   "corr_rows"    correlation form: image rows per band (0 auto by image height, or 4 / 6 / 8)
+ *   "corr_rows"    correlation form: image rows per band (0 auto by image height, or 4 / 6 / 8; 8 only when X~ == X,
+ *                  the one-pass G1 + G2 kernel of X~ != X has bands of 4 or 6 rows and plans its own height otherwise)
  *   "corr_strip"   correlation form on small images (widths 8, 14, 16, 28, 32, 56, 64): 0 the strip kernel (whole strips of <= 16 columns as
  *                  straight-line code), 2 the band kernel
  *   "sweep_walk"   range walk of the Gram-row sweep for one symmetric equispaced alphabet: 0 auto (the tensor-core walk

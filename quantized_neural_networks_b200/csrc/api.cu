@@ -29,14 +29,14 @@ int im2col_stage(gpfq_ctx *, const float *, int64_t, int, int, int64_t, int64_t,
                  int, int, int, int, float *, int64_t);
 int msq_stage(gpfq_ctx *, const void *, int, int64_t, const double *, int, int, double *, const double *, int64_t);  // ctx->d_seeds
 int nhwc9_plan(int, int, int, int, int, int, int, int, int *, int *);
-int corr9_plan(int, int, int, int, int, int, int, int, int, int);
+int corr9_plan(int, int, int, int, int, int, int, int, int, int, bool);
 int corr9_pack_stage(gpfq_ctx *, const float *, int64_t, int, int, int64_t, int64_t, int, int, int64_t, int64_t, float *);
 int corr9_pick_slots(gpfq_ctx *, int, bool, int64_t, int, int64_t, int);
 int corr9_uses_strips(gpfq_ctx *, int);
 int corr9_tensor_ok(const float *, const float *);
 int conv_corr9_stage(gpfq_ctx *, const float *, const float *, bool, int64_t, int64_t, int64_t, int, int, int64_t, int64_t, int,
                      int, double *, int, int, int, double *, int, int, int);
-int conv_corr9_assemble_stage(gpfq_ctx *, const double *, int, const double *, int, bool, int, int, double *);
+int conv_corr9_assemble_stage(gpfq_ctx *, const double *, int, const double *, int, bool, int, int, int, double *);
 int conv_gram9_nhwc_stage(gpfq_ctx *, const float *, const float *, bool, int64_t, int64_t, int, int, int64_t, int64_t, int,
                           int, int, int, int, int, int, int, double *, int);
 
@@ -1072,7 +1072,7 @@ static int conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float *actq, i
         }
     }
     CUDA_TRY(ctx, gpfq_record(ctx, 5, s));
-    const int corr_rb = ctx->conv_variant == 0 ? corr9_plan(kh, kw, sh, sw, rh, rw, padding_same, (int)H, (int)Wd, ctx->corr_rb) : 0;
+    const int corr_rb = ctx->conv_variant == 0 ? corr9_plan(kh, kw, sh, sw, rh, rw, padding_same, (int)H, (int)Wd, ctx->corr_rb, same) : 0;
     // what a tensor map of the activations needs: 32-channel boxes on a 16-byte channel pitch; and lane = channel wants a
     // full warp of channels.  Otherwise G images are packed side by side as virtual channels first (conv_corr.cu).
     // Measured (tools/vgg_bench.py --net cifar / --conv-kernel 3): on 8 x 8 images the per-band start-up outweighs the 6.5x
@@ -1152,7 +1152,7 @@ static int conv_layer_nhwc(gpfq_ctx *ctx, const float *act, const float *actq, i
                                           ic * per_ic, per_ic, bpartial, bslots, ic * bper_ic, bper_ic));
             }
         }
-        GPFQ_TRY(conv_corr9_assemble_stage(ctx, partial, slots, bpartial, bslots, same, (int)n_ch, pack ? corr_G : 1, gram));
+        GPFQ_TRY(conv_corr9_assemble_stage(ctx, partial, slots, bpartial, bslots, same, (int)Wd, (int)n_ch, pack ? corr_G : 1, gram));
         CUDA_TRY(ctx, gpfq_record(ctx, 3, s));
         GPFQ_TRY(conv_finish(ctx, kk, nullptr, (int)n_ch, 0, same, W, C, F, c0, al, n_alph, Q_out, flags, gram, groups, d_scales));
         CUDA_TRY(ctx, gpfq_record(ctx, 1, s));

@@ -19,16 +19,25 @@
 // order (tasks per warp in index order, warps in index order): bit-reproducible, and equal to the patch form up to fp64
 // re-association (1e-16 relative; the parity budget is 1e-9, SURVEY.md App. C).
 //
-//   conv_corr9_tma_kernel<RB, CROSS>  lane = channel (NHWC: 32 channels = one 128-byte line per pixel); a warp walks a band
-//                                  of RB image rows left to right with a (RB+2) x 5 fp64 register window of the displaced
-//                                  operand and 13 accumulators per lane.  Operands arrive by TMA (cp.async.bulk.tensor.4d
-//                                  over the (N, H, W, C) tensor, box = 32 channels x 5 columns x RB+2 rows, zero fill
-//                                  outside the image = the 'SAME' padding) into a per-warp mbarrier ring; the warp is its
-//                                  own producer (lane 0 issues the next box before multiplying the current one).
-//                                  CROSS: xq centre x x window (G1), else xq x xq (G2).  The first and the last pixel
-//                                  column of a band go to the left / right region records.  One launch with RB in
-//                                  {8, 6, 4} covers rows 1 .. H-2, one with RB = 1 the top and bottom rows.
-//                                  Bound by the fp64 pipe: 13 DFMA + 1.3-2.3 F2F per pixel and pass.
+//   conv_corr9_tma_kernel<RB, BOTH>  lane = channel (NHWC: 32 channels = one 128-byte line per pixel); a warp walks a band
+//                                  of RB image rows left to right with a rotating 5-column fp64 register window of xq and
+//                                  13 accumulators per lane and Gram.  Operands arrive by TMA (cp.async.bulk.tensor.4d over
+//                                  the (N, H, W, C) tensor, zero fill outside the image = the 'SAME' padding) into a
+//                                  per-warp mbarrier ring; the warp is its own producer (lane 0 issues the next box before
+//                                  multiplying the current one).  X~ == X: G2 = xq x xq from (RB+2)-row windows.  BOTH
+//                                  (X~ != X): G1 and G2 in ONE pass.  Substituting t = s + d in G1 makes it
+//                                      G1[a, b] = sum over pixels t of  x[t] * xq[t - d],   -d lexicographically >= 0,
+//                                  restricted to t - b + 1 inside the image: x centre times the xq window at and BELOW it,
+//                                  while G2 is xq centre times the xq window at and ABOVE it.  Both read one (RB+4)-row
+//                                  window of xq plus the RB x 5 centre pixels of x: 26 DFMA and (RB+4)/RB + 1 fp32 -> fp64
+//                                  conversions per pixel, 8 B per pixel and channel from HBM.  G1's records are split by
+//                                  the region of the x pixel t, the assembly adds for G1[a, b] the regions of tap b.  The
+//                                  first and the last pixel column of a band go to the left / right region records.  One
+//                                  launch covers rows 1 .. H-2 (RB in {8, 6, 4}; {6, 4} with BOTH), one with RB = 1 the top
+//                                  and bottom rows.
+//   conv_corr9_strip_kernel<SW, RB, CROSS>  the same sums on images 14-64 pixels wide as whole strips of <= 16 columns, in
+//                                  two launches (CROSS: xq centre x x window, G1 records split by the xq pixel)
+//   conv_corr9_strip1_kernel<SW, RB>  both Grams in one pass on strips, the band kernel's form; picked by width (8 pixels)
 //   conv_corr9_assemble_kernel     fixed-order slot sums + the per-tap region sums -> [G1 | G2] per channel in the
 //                                  layout conv_sweep_kernel reads
 //   corr9_pack_kernel              channel counts a tensor map cannot serve (C < 32, C % 4 != 0) on large images: G images
@@ -80,24 +89,47 @@ __device__ __forceinline__ void tma_load_4d(void *dst, const CUtensorMap *map, u
             smem_u32(dst)), "l"(map), "r"(smem_u32(bar)), "r"(c), "r"(x), "r"(y), "r"(n)
         : "memory");
 }
-template <int RB, bool CROSS>
+template <int RB, bool BOTH>
 struct Ring {
-    static constexpr int NS = CROSS ? 2 : 3;                 // boxes in flight per warp
-    static constexpr int B_FLOATS = (RB + 2) * WC * 32;      // window operand: RB + 2 rows x 5 columns x 32 channels
-    static constexpr int A_FLOATS = CROSS ? RB * WC * 32 : 0;  // xq centre pixels, two columns behind
+    static constexpr int NS = BOTH ? 2 : 3;                  // boxes in flight per warp
+    static constexpr int WR = BOTH ? RB + 4 : RB + 2;        // window rows: two above the band, and two below it for G1
+    static constexpr int B_FLOATS = WR * WC * 32;            // xq window: WR rows x 5 columns x 32 channels
+    static constexpr int A_FLOATS = BOTH ? RB * WC * 32 : 0;  // x centre pixels, two columns behind
     static constexpr int STAGE_FLOATS = B_FLOATS + A_FLOATS;
     static constexpr size_t WARP_BYTES = (size_t)NS * STAGE_FLOATS * sizeof(float);
     static constexpr size_t SMEM = WARPS * WARP_BYTES + WARPS * NS * sizeof(uint64_t);
 };
+// One pixel row i of the band into the 13 sums `o`; the window's logical column L (pixel column - 2 + L) sits in physical slot
+// (ph + 1 + L) % 5.  G2: xq centre x the xq window at the displacements d (lexicographically <= 0) above it.  G1: x centre x
+// the xq window at -d, below it -- the point reflection of the G2 pattern through the centre (row i + 2 + r <-> i + 2 - r,
+// column 2 + c <-> 2 - c), so that G1 reads the same window as G2 and lands in the same 13 displacement slots.
+template <int WR>
+__device__ __forceinline__ void mac_g2(double a, const double (&win)[WR][5], int i, int ph, double (&o)[ND]) {
+#pragma unroll
+    for (int dy = 0; dy < 2; ++dy)
+#pragma unroll
+        for (int dx = 0; dx < 5; ++dx) o[dy * 5 + dx] = fma(a, win[i + dy][(ph + 1 + dx) % 5], o[dy * 5 + dx]);
+#pragma unroll
+    for (int dx = 0; dx < 3; ++dx) o[10 + dx] = fma(a, win[i + 2][(ph + 1 + dx) % 5], o[10 + dx]);
+}
+template <int WR>
+__device__ __forceinline__ void mac_g1(double a, const double (&win)[WR][5], int i, int ph, double (&o)[ND]) {
+#pragma unroll
+    for (int dy = 0; dy < 2; ++dy)
+#pragma unroll
+        for (int dx = 0; dx < 5; ++dx) o[dy * 5 + dx] = fma(a, win[i + 4 - dy][(ph + 5 - dx) % 5], o[dy * 5 + dx]);
+#pragma unroll
+    for (int dx = 0; dx < 3; ++dx) o[10 + dx] = fma(a, win[i + 2][(ph + 5 - dx) % 5], o[10 + dx]);
+}
 }  // namespace corr9
 
-template <int RB, bool CROSS>
-__global__ void __launch_bounds__(corr9::WARPS * 32, RB <= 4 ? 3 : 2)
-conv_corr9_tma_kernel(const __grid_constant__ CUtensorMap mapB, const __grid_constant__ CUtensorMap mapA, Corr9Geom gm,
+template <int RB, bool BOTH>
+__global__ void __launch_bounds__(corr9::WARPS * 32, (RB <= 4 && !BOTH) || RB == 1 ? 3 : 2)
+conv_corr9_tma_kernel(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUtensorMap mapX, Corr9Geom gm,
                       double *__restrict__ partial, int slot_stride, int slot0) {
     using namespace corr9;
-    using R = Ring<RB, CROSS>;
-    constexpr int NS = R::NS;
+    using R = Ring<RB, BOTH>;
+    constexpr int NS = R::NS, WR = R::WR;
     extern __shared__ __align__(128) unsigned char corr9_smem[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int slot = blockIdx.x * WARPS + warp;
@@ -120,13 +152,13 @@ conv_corr9_tma_kernel(const __grid_constant__ CUtensorMap mapB, const __grid_con
     const int64_t ntasks = gm.two_rows ? gm.n_img : gm.n_img * nbands;
     const int64_t t_first = gm.two_rows ? slot / 2 : slot, t_step = gm.two_rows ? gm.slots / 2 : gm.slots;
     const int nstages = (W + 2 + WC - 1) / WC;
-    // this lane's record: [pass][first column | between | last column][13]; first / last are read-modify-written in
+    // this lane's record: [pass: G1, G2][first column | between | last column][13]; first / last are read-modify-written in
     // task order by this lane only (the API zeroes the records), `between` is stored once at the end
-    double *rec = partial + ((size_t)(chok ? chl : 0) * slot_stride + slot0 + slot) * REC + (CROSS ? 0 : 3 * ND);
+    double *rec = partial + ((size_t)(chok ? chl : 0) * slot_stride + slot0 + slot) * REC;
     uint32_t it = 0;  // boxes this warp has consumed so far: ring position and mbarrier parity
-    double acc[ND];
+    double acc[ND], acc1[ND];   // G2, G1 (BOTH)
 #pragma unroll
-    for (int d = 0; d < ND; ++d) acc[d] = 0.0;
+    for (int d = 0; d < ND; ++d) acc[d] = acc1[d] = 0.0;
 
     // The boxes of this warp's tasks form one stream (task after task, columns left to right); the producer cursor runs
     // NS - 1 boxes ahead of the consumer, across task boundaries, so a new band never starts with an empty ring.
@@ -145,8 +177,8 @@ conv_corr9_tma_kernel(const __grid_constant__ CUtensorMap mapB, const __grid_con
                 const int s = (int)(ppos % NS);
                 float *dst = ring + s * R::STAGE_FLOATS;
                 mbar_expect_tx(&bars[s], (uint32_t)(R::STAGE_FLOATS * sizeof(float)));
-                tma_load_4d(dst, &mapB, &bars[s], c0, pk * WC, py0 - 2, pimg);
-                if (CROSS) tma_load_4d(dst + R::B_FLOATS, &mapA, &bars[s], c0, pk * WC - 2, py0, pimg);
+                tma_load_4d(dst, &mapQ, &bars[s], c0, pk * WC, py0 - 2, pimg);
+                if (BOTH) tma_load_4d(dst + R::B_FLOATS, &mapX, &bars[s], c0, pk * WC - 2, py0, pimg);
             }
             ++ppos;
             if (++pk == nstages) {
@@ -170,11 +202,11 @@ conv_corr9_tma_kernel(const __grid_constant__ CUtensorMap mapB, const __grid_con
 #pragma unroll
         for (int i = 0; i < RB; ++i) rowmask |= (y0 + i <= gm.y_last) ? (1u << i) : 0u;
         const bool allrows = rowmask == (1u << RB) - 1u;
-        double win[RB + 2][5];
+        double win[WR][5];
         double ac[RB];
         (void)ac;
 #pragma unroll
-        for (int r = 0; r < RB + 2; ++r)
+        for (int r = 0; r < WR; ++r)
 #pragma unroll
             for (int c = 0; c < 5; ++c) win[r][c] = 0.0;
         for (int k = 0; k < nstages; ++k) {
@@ -190,34 +222,27 @@ conv_corr9_tma_kernel(const __grid_constant__ CUtensorMap mapB, const __grid_con
 #pragma unroll
                 for (int ph = 0; ph < WC; ++ph) {
 #pragma unroll
-                    for (int r = 0; r < RB + 2; ++r) win[r][ph] = (double)tb[(r * WC + ph) * 32];
-                    if (CROSS) {
+                    for (int r = 0; r < WR; ++r) win[r][ph] = (double)tb[(r * WC + ph) * 32];
+                    if (BOTH) {
 #pragma unroll
                         for (int i = 0; i < RB; ++i) ac[i] = (double)ta[(i * WC + ph) * 32];
                     }
 #pragma unroll
                     for (int i = 0; i < RB; ++i) {
-                        const double a = CROSS ? ac[i] : win[i + 2][(ph + 3) % 5];
-#pragma unroll
-                        for (int dy = 0; dy < 2; ++dy)
-#pragma unroll
-                            for (int dx = 0; dx < 5; ++dx)
-                                acc[dy * 5 + dx] = fma(a, win[i + dy][(ph + 1 + dx) % 5], acc[dy * 5 + dx]);
-#pragma unroll
-                        for (int dx = 0; dx < 3; ++dx)
-                            acc[10 + dx] = fma(a, win[i + 2][(ph + 1 + dx) % 5], acc[10 + dx]);
+                        mac_g2(win[i + 2][(ph + 3) % 5], win, i, ph, acc);
+                        if (BOTH) mac_g1(ac[i], win, i, ph, acc1);
                     }
                 }
             } else {
                 // ---- band ends, ragged last band: one column at a time into `e`, then to the record it belongs to.  The raw
                 // fp32 values of a column are read from the box one column ahead (the branches between the columns keep the
                 // compiler from hoisting the loads itself, and LDS -> F2F -> DFMA back to back is all latency: ncu, conv10)
-                float rawb[RB + 2], rawa[RB];
+                float rawb[WR], rawa[RB];
                 (void)rawa;
                 auto fetch = [&](int ph) {
 #pragma unroll
-                    for (int r = 0; r < RB + 2; ++r) rawb[r] = tb[(r * WC + ph) * 32];
-                    if (CROSS) {
+                    for (int r = 0; r < WR; ++r) rawb[r] = tb[(r * WC + ph) * 32];
+                    if (BOTH) {
 #pragma unroll
                         for (int i = 0; i < RB; ++i) rawa[i] = ta[(i * WC + ph) * 32];
                     }
@@ -228,41 +253,42 @@ conv_corr9_tma_kernel(const __grid_constant__ CUtensorMap mapB, const __grid_con
                     const int cx = k * WC + ph;  // newest window column (image column cx) lives in physical slot ph
                     if (cx < W + 2) {
 #pragma unroll
-                        for (int r = 0; r < RB + 2; ++r) win[r][ph] = (double)rawb[r];
-                        if (CROSS) {
+                        for (int r = 0; r < WR; ++r) win[r][ph] = (double)rawb[r];
+                        if (BOTH) {
 #pragma unroll
                             for (int i = 0; i < RB; ++i) ac[i] = (double)rawa[i];
                         }
                         if (ph + 1 < WC) fetch(ph + 1);   // inside the box even when that column lies past the image (zeros)
                         if (cx >= 2) {
-                            // pixel column cx - 2 = logical window column 2 = physical slot (ph + 3) % 5
-                            double e[ND];
+                            // pixel column cx - 2 = logical window column 2 = physical slot (ph + 3) % 5; the first / last
+                            // pixel column have their own records
+                            const bool edge = cx == 2 || cx == W + 1;
+                            double *o = rec + (cx == 2 ? 0 : 2 * ND);
 #pragma unroll
-                            for (int d = 0; d < ND; ++d) e[d] = 0.0;
+                            for (int pass = BOTH ? 0 : 1; pass < 2; ++pass) {
+                                double e[ND];
 #pragma unroll
-                            for (int i = 0; i < RB; ++i) {
-                                double a = CROSS ? ac[i] : win[i + 2][(ph + 3) % 5];
-                                a = (rowmask >> i) & 1u ? a : 0.0;
+                                for (int d = 0; d < ND; ++d) e[d] = 0.0;
 #pragma unroll
-                                for (int dy = 0; dy < 2; ++dy)
-#pragma unroll
-                                    for (int dx = 0; dx < 5; ++dx)
-                                        e[dy * 5 + dx] = fma(a, win[i + dy][(ph + 1 + dx) % 5], e[dy * 5 + dx]);
-#pragma unroll
-                                for (int dx = 0; dx < 3; ++dx)
-                                    e[10 + dx] = fma(a, win[i + 2][(ph + 1 + dx) % 5], e[10 + dx]);
-                            }
-                            if (cx == 2 || cx == W + 1) {   // first / last pixel column: their own records
-                                if (chok) {
-                                    // fire-and-forget reductions (RED.ADD.F64): nothing waits for the round trip to L2;
-                                    // only this lane ever touches the record, and its updates apply in program order
-                                    double *o = rec + (cx == 2 ? 0 : 2 * ND);
-#pragma unroll
-                                    for (int d = 0; d < ND; ++d) atomicAdd(o + d, e[d]);
+                                for (int i = 0; i < RB; ++i) {
+                                    const bool live = (rowmask >> i) & 1u;
+                                    if (pass == 1) mac_g2(live ? win[i + 2][(ph + 3) % 5] : 0.0, win, i, ph, e);
+                                    else mac_g1(live ? ac[i] : 0.0, win, i, ph, e);
                                 }
-                            } else {
+                                if (edge) {
+                                    if (chok) {
+                                        // fire-and-forget reductions (RED.ADD.F64): nothing waits for the round trip to L2;
+                                        // only this lane ever touches the record, and its updates apply in program order
 #pragma unroll
-                                for (int d = 0; d < ND; ++d) acc[d] += e[d];
+                                        for (int d = 0; d < ND; ++d) atomicAdd(o + pass * 3 * ND + d, e[d]);
+                                    }
+                                } else if (pass == 1) {
+#pragma unroll
+                                    for (int d = 0; d < ND; ++d) acc[d] += e[d];
+                                } else {
+#pragma unroll
+                                    for (int d = 0; d < ND; ++d) acc1[d] += e[d];
+                                }
                             }
                         }
                     }
@@ -273,7 +299,10 @@ conv_corr9_tma_kernel(const __grid_constant__ CUtensorMap mapB, const __grid_con
     }
     if (chok) {
 #pragma unroll
-        for (int d = 0; d < ND; ++d) rec[ND + d] = acc[d];
+        for (int d = 0; d < ND; ++d) {
+            rec[3 * ND + ND + d] = acc[d];
+            if (BOTH) rec[ND + d] = acc1[d];
+        }
     }
 }
 
@@ -285,7 +314,8 @@ conv_corr9_tma_kernel(const __grid_constant__ CUtensorMap mapB, const __grid_con
 // TMA box of (RB + 2) x (SW + 4) pixels x 32 channels, zero fill outside the image = the padding, plus the RB x SW centre pixels
 // of xq for the xq x x pass) and walked as straight-line code: the column index is a compile-time constant, so the rotating
 // register window, the column class (first / between / last pixel column) and every shared-memory offset are static, there are
-// no edge stages and the three column classes are three register accumulator sets stored once per warp.  W = 28 / 32 are two
+// no edge stages and the three column classes are three register accumulator sets stored once per warp.  G1 and G2 stay two
+// launches here: one pass would need the (RB + 4)-row window and 3 x 26 accumulators, past what fits in registers at this occupancy.  W = 28 / 32 are two
 // strips (the inner strip boundary is an ordinary "between" column: the halo columns hold real pixels).  Same records as the
 // band kernel (conv_corr9_assemble_kernel reads both), same exact products, fixed summation order.
 namespace corr9s {
@@ -458,12 +488,181 @@ conv_corr9_strip_kernel(const __grid_constant__ CUtensorMap mapWin, const __grid
     }
 }
 
+// One pass for both Grams on strips (X~ != X): a box of RB + 4 rows of xq x (SW + 4) columns plus the RB x SW centre pixels of x
+// per task; G2 = xq centre x the window above it, G1 = x centre x the window below it (conv_corr9_tma_kernel's mac_g1).  The
+// columns between the first and the last one accumulate in registers (2 x 13 sums); 3 x 26 sums and the (RB + 4)-row window do not
+// fit in registers, so the image's first / last pixel column add their sums to lane-private shared-memory records (plain
+// read-add-write by the owning lane, in task order) that are stored once per warp like the register sums.
+namespace corr9s {
+template <int SW, int RB>
+struct Cfg1 {
+    static constexpr int BW = SW + 4, WR = RB + 4;
+    static constexpr int WIN_FLOATS = WR * BW * 32;
+    static constexpr int CTR_FLOATS = RB * SW * 32;
+    static constexpr int STAGE_FLOATS = WIN_FLOATS + CTR_FLOATS;
+    static constexpr int NS = Boxes<RB>::NS;
+    static constexpr size_t WARP_BYTES = (size_t)NS * STAGE_FLOATS * sizeof(float);
+    static constexpr size_t REC_BYTES = (size_t)2 * 2 * ND * 32 * sizeof(double);   // [first, last][G1, G2][13] x 32 lanes
+    static constexpr size_t SMEM = WARPS * (WARP_BYTES + REC_BYTES) + WARPS * NS * sizeof(uint64_t);
+};
+}  // namespace corr9s
+
+template <int SW, int RB>
+__global__ void __launch_bounds__(corr9s::WARPS * 32)
+conv_corr9_strip1_kernel(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUtensorMap mapX, Corr9Geom gm,
+                         double *__restrict__ partial, int slot_stride, int slot0) {
+    using namespace corr9s;
+    using corr9::mbar_expect_tx;
+    using corr9::mbar_init;
+    using corr9::mbar_wait;
+    using corr9::tma_load_4d;
+    using C = Cfg1<SW, RB>;
+    constexpr int BW = C::BW, WR = C::WR, NS = C::NS;
+    extern __shared__ __align__(128) unsigned char corr9_smem[];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int slot = blockIdx.x * WARPS + warp;
+    const int c0 = (int)(gm.c_first & ~(int64_t)3) + (int)blockIdx.y * 32;
+    const int chl = c0 + lane - (int)gm.c_first;
+    const bool chok = chl >= 0 && chl < gm.n_ch;
+    float *ring = reinterpret_cast<float *>(corr9_smem + warp * C::WARP_BYTES);
+    double *srec = reinterpret_cast<double *>(corr9_smem + WARPS * C::WARP_BYTES + warp * C::REC_BYTES) + lane;  // [j * 32]
+    uint64_t *bars = reinterpret_cast<uint64_t *>(corr9_smem + WARPS * (C::WARP_BYTES + C::REC_BYTES)) + warp * NS;
+#pragma unroll
+    for (int j = 0; j < 4 * ND; ++j) srec[j * 32] = 0.0;
+    if (lane == 0) {
+#pragma unroll
+        for (int s = 0; s < NS; ++s) mbar_init(&bars[s], 1);
+        asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
+    }
+    __syncwarp();
+    const int nstrips = gm.W / SW;
+    const int nrows = gm.y_last - gm.y_first + 1;
+    const int nbands = gm.two_rows ? 1 : (nrows + RB - 1) / RB;
+    const int per_img = nbands * nstrips;
+    const int64_t ntasks = gm.n_img * per_img;
+    const int64_t t_first = gm.two_rows ? slot / 2 : slot, t_step = gm.two_rows ? gm.slots / 2 : gm.slots;
+    const int row_fixed = (slot & 1) ? gm.y_last : gm.y_first;
+    const int step_img = (int)(t_step / per_img), step_in = (int)(t_step % per_img);
+    auto fetch = [&](int img, int in, uint32_t pos) {
+        const int band = in / nstrips, strip = in - band * nstrips;
+        const int y0 = gm.two_rows ? row_fixed : gm.y_first + band * RB, x0 = strip * SW;
+        const int s = (int)(pos % NS);
+        float *dst = ring + s * C::STAGE_FLOATS;
+        mbar_expect_tx(&bars[s], (uint32_t)(C::STAGE_FLOATS * sizeof(float)));
+        tma_load_4d(dst, &mapQ, &bars[s], c0, x0 - 2, y0 - 2, img);
+        tma_load_4d(dst + C::WIN_FLOATS, &mapX, &bars[s], c0, x0, y0, img);
+    };
+    double acc1[ND], acc2[ND];
+#pragma unroll
+    for (int d = 0; d < ND; ++d) acc1[d] = acc2[d] = 0.0;
+    int img = (int)(gm.img0 + t_first / per_img), in = (int)(t_first % per_img);
+    if (t_first < ntasks && lane == 0) fetch(img, in, 0);
+    uint32_t pos = 0;
+    for (int64_t task = t_first; task < ntasks; task += t_step, ++pos) {
+        int nimg = img + step_img, nin = in + step_in;
+        if (nin >= per_img) { nin -= per_img; ++nimg; }
+        if (NS > 1) {
+            __syncwarp();
+            if (task + t_step < ntasks && lane == 0) fetch(nimg, nin, pos + 1);
+        }
+        const int band = in / nstrips, strip = in - band * nstrips;
+        const int y0 = gm.two_rows ? row_fixed : gm.y_first + band * RB;
+        const bool left_edge = strip == 0, right_edge = strip == nstrips - 1;
+        unsigned rowmask = 0;
+#pragma unroll
+        for (int i = 0; i < RB; ++i) rowmask |= (y0 + i <= gm.y_last) ? (1u << i) : 0u;
+        const int s = (int)(pos % NS);
+        mbar_wait(&bars[s], (pos / NS) & 1u);
+        const float *tb = ring + s * C::STAGE_FLOATS + lane;
+        const float *ta = tb + C::WIN_FLOATS;
+        // window: box columns p .. p + 4 in physical slots (p + k) % 6; box column p + 5 is converted during column p
+        double win[WR][6];
+        double ctr[RB], ctr_n[RB];
+#pragma unroll
+        for (int bc = 0; bc < 5; ++bc)
+#pragma unroll
+            for (int r = 0; r < WR; ++r) win[r][bc] = (double)tb[(r * BW + bc) * 32];
+#pragma unroll
+        for (int i = 0; i < RB; ++i) ctr[i] = (double)ta[(i * SW) * 32];
+#pragma unroll
+        for (int p = 0; p < SW; ++p) {
+            const bool edge = p == 0 || p == SW - 1;
+            double e1[ND], e2[ND];
+            if (edge) {
+#pragma unroll
+                for (int d = 0; d < ND; ++d) e1[d] = e2[d] = 0.0;
+            }
+#pragma unroll
+            for (int i = 0; i < RB; ++i) {
+                const bool live = (rowmask >> i) & 1u;
+                const double q = live ? win[i + 2][(p + 2) % 6] : 0.0, xc = live ? ctr[i] : 0.0;
+                double *o1 = edge ? e1 : acc1, *o2 = edge ? e2 : acc2;
+#pragma unroll
+                for (int dy = 0; dy < 2; ++dy)
+#pragma unroll
+                    for (int dx = 0; dx < 5; ++dx) {
+                        o2[dy * 5 + dx] = fma(q, win[i + dy][(p + dx) % 6], o2[dy * 5 + dx]);
+                        o1[dy * 5 + dx] = fma(xc, win[i + 4 - dy][(p + 4 - dx) % 6], o1[dy * 5 + dx]);
+                    }
+#pragma unroll
+                for (int dx = 0; dx < 3; ++dx) {
+                    o2[10 + dx] = fma(q, win[i + 2][(p + dx) % 6], o2[10 + dx]);
+                    o1[10 + dx] = fma(xc, win[i + 2][(p + 4 - dx) % 6], o1[10 + dx]);
+                }
+                // the next column's operands, spread over the rows: window rows i, i + RB, ..., centre pixel of row i
+                if (p + 5 < BW) {
+#pragma unroll
+                    for (int r = i; r < WR; r += RB) win[r][(p + 5) % 6] = (double)tb[(r * BW + p + 5) * 32];
+                }
+                if (p + 1 < SW) ctr_n[i] = (double)ta[(i * SW + p + 1) * 32];
+            }
+#pragma unroll
+            for (int i = 0; i < RB; ++i) ctr[i] = ctr_n[i];
+            if (edge) {   // the image's first / last pixel column: the shared-memory records; a strip boundary inside the image: between
+                const bool first = p == 0 && left_edge, last = p == SW - 1 && right_edge;
+                if (first || last) {
+                    double *r = srec + (last ? 2 * ND * 32 : 0);
+#pragma unroll
+                    for (int d = 0; d < ND; ++d) {
+                        r[d * 32] += e1[d];
+                        r[(ND + d) * 32] += e2[d];
+                    }
+                } else {
+#pragma unroll
+                    for (int d = 0; d < ND; ++d) {
+                        acc1[d] += e1[d];
+                        acc2[d] += e2[d];
+                    }
+                }
+            }
+        }
+        if (NS == 1) {
+            __syncwarp();
+            if (task + t_step < ntasks && lane == 0) fetch(nimg, nin, pos + 1);
+        }
+        img = nimg;
+        in = nin;
+    }
+    if (chok) {
+        double *rec = partial + ((size_t)chl * slot_stride + slot0 + slot) * REC;   // [G1, G2][first, between, last][13]
+#pragma unroll
+        for (int d = 0; d < ND; ++d) {
+            rec[d] = srec[d * 32];
+            rec[ND + d] = acc1[d];
+            rec[2 * ND + d] = srec[(2 * ND + d) * 32];
+            rec[3 * ND + d] = srec[(ND + d) * 32];
+            rec[4 * ND + d] = acc2[d];
+            rec[5 * ND + d] = srec[(3 * ND + d) * 32];
+        }
+    }
+}
+
 // gram: (n_channels, 2 * 81): [G1 | G2], lower triangle + diagonal valid, zeros above (conv_finalize_kernel's layout).
 // partial: records of the launch over rows 1 .. H-2 (left column, interior, right column); rpartial: records of the
 // top / bottom row launch (even slots: top-left corner, top row, top-right corner; odd slots: the bottom ones).
 __global__ void __launch_bounds__(1024)
 conv_corr9_assemble_kernel(const double *__restrict__ partial, int slots, const double *__restrict__ rpartial, int rslots,
-                           int same, int n_ch, int G, double *__restrict__ gram) {
+                           int same, int g1_by_x, int n_ch, int G, double *__restrict__ gram) {
     using namespace corr9;
     // S[pass][row class: 0 top, 1 between, 2 bottom][column class: 0 first, 1 between, 2 last][13]
     constexpr int NV = 2 * 9 * ND, NP = 4;            // values per channel; slot partitions (one quarter of the CTA each)
@@ -513,8 +712,12 @@ conv_corr9_assemble_kernel(const double *__restrict__ partial, int slots, const 
             const int ar = t / 3, ac = t % 3, dy = s / 3 - ar, dx = s % 3 - ac;
             const int id = dy < 0 ? (dy + 2) * 5 + dx + 2 : 12 + dx;
             const int pass = (which == 0 && !same) ? 0 : 1;
-            // tap row 0 never sits on the bottom image row, tap row 2 never on the top row; columns alike
-            const int r_lo = ar == 2 ? 1 : 0, r_hi = ar == 0 ? 1 : 2, c_lo = ac == 2 ? 1 : 0, c_hi = ac == 0 ? 1 : 2;
+            // The records are split by the region of the window's centre pixel: the xq pixel tap t reads, or for G1 from the
+            // one-pass band kernel (g1_by_x) the x pixel tap s reads (the patch position is the same pixel either way).
+            // Tap row 0 never sits on the bottom image row, tap row 2 never on the top row; columns alike.
+            const bool by_s = pass == 0 && g1_by_x;
+            const int cr = by_s ? s / 3 : ar, ccl = by_s ? s % 3 : ac;
+            const int r_lo = cr == 2 ? 1 : 0, r_hi = cr == 0 ? 1 : 2, c_lo = ccl == 2 ? 1 : 0, c_hi = ccl == 0 ? 1 : 2;
             for (int rc = r_lo; rc <= r_hi; ++rc)
                 for (int cc = c_lo; cc <= c_hi; ++cc) v += S[pass][rc][cc][id];
         }
@@ -525,11 +728,19 @@ conv_corr9_assemble_kernel(const double *__restrict__ partial, int slots, const 
 // ---- host side ---------------------------------------------------------------------------------------------------
 // Is the geometry eligible, and with how many rows per band?  (0: keep the patch form.)  The channel conditions of the
 // tensor map (C >= 32, C % 4 == 0) are the caller's: it can meet them by packing images side by side (corr9_pack_kernel).
-int corr9_plan(int kh, int kw, int sh, int sw, int rh, int rw, int padding_same, int H, int W, int force_rb) {
+int corr9_plan(int kh, int kw, int sh, int sw, int rh, int rw, int padding_same, int H, int W, int force_rb, bool same) {
     if (kh != 3 || kw != 3 || sh != 1 || sw != 1 || rh != 1 || rw != 1 || !padding_same) return 0;
     if (H < 6 || W < corr9::WC) return 0;            // a TMA box (RB + 2 >= 6 rows x 5 columns) must fit in the image
     if ((int64_t)H * W >= ((int64_t)1 << 28)) return 0;
-    if ((force_rb == 8 || force_rb == 6 || force_rb == 4) && force_rb + 2 <= H) return force_rb;
+    if ((force_rb == 8 || force_rb == 6 || force_rb == 4) && force_rb + 2 <= H && (same || force_rb != 8)) return force_rb;
+    if (!same) {
+        // G1 and G2 in one pass: bands of 6 or 4 rows (an 8-row band's 12 x 5 window and 26 sums spill).
+        // RB = 6 converts 2.67 values per pixel against RB = 4's 3.0 and moves fewer halo rows: it wins unless it wastes
+        // more than 15 % of its band rows.
+        const int rows = H - 2;
+        const int bands6 = (rows + 5) / 6, bands4 = (rows + 3) / 4;
+        return 6 + 2 <= H && ((double)rows >= 0.85 * bands6 * 6 || bands6 * 6 <= bands4 * 4) ? 6 : 4;
+    }
     // Rows 1 .. H-2 in bands of RB rows.  Measured (tools/vgg_bench.py --corr-rows, VGG16 and CIFAR10 shapes): RB = 8 wins
     // whenever at least 85 % of its band rows are live (224, 112, 56, 32, 16 rows high), otherwise the band height that
     // wastes fewest rows, with RB = 4 handicapped by 0.1 (more conversions and box traffic per DFMA: on 28 x 28 it wastes
@@ -616,43 +827,56 @@ int corr9_pack_stage(gpfq_ctx *ctx, const float *act, int64_t n_img, int H, int 
     return GPFQ_OK;
 }
 
-template <int RB>
-static int corr9_resident_ctas(bool same) {
+template <int RB, bool BOTH>
+static int corr9_resident_ctas() {
     using namespace corr9;
     // a failed query only costs launch geometry (the caller plans for one CTA per SM): its error is consumed HERE, where it
     // arose, so that it can neither leak into the next launch check nor swallow an unrelated pending error
-    int a = 0, b = 0;
-    if (cudaFuncSetAttribute(conv_corr9_tma_kernel<RB, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Ring<RB, false>::SMEM) != cudaSuccess ||
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&a, conv_corr9_tma_kernel<RB, false>, WARPS * 32, Ring<RB, false>::SMEM) != cudaSuccess) {
+    int a = 0;
+    if (cudaFuncSetAttribute(conv_corr9_tma_kernel<RB, BOTH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Ring<RB, BOTH>::SMEM) != cudaSuccess ||
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&a, conv_corr9_tma_kernel<RB, BOTH>, WARPS * 32, Ring<RB, BOTH>::SMEM) != cudaSuccess) {
         cudaGetLastError();
         return 0;
     }
-    if (same) return a;
-    if (cudaFuncSetAttribute(conv_corr9_tma_kernel<RB, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Ring<RB, true>::SMEM) != cudaSuccess ||
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, conv_corr9_tma_kernel<RB, true>, WARPS * 32, Ring<RB, true>::SMEM) != cudaSuccess) {
-        cudaGetLastError();
-        return 0;
-    }
-    return a < b ? a : b;
+    return a;
 }
 
+// X~ != X on strips: both Grams in one pass (conv_corr9_strip1_kernel) or the two-pass pair, by strip width.  Measured per layer
+// (B200, VGG16 and CIFAR10 benches, profiles/r3_corr9_onepass.md): one pass wins on 8-pixel images (0.305 -> 0.219 ms, 0.342 ->
+// 0.331 ms) and loses on 14- to 64-wide ones (VGG16 56 x 56 x 256: 3.66 -> 5.39 ms), where its shared-memory records and
+// (RB + 4)-row boxes leave one CTA of four warps per SM against the pair's eight warps.
+static constexpr bool corr9_strip_onepass_sw(int sw) { return sw == 8; }
 static int corr9_strip_width(int Wd);
+static bool corr9_strip_onepass(int Wd);
 template <int SW, int RB>
 static int corr9_strip_resident_ctas(bool same) {
     using namespace corr9s;
     int a = 0, b = 0;
+    if constexpr (corr9_strip_onepass_sw(SW)) {
+        if (!same) {
+            if (cudaFuncSetAttribute(conv_corr9_strip1_kernel<SW, RB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg1<SW, RB>::SMEM) != cudaSuccess ||
+                cudaOccupancyMaxActiveBlocksPerMultiprocessor(&a, conv_corr9_strip1_kernel<SW, RB>, WARPS * 32, Cfg1<SW, RB>::SMEM) != cudaSuccess) {
+                cudaGetLastError();
+                return 0;
+            }
+            return a;
+        }
+    }
     if (cudaFuncSetAttribute(conv_corr9_strip_kernel<SW, RB, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg<SW, RB, false>::SMEM) != cudaSuccess ||
         cudaOccupancyMaxActiveBlocksPerMultiprocessor(&a, conv_corr9_strip_kernel<SW, RB, false>, WARPS * 32, Cfg<SW, RB, false>::SMEM) != cudaSuccess) {
         cudaGetLastError();
         return 0;
     }
-    if (same) return a;
-    if (cudaFuncSetAttribute(conv_corr9_strip_kernel<SW, RB, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg<SW, RB, true>::SMEM) != cudaSuccess ||
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, conv_corr9_strip_kernel<SW, RB, true>, WARPS * 32, Cfg<SW, RB, true>::SMEM) != cudaSuccess) {
-        cudaGetLastError();
-        return 0;
+    if constexpr (!corr9_strip_onepass_sw(SW)) {
+        if (same) return a;
+        if (cudaFuncSetAttribute(conv_corr9_strip_kernel<SW, RB, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg<SW, RB, true>::SMEM) != cudaSuccess ||
+            cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b, conv_corr9_strip_kernel<SW, RB, true>, WARPS * 32, Cfg<SW, RB, true>::SMEM) != cudaSuccess) {
+            cudaGetLastError();
+            return 0;
+        }
+        return a < b ? a : b;
     }
-    return a < b ? a : b;
+    return a;
 }
 
 // Slots (warps per channel group) that fill every SM with as many CTAs of four warps as stay resident.  Wd: the image width (the
@@ -676,8 +900,9 @@ int corr9_pick_slots(gpfq_ctx *ctx, int RB, bool same, int64_t c_first, int n_ch
     }
     int &occ = ctx->corr_occ[same ? 1 : 0][RB];      // per context (= per device): no state shared between engines / threads
     if (!occ) {
-        occ = RB == 8 ? corr9_resident_ctas<8>(same) : RB == 6 ? corr9_resident_ctas<6>(same)
-              : RB == 4 ? corr9_resident_ctas<4>(same) : corr9_resident_ctas<1>(same);
+        occ = same ? (RB == 8 ? corr9_resident_ctas<8, false>() : RB == 6 ? corr9_resident_ctas<6, false>()
+                      : RB == 4 ? corr9_resident_ctas<4, false>() : corr9_resident_ctas<1, false>())
+                   : (RB == 6 ? corr9_resident_ctas<6, true>() : RB == 4 ? corr9_resident_ctas<4, true>() : corr9_resident_ctas<1, true>());
         if (occ < 1) occ = 1;                        // the occupancy query failed: plan for one CTA per SM
     }
     const int64_t groups = ceil_div64(n_ch + (c_first & 3), 32);
@@ -720,29 +945,21 @@ static bool corr9_make_map(CUtensorMap *map, const float *act, int64_t n_img_tot
                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-template <int RB>
-static int launch_corr9(gpfq_ctx *ctx, const float *actq, const float *actx, bool same, const Corr9Geom &gm, int64_t C,
-                        int64_t n_img_total, double *partial, int slot_stride, int slot0) {
+// X~ == X: G2 only; otherwise G1 and G2 in one pass (an (RB + 4)-row window of xq and the RB x 5 centre pixels of x per box)
+template <int RB, bool BOTH>
+static int launch_corr9(gpfq_ctx *ctx, const float *actq, const float *actx, const Corr9Geom &gm, int64_t C, int64_t n_img_total,
+                        double *partial, int slot_stride, int slot0) {
     using namespace corr9;
-    cudaStream_t st = ctx->stream;
+    using R = Ring<RB, BOTH>;
     dim3 grid((unsigned)(gm.slots / WARPS), (unsigned)ceil_div64(gm.n_ch + (gm.c_first & 3), 32));
-    CUtensorMap mq_win, mq_ctr, mx_win;
-    bool ok = corr9_make_map(&mq_win, actq, n_img_total, gm.H, gm.W, C, RB + 2);
-    if (ok && !same)
-        ok = corr9_make_map(&mq_ctr, actq, n_img_total, gm.H, gm.W, C, RB) &&
-             corr9_make_map(&mx_win, actx, n_img_total, gm.H, gm.W, C, RB + 2);
+    CUtensorMap mq_win, mx_ctr;
+    bool ok = corr9_make_map(&mq_win, actq, n_img_total, gm.H, gm.W, C, R::WR);
+    if (ok && BOTH) ok = corr9_make_map(&mx_ctr, actx, n_img_total, gm.H, gm.W, C, RB);
     if (!ok) return gpfq_fail(ctx, GPFQ_ERR_CUDA, "cuTensorMapEncodeTiled failed for the (%lld, %d, %d, %lld) activations",
                               (long long)n_img_total, gm.H, gm.W, (long long)C);
-    CUDA_TRY(ctx, cudaFuncSetAttribute(conv_corr9_tma_kernel<RB, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       (int)Ring<RB, false>::SMEM));
-    conv_corr9_tma_kernel<RB, false><<<grid, WARPS * 32, Ring<RB, false>::SMEM, st>>>(mq_win, mq_win, gm, partial, slot_stride, slot0);
+    CUDA_TRY(ctx, cudaFuncSetAttribute(conv_corr9_tma_kernel<RB, BOTH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)R::SMEM));
+    conv_corr9_tma_kernel<RB, BOTH><<<grid, WARPS * 32, R::SMEM, ctx->stream>>>(mq_win, BOTH ? mx_ctr : mq_win, gm, partial, slot_stride, slot0);
     KERNEL_CHECK(ctx);
-    if (!same) {
-        CUDA_TRY(ctx, cudaFuncSetAttribute(conv_corr9_tma_kernel<RB, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                           (int)Ring<RB, true>::SMEM));
-        conv_corr9_tma_kernel<RB, true><<<grid, WARPS * 32, Ring<RB, true>::SMEM, st>>>(mx_win, mq_ctr, gm, partial, slot_stride, slot0);
-        KERNEL_CHECK(ctx);
-    }
     return GPFQ_OK;
 }
 
@@ -754,6 +971,19 @@ static int launch_corr9_strip(gpfq_ctx *ctx, const float *actq, const float *act
     cudaStream_t st = ctx->stream;
     dim3 grid((unsigned)(gm.slots / WARPS), (unsigned)ceil_div64(gm.n_ch + (gm.c_first & 3), 32));
     CUtensorMap mq_win, mq_ctr, mx_win;
+    if constexpr (corr9_strip_onepass_sw(SW)) {
+        if (!same) {   // both Grams in one launch
+        using C1 = Cfg1<SW, RB>;
+        if (!corr9_make_map(&mq_win, actq, n_img_total, gm.H, gm.W, C, C1::WR, SW + 4) ||
+            !corr9_make_map(&mq_ctr, actx, n_img_total, gm.H, gm.W, C, RB, SW))
+            return gpfq_fail(ctx, GPFQ_ERR_CUDA, "cuTensorMapEncodeTiled failed for the (%lld, %d, %d, %lld) activations",
+                             (long long)n_img_total, gm.H, gm.W, (long long)C);
+        CUDA_TRY(ctx, cudaFuncSetAttribute(conv_corr9_strip1_kernel<SW, RB>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C1::SMEM));
+        conv_corr9_strip1_kernel<SW, RB><<<grid, WARPS * 32, C1::SMEM, st>>>(mq_win, mq_ctr, gm, partial, slot_stride, slot0);
+        KERNEL_CHECK(ctx);
+        return GPFQ_OK;
+        }
+    }
     bool ok = corr9_make_map(&mq_win, actq, n_img_total, gm.H, gm.W, C, RB + 2, SW + 4);
     if (ok && !same)
         ok = corr9_make_map(&mq_ctr, actq, n_img_total, gm.H, gm.W, C, RB, SW) &&
@@ -764,11 +994,13 @@ static int launch_corr9_strip(gpfq_ctx *ctx, const float *actq, const float *act
                                        (int)Cfg<SW, RB, false>::SMEM));
     conv_corr9_strip_kernel<SW, RB, false><<<grid, WARPS * 32, Cfg<SW, RB, false>::SMEM, st>>>(mq_win, mq_win, gm, partial, slot_stride, slot0);
     KERNEL_CHECK(ctx);
-    if (!same) {
-        CUDA_TRY(ctx, cudaFuncSetAttribute(conv_corr9_strip_kernel<SW, RB, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                           (int)Cfg<SW, RB, true>::SMEM));
-        conv_corr9_strip_kernel<SW, RB, true><<<grid, WARPS * 32, Cfg<SW, RB, true>::SMEM, st>>>(mx_win, mq_ctr, gm, partial, slot_stride, slot0);
-        KERNEL_CHECK(ctx);
+    if constexpr (!corr9_strip_onepass_sw(SW)) {
+        if (!same) {
+            CUDA_TRY(ctx, cudaFuncSetAttribute(conv_corr9_strip_kernel<SW, RB, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                               (int)Cfg<SW, RB, true>::SMEM));
+            conv_corr9_strip_kernel<SW, RB, true><<<grid, WARPS * 32, Cfg<SW, RB, true>::SMEM, st>>>(mx_win, mq_ctr, gm, partial, slot_stride, slot0);
+            KERNEL_CHECK(ctx);
+        }
     }
     return GPFQ_OK;
 }
@@ -776,6 +1008,7 @@ static int launch_corr9_strip(gpfq_ctx *ctx, const float *actq, const float *act
 // strip width of the small-image variant for an image width (0: none)
 // (measured on VGG16: 56-wide layers 4.00 -> 3.66 ms as four strips, 112-wide ones 3.50 -> 3.65 ms: those keep the band kernel)
 static int corr9_strip_width(int Wd) { return Wd == 8 ? 8 : (Wd == 14 || Wd == 28 || Wd == 56) ? 14 : (Wd == 16 || Wd == 32 || Wd == 64) ? 16 : 0; }
+static bool corr9_strip_onepass(int Wd) { return corr9_strip_onepass_sw(corr9_strip_width(Wd)); }
 
 template <int SW>
 static int corr9_strip_stage(gpfq_ctx *ctx, const float *actq, const float *act, bool same, Corr9Geom gm, int64_t C, int64_t n_img_total,
@@ -813,15 +1046,19 @@ int conv_corr9_stage(gpfq_ctx *ctx, const float *act, const float *actq, bool sa
     }
     if (H > 2) {
         gm.slots = slots; gm.y_first = 1; gm.y_last = H - 2; gm.two_rows = 0;
-        switch (RB) {
-            case 8: GPFQ_TRY(launch_corr9<8>(ctx, actq, act, same, gm, C, n_img_total, partial, slot_stride, slot0)); break;
-            case 6: GPFQ_TRY(launch_corr9<6>(ctx, actq, act, same, gm, C, n_img_total, partial, slot_stride, slot0)); break;
-            case 4: GPFQ_TRY(launch_corr9<4>(ctx, actq, act, same, gm, C, n_img_total, partial, slot_stride, slot0)); break;
-            default: return gpfq_fail(ctx, GPFQ_ERR_ARG, "corr9: no kernel for %d rows per band", RB);
+        const int rc = same ? RB : -RB;
+        switch (rc) {
+            case 8: GPFQ_TRY((launch_corr9<8, false>(ctx, actq, act, gm, C, n_img_total, partial, slot_stride, slot0))); break;
+            case 6: GPFQ_TRY((launch_corr9<6, false>(ctx, actq, act, gm, C, n_img_total, partial, slot_stride, slot0))); break;
+            case 4: GPFQ_TRY((launch_corr9<4, false>(ctx, actq, act, gm, C, n_img_total, partial, slot_stride, slot0))); break;
+            case -6: GPFQ_TRY((launch_corr9<6, true>(ctx, actq, act, gm, C, n_img_total, partial, slot_stride, slot0))); break;
+            case -4: GPFQ_TRY((launch_corr9<4, true>(ctx, actq, act, gm, C, n_img_total, partial, slot_stride, slot0))); break;
+            default: return gpfq_fail(ctx, GPFQ_ERR_ARG, "corr9: no kernel for %d rows per band (X~ %s X)", RB, same ? "==" : "!=");
         }
     }
     gm.slots = rslots; gm.y_first = 0; gm.y_last = H - 1; gm.two_rows = 1;
-    GPFQ_TRY(launch_corr9<1>(ctx, actq, act, same, gm, C, n_img_total, rpartial, rslot_stride, rslot0));
+    if (same) GPFQ_TRY((launch_corr9<1, false>(ctx, actq, act, gm, C, n_img_total, rpartial, rslot_stride, rslot0)));
+    else GPFQ_TRY((launch_corr9<1, true>(ctx, actq, act, gm, C, n_img_total, rpartial, rslot_stride, rslot0)));
     return GPFQ_OK;
 }
 
@@ -837,7 +1074,8 @@ __global__ void conv_corr9_sum_groups_kernel(const double *__restrict__ gv, int 
 }
 
 int conv_corr9_assemble_stage(gpfq_ctx *ctx, const double *partial, int slots, const double *rpartial, int rslots,
-                              bool same, int n_ch, int G, double *gram) {
+                              bool same, int Wd, int n_ch, int G, double *gram) {
+    const int g1_by_x = corr9_uses_strips(ctx, Wd) && !corr9_strip_onepass(Wd) ? 0 : 1;   // which kernel wrote the G1 records (conv_corr9_stage)
     if (G > 1) {
         // Packed layers (VGG16's first layer: 3 real channels, G = 32): one CTA per REAL channel would walk G x slots records
         // alone (measured: 1.05 ms of that layer's 1.95).  Assemble every virtual channel on its own CTA, then add the G
@@ -845,13 +1083,13 @@ int conv_corr9_assemble_stage(gpfq_ctx *ctx, const double *partial, int slots, c
         double *gv = nullptr;
         GPFQ_TRY(gpfq_ws(ctx, WS_MISC, (size_t)G * n_ch * 162 * sizeof(double), (void **)&gv));
         conv_corr9_assemble_kernel<<<(unsigned)(G * n_ch), 1024, 0, ctx->stream>>>(partial, slots, rpartial, rslots, same ? 1 : 0,
-                                                                                    G * n_ch, 1, gv);
+                                                                                    g1_by_x, G * n_ch, 1, gv);
         KERNEL_CHECK(ctx);
         conv_corr9_sum_groups_kernel<<<(unsigned)n_ch, 192, 0, ctx->stream>>>(gv, n_ch, G, gram);
         KERNEL_CHECK(ctx);
         return GPFQ_OK;
     }
-    conv_corr9_assemble_kernel<<<(unsigned)n_ch, 1024, 0, ctx->stream>>>(partial, slots, rpartial, rslots, same ? 1 : 0, n_ch, G, gram);
+    conv_corr9_assemble_kernel<<<(unsigned)n_ch, 1024, 0, ctx->stream>>>(partial, slots, rpartial, rslots, same ? 1 : 0, g1_by_x, n_ch, G, gram);
     KERNEL_CHECK(ctx);
     return GPFQ_OK;
 }
