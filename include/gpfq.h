@@ -12,7 +12,9 @@
  *           (kh*kw, n_patches) `wX_channel{c}`/`qX_channel{c}` datasets, :789-797)
  *   W      float32 Keras kernel, (N0, N1) row-major for Dense -- a neuron is a COLUMN (:553);
  *          (kh, kw, C, F) for Conv2D -- the "neuron" is W[:, :, c, f] flattened C-order (:215)
- *   alphabet  float64, K levels, as produced by `rad * linspace(-1, 1, K)` (:396, :544-545)
+ *   alphabet  float64, K levels, as produced by `rad * linspace(-1, 1, K)` (:396, :544-545).  Any levels are accepted and
+ *          rounded to literally; the fast kernels are chosen from the levels themselves (ascending within 1 % of a step of a
+ *          grid: windowed rounding; on the symmetric grid, see "sweep_walk": the tensor-core walk and the int8 residual form)
  *   Q      float64, same shape/strides convention as W (`Q = zeros(W.shape)`, :535, :833)
  */
 #ifndef GPFQ_H_
@@ -95,9 +97,11 @@ int gpfq_set_stream(gpfq_ctx *ctx, void *cuda_stream);
  *                  the one-pass G1 + G2 kernel of X~ != X has bands of 4 or 6 rows and plans its own height otherwise)
  *   "corr_strip"   correlation form on small images (widths 8, 14, 16, 28, 32, 56, 64): 0 the strip kernel (whole strips of <= 16 columns as
  *                  straight-line code), 2 the band kernel
- *   "sweep_walk"   range walk of the Gram-row sweep for one symmetric equispaced alphabet: 0 auto (the tensor-core walk
- *                  sweep_tc_kernel from 2048 directions, below that sweep_pipe / sweep_tile), 1 always the tensor-core walk,
- *                  2 always sweep_pipe / sweep_tile.  The residual form walks with sweep_tc_kernel when its contractions run on
+ *   "sweep_walk"   range walk of the Gram-row sweep for one alphabet on the symmetric grid (every level within 2^-40 a of
+ *                  -a + k 2a / (K - 1), a = the top level; for odd K the middle level exactly 0, three levels exactly {-a, 0, a}):
+ *                  0 auto (the tensor-core walk sweep_tc_kernel from 2048 directions, below that sweep_pipe / sweep_tile),
+ *                  1 always the tensor-core walk, 2 always sweep_pipe / sweep_tile; other alphabets always walk with
+ *                  sweep_pipe / sweep_tile.  The residual form walks with sweep_tc_kernel when its contractions run on
  *                  tcgen05, with sweep_pipe / sweep_tile when they run on the fp64 pipe ("sweep_i8")
  *   "sweep_i8"     contractions of the residual-form sweep: 0 auto, 1 int8 slices on tcgen05, 2 fp64 DMMA
  *   "sweep_outer"  0 auto, 1 Gram rows of all earlier directions, 2 carried residuals (3 m N0 N1 MACs: wins when m << N0),

@@ -202,7 +202,7 @@ extern "C" int gpfq_set_option(gpfq_ctx *ctx, const char *key, int64_t value) {
         // 3 carried residuals as ONE chain (no two-stream split of the neurons)
         if (value < 0 || value > 3) return gpfq_fail(ctx, GPFQ_ERR_ARG, "sweep_outer must be 0, 1, 2 or 3");
         ctx->lowrank_variant = (int)value;
-    } else if (!strcmp(key, "sweep_walk")) {    // range walk of the Gram-row sweep (one symmetric equispaced alphabet): 0 auto,
+    } else if (!strcmp(key, "sweep_walk")) {    // range walk of the Gram-row sweep (one alphabet on the symmetric grid): 0 auto,
                                                  // 1 tensor-core walk (sweep_tc.cu), 2 sweep_pipe / sweep_tile kernels
         if (value < 0 || value > 2) return gpfq_fail(ctx, GPFQ_ERR_ARG, "sweep_walk must be 0, 1 or 2");
         ctx->sweep_walk = (int)value;

@@ -1105,23 +1105,44 @@ static int dense_lowrank_sweep(gpfq_ctx *ctx, const float *X, const float *Xq, i
 // ---------------------------------------------------------------------------------------------
 // The same residual-form sweep with its contractions on the 5th-generation tensor cores (slgemm_i8.cu): X, X~ and W as five
 // int8 digit slices each (sliced ONCE per layer; X^T / X~^T with one exponent per sample, X~ and W with one per row), the
-// decisions of a range as ONE slice of level indices k' = q / h (symmetric equispaced alphabets: q = h k', |k'| <= K - 1,
+// decisions of a range as ONE slice of level indices k' = q / h (alphabets on the symmetric grid: q = h k', |k'| <= K - 1,
 // the literal 0 of a dead direction is k' = 0), the fp64 residuals U re-sliced after every range.  Per range:
 //     U += W_r X_r  (19 slice pairs, dropped terms < 2^-46 of 2^(eW + eX) per direction)  -  h K'_r X~_r  (5 pairs, exact)
 //     D_r = U X~_r^T (15 pairs, < 2^-38 of 2^(eU + eX~) per sample: ~1e-11 of the decision argument, as the tcgen05 Gram)
 // every slice-pair sum is an exact integer in TMEM, the fp64 combination has a fixed order: bit-reproducible.
 // ---------------------------------------------------------------------------------------------
-static bool alphabet_symmetric_equispaced(const double *a, int K, int flag, double *h) {
-    if (!flag || K < 2 || !(a[K - 1] > 0.0)) return false;
-    if (!(fabs(a[0] + a[K - 1]) <= 1e-13 * a[K - 1])) return false;
-    *h = a[K - 1] / (double)(K - 1);
-    return K - 1 <= 127;
+// The gate of sweep_tc_kernel and of the int8 residual form: an alphabet whose levels lie on the symmetric grid
+// a_k = -a + k 2a / (K - 1), a = a[K-1] > 0.  Both decide on that grid (the rounded grid position for K > 3, the thresholds +-a/2
+// for K = 3) and carry the range's decisions as h k' with h = a / (K - 1); only the output values are looked up from the real
+// levels.  So the levels must sit on the grid more tightly than the walk's flag windows resolve: a level delta off the grid
+// moves a decision threshold by at most delta, and an unflagged decision is literal only while that shift stays well inside
+// the window -- 2^-30 of a step for K > 3 (>= 2^-36 a for K <= 128), ~2^-20 relative for K = 3.  delta <= 2^-40 a keeps the
+// shift below 1/16 of the window, and the h k' residual within 2^-40 a of the real one per direction (below what the int8
+// contractions drop).  `c * median|W| * linspace(-1, 1, K)` is off the grid by a few ulp and passes.  Two levels must be exact:
+// for odd K the middle one is 0.0, since the level index k' = 0 is also the literal 0 of a dead direction and is written out
+// as 0.0 (stc_q_from_kq_kernel: a middle level of 1e-14 a, inside the tolerance, would come out as 0.0, not as a level); and
+// K = 3 is decided with exact comparisons against +-a / 2, so its ends must be exact negatives (gpfq_ternary_radius).
+// Anything else -- levels within the 1 % equispaced window but off the grid, an asymmetric or non-uniform alphabet -- walks
+// with sweep_pipe / sweep_tile and the fp64 residual form, which compare the real levels.
+static bool alphabet_on_symmetric_grid(const double *a, int K, int flag, double *h) {
+    if (!flag || K < 2 || K - 1 > 127 || !(a[K - 1] > 0.0)) return false;
+    const double top = a[K - 1];
+    if (K % 2 == 1 && a[K / 2] != 0.0) return false;
+    if (K == 3) {
+        if (a[0] != -top) return false;
+    } else {
+        const double step = 2.0 * top / (double)(K - 1), tol = 0x1p-40 * top;
+        for (int k = 0; k < K; ++k)
+            if (!(fabs(a[k] - (-top + k * step)) <= tol)) return false;
+    }
+    *h = top / (double)(K - 1);
+    return true;
 }
 
 static bool dense_lowrank_uses_i8(gpfq_ctx *ctx, int64_t N0, int64_t m, int64_t nj, int n_alph, double *h) {
     if (ctx->sweep_i8 == 2 || n_alph != 1 || !ctx->h_alph || !ctx->h_koff || !ctx->h_flags) return false;
     if (m > 204 * 128 || N0 >= ((int64_t)1 << 30)) return false;   // one K chunk of the s32 accumulators
-    return alphabet_symmetric_equispaced(ctx->h_alph + ctx->h_koff[0], ctx->h_koff[1] - ctx->h_koff[0], ctx->h_flags[0], h);
+    return alphabet_on_symmetric_grid(ctx->h_alph + ctx->h_koff[0], ctx->h_koff[1] - ctx->h_koff[0], ctx->h_flags[0], h);
 }
 
 // h_j = fl(s_j a) / (K - 1): the level step of neuron j with per-channel alphabets, computed as sweep_tc_kernel computes it
@@ -1413,14 +1434,15 @@ int dense_gram_path(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ldx,
     const int64_t tiles_m = ceil_div64(nj, 128) * n_alph;
     int64_t R = pick_range_length(ctx, nj, n_alph);
     double *Do = nullptr, *Dpart = nullptr;
-    // One symmetric equispaced alphabet: the tensor-core range walk (sweep_tc.cu).  P = (what the earlier ranges contribute:
-    // the Gram-row contraction below) + (the W terms of the range itself: one batched product on the fp64 pipe up front).
+    // One alphabet on the symmetric grid (alphabet_on_symmetric_grid): the tensor-core range walk (sweep_tc.cu).  P = (what the
+    // earlier ranges contribute: the Gram-row contraction below) + (the W terms of the range itself: one batched product on the
+    // fp64 pipe up front).
     double h_tc = 0.0;
     // (measured, profiles/dense_methods_r2.md: below ~2048 directions the few extra launches of the preparation cost more than the
     //  walk saves -- MNIST's layers 0.65 -> 0.73 ms -- so those keep sweep_pipe_kernel; sweep_walk = 1 forces the new walk)
     const bool use_tc = n_alph == 1 && ctx->sweep_walk != 2 && (N0 >= 2048 || ctx->sweep_walk == 1) && ctx->h_alph && ctx->h_koff &&
                         ctx->h_flags && N0 < ((int64_t)1 << 30) &&
-                        alphabet_symmetric_equispaced(ctx->h_alph + ctx->h_koff[0], ctx->h_koff[1] - ctx->h_koff[0], ctx->h_flags[0], &h_tc);
+                        alphabet_on_symmetric_grid(ctx->h_alph + ctx->h_koff[0], ctx->h_koff[1] - ctx->h_koff[0], ctx->h_flags[0], &h_tc);
     TcTables tct;
     double *Pd = nullptr, *G1m = nullptr;
     float *Wn = nullptr;

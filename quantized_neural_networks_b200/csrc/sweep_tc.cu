@@ -1,5 +1,6 @@
 // sweep_tc.cu -- the range walk of the Dense sweep with one THREAD per neuron and the range's Q terms on the 5th-generation
-// tensor cores (symmetric equispaced alphabets; the ternary one of the VGG16 / MNIST configurations has its own specialisation).
+// tensor cores (alphabets whose levels lie on the symmetric grid -a + k 2a / (K - 1): alphabet_on_symmetric_grid in dense_gram.cu;
+// the ternary one {-a, 0, a} of the VGG16 / MNIST configurations has its own specialisation).
 //
 // What a range of R <= 512 directions [tb, te) has to do for every neuron (quantized_network.py:83-89, :117-119 in Gram form):
 //     d_t = P[t] - sum_{tb <= s < t} q_s G2[t][s],   q_t = Q( (d_t + w_t G1[t][t]) / nrm_t^2 )        (guards of :83-87)

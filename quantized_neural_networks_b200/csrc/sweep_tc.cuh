@@ -51,7 +51,8 @@ int sweep_tc_slice_g1_lower(gpfq_ctx *ctx, const double *G1, int64_t ldg, bool c
 //       both bound once per layer (sweep_tc_bind: rowsP x ldp allocations, rowsP a multiple of 128); this launch's neuron 0 is row row0
 //   Kq  out: the decisions as int8 level indices k' = q / (a / 2) (sl_offset layout, krows rows, neuron 0 at row krow0)
 int sweep_tc_bind(gpfq_ctx *ctx, TcTables *tab, const double *P, const float *Wn, int64_t rowsP, int64_t ldp);
-//   a, levels, K: the symmetric equispaced alphabet (device levels, a = levels[K - 1]); K == 3 runs the ternary specialisation
+//   a, levels, K: an alphabet on the symmetric grid (device levels, a = levels[K - 1]; alphabet_on_symmetric_grid); K == 3 runs the
+//       ternary specialisation
 //   scales (nullable, device, this launch's nj neurons): per-channel alphabets -- neuron j walks with fl(scales[j] levels[k]); the
 //       tables must then be prepared with h = 1
 //   u0: stochastic rounding (ctx->d_seeds set): this launch's neuron j draws as unit u0 + j
