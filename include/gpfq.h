@@ -103,7 +103,9 @@ int gpfq_set_stream(gpfq_ctx *ctx, void *cuda_stream);
  *                  1 always the tensor-core walk, 2 always sweep_pipe / sweep_tile; other alphabets always walk with
  *                  sweep_pipe / sweep_tile.  The residual form walks with sweep_tc_kernel when its contractions run on
  *                  tcgen05, with sweep_pipe / sweep_tile when they run on the fp64 pipe ("sweep_i8")
- *   "sweep_i8"     contractions of the residual-form sweep: 0 auto, 1 int8 slices on tcgen05, 2 fp64 DMMA
+ *   "sweep_i8"     contractions of the residual-form sweep: 0 auto (int8 slices on tcgen05 unless the direction norms spread
+ *                  beyond what one exponent per sample keeps: then fp64 DMMA; one 4-byte read-back decides), 1 always int8
+ *                  slices on tcgen05, 2 fp64 DMMA
  *   "sweep_outer"  0 auto, 1 Gram rows of all earlier directions, 2 carried residuals (3 m N0 N1 MACs: wins when m << N0),
  *                  3 carried residuals as one chain (default: two halves of the neurons on two streams, so that one half's
  *                  contractions fill the other half's latency-bound walk) */

@@ -1145,6 +1145,90 @@ static bool dense_lowrank_uses_i8(gpfq_ctx *ctx, int64_t N0, int64_t m, int64_t 
     return alphabet_on_symmetric_grid(ctx->h_alph + ctx->h_koff[0], ctx->h_koff[1] - ctx->h_koff[0], ctx->h_flags[0], h);
 }
 
+// The int8 residual form slices X^T / X~^T with ONE exponent per sample over all N0 directions, and the range's G1 rows with one per
+// row.  A direction whose norm is far below the largest entries of its samples therefore reaches U, P and D_r through fewer bits:
+// its decision argument moves by up to ~2^-39 N0 (max-sample norm / ||x~_t||) of a step, and no replay can recover what the slices
+// dropped.  So the layer takes the int8 contractions only while sqrt(sum_i colmax_i^2) -- the norm of the per-sample maxima over
+// X and X~, which bounds every direction's norm -- stays within LOWRANK_I8_SPREAD times the smallest live ||x~_t||.  ReLU
+// activations of similar norms sit near 6 (4.2 / 0.71 for N0 = 25088); direction norms spread over 10^+-1 give ~600.
+// A layer past the gate walks with the fp64 contractions of dense_lowrank_sweep.
+static constexpr double LOWRANK_I8_SPREAD = 64.0;
+
+__global__ void __launch_bounds__(256) spread_colmax_kernel(const float *__restrict__ X, int64_t ldx, int64_t N0, int64_t m,
+                                                            int *__restrict__ colmax, int rows_per_cta) {
+    const int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x;
+    if (i >= m) return;
+    const int64_t t0 = (int64_t)blockIdx.y * rows_per_cta, t1 = min(N0, t0 + rows_per_cta);
+    float mx = 0.f;
+    for (int64_t t = t0; t < t1; ++t) mx = fmaxf(mx, fabsf(X[t * ldx + i]));
+    atomicMax(colmax + i, __float_as_int(mx));   // non-negative floats order like their bit patterns
+}
+
+// one warp per direction: the least ||x~_t||^2 over the live directions (fp32(sqrt) >= GPFQ_DEAD_NORM), as fp64 bits
+__global__ void __launch_bounds__(256) spread_min_norm_kernel(const float *__restrict__ Xq, int64_t ldx, int64_t N0, int64_t m,
+                                                              unsigned long long *__restrict__ minn2) {
+    const int64_t t = (int64_t)blockIdx.x * 8 + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (t >= N0) return;
+    double n2 = 0.0;
+    for (int64_t i = lane; i < m; i += 32) {
+        const double x = (double)Xq[t * ldx + i];
+        n2 = fma(x, x, n2);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) n2 += __shfl_xor_sync(0xffffffffu, n2, o);
+    if (lane == 0 && !((double)(float)sqrt(n2) < GPFQ_DEAD_NORM)) atomicMin(minn2, (unsigned long long)__double_as_longlong(n2));
+}
+
+__global__ void __launch_bounds__(256) spread_gate_kernel(const int *__restrict__ colmax, int64_t m,
+                                                          const unsigned long long *__restrict__ minn2, int *__restrict__ wide) {
+    __shared__ double red[8];
+    double s = 0.0;
+    for (int64_t i = threadIdx.x; i < m; i += 256) {
+        const double c = (double)__int_as_float(colmax[i]);
+        s = fma(c, c, s);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = s;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        for (int w = 1; w < 8; ++w) s += red[w];
+        const double mn = __longlong_as_double((long long)*minn2);   // +inf when every direction is dead
+        *wide = !(s <= LOWRANK_I8_SPREAD * LOWRANK_I8_SPREAD * mn);  // (NaN / Inf in the inputs: wide)
+    }
+}
+
+// *ok = the layer passes the spread gate above.  One 4-byte read-back: the choice of form is made on the host.
+static int lowrank_i8_spread_ok(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ldx, int64_t N0, int64_t m, bool *ok) {
+    cudaStream_t st = ctx->stream;
+    unsigned char *ws = nullptr;
+    const size_t cm_bytes = (size_t)ceil_div64(m, 64) * 64 * sizeof(int);
+    GPFQ_TRY(gpfq_ws(ctx, WS_MISC, cm_bytes + 16, (void **)&ws));
+    int *colmax = reinterpret_cast<int *>(ws);
+    unsigned long long *minn2 = reinterpret_cast<unsigned long long *>(ws + cm_bytes);
+    int *wide = reinterpret_cast<int *>(ws + cm_bytes + 8);
+    CUDA_TRY(ctx, cudaMemsetAsync(colmax, 0, cm_bytes, st));
+    CUDA_TRY(ctx, cudaMemsetAsync(minn2, 0x7f, 8, st));   // 0x7f7f7f7f7f7f7f7f: a huge finite double
+    const int rows_per_cta = 256;
+    const dim3 g((unsigned)ceil_div64(m, 256), (unsigned)ceil_div64(N0, rows_per_cta));
+    spread_colmax_kernel<<<g, 256, 0, st>>>(X, ldx, N0, m, colmax, rows_per_cta);
+    KERNEL_CHECK(ctx);
+    if (Xq != X) {
+        spread_colmax_kernel<<<g, 256, 0, st>>>(Xq, ldx, N0, m, colmax, rows_per_cta);
+        KERNEL_CHECK(ctx);
+    }
+    spread_min_norm_kernel<<<(unsigned)ceil_div64(N0, 8), 256, 0, st>>>(Xq, ldx, N0, m, minn2);
+    KERNEL_CHECK(ctx);
+    spread_gate_kernel<<<1, 256, 0, st>>>(colmax, m, minn2, wide);
+    KERNEL_CHECK(ctx);
+    int h_wide = 1;
+    CUDA_TRY(ctx, cudaMemcpyAsync(&h_wide, wide, sizeof(int), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(ctx, cudaStreamSynchronize(st));
+    *ok = h_wide == 0;
+    return GPFQ_OK;
+}
+
 // h_j = fl(s_j a) / (K - 1): the level step of neuron j with per-channel alphabets, computed as sweep_tc_kernel computes it
 __global__ void unit_steps_kernel(const double *__restrict__ scales, int64_t nj, int64_t njP, double a, int K, double *__restrict__ hrow) {
     const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -1380,8 +1464,10 @@ int dense_gram_path(gpfq_ctx *ctx, const float *X, const float *Xq, int64_t ldx,
     double *G1 = nullptr, *G2 = nullptr, *Wt = nullptr, *Qt = nullptr;
     double h_step = 0.0;
     // Stochastic rounding (ctx->d_seeds): every walk below takes it; the shard's first neuron has unit id u0
-    const bool i8_sweep = !pre && dense_lowrank_uses_i8(ctx, N0, m, nj, n_alph, &h_step);
+    bool i8_sweep = !pre && dense_lowrank_uses_i8(ctx, N0, m, nj, n_alph, &h_step);
     const bool lowrank = !pre && dense_uses_lowrank(ctx, N0, m, nj, n_alph, same, i8_sweep);
+    // sweep_i8 = 0: the int8 contractions only for layers within the spread gate (lowrank_i8_spread_ok); 1 forces them
+    if (lowrank && i8_sweep && ctx->sweep_i8 == 0) GPFQ_TRY(lowrank_i8_spread_ok(ctx, X, Xq, ldx, N0, m, &i8_sweep));
     // Neurons per CTA of the range walk: the narrowest tile that still fits every CTA on the chip at once (two per SM, so
     // that one CTA's serial walk overlaps another's contraction).
     const int64_t slots = 2LL * ctx->sm_count;

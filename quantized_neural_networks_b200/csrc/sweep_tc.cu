@@ -94,41 +94,77 @@ __device__ __forceinline__ void tmem_ld_5x16(uint32_t taddr, uint32_t (&v)[S][16
         : "memory");
 }
 
+// sum_{s < n} k'_s (G2s[t][s] - G2[t][s]) for one Gram row g2row = G2[t][tb ..] with slice exponent ex: what the digit slices of the
+// row (G2s, rounded at 2^(ex - 39)) added to the Q terms of this neuron's level indices in the range's earlier blocks (the K-major,
+// 64B-swizzled tile the walkers hand over; `arow` = this neuron's row of K block 0).  Each difference is exact, the sum is fp64.
+static __device__ __noinline__ double q_term_slicing_error(const double *g2row, int n, int ex, const unsigned char *arow, int j) {
+    const double up = ldexp(1.0, 8 * S - 2 - ex), dn = ldexp(1.0, ex - (8 * S - 2));
+    const int sw = (j >> 1) & 3;
+    double c = 0.0;
+    for (int s = 0; s < n; ++s) {
+        const double x = g2row[s];
+        const int k = (int)reinterpret_cast<const int8_t *>(arow)[(s >> 6) * A_KB + ((((s >> 4) & 3) ^ sw) << 4) + (s & 15)];
+        c = fma((double)k, rint(x * up) * dn - x, c);
+    }
+    return c;
+}
+
 // The literal walk of one block from the saved residual dots (own shared-memory column), for a warp that raised a flag:
 // gpfq_decide_rcp_inl of dense_gram.cu with the ternary scan.  Rolled loops; decisions go out as level indices.
 // SCALED: the neuron's levels are fl(s alph[k]) (per-channel alphabets; a = fl(s alph[K - 1]), `alph` the base alphabet); a neuron
 // with s = 0 decides the literal 0 everywhere (its levels are all zero) and never reaches the divisions by a.
 // STOCH: stochastic rounding (common.cuh) with the draw of step t0 + t from the neuron's unit key.
 // L1: the value of step t is shrunk by its tau (lane t's tau_l: the whole warp replays).
+// The saved dots carry the slicing error of the Q terms of the range's earlier blocks, up to bv in units of v (TabA::qe).  Every
+// quantizer is monotone in v, so where q(v - bv) = q(v + bv) the exact dots decide the same; otherwise the step takes the exact Q
+// terms first: d += h sum k'_s (G2s - G2) over the fp64 Gram row g2 + t * ldg (the range's first direction at column 0).
+// One exception to the monotonicity: the :86 guard (|d| < 1e-10 takes v = w) is tested on the sliced d, in the walk and here, so a
+// d whose slicing error carries it across 1e-10 takes the other branch.  That needs |d| within h sum |k'_s| 2^(e_t - 39) of 1e-10,
+// i.e. a residual dot 10 orders below the Gram scale of the direction; no widening is spent on it.
 template <bool SCALED, bool STOCH = false, bool L1 = false>
 static __device__ __noinline__ void replay_block(unsigned char *dset, const unsigned char *wset, int j, const TabA *tab, double a,
-                                                 int8_t *qcol, const double *alph, int K, double s, uint64_t key = 0, int64_t t0 = 0,
-                                                 double tau_l = 0.0) {
+                                                 int8_t *qcol, const double *alph, int K, double s, uint64_t key, int64_t t0,
+                                                 double tau_l, const double *g2, int64_t ldg, int nprev, const unsigned char *arow,
+                                                 double bv) {
     // K == 3: the ternary scan with the levels in registers; else the windowed scan of the equispaced levels (common.cuh)
     const bool zero = SCALED && !(a > 0.0);
     const double inv_step = zero ? 0.0 : (SCALED ? gpfq_inv_step_s(alph, K, 1, s) : 0.5 * (double)(K - 1) / a);
     const double inv_h = zero ? 0.0 : (double)(K - 1) / a;
+    const double h = zero ? 0.0 : a / (double)(K - 1);
+    const double bw = bv * (1.0 + 0x1p-20);
     auto dptr = [&](int t) { return reinterpret_cast<double *>(dset + (t >> 4) * (D_BYTES / 2) + sw128(j, (t & 15) >> 1)) + (t & 1); };
     for (int t = 0; t < NB; ++t) {
-        const double d0 = *dptr(t);
+        double d0 = *dptr(t);
         const double wv = (double)reinterpret_cast<const float *>(wset + sw128(j, t >> 2))[t & 3];
         const double nrm = tab->nrm[t];
         const double tau = L1 ? __shfl_sync(0xffffffffu, tau_l, t) : 0.0;
-        double q = 0.0;
-        if (!(nrm < GPFQ_DEAD_NORM)) {
+        const double r = STOCH ? gpfq_draw(key, t0 + t) : 0.0;
+        auto value = [&](double dd) {
             double v = wv;
-            if (!(fabs(d0) < GPFQ_PERP_DOT)) {
-                const double num = fma(wv, tab->g1dd[t], d0), rinv = tab->rinv[t];
+            if (!(fabs(dd) < GPFQ_PERP_DOT)) {
+                const double num = fma(wv, tab->g1dd[t], dd), rinv = tab->rinv[t];
                 const double q0 = num * rinv;
                 const double e = fma(-q0, tab->den[t], num);
                 v = fma(e, rinv, q0);
             }
+            return v;
+        };
+        auto decide = [&](double v) {
             if (L1) v = gpfq_shrink(v, tau);
-            if (zero) q = 0.0;
-            else if (STOCH && K == 3) q = gpfq_stoc_round_ternary(v, a, gpfq_draw(key, t0 + t));
-            else if (STOCH) q = gpfq_stoc_round_eq<SCALED>(v, alph, K, inv_step, s, gpfq_draw(key, t0 + t));
-            else if (K == 3) q = gpfq_bit_round_ternary(v, a);
-            else q = SCALED ? gpfq_bit_round_eq_s(v, alph, K, inv_step, s) : gpfq_bit_round_eq(v, alph, K, inv_step);
+            if (zero) return 0.0;
+            if (STOCH && K == 3) return gpfq_stoc_round_ternary(v, a, r);
+            if (STOCH) return gpfq_stoc_round_eq<SCALED>(v, alph, K, inv_step, s, r);
+            if (K == 3) return gpfq_bit_round_ternary(v, a);
+            return SCALED ? gpfq_bit_round_eq_s(v, alph, K, inv_step, s) : gpfq_bit_round_eq(v, alph, K, inv_step);
+        };
+        double q = 0.0;
+        if (!(nrm < GPFQ_DEAD_NORM)) {
+            double v = value(d0);
+            q = decide(v);
+            if (nprev > 0 && !zero && decide(v - bw) != decide(v + bw)) {
+                d0 = fma(h, q_term_slicing_error(g2 + t * ldg, nprev, tab->ex[t], arow, j), d0);
+                q = decide(value(d0));
+            }
         }
         qcol[t * NT] = (int8_t)__double2int_rn(q * inv_h);   // level index k' = q / h, h = a / (K - 1); the literal 0 of a dead direction is 0
         for (int u = t + 1; u < NB; ++u) {
@@ -163,7 +199,8 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap mapP, const __grid_constant_
                 const int8_t *__restrict__ g2s, int kbr, int64_t tb, int64_t te, int row0, int64_t nj, int8_t *__restrict__ Kq,
                 int64_t krows, int64_t krow0, double a_base, const double *__restrict__ levels, int K,
                 const double *__restrict__ scales = nullptr, const uint64_t *__restrict__ seeds = nullptr, int64_t u0 = 0,
-                const double *__restrict__ lambdas = nullptr) {
+                const double *__restrict__ lambdas = nullptr, const double *__restrict__ g2rows = nullptr, int64_t ldg2 = 0,
+                int g2compact = 0) {
     using namespace i8g;
     extern __shared__ unsigned char stc_smem_raw[];
     // (offset arithmetic on the array itself: the compiler keeps the shared address space, LDS / STS instead of generic accesses)
@@ -209,15 +246,15 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap mapP, const __grid_constant_
         const bool zero = SCALED && !(a > 0.0);                     // s = 0: every decision is the literal 0, no replay
         const double h_u = SCALED ? (zero ? 0.0 : a / (double)(K - 1)) : 1.0, inv_hu = SCALED ? (zero ? 0.0 : 1.0 / h_u) : 1.0;
         const double hh = 0.5 * a;
-        // flags of the ternary walk, compared as high words: [hi(a / 2) - 1, hi(a / 2) + 1] around the thresholds (a window of ~2^-20
-        // relative: one warp-block in ~300 replays), a * 2^40 and above (NaN / Inf included), 1e-10 and below (:86)
-        const uint32_t near_lo = (uint32_t)__double2hiint(hh) - 1u, big_hi = (uint32_t)__double2hiint(a * 0x1p40),
-                       perp_hi = (uint32_t)__double2hiint(GPFQ_PERP_DOT);
+        // flags of the ternary walk, compared as high words: [hi(a / 2 - B) - 1, hi(a / 2 + B) + 1] around the thresholds (B = 0: a
+        // window of ~2^-20 relative, one warp-block in ~300 replays; B below), a * 2^40 and above (NaN / Inf included), 1e-10 and below (:86)
+        const uint32_t big_hi = (uint32_t)__double2hiint(a * 0x1p40), perp_hi = (uint32_t)__double2hiint(GPFQ_PERP_DOT);
         // more than three levels a_k = -a + k s, s = 2 a / (K - 1): grid position kr = (p + a) / s, nearest level by the 1.5 * 2^52 trick
         const double km1 = (double)(K - 1), step = 2.0 * a / km1, cmid = 0.5 * km1, magic = 6755399441055744.0;
         const uint32_t lane_field = (uint32_t)(warp * 32) << 16;
         const uint64_t key = STOCH ? gpfq_unit_key(seeds[0], u0 + jg) : 0;
         const double lam = L1 ? lambdas[0] : 0.0, inv_st = SCALED ? 0.5 * inv_hu : cmid / a;   // (one step = 2 h)
+        int ksum = 0;   // sum of |k'| over this neuron's decisions in the range's earlier blocks (the A operand of the Q terms)
         for (int b = 0; b < nblk; ++b) {
             const int buf = b & 1;
             const int64_t t0 = tb + (int64_t)b * NB;
@@ -226,6 +263,14 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap mapP, const __grid_constant_
             const unsigned char *wset = smem + OFF_W + buf * W_BYTES;
             const TabA *tab = reinterpret_cast<const TabA *>(smem + OFF_TAB + buf * TAB_BYTES);
             mbar_wait(&in_full[buf], (b >> 1) & 1);
+            // How far the rounding of the Gram digit slices can move this block's decision arguments (TabA::qe): eq steps of the
+            // grid, B = eq * step in units of p (one step = 2 h, a for K = 3).  Every flag window below is widened by it, so a
+            // step whose exact value may lie on the other side of a threshold replays instead of being decided (and the replay
+            // takes the exact Q terms where they matter, replay_block).  eq = 0 in the first block of a range (DESIGN.md 5.4).
+            const double eq = 0.5 * (double)ksum * tab->qe;
+            const double lim = 0.5 - 0x1p-30 - eq, band = 0x1p-30 + eq, ab = a * eq;
+            const uint32_t near_lo = (uint32_t)__double2hiint(fmax(hh - ab, 0.0)) - 1u,
+                           near_span = (uint32_t)__double2hiint(hh + ab) + 1u - near_lo;
             double d[NB];
 #pragma unroll
             for (int c = 0; c < NB / 2; ++c) {
@@ -281,10 +326,10 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap mapP, const __grid_constant_
                     const double rr = STOCH ? gpfq_draw(key, t0 + t) : 0.5;
                     // the step's thresholds and flag window, off the chain (clamped: tau = inf flags nothing, decides 0)
                     const double up_t = fmin(fma(rr, a, tau), DBL_MAX), dn_t = fmax(fma(rr - 1.0, a, -tau), -DBL_MAX);
-                    const double band = 0x1p-30 * fmin(a + tau, DBL_MAX);
+                    const double band_t = fma(0x1p-30, fmin(a + tau, DBL_MAX), ab);
                     const bool up = p > up_t, dn = p <= dn_t;
                     q = up ? a : (dn ? -a : 0.0);
-                    flag |= (int)!(fmin(fabs(p - up_t), fabs(p - dn_t)) > band);
+                    flag |= (int)!(fmin(fabs(p - up_t), fabs(p - dn_t)) > band_t);
                     const uint32_t hp = (uint32_t)__double2hiint(p) & 0x7fffffffu;
                     m_big = max(m_big, hp);
                     m_perp = min(m_perp, ((uint32_t)__double2hiint(d[t]) & 0x7fffffffu) | (uint32_t)tab->deadm[t]);
@@ -301,11 +346,11 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap mapP, const __grid_constant_
                         const double k0 = fmin(fmax(floor(kr), 0.0), km1 - 1.0);
                         const double f = kr - k0;
                         r = rr < f ? k0 + 1.0 : k0;
-                        fl = (int)!(fabs(f) > 0x1p-30) | (int)!(fabs(f - 1.0) > 0x1p-30) | (int)!(fabs(f - rr) > 0x1p-30);
+                        fl = (int)!(fabs(f) > band) | (int)!(fabs(f - 1.0) > band) | (int)!(fabs(f - rr) > band);
                     } else {
                         const double r0 = (kr + magic) - magic;
                         r = fmin(fmax(r0, 0.0), km1);
-                        fl = (int)!(fabs(kr - r0) < 0.5 - 0x1p-30);
+                        fl = (int)!(fabs(kr - r0) < lim);
                     }
                     const bool live = ri != 0.0;
                     q = live ? fma(r, step, -a) : 0.0;
@@ -345,7 +390,7 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap mapP, const __grid_constant_
                     const double r = rr < f ? k0 + 1.0 : k0;
                     const bool live = ri != 0.0;
                     q = live ? fma(r, step, -a) : 0.0;
-                    flag |= ((int)!(fabs(f) > 0x1p-30) | (int)!(fabs(f - 1.0) > 0x1p-30) | (int)!(fabs(f - rr) > 0x1p-30) |
+                    flag |= ((int)!(fabs(f) > band) | (int)!(fabs(f - 1.0) > band) | (int)!(fabs(f - rr) > band) |
                              (int)!(fabs(kr) < 0x1p40) | (int)(fabs(d[t]) < GPFQ_PERP_DOT)) & (int)live;
                     const int kq = live ? __double2int_rn(fma(r, 2.0, -km1)) : 0;
                     pk[t >> 2] |= ((uint32_t)kq & 0xffu) << (8 * (t & 3));
@@ -356,7 +401,7 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap mapP, const __grid_constant_
                     const bool live = ri != 0.0;
                     q = live ? fma(r, step, -a) : 0.0;                       // a dead direction: the literal 0 (:83-84), index 0
                     // a tie between two levels (or anything within 2^-30 of a step of one), a non-finite / huge argument, the :86 guard
-                    flag |= ((int)!(fabs(kr - r0) < 0.5 - 0x1p-30) | (int)!(fabs(kr) < 0x1p40) | (int)(fabs(d[t]) < GPFQ_PERP_DOT)) & (int)live;
+                    flag |= ((int)!(fabs(kr - r0) < lim) | (int)!(fabs(kr) < 0x1p40) | (int)(fabs(d[t]) < GPFQ_PERP_DOT)) & (int)live;
                     const int kq = live ? __double2int_rn(fma(r, 2.0, -km1)) : 0;   // k' = 2 k - (K - 1)
                     pk[t >> 2] |= ((uint32_t)kq & 0xffu) << (8 * (t & 3));
                 }
@@ -372,8 +417,8 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap mapP, const __grid_constant_
                 if (kbr == -1 - t) asm volatile("trap;\n");
             }
             if (TERN && L1) flag |= (int)(m_big >= big_hi) | (int)(m_perp <= perp_hi);
-            else if (TERN && STOCH) flag = (int)!(m_thr > 0x1p-30 * a) | (int)(m_big >= big_hi) | (int)(m_perp <= perp_hi);
-            else if (TERN) flag = (int)(m_near <= 2u) | (int)(m_big >= big_hi) | (int)(m_perp <= perp_hi);
+            else if (TERN && STOCH) flag = (int)!(m_thr > fma(0x1p-30, a, ab)) | (int)(m_big >= big_hi) | (int)(m_perp <= perp_hi);
+            else if (TERN) flag = (int)(m_near <= near_span) | (int)(m_big >= big_hi) | (int)(m_perp <= perp_hi);
             if (SCALED && zero) {
                 flag = 0;
 #pragma unroll
@@ -381,8 +426,12 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap mapP, const __grid_constant_
             }
             if (__any_sync(0xffffffffu, flag != 0 && valid)) {   // (rows beyond nj hold zeros: they would trip the :86 guard at every step)
                 int8_t *qcol = reinterpret_cast<int8_t *>(smem + OFF_Q) + j;
-                if (L1) replay_block<SCALED, STOCH, true>(dset, wset, j, tab, a, qcol, alph, K, s_u, key, t0, tau_l);
-                else replay_block<SCALED, STOCH>(dset, wset, j, tab, a, qcol, alph, K, s_u, key, t0);
+                const double bv = 0.5 * (double)ksum * tab->qe * step;   // eq in units of v (recomputed: not live across the walk)
+                const double *g2row0 = g2rows + t0 * ldg2 + (g2compact ? 0 : tb);   // G2[t0][tb]
+                const unsigned char *arow = smem + j * KB;
+                if (L1) replay_block<SCALED, STOCH, true>(dset, wset, j, tab, a, qcol, alph, K, s_u, key, t0, tau_l, g2row0, ldg2, (int)(t0 - tb),
+                                                          arow, bv);
+                else replay_block<SCALED, STOCH>(dset, wset, j, tab, a, qcol, alph, K, s_u, key, t0, 0.0, g2row0, ldg2, (int)(t0 - tb), arow, bv);
 #pragma unroll
                 for (int i = 0; i < NB / 4; ++i) {
                     uint32_t w4 = 0u;
@@ -391,6 +440,8 @@ sweep_tc_kernel(const __grid_constant__ CUtensorMap mapP, const __grid_constant_
                     pk[i] = w4;
                 }
             }
+#pragma unroll
+            for (int i = 0; i < NB / 4; ++i) ksum = __dp4a((int)__vabsss4(pk[i]), 0x01010101, ksum);
             // ---- hand the decisions over: 32 bytes of this neuron's row of the level-index tile (K block b / 2, 64B swizzle)
             const int sw = (j >> 1) & 3, c16 = 2 * (b & 1);
             if (b + 1 < nblk) {
@@ -554,6 +605,13 @@ stc_prepare_kernel(const double *__restrict__ G1, const double *__restrict__ G2,
         tab->deadm[tt] = nv < GPFQ_DEAD_NORM ? 0x7ff00000 : 0;
         tab->ris[tt] = nv < GPFQ_DEAD_NORM ? 0.0 : (1.0 / (nv * nv)) / (2.0 * h);   // h = a / (K - 1): one step is 2 h
         tab->sc[tt] = bad_s[tt] ? __longlong_as_double(0x7ff8000000000000LL) : ldexp(h, ex_s[tt] - (8 * S - 2));
+        // the slices hold G2[t][s] to 2^(e_t - 39) (rint of x 2^(38 - e_t)), so the Q terms of a neuron whose level indices in the
+        // range's earlier blocks sum to S in magnitude are off by at most h 2^(e_t - 39) S, and p by that times rinv_t
+        double qe = fmin(ldexp(tab->rinv[tt], ex_s[tt] - (8 * S - 1)), DBL_MAX);
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) qe = fmax(qe, __shfl_xor_sync(0xffffffffu, qe, o));
+        if (tt == 0) { tab->qe = qe; tab->qe_pad = 0.0; }
+        tab->ex[tt] = ex_s[tt];
     }
 }
 
@@ -695,6 +753,9 @@ int sweep_tc_prepare(gpfq_ctx *ctx, const double *G1, const double *G2, int64_t 
     KERNEL_CHECK(ctx);
     out->tabs = tabs;
     out->g2s = g2s;
+    out->G2 = G2;
+    out->ldg = ldg;
+    out->compact = compact;
     out->R = R;
     return GPFQ_OK;
 }
@@ -792,26 +853,28 @@ int sweep_tc_range(gpfq_ctx *ctx, const TcTables &tab, int64_t tb, int64_t te, i
                        : (scales ? sweep_tc_kernel<false, true, true, true> : sweep_tc_kernel<false, false, true, true>);
         CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM));
         k<<<grid, THREADS, SMEM, ctx->stream>>>(tab.mapP, tab.mapW, tab.tabs, tab.g2s, (int)(tab.R / KB), tb, te, (int)row0, nj, Kq, krows, krow0,
-                                                a, levels, K, scales, seeds, u0, lambdas);
+                                                a, levels, K, scales, seeds, u0, lambdas, tab.G2, tab.ldg, (int)tab.compact);
     } else if (const uint64_t *seeds = ctx->d_seeds) {   // stochastic rounding: one alphabet on this path, seeds[0]
         auto k = K == 3 ? (scales ? sweep_tc_kernel<true, true, true> : sweep_tc_kernel<true, false, true>)
                         : (scales ? sweep_tc_kernel<false, true, true> : sweep_tc_kernel<false, false, true>);
         CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM));
         k<<<grid, THREADS, SMEM, ctx->stream>>>(tab.mapP, tab.mapW, tab.tabs, tab.g2s, (int)(tab.R / KB), tb, te, (int)row0, nj, Kq, krows, krow0,
-                                                a, levels, K, scales, seeds, u0, nullptr);
+                                                a, levels, K, scales, seeds, u0, nullptr, tab.G2, tab.ldg, (int)tab.compact);
     } else if (scales) {
         auto k = K == 3 ? sweep_tc_kernel<true, true> : sweep_tc_kernel<false, true>;
         CUDA_TRY(ctx, cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM));
         k<<<grid, THREADS, SMEM, ctx->stream>>>(tab.mapP, tab.mapW, tab.tabs, tab.g2s, (int)(tab.R / KB), tb, te, (int)row0, nj, Kq, krows, krow0,
-                                                a, levels, K, scales, nullptr, 0, nullptr);
+                                                a, levels, K, scales, nullptr, 0, nullptr, tab.G2, tab.ldg, (int)tab.compact);
     } else if (K == 3) {
         CUDA_TRY(ctx, cudaFuncSetAttribute(sweep_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM));
         sweep_tc_kernel<true><<<grid, THREADS, SMEM, ctx->stream>>>(tab.mapP, tab.mapW, tab.tabs, tab.g2s, (int)(tab.R / KB), tb, te, (int)row0, nj,
-                                                                    Kq, krows, krow0, a, levels, K);
+                                                                    Kq, krows, krow0, a, levels, K, nullptr, nullptr, 0, nullptr, tab.G2,
+                                                                    tab.ldg, (int)tab.compact);
     } else {
         CUDA_TRY(ctx, cudaFuncSetAttribute(sweep_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM));
         sweep_tc_kernel<false><<<grid, THREADS, SMEM, ctx->stream>>>(tab.mapP, tab.mapW, tab.tabs, tab.g2s, (int)(tab.R / KB), tb, te, (int)row0, nj,
-                                                                     Kq, krows, krow0, a, levels, K);
+                                                                     Kq, krows, krow0, a, levels, K, nullptr, nullptr, 0, nullptr, tab.G2,
+                                                                    tab.ldg, (int)tab.compact);
     }
     KERNEL_CHECK(ctx);
     return GPFQ_OK;

@@ -24,6 +24,10 @@ struct TabA {
     double nrm[NB];        // (double)(float)sqrt(G2[t][t])   (the snrm2 result of quantized_network.py:83)
     double sc[NB];         // h 2^(e_t - 38): scale of the integer Q-term sums of direction t
     int32_t deadm[NB];     // 0x7ff00000 for a dead direction (masks the perpendicularity flag), else 0
+    double qe;             // max over the block's directions t of 2^(e_t - 39) rinv_t: a neuron whose decisions in the range's earlier
+                           // blocks sum to S = sum |k'_s| gets p moved by at most h S qe by the rounding of the Gram digit slices
+    double qe_pad;         // (the bulk copy moves multiples of 16 bytes)
+    int32_t ex[NB];        // e_t: the exponent of the digit slices of row t (a replay takes the exact Q terms from it)
 };
 }  // namespace stc
 
@@ -32,6 +36,9 @@ struct TcTables {
     const int8_t *g2s = nullptr;       // digit slices of G2[block rows][earlier directions of the block's range]:
                                        // [block][K block][slice][32 rows x 64 B, 64B-swizzled]
     int64_t R = 0;                     // directions per range
+    const double *G2 = nullptr;        // the fp64 Gram rows the slices were made from (sweep_tc_prepare), for the replay
+    int64_t ldg = 0;
+    bool compact = false;
     CUtensorMap mapP, mapW;            // P (rowsP, N0P) fp64 and the neuron-major weights (rowsP, N0P) fp32 (sweep_tc_bind)
     int64_t rowsP = 0;
 };
